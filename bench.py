@@ -5,8 +5,11 @@ One "step" = one pass of the hot path (MFE fill + backtrack, partition function,
 target) over a batch of B=4096 random sequences of length L (default L=100; the other lengths
 of the sweep are timed in the same run and reported under "by_length").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--L 100] [--B 4096]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--L 100] [--B 4096] [--dump-outputs DIR]
   python bench.py --impl reference ...      # CPU arm: the oracle port on all host threads
+
+--dump-outputs DIR writes what the last timed step returned to its caller (mfe_dcal, mfe_ss, pf, eval_dcal of
+score_batch_device) as DIR/<name>.npy, so that two builds can be compared output for output on identical inputs.
 
 Our arm prints ONE JSON line with the driver's contract keys plus `roofline`, `cpu_baseline`,
 `e2e`, `by_length`, `clocks`, `gpu_launches`.  Timing: CUDA events on the launch stream, >= 3
@@ -27,9 +30,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: no __pycache__ next to the sources
 
 SWEEP = (50, 100, 200, 400)
 P_PAIR = 6.0 / 16.0
+DUMP_BYTES = (64 << 20) - (1 << 16)   # --dump-outputs: at most 64 MiB in all, .npy headers included
 
 
 # ---------------------------------------------------------------- algorithmic work (SURVEY.md 8d / DESIGN.md)
@@ -54,6 +59,21 @@ def synth(L, B, rank=0):
 def to_strings(codes):
     lut = np.frombuffer(b"ACGU", np.uint8)
     return [bytes(lut[row]).decode() for row in codes]
+
+
+def dump_outputs(path, out):
+    """Write the arrays of `out` (name -> array, one row per sequence) as path/<name>.npy in float64, the structure bytes
+    in float32.  When the batch exceeds DUMP_BYTES a fixed-seed sample of rows is written, with its indices as row.npy."""
+    out = {k: a.astype(np.float32 if a.dtype == np.uint8 else np.float64) for k, a in out.items()}
+    B = len(next(iter(out.values())))
+    row_bytes = sum(a[0].nbytes for a in out.values()) + 8
+    if B * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // row_bytes, replace=False))
+        out = {k: a[rows] for k, a in out.items()}
+        out["row"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 # ---------------------------------------------------------------- clocks
@@ -120,8 +140,7 @@ def cpu_sample(L, budget_s, threads, fast=True):
     """Time the CPU arm (MFE + backtrack, PF inside, eval) on a bounded sample of the L-workload.
     fast: the tuned port (orc_mfe_fast / orc_pf_fast, bit-identical to the oracle, ~5x faster); else the clarity-first oracle.
     With ViennaRNA importable the sample runs get_mfe_e_ss's call sequence over a process pool instead (kind "reference")."""
-    from oracle.pyoracle import Oracle, build
-    build()
+    from oracle.pyoracle import Oracle   # loads the library build() made; compiles nothing into the tree
     O = Oracle(os.path.join(ROOT, "desirna_b200", "params", "turner1999_37C.par"))
     per_fold = (2.6e-8 * L ** 3 + 1.3e-6 * L ** 2) / (5.0 if fast else 1.0)  # rough single-thread seconds, only used to size the sample
     n = int(max(threads, min(65536, budget_s * threads / per_fold)))
@@ -297,6 +316,10 @@ def run_ours(args):
     main = measure(L, B, args.steps, args.warmup)
     launches = eng.kernel_launches() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the "+defect" column below reuses these buffers
+        mb = main["bufs"]
+        dump_outputs(args.dump_outputs, {"mfe_dcal": mb["mfe"].cpu().numpy(), "mfe_ss": mb["ss"].cpu().numpy(),
+                                         "pf": mb["pf"].cpu().numpy(), "eval_dcal": mb["ev"].cpu().numpy()})
     value = world * B * args.steps / (main["total_ms"] * 1e-3)
 
     # ---- e2e: the host-buffer C-ABI call, H2D/D2H inside the timed region (pinned host memory)
@@ -478,8 +501,7 @@ def run_ours(args):
     # form, the GPU kernels read them as +inf / 0 from the ring): reported next to the closed form the roofline uses (SURVEY 8d)
     if not args.no_cpu:
         try:
-            from oracle.pyoracle import Oracle, build
-            build()
+            from oracle.pyoracle import Oracle
             O = Oracle(os.path.join(ROOT, "desirna_b200", "params", "turner1999_37C.par"))
             cnt = np.array([O.mfe(sq, counts=True)[2] for sq in to_strings(synth(L, 32, rank=0))], dtype=np.float64)
             counted = float(cnt.sum(axis=1).mean())
@@ -684,7 +706,13 @@ def main():
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--peaks", action="store_true", help="measure INT32/FP64/smem chip peaks and write profiles/chip_peaks.json")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's sequences)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.peaks or args.impl != "b200" or args.workload != "sweep"):
+        ap.error("--dump-outputs applies to the sweep workload of --impl b200")
     args.warmup = max(3, args.warmup) if args.impl == "b200" else args.warmup
     if args.peaks:
         from desirna_b200 import engine as eng
