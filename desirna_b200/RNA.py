@@ -189,9 +189,8 @@ class fold_compound:
     def second_best_energy(self):
         """(MFE, energy of the second-best structure) in kcal/mol as C floats, or (MFE, None) when the sequence has a single
         structure: bf_second_best, a 2-best DP on the unambiguous grammar -- the number DesiRNA reads off subopt_cb's enumeration
-        (energy_scores.py:453-488) without the enumeration.  Extension of the shim; ViennaRNA has no such call."""
-        if "&" in self.sequence:
-            raise NotImplementedError("second_best_energy on two-strand compounds is not part of the accelerated path")
+        (energy_scores.py:453-488) without the enumeration.  'A&B' compounds: structures of the two-strand loop model of mfe_dimer()
+        and eval_structure(), connected or not.  Extension of the shim; ViennaRNA has no such call."""
         nopair = np.asarray(self._nopair, np.uint8)[None, :] if self._nopair is not None and any(self._nopair) else None
         e1, e2 = _eng.second_best([self.sequence], nopair)
         return f32(int(e1[0]) / 100.0), (f32(int(e2[0]) / 100.0) if int(e2[0]) < 10000000 else None)

@@ -527,8 +527,8 @@ int bf_second_best(const bf_batch_t *b, int32_t *e1_dcal, int32_t *e2_dcal) {
   if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
   if (!b || !e1_dcal || !e2_dcal || b->B < 0 || b->stride <= 0 || (b->B && (!b->seq || !b->len))) return fail(BF_ERR_ARG, "bf_second_best: bad argument");
   if (b->stride > 2000) return fail(BF_ERR_ARG, "bf_second_best: stride > 2000 not supported");
-  if (b->cut) for (int k = 0; k < b->B; k++) if (b->cut[k] > 0) return fail(BF_ERR_UNAVAILABLE, "bf_second_best: single-strand sequences only");
   if (b->B == 0) return BF_OK;
+  const bool two = any_cut(b, b->cut);
   cudaStream_t st = g.stream;
   const size_t B = b->B, S = b->stride;
   CU(g.d_seq.reserve(B * S), "cudaMalloc(seq)");
@@ -538,6 +538,11 @@ int bf_second_best(const bf_batch_t *b, int32_t *e1_dcal, int32_t *e2_dcal) {
   CU(cudaMemcpyAsync(g.d_len.p, b->len, B * sizeof(int), cudaMemcpyHostToDevice, st), "H2D len");
   BfBatchDev db;
   db.B = b->B; db.stride = b->stride; db.seq = (const char *)g.d_seq.p; db.len = (const int *)g.d_len.p; db.cut = nullptr; db.nopair = nullptr;
+  if (two) {
+    CU(g.d_cut.reserve(B * sizeof(int)), "cudaMalloc(cut)");
+    CU(cudaMemcpyAsync(g.d_cut.p, b->cut, B * sizeof(int), cudaMemcpyHostToDevice, st), "H2D cut");
+    db.cut = (const int32_t *)g.d_cut.p;
+  }
   if (b->nopair) {
     CU(g.d_nopair.reserve(B * S), "cudaMalloc(nopair)");
     CU(cudaMemcpyAsync(g.d_nopair.p, b->nopair, B * S, cudaMemcpyHostToDevice, st), "H2D nopair");
@@ -547,7 +552,7 @@ int bf_second_best(const bf_batch_t *b, int32_t *e1_dcal, int32_t *e2_dcal) {
   const int grid = std::min(b->B, 2 * g.sm_count);
   CU(g.w.ws_mfe.reserve((size_t)grid * bf_twobest_slot(wstride) * sizeof(int2)), "cudaMalloc(second-best workspace)");
   int *d_e = (int *)g.d_mfe.p;
-  CU(bf_launch_twobest(g.dP, db, (int2 *)g.w.ws_mfe.p, wstride, grid, g.w.d_counters + 0, d_e, d_e + B, st), "launch bf_k_mfe2");
+  CU(bf_launch_twobest(g.dP, db, (int2 *)g.w.ws_mfe.p, wstride, grid, g.w.d_counters + 0, d_e, d_e + B, st, nullptr, two), "launch bf_k_mfe2");
   g.launches++;
   CU(cudaMemcpyAsync(e1_dcal, d_e, B * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e1");
   CU(cudaMemcpyAsync(e2_dcal, d_e + B, B * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e2");
@@ -719,10 +724,10 @@ int design_score(DesignLoop *h, bool init = false) {
     // negative design: (best, second best) energies of the rows that fold into their target (rare rows; the others are skipped)
     CU(bf_launch_design_nd_flag(h->D, h->B, h->st), "launch bf_k_design_nd_flag");
     BfBatchDev db;
-    db.B = h->B; db.stride = h->D.stride; db.seq = h->D.mut_seq; db.len = h->D.row_len; db.cut = nullptr; db.nopair = nullptr;
+    db.B = h->B; db.stride = h->D.stride; db.seq = h->D.mut_seq; db.len = h->D.row_len; db.cut = h->two ? h->D.row_cut : nullptr; db.nopair = nullptr;
     const int wstride = h->D.stride + 2, grid = std::min(h->B, g.sm_count);
     CU(h->w.ws_mfe.reserve((size_t)grid * bf_twobest_slot(wstride) * sizeof(int2)), "cudaMalloc(second-best workspace)");
-    CU(bf_launch_twobest(g.dP, db, (int2 *)h->w.ws_mfe.p, wstride, grid, h->w.d_counters + 3, h->D.o_e1, h->D.o_e2, h->st, h->D.nd_flag), "launch bf_k_mfe2");
+    CU(bf_launch_twobest(g.dP, db, (int2 *)h->w.ws_mfe.p, wstride, grid, h->w.d_counters + 3, h->D.o_e1, h->D.o_e2, h->st, h->D.nd_flag, h->two), "launch bf_k_mfe2");
     g.launches += 2;
   }
   if (!h->pks) return BF_OK;
@@ -806,7 +811,7 @@ int bf_design_create(const bf_design_t *c, void **handle) {
       if (!sk.empty()) return fail(BF_ERR_ARG, "bf_design_create: unbalanced target");
   }
   if (c->pks && two) return fail(BF_ERR_ARG, "bf_design_create: the pseudoknot overlay needs single-strand jobs");
-  if (c->subopt && (two || c->pks)) return fail(BF_ERR_ARG, "bf_design_create: negative design (subopt) needs single-strand jobs without the pseudoknot overlay");
+  if (c->subopt && c->pks) return fail(BF_ERR_ARG, "bf_design_create: negative design (subopt) does not combine with the pseudoknot overlay");
   if (!two && (bf_fill_mfe_mode(S) == 0 || bf_fill_pf_mode(S) == 0)) return fail(BF_ERR_UNAVAILABLE, "bf_design_create: stride outside the fill path");
   // optional scenario terms: alternative structures, motifs
   const int max_alt = c->alt_targets ? c->max_alt : 0;

@@ -371,7 +371,9 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_accept(BfDesignDev D, B
       rec[kRecEd2] = sum / D.n_alt[job];
       total += rec[kRecEd2] - Epf;
     }
-    if (C.subopt && D.nd_flag && D.nd_flag[row]) {   // -nd on: the mutant folds into the target; second-best structure within 49 kcal/mol, else 0
+    // -nd on: the mutant folds into the target (1 - mcc == 0, as the reference tests it: a fully paired duplex that folds into its
+    // target has mcc 0); second-best structure within 49 kcal/mol, else 0
+    if (C.subopt && D.nd_flag && D.nd_flag[row] && rec[kRecMcc] == 0.0) {
       const int e1 = D.o_e1[row], e2 = D.o_e2[row];
       rec[kRecSubopt] = (e2 < BF_INF && e2 - e1 <= 4900) ? (double)(float)((double)e2 / 100.0) : 0.0;
       total -= rec[kRecSubopt] - Epf;

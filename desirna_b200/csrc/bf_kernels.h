@@ -75,7 +75,8 @@ cudaError_t bf_launch_pf_cl(const BfParams *dP, const BfBatchDev &b, double *qbt
 // ---- second-best structure energy by a 2-best DP on the unambiguous grammar (bf_twobest.cu)
 size_t bf_twobest_slot(int wstride);   // int2 entries of HBM workspace per CTA
 cudaError_t bf_launch_twobest(const BfParams *dP, const BfBatchDev &b, int2 *ws, int wstride, int grid, int *work_counter, int *out_e1, int *out_e2,
-                              cudaStream_t st, const uint8_t *only = nullptr);   // only: optional per-sequence flags, 0 = skip
+                              cudaStream_t st, const uint8_t *only = nullptr,    // only: optional per-sequence flags, 0 = skip
+                              bool two = false);                                 // two: some row has a cut (b.cut), nick-aware grammar
 
 // ---- exterior recursions for small batches (bf_ext.cu): one CTA per sequence
 bool bf_ext_wide_ok(int nmax);

@@ -141,15 +141,14 @@ def subopt(seq, delta_dcal, nopair=None, max_out=4096):
 
 def second_best(seqs, nopair=None):
     """bf_second_best: (e1, e2) int32 arrays, dcal/mol -- energies of the best and the second-best structure of every sequence
-    (single strands); e2 >= 10000000 where a sequence has no second structure."""
+    ('A&B' for two strands); e2 >= 10000000 where a sequence has no second structure."""
     ensure_ready()
     buf, lens, cuts = pack([s.upper().replace("T", "U") for s in seqs])
-    if cuts.any():
-        raise EngineError(3, "second_best: single-strand sequences only")
     b = bf_batch_t()
     b.B, b.stride = len(seqs), buf.shape[1]
     b.seq, b.len = buf.ctypes.data, lens.ctypes.data
-    keep = [buf, lens]
+    b.cut = cuts.ctypes.data if cuts.any() else None
+    keep = [buf, lens, cuts]
     if nopair is not None:
         nopair = np.ascontiguousarray(nopair, np.uint8)
         assert nopair.shape == buf.shape

@@ -321,9 +321,9 @@ class ScoreSeq:
 def get_first_suboptimal_energy(sequence, a):
     """get_first_suboptimal_structure_and_energy(sequence, a, 1)[1] without the enumeration: the reference widens the band from 1 to
     49 kcal/mol until it holds two structures and takes the second of the sorted list -- i.e. the energy of the second-best
-    structure if it lies within 49 kcal/mol of the MFE, else 0 (utils/energy_scores.py:476-488).  Two-strand compounds fall back to
-    the enumeration (which the shim does not provide for them either)."""
-    if "&" in sequence or not hasattr(a, "second_best_energy"):
+    structure if it lies within 49 kcal/mol of the MFE, else 0 (utils/energy_scores.py:476-488).  Single- and two-strand ('A&B')
+    compounds alike; a compound without second_best_energy falls back to the enumeration."""
+    if not hasattr(a, "second_best_energy"):
         return get_first_suboptimal_structure_and_energy(sequence, a, 1)[1]
     e1, e2 = a.second_best_energy()
     if e2 is None or round((e2 - e1) * 100.0) > 4900:

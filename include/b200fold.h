@@ -87,10 +87,12 @@ int bf_score_batch_device(const bf_batch_t *batch, bf_result_t *result, void *cu
  * sorted by energy.  The O(N^3) tables come from the GPU MFE fill; the output-sensitive walk over them runs on the host.
  * ss_out: max_out x (len+1) chars, e_out: max_out energies in dcal/mol, *n_out: structures written (<= max_out),
  * *truncated: 1 if the band holds more than max_out structures.  nopair: optional len bytes (hard constraint 'x'). */
-/* Energies (dcal/mol) of the best and of the second-best secondary structure of every sequence of the batch (seq, len, nopair,
- * stride as in bf_score_batch; single strands), by one DP over (best, second best) pairs on the unambiguous grammar -- what
+/* Energies (dcal/mol) of the best and of the second-best secondary structure of every sequence of the batch (seq, len, cut,
+ * nopair, stride as in bf_score_batch), by one DP over (best, second best) pairs on the unambiguous grammar -- what
  * get_first_suboptimal_structure_and_energy(seq, fc, 1)[1] reads off fc.subopt_cb's enumeration (utils/energy_scores.py:453-488,
- * RNA.cvar.uniq_ML = 1).  e2 >= 10000000: there is no second structure.  Two structures of equal energy count twice (e2 == e1). */
+ * RNA.cvar.uniq_ML = 1).  e2 >= 10000000: there is no second structure.  Two structures of equal energy count twice (e2 == e1).
+ * Rows with cut > 0 are two strands under the loop model of bf_score_batch's two-strand MFE and eval: unconnected structures
+ * count, a connected one pays DuplexInit once; e1 equals that MFE. */
 int bf_second_best(const bf_batch_t *batch, int32_t *e1_dcal, int32_t *e2_dcal);
 int bf_subopt(const char *seq, int32_t len, const uint8_t *nopair, int32_t delta_dcal, int32_t max_out, char *ss_out, int32_t *e_out,
               int32_t *n_out, int32_t *truncated);
@@ -170,7 +172,8 @@ typedef struct {
   const char *snake_letter;  /* n_jobs x stride x 4: letter of the position in each colouring of its graph, 0 = colouring absent;
                                 a move on a graph node sets every node of the graph to another colouring   :1085-1094 */
   int32_t subopt;            /* 1: negative design (-nd on): a mutant that folds into its target also pays Epf - E(second-best
-                                structure), the latter from bf_second_best's DP                 energy_scores.py:104-107,453-488 */
+                                structure), the latter from bf_second_best's DP (two-strand jobs too; not with pks)
+                                                                                                energy_scores.py:104-107,453-488 */
 } bf_design_t;
 
 enum { BF_DESIGN_REC = 15 }; /* doubles per record: scoring_function, edesired, Epf, 1-mcc, 1-precision, 1-recall, MFE,
