@@ -14,6 +14,17 @@
 #include "bf_kernels.h"
 #include "bf_params.h"
 
+// The switches that override a default kernel-selection rule (include/b200fold.h lists what each does).  They are read where the
+// choice is made (BF_FORCE_GENERIC at bf_init, BF_DESIGN_OVERLAP at bf_design_create, the others at every call), so that a host
+// program can flip them between calls on one engine.
+static const char *const kOptions[] = {"BF_CL", "BF_CL_C", "BF_CL_BW", "BF_EXT_WIDE", "BF_WIDE", "BF_FILL3", "BF_FILL3_SMALL",
+                                       "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP"};
+
+int bf_opt(const char *name, int dflt) {
+  const char *v = getenv(name);
+  return (v && *v) ? atoi(v) : dflt;
+}
+
 namespace {
 
 struct DevBuf {
@@ -123,8 +134,8 @@ int validate(const bf_batch_t *b, const bf_result_t *r) {
 
 // exterior recursions by one CTA per sequence instead of one warp per sequence: batches that leave SMs idle (BF_EXT_WIDE=0/1 overrides)
 bool wide_ext(int B, int stride) {
-  const char *v = getenv("BF_EXT_WIDE");
-  if (v && *v) return atoi(v) != 0 && bf_ext_wide_ok(stride);
+  const int v = bf_opt("BF_EXT_WIDE", -1);
+  if (v >= 0) return v != 0 && bf_ext_wide_ok(stride);
   return B <= 2 * g.sm_count && bf_ext_wide_ok(stride);
 }
 
@@ -277,10 +288,8 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
 // up to 400 nt the default scale keeps every scaled quantity far inside the double range (|E| <= 0.9 kcal/mol/nt: < 1e201).
 int overlap_scale(const bf_batch_t *b, const int **ov) {
   *ov = nullptr;
-  const char *v = getenv("BF_SCORE_OVERLAP");
-  if (v && v[0] == '0') return BF_OK;
   if (!(b->want & (BF_WANT_MFE | BF_WANT_SS)) || !(b->want & BF_WANT_PF) || (b->want & (BF_WANT_BPP | BF_WANT_DEFECT)) || b->nopair) return BF_OK;
-  if ((2 * b->B > g.sm_count && !(v && v[0] == '2')) || b->stride > 400) return BF_OK;   // 2: any batch size (experiments)
+  if (2 * b->B > g.sm_count || b->stride > 400) return BF_OK;
   if (g.zero_cap < (size_t)b->B) {
     const size_t n = std::max<size_t>(256, (size_t)b->B);
     CU(g.d_zero.reserve(n * sizeof(int)), "cudaMalloc(zero scale)");
@@ -324,7 +333,7 @@ int bf_init(int device) {
   CU(cudaGetDeviceProperties(&prop, device), "cudaGetDeviceProperties");
   if (prop.major < 10) return fail(BF_ERR_CUDA, std::string("built for sm_100a, found ") + prop.name);
   g.device = device;
-  { const char *fg = getenv("BF_FORCE_GENERIC"); g.force_generic = fg && fg[0] == '1'; }
+  g.force_generic = bf_opt("BF_FORCE_GENERIC", 0) == 1;
   g.sm_count = prop.multiProcessorCount;
   bf_fill_set_sms(g.sm_count);
   CU(cudaStreamCreateWithFlags(&g.stream, cudaStreamNonBlocking), "cudaStreamCreate");
@@ -446,8 +455,7 @@ int bf_score_batch(const bf_batch_t *b, bf_result_t *r) {
                o_tg = o_np + (b->nopair ? up(B * S) : 0), in_bytes = o_tg + up(B * T * S);
   const size_t p_ss = up(B * sizeof(int)), p_pf = p_ss + up(B * (S + 1)), p_ev = p_pf + up(B * 5 * sizeof(double)),
                p_df = p_ev + up(B * std::max<size_t>(T, 1) * sizeof(int)), out_bytes = p_df + up(B * sizeof(double));
-  const char *stage_env = getenv("BF_STAGE");
-  if (in_bytes <= ((size_t)256 << 10) && out_bytes <= ((size_t)256 << 10) && !(stage_env && stage_env[0] == '0')) {
+  if (in_bytes <= ((size_t)256 << 10) && out_bytes <= ((size_t)256 << 10)) {
     CU(reserve_pinned(&g.h_in, &g.h_in_cap, in_bytes), "cudaMallocHost(inputs)");
     CU(reserve_pinned(&g.h_out, &g.h_out_cap, out_bytes), "cudaMallocHost(results)");
     CU(g.d_in.reserve(in_bytes), "cudaMalloc(inputs)");
@@ -613,9 +621,7 @@ int bf_last_kernel_ms(double out[3]) {
 }
 
 int bf_set_option(const char *key, int value) {
-  // Kernel variants are chosen per call from BF_* environment variables (bf_fill.cu, bf_fill3.cu, bf_cluster.cu, this file); this
-  // sets one of them from the host program: key "cl" -> BF_CL, "cl_c" -> BF_CL_C, "ext_wide" -> BF_EXT_WIDE, "wide" -> BF_WIDE, ...
-  // A negative value removes the variable (back to the default rule).
+  // key "cl" -> BF_CL, "cl_c" -> BF_CL_C, ...: one of kOptions.  A negative value removes the variable (back to the default rule).
   if (!key || !*key) return fail(BF_ERR_ARG, "null option key");
   std::string name = "BF_";
   for (const char *p = key; *p; p++) {
@@ -623,6 +629,7 @@ int bf_set_option(const char *key, int value) {
     if (!((ch >= 'a' && ch <= 'z') || (ch >= 'A' && ch <= 'Z') || (ch >= '0' && ch <= '9') || ch == '_')) return fail(BF_ERR_ARG, std::string("bad option key: ") + key);
     name += (char)((ch >= 'a' && ch <= 'z') ? ch - 'a' + 'A' : ch);
   }
+  if (std::find(std::begin(kOptions), std::end(kOptions), name) == std::end(kOptions)) return fail(BF_ERR_ARG, std::string("unknown option: ") + key);
   if (value < 0) unsetenv(name.c_str());
   else setenv(name.c_str(), std::to_string(value).c_str(), 1);
   return BF_OK;
@@ -661,13 +668,6 @@ struct DesignLoop {
   bool two = false;   // some job has two strands: the loop folds with the two-strand kernels
   bool pks = false;   // pseudoknot overlay: three constrained refolds after the MFE fold of every sub-step
   bool overlap = true;  // BF_DESIGN_OVERLAP=0: always fold MFE, then PF
-  int overlap_x2 = 16;  // BF_DESIGN_OVERLAP_X: batch size up to which the two fills run side by side, in units of half the SM count
-                        // (measured: pays at every size tried, 0.76 -> 0.42 ms per sub-step at 64 x 104 nt, 15.5 -> 14.4 ms at 296 x 400 nt)
-  // one global step (re_attempt sub-steps, neighbour swaps) as a CUDA graph: one launch instead of ~8 per sub-step
-  bool use_graph = false;         // BF_DESIGN_GRAPH=1
-  cudaGraphExec_t gexec = nullptr;
-  int graph_B = -1;
-  int64_t graph_nodes = 0;
   std::vector<void *> allocs;
   std::vector<uint8_t> active;
   uint8_t *d_active = nullptr;
@@ -682,8 +682,6 @@ struct DesignLoop {
   }
   void destroy() {
     if (st) cudaStreamSynchronize(st);
-    if (gexec) cudaGraphExecDestroy(gexec);
-    gexec = nullptr;
     for (void *q : allocs) cudaFree(q);
     allocs.clear();
     w.destroy();
@@ -716,8 +714,10 @@ int design_score(DesignLoop *h, bool init = false) {
   bf_result_t r;
   std::memset(&r, 0, sizeof r);
   r.mfe_dcal = h->D.o_mfe; r.mfe_ss = h->D.o_ss; r.pf = h->D.o_pf; r.eval_dcal = h->D.o_eval; r.defect = h->D.o_defect;
-  // small batches: partition function beside the MFE fill, scaled by the parent sequence's MFE (kept per replica)
-  const bool beside = !init && h->overlap && h->B * 2 <= g.sm_count * (h->two ? 1 : h->overlap_x2) && !(h->want & BF_WANT_DEFECT);
+  // small batches: partition function beside the MFE fill, scaled by the parent sequence's MFE (kept per replica).  Single strands
+  // up to 8 x the SM count (measured: pays at every size tried, 0.76 -> 0.42 ms per sub-step at 64 x 104 nt, 15.5 -> 14.4 ms at
+  // 296 x 400 nt), two strands up to half the SM count
+  const bool beside = !init && h->overlap && h->B * 2 <= g.sm_count * (h->two ? 1 : 16) && !(h->want & BF_WANT_DEFECT);
   int rc = run_device(h->w, &b, &r, h->two, h->st, beside ? h->D.row_scale : nullptr, false);
   if (rc) return rc;
   if (h->C.subopt) {
@@ -746,20 +746,6 @@ int design_score(DesignLoop *h, bool init = false) {
     CU(bf_launch_design_pk_paint(h->D, h->B, round, h->st), "launch bf_k_design_pk_paint");
     g.launches += 2;
   }
-  return BF_OK;
-}
-
-// the launches of one global step; gstep < 0: inside a graph capture (the kernels read the step number from device memory)
-int design_enqueue_global_step(DesignLoop *h, int gstep, int64_t *launches) {
-  for (int k = 0; k < h->re_attempt && h->B > 0; k++) {
-    CU(bf_launch_design_propose(h->D, h->C, h->B, false, h->st), "launch bf_k_design_propose");
-    int rc = design_score(h);
-    if (rc) return rc;
-    CU(bf_launch_design_accept(h->D, h->C, h->B, false, gstep, h->st), "launch bf_k_design_accept");
-    *launches += 2;
-  }
-  CU(bf_launch_design_exchange(h->D, h->C, h->d_active, gstep, h->st), "launch bf_k_design_exchange");
-  *launches += 2;
   return BF_OK;
 }
 }  // namespace
@@ -840,12 +826,7 @@ int bf_design_create(const bf_design_t *c, void **handle) {
   DesignLoop *h = new DesignLoop;
   h->two = two;
   h->pks = c->pks != 0;
-  { const char *ov = getenv("BF_DESIGN_OVERLAP"); h->overlap = !(ov && ov[0] == '0'); }
-  { const char *ox = getenv("BF_DESIGN_OVERLAP_X"); h->overlap_x2 = (ox && atoi(ox) > 0) ? atoi(ox) : 16; }
-  // measured (bench.py design_loop, profiles/r02_design_graph.txt): one loop alone gains 2-6 % per sub-step (36 nt x 10: 0.111 ->
-  // 0.104 ms, 104 nt x 64: 0.402 -> 0.396 ms) -- the sub-step is a chain of short kernels, not launch-bound -- while seven loops
-  // advancing side by side lose 16 % (their graphs overlap less than their plain launches): opt-in
-  { const char *gr = getenv("BF_DESIGN_GRAPH"); h->use_graph = gr && gr[0] == '1'; }
+  h->overlap = bf_opt("BF_DESIGN_OVERLAP", 1) != 0;
   std::memset(&h->D, 0, sizeof h->D);
   std::memset(&h->C, 0, sizeof h->C);
   auto bail = [&](cudaError_t e, const char *what) { h->destroy(); delete h; return cuda_fail(e, what); };
@@ -864,7 +845,6 @@ int bf_design_create(const bf_design_t *c, void **handle) {
   DCU(h->alloc(&D.best_rec, (size_t)J * kDesignRec), "cudaMalloc(design)");
   DCU(h->alloc(&D.solved_step, J), "cudaMalloc(design)"); DCU(h->alloc(&D.n_solved, J), "cudaMalloc(design)");
   DCU(h->alloc(&D.re_counts, (size_t)J * 3), "cudaMalloc(design)");
-  DCU(h->alloc(&D.gstep_dev, 1), "cudaMalloc(design)");
   DCU(h->alloc(&D.cur_seq, G * S), "cudaMalloc(design)"); DCU(h->alloc(&D.cur_ss, G * (S + 1)), "cudaMalloc(design)");
   DCU(h->alloc(&D.rec, G * kDesignRec), "cudaMalloc(design)"); DCU(h->alloc(&D.shelf, G), "cudaMalloc(design)");
   DCU(h->alloc(&D.rng, G), "cudaMalloc(design)"); DCU(h->alloc(&D.counts, G * 3), "cudaMalloc(design)");
@@ -968,34 +948,15 @@ int bf_design_run(void *handle, int32_t global_steps) {
   if (!h || global_steps < 0) return fail(BF_ERR_ARG, "bf_design_run: bad argument");
   for (int s = 0; s < global_steps; s++) {
     h->gstep++;
-    if (h->use_graph && h->B > 0) {
-      if (!h->gexec || h->graph_B != h->B) {
-        // (re-)capture: the set of active rows changed, or first use.  Buffers were sized by the uncaptured scoring pass of
-        // bf_design_create; the kernels take the global-step number from device memory.
-        if (h->gexec) { cudaGraphExecDestroy(h->gexec); h->gexec = nullptr; }
-        cudaGraph_t graph = nullptr;
-        int64_t nodes = 0;
-        const int64_t before = g.launches;   // the fold pipeline counts its kernels as it enqueues them: during capture nothing runs
-        CU(cudaStreamBeginCapture(h->st, cudaStreamCaptureModeRelaxed), "cudaStreamBeginCapture");
-        int rc = design_enqueue_global_step(h, -1, &nodes);
-        cudaError_t ce = cudaStreamEndCapture(h->st, &graph);
-        if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-        if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
-        ce = cudaGraphInstantiate(&h->gexec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (ce != cudaSuccess) { h->gexec = nullptr; return cuda_fail(ce, "cudaGraphInstantiate"); }
-        h->graph_B = h->B;
-        h->graph_nodes = nodes + (g.launches - before);   // kernels per launch of the graph
-        g.launches = before;
-      }
-      CU(cudaGraphLaunch(h->gexec, h->st), "cudaGraphLaunch");
-      g.launches += h->graph_nodes;
-    } else {
-      int64_t n = 0;
-      int rc = design_enqueue_global_step(h, h->gstep, &n);
+    for (int k = 0; k < h->re_attempt && h->B > 0; k++) {
+      CU(bf_launch_design_propose(h->D, h->C, h->B, false, h->st), "launch bf_k_design_propose");
+      int rc = design_score(h);
       if (rc) return rc;
-      g.launches += n;
+      CU(bf_launch_design_accept(h->D, h->C, h->B, false, h->gstep, h->st), "launch bf_k_design_accept");
+      g.launches += 2;
     }
+    CU(bf_launch_design_exchange(h->D, h->C, h->d_active, h->gstep, h->st), "launch bf_k_design_exchange");
+    g.launches++;
   }
   return BF_OK;
 }

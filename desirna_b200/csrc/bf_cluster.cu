@@ -110,15 +110,13 @@ MfeClPlan mfe_cl_plan(int nmax, const ClGeom &g) {
 template <int NW, int NT>
 __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__restrict__ P, BfBatchDev b, int *ctri, int *ftri, size_t tri_slot,
                                                           int *ent_ws, size_t ent_slot, const uint32_t *__restrict__ taps, MfeClPlan pl, ClGeom g,
-                                                          int *work_counter, long long *trace) {
+                                                          int *work_counter) {
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ int s_seq;
   __shared__ unsigned char s_meta[96];
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(BF_FULL, tid >> 5, 0);
   const int r = (int)cl_rank(), C = g.C, logC = g.logC, BW = g.BW, logBW = g.logBW, WIN = g.WIN, RS = g.RS, ncl = g.ncl;
-  // BF_CL_TRACE: cycle stamps of cluster 0 / rank 0, [diagonal][warp][8 points]
-#define CL_STAMP(k_) do { if (trace && lane == 0 && r == 0 && cl_index() == 0) trace[((size_t)d * NW + warp) * 8 + (k_)] = clock64(); } while (0)
   int *RG = reinterpret_cast<int *>(dyn + pl.o_ring);
   int *DML = reinterpret_cast<int *>(dyn + pl.o_dml);
   int *FP = reinterpret_cast<int *>(dyn + pl.o_fp);
@@ -274,7 +272,6 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__rest
     int rowd = (BF_TURN + 1) % kDepth;   // ring row of diagonal d
     for (int d = BF_TURN + 1; d <= n; d++, rowd = rowd + 1 == kDepth ? 0 : rowd + 1) {
       const int buf = d & 1;
-      CL_STAMP(0);
       // ------------------------------------------------------------ taps: c(i,j) of this CTA's pairable cells of diagonal d
       if (warp < NT && d <= n - 1) {
         const int np = NP[d];
@@ -342,7 +339,6 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__rest
         else if (ng <= 8) cells(integral_constant<int, 8>(), integral_constant<int, kNS1>(), integral_constant<int, kNSB>());
         else cells(integral_constant<int, kNSG>(), integral_constant<int, kNS1>(), integral_constant<int, kNSB>());
         __syncwarp();
-        CL_STAMP(1);
       }
       // ------------------------------------------------------------ combine of diagonal d-1: this CTA's cells (dealt from the last warp down)
       constexpr int NWS = NW - NT;
@@ -399,9 +395,7 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__rest
       // ------------------------------------------------------------ HBM tables: the last warp writes what the previous phases left in
       // shared memory (c of diagonal d-1, fML of diagonal d-2), so that no thread has a global store in flight when it reaches the
       // cluster barrier's release
-      CL_STAMP(3);
       if (aw == NWS - 1) mfe_flush(d - 1, d - 2);
-      CL_STAMP(4);
       // ------------------------------------------------------------ split partials of diagonal d over this CTA's split positions
       if (aw >= 0 && d <= n - 1) {
         const int ncell = n - d, nch = (ncell + 31) >> 5;
@@ -439,7 +433,6 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__rest
           }
         }
       }
-      CL_STAMP(5);
       cl_arrive();
       // ---- between arrive and wait: work that nobody else sees
       if (warp < NT) {
@@ -455,9 +448,7 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_mfe_cl(const BfParams *__rest
           RG[row * RS + x] = BF_INF; RG[(kDepth + row) * RS + x] = BF_INF; RG[(2 * kDepth + row) * RS + x] = BF_INF;
         }
       }
-      CL_STAMP(6);
       cl_wait();
-      CL_STAMP(7);
     }
     if (warp == NW - 1) mfe_flush(n, n - 1);   // fML of the last diagonal
   }
@@ -830,10 +821,6 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_pf_cl(const BfParams *__restr
   cl_sync();
 }
 
-int env_int(const char *name, int dflt) {
-  const char *v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}
 constexpr size_t kSmemBudgetCl = 232448 - 1024 - 256;
 
 int ilog2(int x) { int l = 0; while ((1 << l) < x) l++; return l; }
@@ -911,8 +898,8 @@ ClCfg mfe_cl_cfg(int nmax, int B) {
   ClCfg c;
   c.ok = c.dflt = false; c.slots = 0;
   if (nmax < 1 || nmax > 2000) return c;
-  const int cforce = env_int("BF_CL_C", 0);
-  const int bw = env_int("BF_CL_BW", 32);
+  const int cforce = bf_opt("BF_CL_C", 0);
+  const int bw = bf_opt("BF_CL_BW", 32);
   if (bw != 16 && bw != 32) return c;
   const ClSlots &sl = cl_slots(g_slots_mfe, bf_k_mfe_cl<kNWcl, kNTcl>);
   int best_rounds = 1 << 30;
@@ -935,8 +922,8 @@ PfClCfg pf_cl_cfg(int nmax, int B) {
   PfClCfg c;
   c.ok = c.dflt = false; c.slots = 0;
   if (nmax < 1 || nmax > 2000) return c;
-  const int cforce = env_int("BF_CL_C", 0);
-  const int bw = env_int("BF_CL_BW", 32);
+  const int cforce = bf_opt("BF_CL_C", 0);
+  const int bw = bf_opt("BF_CL_BW", 32);
   if (bw != 16 && bw != 32) return c;
   const ClSlots &sl = cl_slots(g_slots_pf, bf_k_pf_cl<kNWcl, kNTcl>);
   int best_rounds = 1 << 30;
@@ -974,7 +961,7 @@ cudaError_t cl_launch(K kern, int nclusters, int C, unsigned smem, cudaStream_t 
 // The cluster kernels take a batch when asked to (BF_CL=1, wherever they cover the length) or, by default, when the batch fits in
 // few rounds of the clusters in flight (see *_rounds_allowed); BF_CL=0 switches them off.
 bool bf_cl_mfe_use(int nmax, int B) {
-  const int m = env_int("BF_CL", -1);
+  const int m = bf_opt("BF_CL", -1);
   if (m == 0) return false;
   const ClCfg c = mfe_cl_cfg(nmax, B);
   return c.ok && (m == 1 || c.dflt);
@@ -1002,22 +989,13 @@ cudaError_t bf_launch_mfe_cl(const BfParams *dP, const BfBatchDev &b, int *ctri,
   if (e != cudaSuccess) return e;
   const int ncluster = b.B < c.slots ? b.B : c.slots;
   const size_t tri_slot = bf_tri_slot(b.stride), ent_slot = bf_cl_mfe_ws_slot(b.stride, b.B);
-  static long long *trace = nullptr;
-  const bool tr = env_int("BF_CL_TRACE", 0) != 0;
-  if (tr && !trace) { cudaMallocManaged(&trace, (size_t)2048 * kNWcl * 8 * sizeof(long long)); }
-  if (tr) memset(trace, 0, (size_t)2048 * kNWcl * 8 * sizeof(long long));
-  e = cl_launch(bf_k_mfe_cl<kNWcl, kNTcl>, ncluster, c.g.C, c.pl.total, st, dP, b, ctri, ftri, tri_slot, ws, ent_slot, taps, c.pl, c.g,
-                work_counter, tr ? trace : (long long *)nullptr);
-  if (tr && e == cudaSuccess) {   // debugging aid: dump the stamps of the launch
-    cudaStreamSynchronize(st);
-    if (FILE *f = fopen("gpurun_out/cl_trace.bin", "wb")) { fwrite(trace, sizeof(long long), (size_t)2048 * kNWcl * 8, f); fclose(f); }
-  }
-  return e;
+  return cl_launch(bf_k_mfe_cl<kNWcl, kNTcl>, ncluster, c.g.C, c.pl.total, st, dP, b, ctri, ftri, tri_slot, ws, ent_slot, taps, c.pl, c.g,
+                   work_counter);
 }
 
 // ---------------------------------------------------------------------------------------------------- partition function
 bool bf_cl_pf_use(int nmax, int B) {
-  const int m = env_int("BF_CL", -1);
+  const int m = bf_opt("BF_CL", -1);
   if (m == 0) return false;
   const PfClCfg c = pf_cl_cfg(nmax, B);
   return c.ok && (m == 1 || c.dflt);

@@ -292,8 +292,7 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_propose(BfDesignDev D, 
 // ------------------------------------------------------------------------------------------------ accept
 // score record of the mutant (energy_scores.py:31-125 with the float32 conventions of the ViennaRNA API, sim_score.py:62-147)
 // and the Metropolis test (replica_exchange_monte_carlo.py:26-77)
-__global__ void __launch_bounds__(kWPB * 32) bf_k_design_accept(BfDesignDev D, BfDesignCfg C, int B, int init, int gstep_arg) {
-  const int gstep = gstep_arg >= 0 ? gstep_arg : *D.gstep_dev;   // negative: the launch sits in a captured graph
+__global__ void __launch_bounds__(kWPB * 32) bf_k_design_accept(BfDesignDev D, BfDesignCfg C, int B, int init, int gstep) {
   extern __shared__ __align__(16) unsigned char dyn[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, row = blockIdx.x * kWPB + warp;
   if (row >= B) return;
@@ -422,9 +421,8 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_accept(BfDesignDev D, B
 // ------------------------------------------------------------------------------------------------ exchange
 // End of a global step: record the best state of every job, then the neighbour swaps in temperature order
 // (replica_exchange_monte_carlo.py:113-173: pairs (1,2),(3,4).. on even global steps, (0,1),(2,3).. on odd ones).
-__global__ void bf_k_design_exchange(BfDesignDev D, BfDesignCfg C, const uint8_t *active, int gstep_arg) {
+__global__ void bf_k_design_exchange(BfDesignDev D, BfDesignCfg C, const uint8_t *active, int gstep) {
   const int job = blockIdx.x * blockDim.x + threadIdx.x;
-  const int gstep = gstep_arg >= 0 ? gstep_arg : *D.gstep_dev;   // negative: the launch sits in a captured graph
   if (job >= D.J || (active && !active[job])) return;
   const int R = D.R, S = D.stride;
   double *best = D.best_rec + (size_t)job * kDesignRec;
@@ -505,12 +503,8 @@ cudaError_t bf_launch_design_accept(const BfDesignDev &D, const BfDesignCfg &C, 
   bf_k_design_accept<<<(B + kWPB - 1) / kWPB, kWPB * 32, scratch_bytes(D.stride), st>>>(D, C, B, init ? 1 : 0, gstep);
   return cudaGetLastError();
 }
-// after the exchange: the sub-steps that follow belong to the next global step
-__global__ void bf_k_design_advance(int *gstep_dev, int gstep_arg) { *gstep_dev = (gstep_arg >= 0 ? gstep_arg : *gstep_dev) + 1; }
-
 cudaError_t bf_launch_design_exchange(const BfDesignDev &D, const BfDesignCfg &C, const uint8_t *active, int gstep, cudaStream_t st) {
   if (D.J <= 0) return cudaSuccess;
   bf_k_design_exchange<<<(D.J + 63) / 64, 64, 0, st>>>(D, C, active, gstep);
-  bf_k_design_advance<<<1, 1, 0, st>>>(D.gstep_dev, gstep);
   return cudaGetLastError();
 }

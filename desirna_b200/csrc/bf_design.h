@@ -55,8 +55,6 @@ struct BfDesignDev {
   int *solved_step;              // J            first global step at whose end a replica folds into the target, -1 before
   unsigned int *n_solved;        // J            replica states (at global-step ends) that fold into the target
   unsigned int *re_counts;       // J x 3        neighbour swaps accepted, accepted because not worse, rejected (Stats, :671-792)
-  int *gstep_dev;                // 1            global step the sub-steps in flight belong to (written by the exchange kernel), so
-                                 //              that a captured CUDA graph of a global step does not bake the number in
   // per replica g = job * R + r
   char *cur_seq, *cur_ss;        // G x stride, G x (stride+1)
   double *rec;                   // G x kDesignRec

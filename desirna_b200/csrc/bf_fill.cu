@@ -59,11 +59,10 @@ __device__ __forceinline__ int ptype_sp(const uint8_t *SP, int i, int j) { retur
 // placement flags of the MFE fill: where the tables that are re-read every diagonal live
 constexpr int kMfeFmSmem = 1;   // packed fML table on chip (else: the per-sequence HBM copy, L2-resident while in use)
 constexpr int kMfeRgSmem = 2;   // the three 32-deep pair rings on chip (else: per-CTA HBM workspace)
-constexpr int kTabSmem = 8;     // small loop tables (BfSmallI / BfSmallD) staged per CTA (else: read through L1)
 
 struct MfePlan {
   int rs;  // ring row stride (ints)
-  size_t o_S, o_SP, o_toff, o_pg, o_pb, o_p1, o_fm, o_ring, o_dml, o_pi, o_ps, o_list, o_tab, o_sa, o_f5, total;
+  size_t o_S, o_SP, o_toff, o_pg, o_pb, o_p1, o_fm, o_ring, o_dml, o_pi, o_ps, o_list, o_sa, o_f5, total;
 };
 __host__ __device__ inline MfePlan mfe_plan(int nmax, int nw, int pl, bool blk = false, bool atom = false) {
   MfePlan p;
@@ -82,7 +81,6 @@ __host__ __device__ inline MfePlan mfe_plan(int nmax, int nw, int pl, bool blk =
   p.o_pi = o; o += (size_t)2 * nbuf * p.rs * sizeof(int);
   p.o_ps = o; o += (size_t)2 * nbuf * p.rs * sizeof(int);
   p.o_list = o; o += (size_t)2 * p.rs * sizeof(unsigned short);  // pairable cells of a diagonal, double-buffered
-  p.o_tab = o; o += (pl & kTabSmem) ? (sizeof(BfSmallI) + 15) / 16 * 16 : 0;
   o = (o + 15) / 16 * 16;
   p.o_sa = o; o += blk ? (size_t)3 * ((nmax + 3) / 4) * 16 * sizeof(int) : 0;  // blocked-split minima of three tile-diagonals
   p.o_f5 = o; o += nw == 16 ? (size_t)(nmax + 8) * sizeof(int) : 0;   // exterior recursion inside the fill (16-warp variants)
@@ -155,9 +153,7 @@ __global__ void __launch_bounds__(NW * 32) bf_k_mfe_fill(const BfParams *__restr
 
   for (int k = tid; k < (int)(pl.total / 4); k += blockDim.x) reinterpret_cast<int *>(dyn)[k] = 0;
   __syncthreads();
-  if (PL & kTabSmem) bf_stage(reinterpret_cast<BfSmallI *>(dyn + pl.o_tab), &P->si);
-  const BfSmallI &T = (PL & kTabSmem) ? *reinterpret_cast<const BfSmallI *>(dyn + pl.o_tab) : P->si;
-  __syncthreads();
+  const BfSmallI &T = P->si;
   for (int k = tid; k < 31 * 32; k += blockDim.x) {
     const int s = k >> 5, u1 = (k & 31) + 2;
     int v = BF_INF;
@@ -736,12 +732,11 @@ __global__ void __launch_bounds__(WPB * 32) bf_k_trace(const BfParams *__restric
 //                                   partition function (inside) fill
 // =====================================================================================================
 constexpr int kPfQmSmem = 1;   // packed qm and qm1 tables on chip (else: per-CTA HBM workspace)
-constexpr int kPfR2Smem = 2;   // the 1xn and bulge rings on chip
-constexpr int kPfQgSmem = 4;   // the generic-interior ring on chip
+constexpr int kPfQgSmem = 4;   // the generic-interior ring on chip (the 1xn and bulge rings are always in the workspace)
 
 struct PfPlan {
   int rs;
-  size_t o_S, o_toff, o_wg, o_wb, o_w1, o_scl, o_bu, o_qm, o_qm1, o_qg, o_r2, o_qms, o_au, o_pi, o_ps, o_list, o_tab, o_q5, total;
+  size_t o_S, o_toff, o_wg, o_wb, o_w1, o_scl, o_bu, o_qm, o_qm1, o_qg, o_qms, o_au, o_pi, o_ps, o_list, o_q5, total;
 };
 __host__ __device__ inline PfPlan pf_plan(int nmax, int nw, int pl, bool half = false) {
   PfPlan p;
@@ -755,13 +750,11 @@ __host__ __device__ inline PfPlan pf_plan(int nmax, int nw, int pl, bool half = 
   p.o_qm = o; o += (pl & kPfQmSmem) ? (tri_size(nmax) + 4) * sizeof(double) : 0;
   p.o_qm1 = o; o += (pl & kPfQmSmem) ? (tri_size(nmax) + 4) * sizeof(double) : 0;
   p.o_qg = o; o += (pl & kPfQgSmem) ? (size_t)kRing * p.rs * sizeof(double) : 0;
-  p.o_r2 = o; o += (pl & kPfR2Smem) ? (size_t)2 * kRing * p.rs * sizeof(double) : 0;
   p.o_qms = o; o += (size_t)4 * p.rs * sizeof(double);
   p.o_au = o; o += (size_t)2 * p.rs * sizeof(double);
   const int nb = half ? nw / 2 : nw;  // per-warp partial buffers; half: two warps share one (see bf_k_pf_fill)
   p.o_pi = o; o += (size_t)2 * nb * p.rs * sizeof(double);
   p.o_ps = o; o += (size_t)2 * nb * p.rs * sizeof(double);
-  p.o_tab = o; o += (pl & kTabSmem) ? (sizeof(BfSmallD) + 15) / 16 * 16 : 0;
   p.o_list = o; o += (size_t)2 * p.rs * sizeof(unsigned short);
   p.o_toff = o; o += (size_t)(nmax + 4) / 4 * 4 * sizeof(int);
   p.o_S = o; o += (nmax + 2 + 15) / 16 * 16;
@@ -772,10 +765,9 @@ __host__ __device__ inline PfPlan pf_plan(int nmax, int nw, int pl, bool half = 
 // doubles of per-CTA HBM workspace for the tables that are not on chip
 __host__ __device__ inline size_t pf_ws_doubles(int nmax, int pl) {
   const size_t rs = (nmax + 8 + 3) / 4 * 4;
-  size_t o = 0;
+  size_t o = 2 * kRing * rs;
   if (!(pl & kPfQmSmem)) o += 2 * ((tri_size(nmax) + 7) / 8 * 8);
   if (!(pl & kPfQgSmem)) o += kRing * rs;
-  if (!(pl & kPfR2Smem)) o += 2 * kRing * rs;
   return (o + 7) / 8 * 8;
 }
 
@@ -828,8 +820,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) bf_k_pf_fill(const BfParams *__
   }
   if (PL & kPfQgSmem) QG = reinterpret_cast<double *>(dyn + pl.o_qg);
   else { QG = wsp; wsp += kRing * RS; }
-  if (PL & kPfR2Smem) { Q1 = reinterpret_cast<double *>(dyn + pl.o_r2); QBB = Q1 + kRing * RS; }
-  else { Q1 = wsp; QBB = wsp + kRing * RS; }
+  Q1 = wsp; QBB = wsp + kRing * RS;
   // blocked split: tile-major mirrors of qm / qm1 and the block-product sums of three tile-diagonals, at the end of the slot
   const int NTS = (nmax + 3) / 4;
   const size_t tt = (tile_table_entries(nmax) + 7) / 8 * 8;
@@ -839,8 +830,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) bf_k_pf_fill(const BfParams *__
 
   for (int k = tid; k < (int)(pl.total / 4); k += blockDim.x) reinterpret_cast<int *>(dyn)[k] = 0;
   __syncthreads();
-  if (PL & kTabSmem) bf_stage(reinterpret_cast<BfSmallD *>(dyn + pl.o_tab), &P->sd);
-  const BfSmallD &T = (PL & kTabSmem) ? *reinterpret_cast<const BfSmallD *>(dyn + pl.o_tab) : P->sd;
+  const BfSmallD &T = P->sd;
   for (int k = tid; k < kRing * RS; k += blockDim.x) { QG[k] = 0.0; Q1[k] = 0.0; QBB[k] = 0.0; }
 
   for (;;) {
@@ -1268,19 +1258,14 @@ constexpr size_t kSmemBudget = 232448 - 1024 - 256;  // dynamic budget per CTA (
 // =====================================================================================================
 size_t bf_tri_slot(int nmax) { return (tri_size(nmax) + 7) / 8 * 8; }
 
-// ---- configuration: warps per CTA and table placement.  Defaults come from the tuning sweep on B200
-// (profiles/); BF_MFE_NW / BF_MFE_PL / BF_PF_NW / BF_PF_PL override them for experiments.
-static int env_int(const char *name, int dflt) {
-  const char *v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}
+// ---- configuration: warps per CTA and table placement, from the tuning sweep on B200 (profiles/)
 struct FillCfg { int nw, pl; };
 
 // Small batches (a replica-exchange sub-step: B = replicas x targets, often far fewer sequences than the 148 x 2..3 CTA slots):
 // what matters is the latency of ONE sequence, so a CTA gets 16 warps instead of 8 when every sequence still gets its own SM.
 static int g_fill_sms = 148;
 void bf_fill_set_sms(int sms) { if (sms > 0) g_fill_sms = sms; }
-static bool want_wide(int B) { const int w = env_int("BF_WIDE", 1); return B > 0 && (w == 2 || (B <= g_fill_sms && w != 0)); }   // 2: always (experiments)
+static bool want_wide(int B) { return B > 0 && B <= g_fill_sms && bf_opt("BF_WIDE", 1) != 0; }
 
 static bool mfe_fits(int nmax, int nw, int pl) { return mfe_plan(nmax, nw, pl).total <= kSmemBudget; }
 static bool pf_fits(int nmax, int nw, int pl) { return pf_plan(nmax, nw, pl).total <= kSmemBudget; }
@@ -1288,8 +1273,6 @@ static bool pf_fits(int nmax, int nw, int pl) { return pf_plan(nmax, nw, pl).tot
 static bool mfe_blk(int nmax, const FillCfg &c);
 // shared partial buffers (atomicMin) where they buy occupancy: CTAs per SM by shared memory, capped by the register limit (4 x 256 threads)
 static bool mfe_atom(int nmax, const FillCfg &c, bool blk) {
-  const int a = env_int("BF_MFE_ATOM", -1);
-  if (a >= 0) return a != 0;
   auto occ = [&](bool atom) {
     const size_t t = mfe_plan(nmax, c.nw, c.pl, blk, atom).total + 1024;
     const int cap = c.nw == 16 ? 2 : 4;
@@ -1299,63 +1282,38 @@ static bool mfe_atom(int nmax, const FillCfg &c, bool blk) {
   return occ(true) > occ(false);
 }
 static FillCfg mfe_cfg(int nmax, int B = 0) {
-  FillCfg c;
-  c.nw = env_int("BF_MFE_NW", 8);
-  if (c.nw != 2 && c.nw != 4) c.nw = 8;
-  if (c.nw == 8 && want_wide(B)) {   // same placement rule, 16 warps; only the combinations instantiated below
+  if (want_wide(B))   // same placement rule, 16 warps
     // one CTA per SM: nothing is gained by a small footprint, and with nothing else resident L2 latency is fully exposed --
     // keep on chip whatever fits (fML table + rings, else the rings), shared partial buffers if that is what makes it fit
-    FillCfg w;
-    w.nw = 16;
-    if (env_int("BF_MFE_PL", -1) < 0)
-      for (int pl : {kMfeFmSmem | kMfeRgSmem, kMfeRgSmem, 0}) {
-        w.pl = pl;
-        const bool blk = mfe_blk(nmax, w);
-        if (pl != 0 && nmax >= env_int("BF_BLK_MIN", 280)) continue;   // blocked split: the through-L2 layout measured faster (L=400)
-        if (mfe_plan(nmax, 16, pl, blk, true).total <= kSmemBudget) return w;
-      }
-  }
-  // default (tuning sweep, profiles/r01_sweeps.md): rings on chip while >= 3 CTAs still fit on an SM, else everything through L2
-  const int dflt = mfe_plan(nmax, c.nw, kMfeRgSmem, false, true).total <= (size_t)env_int("BF_MFE_RING_KB", 70) * 1024 ? kMfeRgSmem : 0;
-  const int want = env_int("BF_MFE_PL", dflt);
-  const int tb = want & kTabSmem;
-  const int order[4] = {want & 11, (want & kMfeRgSmem) | tb, want & kMfeRgSmem, 0};
-  for (int k = 0; k < 4; k++)
-    if (mfe_fits(nmax, c.nw, order[k])) { c.pl = order[k]; return c; }
-  c.pl = -1;
-  return c;
+    for (int pl : {kMfeFmSmem | kMfeRgSmem, kMfeRgSmem, 0}) {
+      const FillCfg w{16, pl};
+      if (pl != 0 && nmax >= bf_opt("BF_BLK_MIN", 280)) continue;   // blocked split: the through-L2 layout measured faster (L=400)
+      if (mfe_plan(nmax, 16, pl, mfe_blk(nmax, w), true).total <= kSmemBudget) return w;
+    }
+  // default (tuning sweep, profiles/r01_sweeps.md): rings on chip while >= 3 CTAs still fit on an SM (70 KB), else everything
+  // through L2
+  const int pl = mfe_plan(nmax, 8, kMfeRgSmem, false, true).total <= 70 * 1024 ? kMfeRgSmem : 0;
+  if (mfe_fits(nmax, 8, pl)) return {8, pl};
+  return {8, mfe_fits(nmax, 8, 0) ? 0 : -1};
 }
 static bool pf_blk(int nmax, const FillCfg &c);
 static bool pf_half(int nmax, const FillCfg &c);
 static FillCfg pf_cfg(int nmax, int B = 0) {
-  FillCfg c;
-  c.nw = env_int("BF_PF_NW", 8);
-  if (c.nw != 2 && c.nw != 4) c.nw = 8;
-  if (c.nw == 8 && want_wide(B)) {
-    FillCfg w;   // as for the MFE: one CTA per SM, keep on chip what fits (qm/qm1 + generic ring, else the ring)
-    w.nw = 16;
-    if (env_int("BF_PF_PL", -1) < 0)
-      for (int pl : {kPfQmSmem | kPfQgSmem, kPfQgSmem, 0}) {
-        w.pl = pl;
-        if (pl != 0 && nmax >= env_int("BF_BLK_MIN_PF", 250)) continue;   // blocked split: through-L2 layout only
-        if (pf_plan(nmax, 16, pl, pf_half(nmax, w)).total <= kSmemBudget) return w;
-      }
-  }
-  const int dflt = pf_plan(nmax, c.nw, kPfQgSmem).total <= 74 * 1024 ? kPfQgSmem : 0;
-  const int want = env_int("BF_PF_PL", dflt);
-  const int tb = want & kTabSmem;
-  const int order[4] = {want & 15, (want & (kPfQgSmem | kPfR2Smem)) | tb, (want & kPfQgSmem) | tb, 0};
-  for (int k = 0; k < 4; k++)
-    if (pf_fits(nmax, c.nw, order[k])) { c.pl = order[k]; return c; }
-  c.pl = -1;
-  return c;
+  if (want_wide(B))   // as for the MFE: one CTA per SM, keep on chip what fits (qm/qm1 + generic ring, else the ring)
+    for (int pl : {kPfQmSmem | kPfQgSmem, kPfQgSmem, 0}) {
+      const FillCfg w{16, pl};
+      if (pl != 0 && nmax >= bf_opt("BF_BLK_MIN_PF", 250)) continue;   // blocked split: through-L2 layout only
+      if (pf_plan(nmax, 16, pl, pf_half(nmax, w)).total <= kSmemBudget) return w;
+    }
+  const int pl = pf_plan(nmax, 8, kPfQgSmem).total <= 74 * 1024 ? kPfQgSmem : 0;
+  if (pf_fits(nmax, 8, pl)) return {8, pl};
+  return {8, pf_fits(nmax, 8, 0) ? 0 : -1};
 }
 
-// blocked split (tile-major mirror + block products): for NW = 8 and the two default placements.  It pays once the split
-// operands no longer fit on chip (measured: L=100 3.86 -> 5.18 ms, L=200 16.1 -> 17.8 ms, L=400 143 -> 117 ms): long sequences only
+// blocked split (tile-major mirror + block products): for the two default placements.  It pays once the split operands no longer
+// fit on chip (measured: L=100 3.86 -> 5.18 ms, L=200 16.1 -> 17.8 ms, L=400 143 -> 117 ms): long sequences only
 static bool mfe_blk(int nmax, const FillCfg &c) {
-  return env_int("BF_BLK", 1) && c.nw >= 8 && (c.pl == 0 || c.pl == kMfeRgSmem) && nmax >= env_int("BF_BLK_MIN", 280) &&
-         mfe_plan(nmax, c.nw, c.pl, true).total <= kSmemBudget;
+  return (c.pl == 0 || c.pl == kMfeRgSmem) && nmax >= bf_opt("BF_BLK_MIN", 280) && mfe_plan(nmax, c.nw, c.pl, true).total <= kSmemBudget;
 }
 
 // 0: length not covered by the fill path (the generic kernels take it); else 1 + placement flags
@@ -1371,7 +1329,7 @@ int bf_fill_pf_mode(int nmax) {
 // 16-warp round-1 kernels of this file only what those do not cover (BF_FILL3_SMALL=0: as before round 2's last session)
 // cluster-per-sequence kernels (bf_cluster.cu): small batches of long sequences (rule in bf_cluster.cu; BF_CL=0/1 overrides)
 static bool use_cl_mfe(int nmax, int B) { return B > 0 && bf_cl_mfe_use(nmax, B); }
-static bool small3(int B) { return want_wide(B) && env_int("BF_FILL3_SMALL", 1) != 0; }
+static bool small3(int B) { return want_wide(B) && bf_opt("BF_FILL3_SMALL", 1) != 0; }
 static bool use_fill3_mfe(int nmax, int B) { return !use_cl_mfe(nmax, B) && (!want_wide(B) || small3(B)) && bf_fill3_mfe_ok(nmax, small3(B)); }
 static bool use_cl_pf(int nmax, int B) { return B > 0 && bf_cl_pf_use(nmax, B); }
 static bool use_fill3_pf(int nmax, int B) { return !use_cl_pf(nmax, B) && (!want_wide(B) || small3(B)) && bf_fill3_pf_ok(nmax, small3(B)); }
@@ -1386,15 +1344,12 @@ size_t bf_mfe_ws_slot(int nmax, int B) {  // ints of per-CTA HBM workspace: [rin
   if (mfe_blk(nmax, c)) o += (tile_table_entries(nmax) + 7) / 8 * 8;
   return o;
 }
-static bool pf_blk(int nmax, const FillCfg &c) {
-  return env_int("BF_BLK", 1) && c.nw >= 8 && c.pl == 0 && nmax >= env_int("BF_BLK_MIN_PF", 250);
-}
+static bool pf_blk(int nmax, const FillCfg &c) { return c.pl == 0 && nmax >= bf_opt("BF_BLK_MIN_PF", 250); }
 static bool pf_half(int nmax, const FillCfg &c) {
   // long sequences: with one partial buffer per warp only one CTA fits an SM; sharing buffers between warp pairs fits two
   if (c.nw == 16)   // one CTA per SM: share buffers between warp pairs only when the full set does not fit
-    return c.pl == 0 && env_int("BF_PF_HALF", 1) && pf_plan(nmax, 16, 0, false).total > kSmemBudget;
-  return c.nw == 8 && c.pl == 0 && env_int("BF_PF_HALF", 1) && pf_plan(nmax, 8, 0, false).total > 113 * 1024 &&
-         pf_plan(nmax, 8, 0, true).total <= 113 * 1024;
+    return c.pl == 0 && pf_plan(nmax, 16, 0, false).total > kSmemBudget;
+  return c.pl == 0 && pf_plan(nmax, 8, 0, false).total > 113 * 1024 && pf_plan(nmax, 8, 0, true).total <= 113 * 1024;
 }
 size_t bf_pf_ws_slot(int nmax, int B) {  // doubles of per-CTA HBM workspace: [tables that are not on chip][blocked split: qm/qm1 mirrors, sums]
   if (use_cl_pf(nmax, B)) return bf_cl_pf_ws_slot(nmax, B);
@@ -1425,57 +1380,34 @@ static cudaError_t mfe_fill_t(const BfParams *dP, const BfBatchDev &b, int *ctri
   return cudaGetLastError();
 }
 
-template <int NW>
-static cudaError_t mfe_fill_pl(int pl, const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *grid_out,
-                               bool launch, int *counter, cudaStream_t st) {
-  switch (pl) {
-    case 0: return mfe_fill_t<NW, 0>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 1: return mfe_fill_t<NW, 1>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 2: return mfe_fill_t<NW, 2>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 3: return mfe_fill_t<NW, 3>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 8: return mfe_fill_t<NW, 8>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 9: return mfe_fill_t<NW, 9>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 10: return mfe_fill_t<NW, 10>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-    case 11: return mfe_fill_t<NW, 11>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-  }
-  return cudaErrorInvalidValue;
-}
 static cudaError_t mfe_fill_dispatch(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *grid_out,
                                      bool launch, int *counter, cudaStream_t st) {
   const FillCfg c = mfe_cfg(b.stride, b.B);
   if (c.pl < 0) return cudaErrorInvalidValue;
-  const bool blk = mfe_blk(b.stride, c);
-  const bool atom = (c.nw >= 8) && (c.pl == 0 || c.pl == kMfeRgSmem) && mfe_atom(b.stride, c, blk);
+  const bool blk = mfe_blk(b.stride, c), atom = mfe_atom(b.stride, c, blk);
 #define BF_MFE_GO(NW_, PL_, BLK_, ATOM_) return mfe_fill_t<NW_, PL_, BLK_, ATOM_>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st)
-  if (c.nw == 16 && c.pl == (kMfeFmSmem | kMfeRgSmem)) {
-    if (mfe_atom(b.stride, c, false)) BF_MFE_GO(16, kMfeFmSmem | kMfeRgSmem, false, true);
+  if (c.pl == (kMfeFmSmem | kMfeRgSmem)) {   // 16 warps only, never blocked
+    if (atom) BF_MFE_GO(16, kMfeFmSmem | kMfeRgSmem, false, true);
     BF_MFE_GO(16, kMfeFmSmem | kMfeRgSmem, false, false);
   }
-  if (c.nw == 16 || atom || blk) {
-    const int key = (c.nw == 16 ? 8 : 0) | (c.pl == 0 ? 0 : 4) | (blk ? 2 : 0) | (atom ? 1 : 0);
-    switch (key) {
-      case 0: break;   // <8, 0, false, false>: the generic switch below
-      case 1: BF_MFE_GO(8, 0, false, true);
-      case 2: BF_MFE_GO(8, 0, true, false);
-      case 3: BF_MFE_GO(8, 0, true, true);
-      case 4: break;
-      case 5: BF_MFE_GO(8, kMfeRgSmem, false, true);
-      case 6: BF_MFE_GO(8, kMfeRgSmem, true, false);
-      case 7: BF_MFE_GO(8, kMfeRgSmem, true, true);
-      case 8: BF_MFE_GO(16, 0, false, false);
-      case 9: BF_MFE_GO(16, 0, false, true);
-      case 10: BF_MFE_GO(16, 0, true, false);
-      case 11: BF_MFE_GO(16, 0, true, true);
-      case 12: BF_MFE_GO(16, kMfeRgSmem, false, false);
-      case 13: BF_MFE_GO(16, kMfeRgSmem, false, true);
-      case 14: BF_MFE_GO(16, kMfeRgSmem, true, false);
-      case 15: BF_MFE_GO(16, kMfeRgSmem, true, true);
-    }
+  // the combinations the rules above return
+  switch ((c.nw == 16 ? 8 : 0) | (c.pl == 0 ? 0 : 4) | (blk ? 2 : 0) | (atom ? 1 : 0)) {
+    case 0: BF_MFE_GO(8, 0, false, false);
+    case 1: BF_MFE_GO(8, 0, false, true);
+    case 2: BF_MFE_GO(8, 0, true, false);
+    case 3: BF_MFE_GO(8, 0, true, true);
+    case 4: BF_MFE_GO(8, kMfeRgSmem, false, false);
+    case 5: BF_MFE_GO(8, kMfeRgSmem, false, true);
+    case 6: BF_MFE_GO(8, kMfeRgSmem, true, false);
+    case 7: BF_MFE_GO(8, kMfeRgSmem, true, true);
+    case 9: BF_MFE_GO(16, 0, false, true);
+    case 10: BF_MFE_GO(16, 0, true, false);
+    case 11: BF_MFE_GO(16, 0, true, true);
+    case 12: BF_MFE_GO(16, kMfeRgSmem, false, false);
+    case 13: BF_MFE_GO(16, kMfeRgSmem, false, true);
   }
 #undef BF_MFE_GO
-  if (c.nw == 4) return mfe_fill_pl<4>(c.pl, dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-  if (c.nw == 2) return mfe_fill_pl<2>(c.pl, dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
-  return mfe_fill_pl<8>(c.pl, dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st);
+  return cudaErrorInvalidValue;
 }
 cudaError_t bf_mfe_fill_grid(const BfBatchDev &b, int sms, int *grid) {
   if (use_cl_mfe(b.stride, b.B)) return bf_cl_mfe_grid(b, sms, grid);
@@ -1525,47 +1457,30 @@ static cudaError_t pf_fill_t(const BfParams *dP, const BfBatchDev &b, double *qb
   kern<<<grid, NW * 32, sm, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), ws, bf_pf_ws_slot(b.stride, b.B), qmseq, mfe_for_scale, lnscale, counter, NW == 16 ? g_pf_out5 : nullptr);
   return cudaGetLastError();
 }
-template <int NW>
-static cudaError_t pf_fill_pl(int pl, const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                              double *lnscale, int sms, int *grid_out, bool launch, int *counter, cudaStream_t st) {
-  switch (pl) {
-    case 0: return pf_fill_t<NW, 0>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 4: return pf_fill_t<NW, 4>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 6: return pf_fill_t<NW, 6>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 7: return pf_fill_t<NW, 7>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 8: return pf_fill_t<NW, 8>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 12: return pf_fill_t<NW, 12>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 14: return pf_fill_t<NW, 14>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    case 15: return pf_fill_t<NW, 15>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  }
-  return cudaErrorInvalidValue;
-}
 static cudaError_t pf_fill_dispatch(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
                                     double *lnscale, int sms, int *grid_out, bool launch, int *counter, cudaStream_t st) {
   const FillCfg c = pf_cfg(b.stride, b.B);
   if (c.pl < 0) return cudaErrorInvalidValue;
   const bool half = pf_half(b.stride, c), blk = pf_blk(b.stride, c);
+#define BF_PF_GO(...) return pf_fill_t<__VA_ARGS__>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st)
   if (c.nw == 16) {
-    if (c.pl == (kPfQmSmem | kPfQgSmem)) return pf_fill_t<16, kPfQmSmem | kPfQgSmem>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    if (c.pl == kPfQgSmem) return pf_fill_t<16, kPfQgSmem>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    if (half && blk) return pf_fill_t<16, 0, true, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    if (half) return pf_fill_t<16, 0, true, false>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    if (blk) return pf_fill_t<16, 0, false, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    return pf_fill_t<16, 0>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
+    if (c.pl == (kPfQmSmem | kPfQgSmem)) BF_PF_GO(16, kPfQmSmem | kPfQgSmem);
+    if (c.pl == kPfQgSmem) BF_PF_GO(16, kPfQgSmem);
+    if (half && blk) BF_PF_GO(16, 0, true, true);
+    if (half) BF_PF_GO(16, 0, true, false);
+    if (blk) BF_PF_GO(16, 0, false, true);
+    BF_PF_GO(16, 0);
   }
-  if (half && blk) return pf_fill_t<8, 0, true, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  if (half) return pf_fill_t<8, 0, true, false>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  if (blk) return pf_fill_t<8, 0, false, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  if (c.nw == 8 && c.pl == 0) {   // everything through L2: occupancy is a register question
-    // measured (profiles/r01_s4_sweep_pf_minb.log): 4 CTAs per SM pay up to ~135 nt, 3 up to ~185 nt; beyond, the tables of more
-    // sequences in flight no longer fit in L2 and the 2-CTA build wins
-    const int mb = env_int("BF_PF_MINB", b.stride <= 135 ? 4 : b.stride <= 185 ? 3 : 0);
-    if (mb == 3) return pf_fill_t<8, 0, false, false, 3>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-    if (mb == 4) return pf_fill_t<8, 0, false, false, 4>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  }
-  if (c.nw == 4) return pf_fill_pl<4>(c.pl, dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  if (c.nw == 2) return pf_fill_pl<2>(c.pl, dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
-  return pf_fill_pl<8>(c.pl, dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st);
+  if (c.pl == kPfQgSmem) BF_PF_GO(8, kPfQgSmem);
+  if (half && blk) BF_PF_GO(8, 0, true, true);
+  if (half) BF_PF_GO(8, 0, true, false);
+  if (blk) BF_PF_GO(8, 0, false, true);
+  // everything through L2: occupancy is a register question.  Measured (profiles/r01_s4_sweep_pf_minb.log): 4 CTAs per SM pay up
+  // to ~135 nt, 3 up to ~185 nt; beyond, the tables of more sequences in flight no longer fit in L2 and the 2-CTA build wins
+  if (b.stride <= 135) BF_PF_GO(8, 0, false, false, 4);
+  if (b.stride <= 185) BF_PF_GO(8, 0, false, false, 3);
+  BF_PF_GO(8, 0);
+#undef BF_PF_GO
 }
 
 // grid size the fill will use (the caller sizes the per-CTA workspace with it)

@@ -62,12 +62,12 @@ constexpr bool kPrepassInPhases = false;
 struct Mfe3Plan {
   size_t o_S, o_SP, o_np, o_ring, o_dml, o_fm, o_stg, o_tmpe, o_ps, o_cl, o_pp, total;
 };
-__host__ __device__ inline Mfe3Plan mfe3_plan(int nmax, int rs, int nw, int nwa, bool fms) {
+__host__ __device__ inline Mfe3Plan mfe3_plan(int nmax, int rs, int nw, int nwa) {
   Mfe3Plan p;
   size_t o = 0;
   p.o_ring = o; o += ((size_t)3 * kRing * rs + rs) * sizeof(int);   // three rings + one neutral row
   p.o_dml = o; o += (size_t)4 * rs * sizeof(int);
-  p.o_fm = o; o += fms ? (tri_size(nmax) + 4) * sizeof(int) : 0;
+  p.o_fm = o; o += (tri_size(nmax) + 4) * sizeof(int);
   p.o_stg = o; o += (size_t)2 * 3 * rs * sizeof(int);               // newest ring row, staged by the tap warps (double-buffered)
   p.o_tmpe = o; o += (size_t)2 * rs * sizeof(int);                  // c + MLstem of the newest diagonal
   p.o_ps = o; o += (size_t)2 * nwa * rs * sizeof(int);
@@ -99,17 +99,17 @@ __device__ __forceinline__ int lds_s32(unsigned addr) {
 //   aux warps [NWI, NW): diagonal d-1: staging row -> rings, fML (needs c of d-1, the split minima of d-1 and fML of d-2);
 //                        then their share of the split points of diagonal d
 // Ring row d must not be written while phase d still reads row d-32 (same slot): hence the staging row.
-template <int NW, int NWI, bool FMS>
+template <int NW, int NWI>
 __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_mfe_fill3(const BfParams *__restrict__ P, BfBatchDev b, int *ctri, int *ftri, size_t tri_slot,
                                                           int *ent_ws, size_t ent_slot, const uint32_t *__restrict__ taps, int RS,
-                                                          int *work_counter, int dbg) {
+                                                          int *work_counter) {
   constexpr int NWA = NW - NWI;
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ int s_seq;
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(BF_FULL, tid >> 5, 0);
   const int nmax = b.stride;
-  const Mfe3Plan pl = mfe3_plan(nmax, RS, NW, NWA, FMS);
+  const Mfe3Plan pl = mfe3_plan(nmax, RS, NW, NWA);
   const int seq_pad = (nmax + 2 + 15) / 16 * 16, np_pad = (nmax + 4) / 4 * 4;
   int *RG = reinterpret_cast<int *>(dyn + pl.o_ring);
   int *CG = RG, *C1 = RG + kRing * RS, *CB = RG + 2 * kRing * RS;
@@ -234,7 +234,6 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
     const int *ent = ent_base + (size_t)cur * (ent_slot / 2);
     int *cg_out = ctri + (size_t)sq * tri_slot;
     int *fg_out = ftri + (size_t)sq * tri_slot;
-    int *FM = FMS ? fms : fg_out;
     if (tapw) {
 #pragma unroll
       for (int k = 0; k < kNSlot; k++) {
@@ -258,13 +257,13 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
                      : "memory");
       }
     };
-    if (tapw && n - 1 >= BF_TURN + 1 && !(dbg & 1)) stage(BF_TURN + 1);
+    if (tapw && n - 1 >= BF_TURN + 1) stage(BF_TURN + 1);
 
     for (int d = BF_TURN + 1; d <= n; d++) {
       const int buf = d & 1;
       if (tapw) {
         // ------------------------------------------------------------ tap warps: c(i,j) of every pairable cell of diagonal d
-        if (d <= n - 1 && !(dbg & 1)) {
+        if (d <= n - 1) {
           const int np = NP[d];
           const int od = tri_off(n, d);
           const unsigned sdml = (unsigned)__cvta_generic_to_shared(DML + ((d - 2) & 3) * RS + 1);
@@ -323,7 +322,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
       } else {
         const int a = warp - NWI;   // auxiliary warp index
         // ------------------------------------------------------------ diagonal d-1: staging row -> rings, fML
-        if (d > BF_TURN + 1 && !(dbg & 8)) {
+        if (d > BF_TURN + 1) {
           const int dd = d - 1, ncell = n - dd, pb = dd & 1;
           int *stg = STG + pb * 3 * RS, *tmpe = TMPE + pb * RS;
           const int *ps = PS + pb * NWA * RS;
@@ -339,72 +338,54 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
             stg[i] = BF_INF; stg[RS + i] = BF_INF; stg[2 * RS + i] = BF_INF; tmpe[i] = BF_INF;   // only pairable cells are written
             CG[row + i] = eg; C1[row + i] = e1; CB[row + i] = eb;
             int m = min(sp, te);
-            if (dd > BF_TURN + 1) m = min(m, min(FM[om + i], FM[om + i - 1]) + T.MLbase);
+            if (dd > BF_TURN + 1) m = min(m, min(fms[om + i], fms[om + i - 1]) + T.MLbase);
             if (m >= kInfThr) m = BF_INF;
             fg_out[o0 + i - 1] = m;
-            if (FMS) fms[o0 + i - 1] = m;
+            fms[o0 + i - 1] = m;
             DML[(dd & 3) * RS + i] = sp;
           }
         }
         if (d <= n - 1) {
           const int ncell = n - d;
           // ------------------------------------------------------------ fML split: this warp's share of the split points, every cell
-          if (!(dbg & 2)) {
-            int *ps = PS + (buf * NWA + a) * RS;
-            constexpr int Q = NWA;
-            // operands of split point k: fML(i, i+k-1) at off(k-1) + cell, fML(i+k, j) at off(d-k) + k + cell.  The offsets are
-            // warp-uniform and advance by second-order increments (off(x+Q) - off(x) = Q(n-x) - Q(Q-1)/2): they live in uniform
-            // registers, a load is LDS [lane's cell offset + uniform].
-            for (int c0 = 0; c0 < ncell; c0 += 128) {
-              int ii[4], acc[4];
+          int *ps = PS + (buf * NWA + a) * RS;
+          constexpr int Q = NWA;
+          // operands of split point k: fML(i, i+k-1) at off(k-1) + cell, fML(i+k, j) at off(d-k) + k + cell.  The offsets are
+          // warp-uniform and advance by second-order increments (off(x+Q) - off(x) = Q(n-x) - Q(Q-1)/2): they live in uniform
+          // registers, a load is LDS [lane's cell offset + uniform].
+          for (int c0 = 0; c0 < ncell; c0 += 128) {
+            int ii[4], acc[4];
 #pragma unroll
-              for (int u = 0; u < 4; u++) { ii[u] = 4 * min(c0 + 32 * u + lane, ncell - 1); acc[u] = BF_INF; }   // byte offset of the lane's cell
-              const bool many = c0 + 64 < ncell;   // warp-uniform: more than two chunks left
-              int k = 5 + a;
-              if (k <= d - 4) {
-                // running byte addresses of the two operands of every chunk; both advance by the same (uniform) first differences
-                const int oL = 4 * tri_off(n, k - 1), oR = 4 * (tri_off(n, d - k) + k);
-                int dL = 4 * (Q * (n - k + 1) - Q * (Q - 1) / 2), dR = 4 * (-Q * (n - d + k + Q) + Q * (Q - 1) / 2 + Q);
-                if (FMS) {
-                  unsigned pL[4], pR[4];
+            for (int u = 0; u < 4; u++) { ii[u] = 4 * min(c0 + 32 * u + lane, ncell - 1); acc[u] = BF_INF; }   // byte offset of the lane's cell
+            const bool many = c0 + 64 < ncell;   // warp-uniform: more than two chunks left
+            int k = 5 + a;
+            if (k <= d - 4) {
+              // running byte addresses of the two operands of every chunk; both advance by the same (uniform) first differences
+              const int oL = 4 * tri_off(n, k - 1), oR = 4 * (tri_off(n, d - k) + k);
+              int dL = 4 * (Q * (n - k + 1) - Q * (Q - 1) / 2), dR = 4 * (-Q * (n - d + k + Q) + Q * (Q - 1) / 2 + Q);
+              unsigned pL[4], pR[4];
 #pragma unroll
-                  for (int u = 0; u < 4; u++) { pL[u] = sFM + (unsigned)(oL + ii[u]); pR[u] = sFM + (unsigned)(oR + ii[u]); }
-                  if (many) {
+              for (int u = 0; u < 4; u++) { pL[u] = sFM + (unsigned)(oL + ii[u]); pR[u] = sFM + (unsigned)(oR + ii[u]); }
+              if (many) {
 #pragma unroll 2
-                    for (; k <= d - 4; k += Q) {
+                for (; k <= d - 4; k += Q) {
 #pragma unroll
-                      for (int u = 0; u < 4; u++) { acc[u] = min(acc[u], lds_s32(pL[u]) + lds_s32(pR[u])); pL[u] += dL; pR[u] += dR; }
-                      dL -= 4 * Q * Q; dR -= 4 * Q * Q;
-                    }
-                  } else {
+                  for (int u = 0; u < 4; u++) { acc[u] = min(acc[u], lds_s32(pL[u]) + lds_s32(pR[u])); pL[u] += dL; pR[u] += dR; }
+                  dL -= 4 * Q * Q; dR -= 4 * Q * Q;
+                }
+              } else {
 #pragma unroll 4
-                    for (; k <= d - 4; k += Q) {
+                for (; k <= d - 4; k += Q) {
 #pragma unroll
-                      for (int u = 0; u < 2; u++) { acc[u] = min(acc[u], lds_s32(pL[u]) + lds_s32(pR[u])); pL[u] += dL; pR[u] += dR; }
-                      dL -= 4 * Q * Q; dR -= 4 * Q * Q;
-                    }
-                  }
-                } else {
-                  const char *pL[4], *pR[4];
-#pragma unroll
-                  for (int u = 0; u < 4; u++) { pL[u] = reinterpret_cast<const char *>(FM) + oL + ii[u]; pR[u] = reinterpret_cast<const char *>(FM) + oR + ii[u]; }
-                  const int nu = many ? 4 : 2;
-                  for (; k <= d - 4; k += Q) {
-#pragma unroll
-                    for (int u = 0; u < 4; u++)
-                      if (u < nu) {
-                        acc[u] = min(acc[u], *reinterpret_cast<const int *>(pL[u]) + *reinterpret_cast<const int *>(pR[u]));
-                        pL[u] += dL; pR[u] += dR;
-                      }
-                    dL -= 4 * Q * Q; dR -= 4 * Q * Q;
-                  }
+                  for (int u = 0; u < 2; u++) { acc[u] = min(acc[u], lds_s32(pL[u]) + lds_s32(pR[u])); pL[u] += dL; pR[u] += dR; }
+                  dL -= 4 * Q * Q; dR -= 4 * Q * Q;
                 }
               }
+            }
 #pragma unroll
-              for (int u = 0; u < 4; u++) {
-                const int cell = c0 + 32 * u + lane;
-                if (cell < ncell) ps[cell] = acc[u];
-              }
+            for (int u = 0; u < 4; u++) {
+              const int cell = c0 + 32 * u + lane;
+              if (cell < ncell) ps[cell] = acc[u];
             }
           }
         }
@@ -478,7 +459,7 @@ template <int NW, int NWI, bool QMSM, bool PAIR = false>
 __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const BfParams *__restrict__ P, BfBatchDev b, double *qbtri, size_t tri_slot,
                                                                           double *ws, size_t ws_slot, double *qm_perseq,
                                                                           const int *__restrict__ mfe_for_scale, double *lnscale_out,
-                                                                          const uint32_t *__restrict__ taps, int RS, int *work_counter, int dbg) {
+                                                                          const uint32_t *__restrict__ taps, int RS, int *work_counter) {
   constexpr int NWA = NW - NWI;
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ int s_seq;
@@ -561,7 +542,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
     // ------------------------------------------------------------ pre-pass: per-cell constants of every diagonal
     {
       unsigned short *cl = reinterpret_cast<unsigned short *>(dyn + pl.o_pp) + (size_t)warp * ((nmax + 7) / 8 * 8);
-      for (int d = BF_TURN + 1 + warp; d <= n - 1 && !(dbg & 4); d += NW) {
+      for (int d = BF_TURN + 1 + warp; d <= n - 1; d += NW) {
         int count = 0;
         const int od = tri_off(n, d);
         for (int base = 1; base <= n - d; base += 32) {
@@ -617,13 +598,13 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
                      : "memory");
       }
     };
-    if (tapw && n - 1 >= BF_TURN + 1 && !(dbg & 1)) stage(BF_TURN + 1);
+    if (tapw && n - 1 >= BF_TURN + 1) stage(BF_TURN + 1);
 
     for (int d = BF_TURN + 1; d <= n; d++) {
       const int buf = d & 1;
       if (tapw) {
         // ------------------------------------------------------------ tap warps: qb(i,j) of every pairable cell of diagonal d
-        if (d <= n - 1 && !(dbg & 1)) {
+        if (d <= n - 1) {
           const int np = NP[d];
           const int od = tri_off(n, d);
           const unsigned sqms = (unsigned)__cvta_generic_to_shared(QMS + ((d - 2) & 3) * RS + 1);
@@ -722,7 +703,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
       } else {
         const int a = warp - NWI;
         // ------------------------------------------------------------ diagonal d-1: staging row -> rings, qm1, au, qm
-        if (d > BF_TURN + 1 && !(dbg & 8)) {
+        if (d > BF_TURN + 1) {
           const int dd = d - 1, ncell = n - dd, pb = dd & 1;
           double *stg = STG + pb * 3 * RS, *tmpq = TMPQ + pb * RS;
           const double *ps = PS + pb * NWA * RS;
@@ -749,7 +730,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
             AU[(dd & 1) * RS + i] = au;
           }
         }
-        if (d <= n - 1 && !(dbg & 2)) {
+        if (d <= n - 1) {
           const int ncell = n - d;
           // ------------------------------------------------------------ qm split: this warp's share of the split points, every cell
           double *ps = PS + (buf * NWA + a) * RS;
@@ -825,32 +806,20 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
 
 constexpr size_t kSmemBudget = 232448 - 1024 - 256;
 
-int env_int(const char *name, int dflt) {
-  const char *v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}
-
-struct Mfe3Cfg { bool ok; int rs; bool fms; size_t smem; int nw, nwi; };
+struct Mfe3Cfg { bool ok; int rs; size_t smem; };
 // small: a batch that leaves SMs idle (a replica-exchange sub-step) -- one 16-warp CTA (12 tap + 4 auxiliary warps) per sequence with the
 // whole shared memory of its SM; measured against the 16-warp round-1 kernels at B = 64 (profiles/r02_small_batch_fill3.txt): 36 nt 0.089 ->
 // 0.076 ms, 100 nt 0.340 -> 0.257, 148 nt 0.678 -> 0.427, 200 nt 1.07 -> 0.66, as long as the fML table fits on chip (~230 nt)
 Mfe3Cfg mfe3_cfg(int nmax, bool small) {
   Mfe3Cfg c;
   c.ok = false;
-  if (nmax < 1 || env_int("BF_FILL3", 1) == 0 || env_int("BF_FILL3_MFE", 1) == 0) return c;
+  if (nmax < 1 || bf_opt("BF_FILL3", 1) == 0) return c;
   c.rs = pick_rs(nmax, 32);
-  c.nw = env_int("BF_FILL3_NW", small ? 16 : 8);
-  c.nwi = env_int("BF_FILL3_NWI", c.nw == 8 ? 6 : c.nw * 3 / 4);
-  const int NWA = c.nw - c.nwi;
-  // The fML table has to be on chip: with two auxiliary warps per CTA the split cannot hide L2 latency (measured: L = 120 7.8 ms
-  // per 4096 folds against 5.96 ms of the round-1 kernel, L = 200 33 against 16).  Three CTAs per SM up to ~105 nt, two up to
-  // ~150 nt; longer sequences stay on the round-1 kernels (bf_fill.cu).
-  const size_t with = mfe3_plan(nmax, c.rs, c.nw, NWA, true).total, without = mfe3_plan(nmax, c.rs, c.nw, NWA, false).total;
-  const int fm_env = env_int("BF_FILL3_FMS", -1);
-  c.fms = fm_env >= 0 ? fm_env != 0 : true;
-  c.smem = c.fms ? with : without;
-  const size_t cap = (fm_env >= 0 || small) ? kSmemBudget : (size_t)env_int("BF_FILL3_MFE_KB", 112) * 1024;
-  c.ok = c.smem <= cap && c.smem <= kSmemBudget && nmax <= env_int("BF_FILL3_MAXN", 2000);
+  // 8 warps: 6 tap + 2 auxiliary.  The fML table has to be on chip: with two auxiliary warps per CTA the split cannot hide L2
+  // latency (measured: L = 120 7.8 ms per 4096 folds against 5.96 ms of the round-1 kernel, L = 200 33 against 16).  Three CTAs
+  // per SM up to ~105 nt, two up to ~150 nt (112 KB); longer sequences stay on the round-1 kernels (bf_fill.cu).
+  c.smem = small ? mfe3_plan(nmax, c.rs, 16, 4).total : mfe3_plan(nmax, c.rs, 8, 2).total;
+  c.ok = c.smem <= (small ? kSmemBudget : 112 * 1024);
   return c;
 }
 
@@ -859,10 +828,10 @@ Mfe3Cfg mfe3_cfg(int nmax, bool small) {
 bool bf_fill3_mfe_ok(int nmax, bool small) { return mfe3_cfg(nmax, small).ok; }
 size_t bf_fill3_mfe_ws_slot(int nmax) { return 2 * ((tri_size(nmax) * kEntWords + 7) / 8 * 8); }   // ints per CTA: entries of every cell, two sequences
 
-template <int NW, int NWI, bool FMS>
+template <int NW, int NWI>
 static cudaError_t mfe3_launch(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, const Mfe3Cfg &c, int sms, int *counter,
                                cudaStream_t st, int *grid_out) {
-  auto kern = bf_k_mfe_fill3<NW, NWI, FMS>;
+  auto kern = bf_k_mfe_fill3<NW, NWI>;
   static int occ_cache[4096];   // per stride: CTAs per SM (0 = not asked yet); the attribute is set once per instance
   static bool attr_set = false;
   cudaError_t e;
@@ -878,15 +847,12 @@ static cudaError_t mfe3_launch(const BfParams *dP, const BfBatchDev &b, int *ctr
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
   }
-  const int cap = env_int("BF_FILL3_MFE_CTAS", 0), per_sm = cap > 0 && cap < occ ? cap : occ;   // fewer CTAs per SM: room for the other fill beside it
-  if (env_int("BF_CFG_PRINT", 0)) fprintf(stderr, "mfe_fill3<%d,%d,%d> stride %d smem %zu occ %d per_sm %d\n", NW, NWI, (int)FMS, b.stride, c.smem, occ, per_sm);
-  const int grid = b.B < sms * per_sm ? b.B : sms * per_sm;
+  const int grid = b.B < sms * occ ? b.B : sms * occ;
   if (grid_out) { *grid_out = grid; return cudaSuccess; }
   const uint32_t *taps = nullptr;
   e = taps_device(c.rs, 32, &taps);
   if (e != cudaSuccess) return e;
-  kern<<<grid, NW * 32, c.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, bf_fill3_mfe_ws_slot(b.stride), taps, c.rs, counter,
-                                      env_int("BF_FILL3_DBG", 0));
+  kern<<<grid, NW * 32, c.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, bf_fill3_mfe_ws_slot(b.stride), taps, c.rs, counter);
   return cudaGetLastError();
 }
 
@@ -894,13 +860,8 @@ static cudaError_t mfe3_dispatch(const BfParams *dP, const BfBatchDev &b, int *c
                                  cudaStream_t st, int *grid_out, bool small) {
   const Mfe3Cfg c = mfe3_cfg(b.stride, small);
   if (!c.ok) return cudaErrorInvalidValue;
-#define BF_GO(NW_, NWI_)                                                                                          \
-  if (c.nw == NW_ && c.nwi == NWI_)                                                                                \
-    return c.fms ? mfe3_launch<NW_, NWI_, true>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out)         \
-                 : mfe3_launch<NW_, NWI_, false>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out)
-  BF_GO(8, 4); BF_GO(8, 5); BF_GO(8, 6); BF_GO(12, 9); BF_GO(16, 12);
-#undef BF_GO
-  return cudaErrorInvalidValue;
+  if (small) return mfe3_launch<16, 12>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out);
+  return mfe3_launch<8, 6>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out);
 }
 
 cudaError_t bf_fill3_mfe_grid(const BfBatchDev &b, int sms, int *grid, bool small) {
@@ -916,32 +877,29 @@ cudaError_t bf_launch_mfe_fill3(const BfParams *dP, const BfBatchDev &b, int *ct
 
 // ---------------------------------------------------------------------------------------------------- partition function, host side
 namespace {
-struct Pf3Cfg { bool ok; int rs; bool qms; size_t smem; int nw, nwi; };
+struct Pf3Cfg { bool ok; int rs; bool qms, pair; size_t smem; int nw, nwi; };
 Pf3Cfg pf3_cfg(int nmax, bool small) {
   Pf3Cfg c;
   c.ok = false;
-  if (nmax < 1 || env_int("BF_FILL3", 1) == 0 || env_int("BF_FILL3_PF", 1) == 0) return c;
+  if (nmax < 1 || bf_opt("BF_FILL3", 1) == 0) return c;
   c.rs = pick_rs(nmax, 16);
   // One CTA of 16 warps (12 tap + 4 auxiliary) per SM with qm / qm1 on chip while they fit (~105 nt), through L2 beyond.  Measured
   // at L = 100 (4096 folds): 16 warps on chip 5.01 ms, 12 warps with paired cells 5.13, two CTAs of 8 warps (qm / qm1 in L2) 5.14;
   // at L = 120 / 150 the 16-warp CTA is ahead of the 8-warp pair by 20 / 30 % (profiles/r02_sweep_len.txt).
-  const int nw_env = env_int("BF_FILL3_PF_NW", 0);
   // 16 warps with cells in pairs from 90 nt (L = 100: 4.90 ms per 4096 folds against 5.14 for two 8-warp CTAs); below, two or three
-  // 8-warp CTAs per SM are ahead (L = 30 / 50 / 75: 0.60 / 1.26 / 2.79 ms against 0.88 / 1.71 / 3.13; scripts/sweep_pfnw.sh)
+  // 8-warp CTAs per SM are ahead (L = 30 / 50 / 75: 0.60 / 1.26 / 2.79 ms against 0.88 / 1.71 / 3.13)
   // small batches (see mfe3_cfg): 16 warps at every length (B = 64: 36 nt 0.071 -> 0.058 ms, 100 nt 0.336 -> 0.227, 148 nt 0.776 -> 0.550,
   // 170 nt 1.00 -> 0.69, 176 nt 1.10 -> 0.72; the plan stops fitting the shared memory at ~178 nt, longer sequences stay on the round-1 kernel)
   // (beyond ~110 nt, qm / qm1 off chip, the split wants more auxiliary warps: paired cells with 10 tap + 6 auxiliary warps, B = 64 x 140 nt 0.51 -> 0.46 ms)
-  c.nw = nw_env ? nw_env : small ? (nmax > 110 ? 116 : 16) : (nmax < 90 ? 8 : 116);
-  const int nwr = c.nw % 100;   // (100 + warps: the paired variant)
-  c.nwi = env_int("BF_FILL3_PF_NWI", nwr == 8 ? 6 : nwr == 16 ? ((small && nmax > 110) ? 10 : 12) : nwr * 3 / 4);
-  const int nwa = nwr - c.nwi;
-  const size_t with = pf3_plan(nmax, c.rs, nwr, nwa, true).total, without = pf3_plan(nmax, c.rs, nwr, nwa, false).total;
-  const int q_env = env_int("BF_FILL3_PF_QMS", -1);
-  c.qms = q_env >= 0 ? q_env != 0 : (nwr >= 12 && with <= kSmemBudget);
-  if (c.qms && with > kSmemBudget) c.qms = false;
-  c.smem = c.qms ? with : without;
+  c.nw = small || nmax >= 90 ? 16 : 8;
+  c.pair = small ? nmax > 110 : nmax >= 90;
+  c.nwi = c.nw == 8 ? 6 : (small && nmax > 110) ? 10 : 12;
+  const int nwa = c.nw - c.nwi;
+  const size_t with = pf3_plan(nmax, c.rs, c.nw, nwa, true).total;
+  c.qms = c.nw == 16 && with <= kSmemBudget;
+  c.smem = c.qms ? with : pf3_plan(nmax, c.rs, c.nw, nwa, false).total;
   // measured against the round-1 kernel (profiles/r02_sweep_len.txt): ahead up to 150 nt, level beyond
-  c.ok = c.smem <= kSmemBudget && nmax <= (small ? env_int("BF_FILL3_PF_MAXN_SMALL", 230) : env_int("BF_FILL3_PF_MAXN", 150));
+  c.ok = c.smem <= kSmemBudget && nmax <= (small ? 230 : 150);
   return c;
 }
 }  // namespace
@@ -971,15 +929,13 @@ static cudaError_t pf3_launch(const BfParams *dP, const BfBatchDev &b, double *q
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
   }
-  const int cap = env_int("BF_FILL3_PF_CTAS", 0), per_sm = cap > 0 && cap < occ ? cap : occ;
-  if (env_int("BF_CFG_PRINT", 0)) fprintf(stderr, "pf_fill3<%d,%d,%d,%d> stride %d smem %zu occ %d per_sm %d\n", NW, NWI, (int)QMSM, (int)PAIR, b.stride, c.smem, occ, per_sm);
-  const int grid = b.B < sms * per_sm ? b.B : sms * per_sm;
+  const int grid = b.B < sms * occ ? b.B : sms * occ;
   if (grid_out) { *grid_out = grid; return cudaSuccess; }
   const uint32_t *taps = nullptr;
   e = taps_device(c.rs, 16, &taps);
   if (e != cudaSuccess) return e;
   kern<<<grid, NW * 32, c.smem, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), ws, bf_fill3_pf_ws_slot(b.stride), qmseq, mfe_for_scale, lnscale,
-                                      taps, c.rs, counter, env_int("BF_FILL3_DBG", 0));
+                                      taps, c.rs, counter);
   return cudaGetLastError();
 }
 
@@ -987,19 +943,11 @@ static cudaError_t pf3_dispatch(const BfParams *dP, const BfBatchDev &b, double 
                                 double *lnscale, int sms, int *counter, cudaStream_t st, int *grid_out, bool small) {
   const Pf3Cfg c = pf3_cfg(b.stride, small);
   if (!c.ok) return cudaErrorInvalidValue;
-#define BF_GO(NW_, NWI_)                                                                                                              \
-  if (c.nw == NW_ && c.nwi == NWI_)                                                                                                    \
-    return c.qms ? pf3_launch<NW_, NWI_, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)         \
-                 : pf3_launch<NW_, NWI_, false>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)
-  BF_GO(8, 6); BF_GO(16, 12); BF_GO(16, 10); BF_GO(12, 9);
+#define BF_GO(NW_, NWI_, QMSM_, PAIR_)                                                                                                \
+  if (c.nw == NW_ && c.nwi == NWI_ && c.qms == QMSM_ && c.pair == PAIR_)                                                             \
+    return pf3_launch<NW_, NWI_, QMSM_, PAIR_>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)
+  BF_GO(8, 6, false, false); BF_GO(16, 12, true, false); BF_GO(16, 12, true, true); BF_GO(16, 12, false, true); BF_GO(16, 10, false, true);
 #undef BF_GO
-  // 12 warps, one CTA per SM: 170 registers per thread -- tap warps take their cells in pairs
-#define BF_GO2(NW_, NWI_)                                                                                                                   \
-  if (c.nw == NW_ + 100 && c.nwi == NWI_)                                                                                                    \
-    return c.qms ? pf3_launch<NW_, NWI_, true, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)         \
-                 : pf3_launch<NW_, NWI_, false, true>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)
-  BF_GO2(12, 8); BF_GO2(12, 9); BF_GO2(12, 10); BF_GO2(16, 12); BF_GO2(16, 10);
-#undef BF_GO2
   return cudaErrorInvalidValue;
 }
 

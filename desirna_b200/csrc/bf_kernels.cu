@@ -1235,19 +1235,15 @@ size_t bf_pf_slot_doubles(int wstride) { return (size_t)6 * wstride * wstride; }
 
 // The generic kernels (two strands; any length the fill path does not cover) keep three W x W tables per CTA.  Short sequences --
 // the reference's two-strand examples are 17 & 18 nt -- fit in shared memory next to the per-sequence arrays, which takes the L2
-// round trip out of every table access (BF_GEN_SMEM=0: always HBM).  Capped so that at least two CTAs share an SM.
+// round trip out of every table access.  Capped so that at least two CTAs share an SM.
 static bool gen_wide(int B) {
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const char *v = getenv("BF_WIDE");
-  return B > 0 && B <= sms && !(v && *v && atoi(v) == 0);
+  return B > 0 && B <= sms && bf_opt("BF_WIDE", 1) != 0;
 }
 // the two-barrier variants: batches that leave SMs idle, i.e. latency matters (measured: 17 & 18 nt x 64 MFE 0.164 -> 0.150 ms, but
-// 50 & 50 nt x 4096 16.7 -> 25.5 ms); BF_GEN_PRE=0: the four-barrier ones everywhere
-static bool gen_pre(int wstride, bool wide) {
-  const char *v = getenv("BF_GEN_PRE");
-  return wide && wstride - 2 <= kPreMax && !(v && *v && atoi(v) == 0);
-}
+// 50 & 50 nt x 4096 16.7 -> 25.5 ms)
+static bool gen_pre(int wstride, bool wide) { return wide && wstride - 2 <= kPreMax; }
 static size_t mfe_smem(int wstride, bool pre) {
   size_t nmax = wstride - 2;
   const size_t arrays = pre ? 3 + 2 + 2 * kPreArr : 3 + 8;
@@ -1257,18 +1253,14 @@ static size_t pf_smem(int wstride, bool pre) {
   size_t nmax = wstride - 2;
   return (pre ? 5 + 2 + 2 * kPreArrD : 5 + 6) * (nmax + 4) * sizeof(double) + (pre ? 4 : 2) * (nmax + 4) * sizeof(int) + 2 * ((nmax + 2 + 15) / 16 * 16);
 }
-static size_t gen_tables_cap() {
-  const char *v = getenv("BF_GEN_SMEM");
-  if (v && *v && atoi(v) == 0) return 0;
-  return (size_t)100 * 1024;
-}
+static const size_t kGenTablesCap = 100 * 1024;
 static unsigned mfe_tables_off(int wstride, bool pre) {   // 0: tables in HBM
   const size_t base = (mfe_smem(wstride, pre) + 15) / 16 * 16;
-  return base + bf_mfe_slot_ints(wstride) * sizeof(int) <= gen_tables_cap() ? (unsigned)base : 0u;
+  return base + bf_mfe_slot_ints(wstride) * sizeof(int) <= kGenTablesCap ? (unsigned)base : 0u;
 }
 static unsigned pf_tables_off(int wstride, bool pre) {
   const size_t base = (pf_smem(wstride, pre) + 15) / 16 * 16;
-  return base + bf_pf_slot_doubles(wstride) * sizeof(double) <= gen_tables_cap() ? (unsigned)base : 0u;
+  return base + bf_pf_slot_doubles(wstride) * sizeof(double) <= kGenTablesCap ? (unsigned)base : 0u;
 }
 static size_t mfe_smem_total(int wstride, bool pre) { const unsigned o = mfe_tables_off(wstride, pre); return o ? o + bf_mfe_slot_ints(wstride) * sizeof(int) : mfe_smem(wstride, pre); }
 static size_t pf_smem_total(int wstride, bool pre) { const unsigned o = pf_tables_off(wstride, pre); return o ? o + bf_pf_slot_doubles(wstride) * sizeof(double) : pf_smem(wstride, pre); }

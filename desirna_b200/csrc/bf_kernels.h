@@ -8,6 +8,10 @@
 
 struct BfBatchDev;
 
+// Switches that override a default kernel-selection rule, read from the environment variable of that name at call time
+// (bf_capi.cu holds the list; bf_set_option sets them from the host program).  Unset or empty: dflt.
+int bf_opt(const char *name, int dflt);
+
 cudaError_t bf_upload_constants();
 size_t bf_mfe_slot_ints(int wstride);
 size_t bf_pf_slot_doubles(int wstride);

@@ -587,18 +587,14 @@ __global__ void __launch_bounds__(NW * 32) bf_k_pf_out2(const BfParams *__restri
 
 // ---- host side: v2 whenever its plan fits the CTA's shared memory (generic ring on chip when that still leaves two CTAs per
 // SM), else the first version
-#include <cstdlib>
 namespace {
 constexpr size_t kOutSmemBudget = 232448 - 1024 - 256;
 int out_version(int nmax, bool *rgs, bool *hsm = nullptr, int B = 0, int sms = 148) {
-  const char *v = getenv("BF_OUT_V");
   if (hsm) *hsm = false;
-  if (v && v[0] == '1') return 1;
   // H / qm / qm1 of the sequence on chip as well: measured against reading them through L2 (profiles/r02_outside_hsm.txt) -- ahead
   // while two CTAs still share an SM (<= ~60 nt: 3-5 %) and for batches that leave SMs idle (B = 64: 0.96 -> 0.82 ms at 100 nt);
-  // behind for big batches once it costs the second CTA (4096 x 100 nt: 16.2 against 11.3 ms).  BF_OUT_HSM=0 / 1: never / whenever it fits.
-  const char *h = getenv("BF_OUT_HSM");
-  const bool want = h && *h ? h[0] != '0' : (out2_plan(nmax, 8, true, true).total <= 113 * 1024 || (B > 0 && B <= sms));
+  // behind for big batches once it costs the second CTA (4096 x 100 nt: 16.2 against 11.3 ms).
+  const bool want = out2_plan(nmax, 8, true, true).total <= 113 * 1024 || (B > 0 && B <= sms);
   if (hsm && want && out2_plan(nmax, 8, true, true).total <= kOutSmemBudget) { *rgs = true; *hsm = true; return 2; }
   if (out2_plan(nmax, 8, true).total <= 113 * 1024) { *rgs = true; return 2; }
   if (out2_plan(nmax, 8, false).total <= kOutSmemBudget) { *rgs = false; return 2; }

@@ -160,8 +160,9 @@ def second_best(seqs, nopair=None):
 
 
 def set_option(key, value):
-    """Tuning / test hook (bf_set_option): sets the engine's BF_<KEY> variable, e.g. set_option("cl", 0) switches the
-    cluster-per-sequence fill kernels off, set_option("cl", -1) restores the default rule."""
+    """Test / measurement hook (bf_set_option): sets the engine's BF_<KEY> variable, e.g. set_option("cl", 0) switches the
+    cluster-per-sequence fill kernels off, set_option("cl", -1) restores the default rule.  The keys are listed in
+    include/b200fold.h; any other key raises."""
     ensure_ready()
     _check(lib().bf_set_option(key.encode(), int(value)))
 

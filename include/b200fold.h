@@ -108,13 +108,18 @@ int bf_microbench(double out[3]);
 int64_t bf_kernel_launches(void);
 /* SM count of the device in use */
 int bf_sm_count(void);
-/* Tuning / test hook.  Kernel variants are chosen per call by default rules that BF_* environment variables override; this sets
- * the variable BF_<KEY> from the host program (value < 0: remove it).  E.g. "cl" 0 / 1: never / always use the cluster-per-sequence
- * fill kernels where they cover the length, "cl_c" 4 | 8 | 16: their cluster size, "ext_wide" 0 / 1: exterior recursions by one warp /
- * one CTA per sequence, "wide" 0: no 16-warp variants for small batches, "fill3_small" 0: small batches on the 16-warp round-1 kernels
- * instead of the 16-warp third-generation ones, "gen_pre" 0: two-strand kernels with four barriers per diagonal at every batch size,
- * "score_overlap" 0: bf_score_batch[_device] never runs the partition function beside the MFE fill, "stage" 0: bf_score_batch copies
- * every host array on its own instead of one pinned block each way for small batches. */
+/* Test / measurement hook.  Kernel variants are chosen per call by default rules that a few BF_* environment variables override;
+ * this sets the variable BF_<KEY> from the host program (value < 0: remove it, back to the default rule).  The keys:
+ *   "cl" 0 / 1: never / always use the cluster-per-sequence fill kernels where they cover the length; "cl_c" 4 | 8 | 16: their
+ *   cluster size; "cl_bw" 16 | 32: their block width;
+ *   "ext_wide" 0 / 1: exterior recursions by one warp / one CTA per sequence;
+ *   "wide" 0: no 16-warp variants for small batches;
+ *   "fill3" 0: the round-1 fill kernels instead of the third-generation ones; "fill3_small" 0: small batches on the 16-warp round-1
+ *   kernels instead of the 16-warp third-generation ones;
+ *   "blk_min" / "blk_min_pf" N: the round-1 MFE / PF fills use the blocked split from N nt on (default 280 / 250);
+ *   "force_generic" 1: single strands on the generic kernels too (read by bf_init);
+ *   "design_overlap" 0: the device design loop always folds MFE, then PF.
+ * Any other key is refused with BF_ERR_ARG. */
 int bf_set_option(const char *key, int value);
 /* Test hook: copy one engine-internal DP table of the most recent call to host memory.
  * which: 0 = c (int32), 1 = fML (int32), 2 = qb (double); layout: per sequence a packed, diagonal-major triangle of

@@ -33,7 +33,7 @@ def main():
                 km += np.array(engine.last_kernel_ms())
             ms = (time.perf_counter() - t0) / n * 1e3
             out[f"L{L}_B{B}"] = {"call_ms": round(ms, 3), "mfe_ms": round(km[0] / n, 3), "pf_ms": round(km[1] / n, 3), "eval_ms": round(km[2] / n, 3)}
-    print(json.dumps({"nw": [os.environ.get("BF_MFE_NW", "default"), os.environ.get("BF_PF_NW", "default")], "latency": out}))
+    print(json.dumps({"latency": out}))
 
 
 if __name__ == "__main__":

@@ -72,6 +72,16 @@ def test_param_loader_matches_oracle_loader(oracle):
         assert g("int22", *idx) == oracle.get("int22", *idx), idx
 
 
+def test_set_option_refuses_unknown_keys():
+    """bf_set_option sets only the switches include/b200fold.h lists; a removed or misspelt key is an error, not a no-op."""
+    from desirna_b200 import engine
+    L = engine.lib()
+    assert L.bf_set_option(b"mfe_nw", 4) == 5  # BF_ERR_ARG
+    assert L.bf_set_option(b"design_graph", 1) == 5
+    assert L.bf_set_option(b"wide", 0) == 0
+    assert L.bf_set_option(b"wide", -1) == 0  # back to the default rule
+
+
 def test_params_2004_is_reported_unavailable():
     from desirna_b200 import engine
     with pytest.raises(engine.EngineError) as ei:

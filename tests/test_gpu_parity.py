@@ -149,7 +149,6 @@ def test_bpp_ragged_and_unavailable_cases(engine, oracle):
 def test_blocked_split_matches_oracle(engine, oracle, monkeypatch):
     """The blocked split (tile-major mirrors + 4x4 block products, long sequences by default) forced on for every length:
     MFE energies and structures bit-exact, ensemble free energy within 1e-6 relative of the oracle."""
-    monkeypatch.setenv("BF_BLK", "1")
     monkeypatch.setenv("BF_BLK_MIN", "1")
     monkeypatch.setenv("BF_BLK_MIN_PF", "1")
     rng = np.random.default_rng(77)
@@ -161,6 +160,23 @@ def test_blocked_split_matches_oracle(engine, oracle, monkeypatch):
         assert out["mfe_dcal"][k] == e and out["mfe_ss"][k] == ss, (len(s), k)
         f = oracle.pf(s)[4]
         assert abs(out["pf"][k, 4] - f) <= 1e-6 * max(1.0, abs(f)), (len(s), k)
+
+
+@pytest.mark.parametrize("thr, L, B", [(300, 253, 1), (400, 365, 1), (400, 317, 149)])
+def test_raised_blocked_split_threshold(engine, oracle, monkeypatch, thr, L, B):
+    """BF_BLK_MIN_PF raised above a length: the round-1 PF fill runs that length without the blocked split (16 warps with the
+    full or the shared partial buffers, 8 warps with shared ones).  Same ensemble energies as the default rule and the oracle."""
+    monkeypatch.setenv("BF_CL", "0")
+    seqs = rand_seqs(900 + L, B, L)
+    want = engine.WANT_MFE | engine.WANT_PF
+    ref = engine.score_batch(seqs, want=want)
+    monkeypatch.setenv("BF_BLK_MIN_PF", str(thr))
+    out = engine.score_batch(seqs, want=want)
+    assert (out["mfe_dcal"] == ref["mfe_dcal"]).all()
+    assert np.allclose(out["pf"][:, 4], ref["pf"][:, 4], rtol=1e-10, atol=0)
+    for k in range(0, B, 50):
+        f = oracle.pf(seqs[k])[4]
+        assert abs(out["pf"][k, 4] - f) <= 1e-6 * max(1.0, abs(f))
 
 
 @pytest.mark.parametrize("L", [30, 100, 260, 400])
