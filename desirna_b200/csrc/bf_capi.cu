@@ -668,6 +668,11 @@ struct DesignLoop {
   bool two = false;   // some job has two strands: the loop folds with the two-strand kernels
   bool pks = false;   // pseudoknot overlay: three constrained refolds after the MFE fold of every sub-step
   bool overlap = true;  // BF_DESIGN_OVERLAP=0: always fold MFE, then PF
+  // avoid designs (oligo 3): the self-dimer fold runs on a stream of its own beside the single-strand fills.  It needs its own
+  // workspace: run_device takes the work counters and ws_pf from the workspace it is given
+  Workspace wd;
+  cudaStream_t st_dimer = nullptr;
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   std::vector<void *> allocs;
   std::vector<uint8_t> active;
   uint8_t *d_active = nullptr;
@@ -682,11 +687,17 @@ struct DesignLoop {
   }
   void destroy() {
     if (st) cudaStreamSynchronize(st);
+    if (st_dimer) cudaStreamSynchronize(st_dimer);
     for (void *q : allocs) cudaFree(q);
     allocs.clear();
     w.destroy();
+    wd.destroy();
+    if (ev_fork) cudaEventDestroy(ev_fork);
+    if (ev_join) cudaEventDestroy(ev_join);
     if (st) cudaStreamDestroy(st);
-    st = nullptr;
+    if (st_dimer) cudaStreamDestroy(st_dimer);
+    st = st_dimer = nullptr;
+    ev_fork = ev_join = nullptr;
   }
 };
 
@@ -707,6 +718,21 @@ int design_rows(DesignLoop *h) {
 
 // one scoring pass over the rows: the same pipeline bf_score_batch_device runs (MFE fill + backtrack, PF fill + exterior, eval)
 int design_score(DesignLoop *h, bool init = false) {
+  if (h->C.oligo == 3) {
+    // avoid: two-strand partition function of the self-dimers (bf_k_design_propose wrote them), forked after propose.  PF only and
+    // no scale override: ViennaRNA's default scale, as the host's fc.pf_dimer() of seq&seq.  Joined before the accept kernel.
+    bf_batch_t bd;
+    std::memset(&bd, 0, sizeof bd);
+    bd.B = h->B; bd.stride = 2 * h->D.stride; bd.seq = h->D.dimer_seq; bd.len = h->D.dimer_len; bd.cut = h->D.dimer_cut; bd.want = BF_WANT_PF;
+    bf_result_t rd;
+    std::memset(&rd, 0, sizeof rd);
+    rd.pf = h->D.o_dimer_pf;
+    CU(cudaEventRecord(h->ev_fork, h->st), "fork self-dimer fold");
+    CU(cudaStreamWaitEvent(h->st_dimer, h->ev_fork, 0), "fork self-dimer fold");
+    const int rc = run_device(h->wd, &bd, &rd, true, h->st_dimer, nullptr, false);
+    if (rc) return rc;
+    CU(cudaEventRecord(h->ev_join, h->st_dimer), "join self-dimer fold");
+  }
   bf_batch_t b;
   std::memset(&b, 0, sizeof b);
   b.B = h->B; b.stride = h->D.stride; b.seq = h->D.mut_seq; b.len = h->D.row_len; b.targets = h->D.row_tgt; b.n_targets = h->D.T; b.want = h->want;
@@ -730,22 +756,24 @@ int design_score(DesignLoop *h, bool init = false) {
     CU(bf_launch_twobest(g.dP, db, (int2 *)h->w.ws_mfe.p, wstride, grid, h->w.d_counters + 3, h->D.o_e1, h->D.o_e2, h->st, h->D.nd_flag, h->two), "launch bf_k_mfe2");
     g.launches += 2;
   }
-  if (!h->pks) return BF_OK;
-  // pseudoknot overlay (sequence_utils.py:1166-1228): forbid what is paired, fold again, paint the new pairs with the next bracket
-  // family; three rounds.  A round that finds no pair leaves the overlay and the mask as they are, so the rounds the reference
-  // skips are no-ops here; all rows go through all rounds.
-  bf_batch_t b2 = b;
-  b2.want = BF_WANT_MFE | BF_WANT_SS; b2.nopair = h->D.pk_nopair; b2.targets = nullptr; b2.n_targets = 0;
-  bf_result_t r2;
-  std::memset(&r2, 0, sizeof r2);
-  r2.mfe_dcal = h->D.o_mfe2; r2.mfe_ss = h->D.o_ss2;
-  for (int round = 0; round < 3; round++) {
-    CU(bf_launch_design_pk_mask(h->D, h->B, h->st), "launch bf_k_design_pk_mask");
-    rc = run_device(h->w, &b2, &r2, false, h->st, nullptr, false);
-    if (rc) return rc;
-    CU(bf_launch_design_pk_paint(h->D, h->B, round, h->st), "launch bf_k_design_pk_paint");
-    g.launches += 2;
+  if (h->pks) {
+    // pseudoknot overlay (sequence_utils.py:1166-1228): forbid what is paired, fold again, paint the new pairs with the next bracket
+    // family; three rounds.  A round that finds no pair leaves the overlay and the mask as they are, so the rounds the reference
+    // skips are no-ops here; all rows go through all rounds.
+    bf_batch_t b2 = b;
+    b2.want = BF_WANT_MFE | BF_WANT_SS; b2.nopair = h->D.pk_nopair; b2.targets = nullptr; b2.n_targets = 0;
+    bf_result_t r2;
+    std::memset(&r2, 0, sizeof r2);
+    r2.mfe_dcal = h->D.o_mfe2; r2.mfe_ss = h->D.o_ss2;
+    for (int round = 0; round < 3; round++) {
+      CU(bf_launch_design_pk_mask(h->D, h->B, h->st), "launch bf_k_design_pk_mask");
+      rc = run_device(h->w, &b2, &r2, false, h->st, nullptr, false);
+      if (rc) return rc;
+      CU(bf_launch_design_pk_paint(h->D, h->B, round, h->st), "launch bf_k_design_pk_paint");
+      g.launches += 2;
+    }
   }
+  if (h->C.oligo == 3) CU(cudaStreamWaitEvent(h->st, h->ev_join, 0), "join self-dimer fold");
   return BF_OK;
 }
 }  // namespace
@@ -797,6 +825,7 @@ int bf_design_create(const bf_design_t *c, void **handle) {
       if (!sk.empty()) return fail(BF_ERR_ARG, "bf_design_create: unbalanced target");
   }
   if (c->pks && two) return fail(BF_ERR_ARG, "bf_design_create: the pseudoknot overlay needs single-strand jobs");
+  if (c->oligo == 3 && two) return fail(BF_ERR_ARG, "bf_design_create: avoid designs (oligo = 3) need single-strand jobs");
   if (c->subopt && c->pks) return fail(BF_ERR_ARG, "bf_design_create: negative design (subopt) does not combine with the pseudoknot overlay");
   if (!two && (bf_fill_mfe_mode(S) == 0 || bf_fill_pf_mode(S) == 0)) return fail(BF_ERR_UNAVAILABLE, "bf_design_create: stride outside the fill path");
   // optional scenario terms: alternative structures, motifs
@@ -877,6 +906,14 @@ int bf_design_create(const bf_design_t *c, void **handle) {
   DCU(h->alloc(&D.o_eval, G * D.T), "cudaMalloc(design)");
   if (c->subopt) { DCU(h->alloc(&D.nd_flag, G), "cudaMalloc(design)"); DCU(h->alloc(&D.o_e1, G), "cudaMalloc(design)"); DCU(h->alloc(&D.o_e2, G), "cudaMalloc(design)"); }
   if (h->pks) { DCU(h->alloc(&D.pk_nopair, G * S), "cudaMalloc(design)"); DCU(h->alloc(&D.o_mfe2, G), "cudaMalloc(design)"); DCU(h->alloc(&D.o_ss2, G * (S + 1)), "cudaMalloc(design)"); }
+  if (c->oligo == 3) {   // self-dimer rows (stride 2 S <= 4000, bf_score_batch's limit), their PF columns, a second workspace and stream
+    DCU(h->alloc(&D.dimer_seq, G * 2 * S), "cudaMalloc(design)"); DCU(h->alloc(&D.dimer_len, G), "cudaMalloc(design)"); DCU(h->alloc(&D.dimer_cut, G), "cudaMalloc(design)");
+    DCU(h->alloc(&D.o_dimer_pf, G * 5), "cudaMalloc(design)");
+    DCU(h->wd.create(), "create self-dimer workspace");
+    DCU(cudaStreamCreateWithFlags(&h->st_dimer, cudaStreamNonBlocking), "cudaStreamCreate(self-dimer)");
+    DCU(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming), "cudaEventCreate(self-dimer)");
+    DCU(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming), "cudaEventCreate(self-dimer)");
+  }
   h->want = BF_WANT_MFE | BF_WANT_SS | BF_WANT_PF | BF_WANT_EVAL;
   BfDesignCfg &C = h->C;
   C.n_terms = c->n_terms;

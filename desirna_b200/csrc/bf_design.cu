@@ -159,6 +159,15 @@ __global__ void bf_k_design_pk_paint(BfDesignDev D, int B, int round) {
 }
 
 // ------------------------------------------------------------------------------------------------ propose
+// avoid designs: the row's self-dimer, the finished mutant twice ('&' is the cut, n + 1, as engine.pack sets it)
+__device__ __forceinline__ void self_dimer_row(const BfDesignDev &D, const BfDesignCfg &C, int row, const char *mut, int n, int lane) {
+  if (C.oligo != 3) return;
+  __syncwarp();
+  char *d = D.dimer_seq + (size_t)row * 2 * D.stride;
+  for (int k = lane; k < 2 * n; k += 32) d[k] = mut[k < n ? k : k - n];
+  if (lane == 0) { D.dimer_len[row] = 2 * n; D.dimer_cut[row] = n + 1; }
+}
+
 // mutate_sequence + get_mutation_position (sequence_utils.py:926-1136) without the scoring call at its end
 __global__ void __launch_bounds__(kWPB * 32) bf_k_design_propose(BfDesignDev D, BfDesignCfg C, int B, int copy_only) {
   extern __shared__ __align__(16) unsigned char dyn[];
@@ -169,12 +178,14 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_propose(BfDesignDev D, 
   char *mut = D.mut_seq + (size_t)row * S;
   for (int k = lane; k < S; k += 32) mut[k] = cur[k];
   if (lane == 0) D.row_scale[row] = D.cur_mfe[g];
-  if (copy_only) return;   // initial scoring: the "mutant" is the start sequence itself
+  const int n_avail = D.n_avail[job];
+  if (copy_only || n_avail == 0) {   // initial scoring: the "mutant" is the start sequence itself; or nothing to mutate
+    self_dimer_row(D, C, row, mut, n, lane);
+    return;
+  }
   const short *tpt = D.tpt + (size_t)job * S;
   const uint8_t *allowed = D.allowed + (size_t)job * S;
   const unsigned short *avail = D.avail + (size_t)job * S;
-  const int n_avail = D.n_avail[job];
-  if (n_avail == 0) return;
   unsigned long long rng = D.rng[g];   // every lane advances an identical copy; lane 0 writes it back
   WarpScratch w = scratch(dyn, S, warp);
 
@@ -287,6 +298,7 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_propose(BfDesignDev D, 
       }
     }
   }
+  self_dimer_row(D, C, row, mut, n, lane);
 }
 
 // ------------------------------------------------------------------------------------------------ accept
@@ -377,14 +389,17 @@ __global__ void __launch_bounds__(kWPB * 32) bf_k_design_accept(BfDesignDev D, B
       rec[kRecSubopt] = (e2 < BF_INF && e2 - e1 <= 4900) ? (double)(float)((double)e2 / 100.0) : 0.0;
       total -= rec[kRecSubopt] - Epf;
     }
-    if (two && C.oligo >= 1) {
-      // equilibrium dimer fraction at 1 mM from FcAB - FA - FB (dimer_multichain_energy.py:36-63), float32 API values first
+    const bool avoid = C.oligo == 3;   // one-strand jobs only: the fraction is the self-dimer's (energy_scores.py:118-119,412-419)
+    if ((two && C.oligo >= 1) || avoid) {
+      // equilibrium dimer fraction at 1 mM from FcAB - FA - FB (dimer_multichain_energy.py:36-63), float32 API values first.
+      // FcAB = 999 (no inter-strand pair) gives rhs = 0 and a NaN fraction, as the host arithmetic does.
+      const double *pf = (avoid ? D.o_dimer_pf : D.o_pf) + (size_t)row * 5;
       const double kT = 0.001987204259 * (273.15 + 37);
-      const double dF = (double)(float)D.o_pf[(size_t)row * 5 + 2] - (double)(float)D.o_pf[(size_t)row * 5 + 0] - (double)(float)D.o_pf[(size_t)row * 5 + 1];
+      const double dF = (double)(float)pf[2] - (double)(float)pf[0] - (double)(float)pf[1];
       const double rhs = 1e-3 / 55.14 * exp(-dF / kT);
       const double frac = 1 - (sqrt(1 + 4 * rhs) - 1) / (2 * rhs);
       rec[kRecOligoFraction] = frac;
-      rec[kRecOligoBonus] = (C.oligo == 2 && D.same_halves[job]) ? -kT * log(1 - frac) : -kT * log(frac);
+      rec[kRecOligoBonus] = (avoid || (C.oligo == 2 && D.same_halves[job])) ? -kT * log(1 - frac) : -kT * log(frac);
       total += rec[kRecOligoBonus];
     }
     for (int m = 0; m < C.n_motifs; m++)

@@ -3,7 +3,8 @@
 // The reference runs this loop on the host: utils/replica_exchange_monte_carlo.py:176-271 (Metropolis sub-steps and
 // neighbour swaps) around utils/sequence_utils.py:926-1136 (move generator).  Here the state of every replica of every
 // design problem ("job") stays in HBM; one sub-step is  propose -> MFE fill + backtrack -> PF fill + exterior -> eval ->
-// accept  on one stream, with no host round trip.
+// accept  on one stream, with no host round trip.  Avoid designs (oligo 3) fold the self-dimers of the rows on a second stream,
+// forked after propose and joined before accept.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -24,7 +25,8 @@ struct BfDesignCfg {
   double nt_weight[4];   // A C G U
   int oligo;             // two-strand jobs: 1 heterodimer, adds -kT ln(dimer fraction); 2 homodimer, strands kept identical and
                          // -kT ln(dimer fraction) (different target halves) or -kT ln(1 - fraction) (identical halves)
-                         // (energy_scores.py:120-125,421-441, dimer_multichain_energy.py:36-76, sequence_utils.py:1102-1128)
+                         // (energy_scores.py:120-125,421-441, dimer_multichain_energy.py:36-76, sequence_utils.py:1102-1128);
+                         // one-strand jobs: 3 avoid (-o on), adds -kT ln(1 - fraction) of the self-dimer seq&seq (energy_scores.py:118-119,412-419)
   int subopt;            // -nd on: Epf - E(second-best structure) for mutants that fold into the target (energy_scores.py:104-107)
   int n_motifs;          // -motifs: IUPAC motifs, bonus added when the motif occurs in the sequence (sequence_utils.py:1231-1256)
   int motif_len[8];
@@ -83,6 +85,11 @@ struct BfDesignDev {
   // negative design: rows whose structure equals the target, and their (best, second-best) energies from bf_k_mfe2
   uint8_t *nd_flag;              // B
   int *o_e1, *o_e2;              // B
+  // avoid (oligo 3): the self-dimer of every row, the mutant twice without '&' (written by bf_k_design_propose), and its
+  // two-strand partition function
+  char *dimer_seq;               // B x 2 stride
+  int *dimer_len, *dimer_cut;    // B            2 n, n + 1
+  double *o_dimer_pf;            // B x 5        FA, FB, FcAB, FAB, F0AB
 };
 
 cudaError_t bf_launch_design_gather(const BfDesignDev &D, int B, cudaStream_t st);

@@ -41,7 +41,7 @@ class DesignOptions:
         self.nt_percentages = nt_percentages or {"A": 15, "C": 30, "G": 30, "U": 15}
         self.diff_start_replicas = diff_start_replicas
         self.L = 504.12
-        self.oligo_state, self.pks, self.subopt = oligo_state, pks, subopt   # "none" | "heterodimer" | "homodimer"
+        self.oligo_state, self.pks, self.subopt = oligo_state, pks, subopt   # "none" | "heterodimer" | "homodimer" | "avoid" (-o on)
         # -motifs "KEY,bonus,KEY,bonus": IUPAC motif -> (compiled regex, bonus) as DesiRNA.py:212-224 builds it
         self.motifs = {k: (re.compile("".join("[%s]" % seq_utils.IUPAC.get(ch, ch) for ch in k)), float(v)) for k, v in (motifs or {}).items()} or None
         self.rep_temps_shelfs = seq_utils.get_rep_temps(self)
@@ -131,7 +131,7 @@ class DesignLoop:
                       np.array(sim_options.rep_temps_shelfs, np.float64), np.array(seq_utils.targeted_move_probabilities(sim_options), np.float64)]
         cfg.n_jobs, cfg.replicas, cfg.stride = self.J, self.R, self.stride
         cfg.target, cfg.len, cfg.len_a, cfg.allowed, cfg.init_seq, cfg.temps, cfg.tm_prob = (a.ctypes.data for a in self._keep)
-        cfg.oligo = {"heterodimer": 1, "homodimer": 2}.get(sim_options.oligo_state, 0)
+        cfg.oligo = {"heterodimer": 1, "homodimer": 2, "avoid": 3}.get(sim_options.oligo_state, 0)
         cfg.n_terms = len(terms)
         for k, (t, w) in enumerate(terms):
             cfg.term[k], cfg.weight[k] = t, w
@@ -260,6 +260,8 @@ class DesignLoop:
                     row["ensemble_defect"] = v["ensemble_defect"]
                 if self.len_a[j] > 0:
                     row["oligo_fraction"], row["oligomer_bonus"] = v["oligo_fraction"], v["oligomer_bonus"]
+                elif sim_options.oligo_state == "avoid":   # ScoreSeq.get_scoring_function_monomer's fields; the record slot is shared
+                    row["oligo_fraction"], row["monomer_bonus"] = v["oligo_fraction"], v["oligomer_bonus"]
                 rows.append(row)
             out.append(rows)
         return out
@@ -355,7 +357,8 @@ def design_batch(inputs, sim_options, time_limit=None, global_steps=None, stop_w
 
     Stops when every job is solved (stop_when_solved, the reference's `-sws on` with `-r 1`), after `global_steps` global
     steps (`-s`), or after `time_limit` seconds (`-t`), whichever comes first.  Returns (results, info): one dict per input
-    (REC_FIELDS + name, sequence, mfe_ss, solved, solved_step, solved_after_s) and run statistics.
+    (REC_FIELDS + name, sequence, mfe_ss, solved, solved_step, solved_after_s; + monomer_bonus with oligo_state="avoid") and run
+    statistics.
 
     trajectory=True (use poll_steps=1) also records, per job, what DesiRNA.py keeps as `simulation_data` -- the state of every
     replica after each global step -- and a Stats object, as info["simulation_data"][k] / info["stats"][k]: the inputs of
@@ -393,6 +396,8 @@ def design_batch(inputs, sim_options, time_limit=None, global_steps=None, stop_w
             res = {"name": inputs[k].name, "sequence": jb["sequence"][pos], "mfe_ss": jb["mfe_ss"][pos], "solved": bool(solved),
                    "solved_step": int(jb["solved_step"][pos]), "solved_after_s": solved_at[k]}
             res.update({f: float(jb["rec"][pos, c]) for c, f in enumerate(REC_FIELDS)})
+            if sim_options.oligo_state == "avoid":
+                res["monomer_bonus"] = res["oligomer_bonus"]
             results[k] = res
             if solved and stop_when_solved:
                 mask[pos] = 0

@@ -4,8 +4,9 @@
 `get_first_suboptimal_structure_and_energy` keep the reference's names, arguments and return values.
 New here: `score_sequences(seqs, input_file, sim_options)`, the batched form the lock-step replica
 loop uses -- ONE engine call (MFE + backtrack + partition function + eval of the target and of every
-alternative structure) for all mutants of a Monte-Carlo sub-step, then the reference's double-precision
-score arithmetic on float32-rounded energies (SURVEY.md 8b "Derived-score arithmetic").
+alternative structure) for all mutants of a Monte-Carlo sub-step, one more for their self-dimers in
+avoid mode (`-o on`), then the reference's double-precision score arithmetic on float32-rounded energies
+(SURVEY.md 8b "Derived-score arithmetic").
 
 Quirks kept for score parity (SURVEY.md App. C): only the scoring terms present in `sim_options.scoring_f`
 are evaluated (the reference's option parser keeps the first `-sf` term only, stats_inputs_outputs.py:232-237,
@@ -90,7 +91,7 @@ def get_mfe_e_ss(seq, sim_options):
     return energy, structure, fc
 
 
-def _score_with_compound(seq, input_file, sim_options, pf_energy, mfe_structure, fold_comp):
+def _score_with_compound(seq, input_file, sim_options, pf_energy, mfe_structure, fold_comp, dimer_comp=None):
     s = ScoreSeq(sequence=seq)
     s.get_Epf(pf_energy)
     s.get_mfe_ss(mfe_structure)
@@ -132,7 +133,7 @@ def _score_with_compound(seq, input_file, sim_options, pf_energy, mfe_structure,
         else:
             s.get_scoring_function_homomonomer(fold_comp)
     if sim_options.oligo_state == "avoid":
-        s.get_scoring_function_monomer()
+        s.get_scoring_function_monomer(dimer_comp)
 
     if sim_options.motifs:
         s.update_scoring_function_w_motifs(score_motifs(seq, sim_options))
@@ -179,7 +180,14 @@ def score_sequences(seqs, input_file, sim_options):
     structures = [f[1] for f in folded]
     if not dimer and sim_options.pks == "on":
         structures = get_pk_structs(structures, compounds)
-    return [_score_with_compound(seq, input_file, sim_options, f[0], ss, fc) for seq, f, ss, fc in zip(seqs, folded, structures, compounds)]
+    dimers = [None] * len(seqs)
+    if sim_options.oligo_state == "avoid":
+        # the self-dimers seq&seq of all mutants in one more engine call: partition function only, as get_scoring_function_monomer
+        # asks of each on its own
+        dimers = [RNA.fold_compound(s + "&" + s) for s in seqs]
+        RNA.fold_compound.prefetch(dimers, want=RNA._eng.WANT_PF)
+    return [_score_with_compound(seq, input_file, sim_options, f[0], ss, fc, dc)
+            for seq, f, ss, fc, dc in zip(seqs, folded, structures, compounds, dimers)]
 
 
 class ScoreSeq:
@@ -297,9 +305,11 @@ class ScoreSeq:
     def get_scoring_function_w_subopt(self):
         self.scoring_function = self.scoring_function - self.esubopt_minus_Epf
 
-    def get_scoring_function_monomer(self):
+    def get_scoring_function_monomer(self, fc=None):
+        """fc: the fold compound of sequence&sequence, if the caller folded it already (score_sequences)"""
         dimer = self.sequence + "&" + self.sequence
-        fc = RNA.fold_compound(dimer)
+        if fc is None:
+            fc = RNA.fold_compound(dimer)
         self.oligo_fraction = dme.oligo_fraction(dimer, fc)
         self.monomer_bonus = dme.kTlog_monomer_fraction(self.oligo_fraction)
         self.scoring_function = self.scoring_function + self.monomer_bonus

@@ -130,7 +130,7 @@ int bf_debug_copy_table(int which, int32_t n_seq, void *host, size_t host_bytes,
 /* ---------------------------------------------------------------------------------------------------------
  * Device-resident Replica-Exchange Monte-Carlo design loop: many design problems ("jobs") x replicas advance
  * in lock step with sequences, scores, temperature shelves and random streams resident in HBM.  Replaces,
- * for targets made of . ( ), one strand or two (heterodimer, homodimer):
+ * for targets made of . ( ), one strand (with or without avoiding self-dimers) or two (heterodimer, homodimer):
  *   remc.mutate_sequence_re / single_replica_design / mc_delta      utils/replica_exchange_monte_carlo.py:26-110,176-271
  *   remc.replica_exchange / replica_exchange_attempt                utils/replica_exchange_monte_carlo.py:80-173
  *   seq_utils.mutate_sequence / get_mutation_position / expand_cases  utils/sequence_utils.py:926-1136
@@ -155,7 +155,10 @@ typedef struct {
   int32_t acgu;            /* -acgu on: paired letters drawn with nt_weight */
   double nt_weight[4];     /* A C G U */
   int32_t oligo;           /* two-strand jobs: 1 heterodimer (-kT ln(dimer fraction)), 2 homodimer (strands kept identical;
-                              -kT ln(fraction) or, for identical target halves, -kT ln(1 - fraction))   energy_scores.py:120-125,421-441 */
+                              -kT ln(fraction) or, for identical target halves, -kT ln(1 - fraction))   energy_scores.py:120-125,421-441;
+                              one-strand jobs: 3 avoid (-o on): every mutant's self-dimer seq&seq is folded too (partition function
+                              only, default scale) and -kT ln(1 - fraction) of that dimer is added; BF_ERR_ARG with a two-strand job
+                                                                                                energy_scores.py:118-119,412-419 */
   uint64_t seed;
   /* optional scenario terms (all zero = absent) */
   const char *alt_targets;   /* n_jobs x max_alt x stride: alternative structures (input_file.alt_sec_structs), only . ( );
@@ -183,7 +186,8 @@ typedef struct {
 
 enum { BF_DESIGN_REC = 15 }; /* doubles per record: scoring_function, edesired, Epf, 1-mcc, 1-precision, 1-recall, MFE,
                                 ensemble_defect, positions whose partner differs from the target's (0 = solved), global step,
-                                oligo_fraction, oligomer_bonus, edesired2 (mean energy of the alternative structures), motif bonus, subopt_e */
+                                oligo_fraction, oligomer_bonus (avoid designs: the monomer bonus), edesired2 (mean energy of the
+                                alternative structures), motif bonus, subopt_e */
 
 /* Allocates the loop on the engine's GPU, scores the start sequences (global step 0). */
 int bf_design_create(const bf_design_t *cfg, void **handle);
