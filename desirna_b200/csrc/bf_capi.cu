@@ -25,6 +25,20 @@ int bf_opt(const char *name, int dflt) {
   return (v && *v) ? atoi(v) : dflt;
 }
 
+BfOpts bf_opts() {
+  BfOpts o;
+  o.wide = bf_opt("BF_WIDE", 1);
+  o.fill3 = bf_opt("BF_FILL3", 1);
+  o.fill3_small = bf_opt("BF_FILL3_SMALL", 1);
+  o.blk_min = bf_opt("BF_BLK_MIN", 280);
+  o.blk_min_pf = bf_opt("BF_BLK_MIN_PF", 250);
+  o.cl = bf_opt("BF_CL", -1);
+  o.cl_c = bf_opt("BF_CL_C", 0);
+  o.cl_bw = bf_opt("BF_CL_BW", 32);
+  o.ext_wide = bf_opt("BF_EXT_WIDE", -1);
+  return o;
+}
+
 namespace {
 
 struct DevBuf {
@@ -132,13 +146,6 @@ int validate(const bf_batch_t *b, const bf_result_t *r) {
   return BF_OK;
 }
 
-// exterior recursions by one CTA per sequence instead of one warp per sequence: batches that leave SMs idle (BF_EXT_WIDE=0/1 overrides)
-bool wide_ext(int B, int stride) {
-  const int v = bf_opt("BF_EXT_WIDE", -1);
-  if (v >= 0) return v != 0 && bf_ext_wide_ok(stride);
-  return B <= 2 * g.sm_count && bf_ext_wide_ok(stride);
-}
-
 // all pointers are device pointers
 // scale_override (device, B ints, dcal/mol): energies that set the partition function's per-nucleotide scale instead of this
 // call's own MFE.  The result does not depend on the scale beyond rounding, and without that dependency the partition function
@@ -148,7 +155,6 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
   if (b->B == 0) return BF_OK;
   BfBatchDev db;
   db.B = b->B; db.stride = b->stride; db.seq = b->seq; db.len = b->len; db.cut = b->cut; db.nopair = b->nopair;
-  const int wstride = b->stride + 2;
   if (&w == &g.w) g.last_stride = b->stride;
   if (scale_override) CU(cudaEventRecord(w.ev_fork, st), "fork");   // what the second stream has to wait for: the work before this call
   const int *mfe_for_scale = nullptr;
@@ -165,47 +171,34 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     g.launches++;
     eval_done = true;
   }
-  const bool fill_mfe = !two && !g.force_generic && bf_fill_mfe_mode(b->stride) != 0;
-  const bool fill_pf = !two && !g.force_generic && bf_fill_pf_mode(b->stride) != 0;
   if (b->want & (BF_WANT_MFE | BF_WANT_SS)) {
     int *out_mfe = r->mfe_dcal;
     if (!out_mfe) { CU(w.d_mfe_scratch.reserve((size_t)b->B * sizeof(int)), "cudaMalloc(mfe scratch)"); out_mfe = (int *)w.d_mfe_scratch.p; }
+    char *out_ss = (b->want & BF_WANT_SS) ? r->mfe_ss : nullptr;
+    BfPlan p;
+    CU(bf_plan_mfe(b->stride, b->B, two, g.force_generic, g.sm_count, &p), "plan the MFE fill");
     if (timing) cudaEventRecord(w.ev[0], st);
-    if (fill_mfe) {
+    if (p.family != BF_FAM_GENERIC) {
       const size_t slot = bf_tri_slot(b->stride) * sizeof(int);
       CU(w.tri_c.reserve((size_t)b->B * slot), "cudaMalloc(c table)");
       CU(w.tri_f.reserve((size_t)b->B * slot), "cudaMalloc(fML table)");
+      CU(w.ws_ring.reserve((size_t)p.grid * p.ws * sizeof(int)), "cudaMalloc(ring workspace)");
       int *f5 = nullptr;
-      const size_t wsi = bf_mfe_ws_slot(b->stride, b->B) * sizeof(int);
-      if (wsi) {
-        int grid = 0;
-        CU(bf_mfe_fill_grid(db, g.sm_count, &grid), "size bf_k_mfe_fill");
-        CU(w.ws_ring.reserve((size_t)grid * wsi), "cudaMalloc(ring workspace)");
-      }
-      if (bf_mfe_fill_does_ext(b->stride, b->B)) {
+      if (p.ext != BF_EXT_WARP) {
         CU(w.f5buf.reserve((size_t)b->B * (b->stride + 4) * sizeof(int)), "cudaMalloc(f5)");
         f5 = (int *)w.f5buf.p;
       }
-      CU(bf_launch_mfe_fill(g.dP, db, (int *)w.tri_c.p, (int *)w.tri_f.p, (int *)w.ws_ring.p, g.sm_count, w.d_counters + 0, st, f5),
-         "launch bf_k_mfe_fill");
-      if (!f5 && wide_ext(b->B, b->stride)) {   // few sequences: the exterior recursion by one CTA per sequence (bf_ext.cu)
-        CU(w.f5buf.reserve((size_t)b->B * (b->stride + 4) * sizeof(int)), "cudaMalloc(f5)");
-        f5 = (int *)w.f5buf.p;
+      CU(bf_launch_mfe_fill(p, g.dP, db, (int *)w.tri_c.p, (int *)w.tri_f.p, (int *)w.ws_ring.p, w.d_counters + 0,
+                            p.ext == BF_EXT_IN_FILL ? f5 : nullptr, st), "launch bf_k_mfe_fill");
+      if (p.ext == BF_EXT_CTA) {
         CU(bf_launch_f5_wide(g.dP, db, (const int *)w.tri_c.p, f5, st), "launch bf_k_f5_wide");
         g.launches++;
       }
-      CU(bf_launch_trace(g.dP, db, (const int *)w.tri_c.p, (const int *)w.tri_f.p, out_mfe, (b->want & BF_WANT_SS) ? r->mfe_ss : nullptr,
-                         b->stride + 1, st, f5), "launch bf_k_trace");
+      CU(bf_launch_trace(g.dP, db, (const int *)w.tri_c.p, (const int *)w.tri_f.p, out_mfe, out_ss, b->stride + 1, st, f5), "launch bf_k_trace");
       g.launches += 2;
     } else {
-      int occ = bf_occupancy_mfe(two, wstride);
-      int grid = std::min(b->B, g.sm_count * occ);
-      size_t slot = bf_mfe_slot_ints(wstride) * sizeof(int);
-      // keep the workspace within a sane share of HBM
-      while (grid > g.sm_count && (size_t)grid * slot > ((size_t)48 << 30)) grid -= g.sm_count;
-      CU(w.ws_mfe.reserve((size_t)grid * slot), "cudaMalloc(mfe workspace)");
-      CU(bf_launch_mfe(g.dP, db, two, (int *)w.ws_mfe.p, wstride, grid, w.d_counters + 0, out_mfe,
-                       (b->want & BF_WANT_SS) ? r->mfe_ss : nullptr, b->stride + 1, st), "launch bf_k_mfe");
+      CU(w.ws_mfe.reserve((size_t)p.grid * p.ws * sizeof(int)), "cudaMalloc(mfe workspace)");
+      CU(bf_launch_mfe(p, g.dP, db, (int *)w.ws_mfe.p, w.d_counters + 0, out_mfe, out_ss, b->stride + 1, st), "launch bf_k_mfe");
       g.launches++;
     }
     if (timing) cudaEventRecord(w.ev[1], st);
@@ -213,9 +206,11 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     mfe_for_scale = out_mfe;
   }
   const bool want_out = (b->want & (BF_WANT_BPP | BF_WANT_DEFECT)) != 0;
-  if (want_out && (two || !fill_pf))
-    return fail(BF_ERR_UNAVAILABLE, "base-pair probabilities / ensemble defect: single-strand sequences within the fill path's length range only");
   if ((b->want & BF_WANT_PF) || want_out) {
+    BfPlan p;
+    CU(bf_plan_pf(b->stride, b->B, two, g.force_generic, g.sm_count, &p), "plan the PF fill");
+    if (want_out && p.family == BF_FAM_GENERIC)
+      return fail(BF_ERR_UNAVAILABLE, "base-pair probabilities / ensemble defect: single-strand sequences within the fill path's length range only");
     BfBatchDev dbp = db;
     dbp.nopair = nullptr;  // hard constraints are added after fc.pf() in the reference (sequence_utils.py:1181)
     // a constrained MFE is not a bound on the unconstrained ensemble: only use it for scaling when unconstrained
@@ -224,47 +219,40 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     if (beside) CU(cudaStreamWaitEvent(sp, w.ev_fork, 0), "fork");
     const int *scale_src = beside ? scale_override : (b->nopair ? nullptr : mfe_for_scale);
     if (timing) cudaEventRecord(w.ev[2], sp);
-    if (fill_pf) {
+    if (p.family != BF_FAM_GENERIC) {
       const size_t slot = bf_tri_slot(b->stride) * sizeof(double);
       CU(w.tri_qb.reserve((size_t)b->B * slot), "cudaMalloc(qb table)");
       CU(w.d_lnscale.reserve((size_t)b->B * sizeof(double)), "cudaMalloc(lnscale)");
-      int grid = 0;
-      CU(bf_pf_fill_grid(dbp, g.sm_count, &grid), "size bf_k_pf_fill");
-      const size_t ws = bf_pf_ws_slot(b->stride, b->B) * sizeof(double);
-      if (ws) CU(w.ws_qm.reserve((size_t)grid * ws), "cudaMalloc(qm workspace)");
+      CU(w.ws_qm.reserve((size_t)p.grid * p.ws * sizeof(double)), "cudaMalloc(qm workspace)");
       double *qmseq = nullptr;
       if (want_out) {
         CU(w.qm_seq.reserve((size_t)b->B * 2 * slot), "cudaMalloc(per-sequence qm/qm1)");
         qmseq = (double *)w.qm_seq.p;
       }
-      CU(bf_launch_pf_fill(g.dP, dbp, (double *)w.tri_qb.p, (double *)w.ws_qm.p, qmseq, scale_src, (double *)w.d_lnscale.p, g.sm_count,
-                           w.d_counters + 1, sp, r->pf), "launch bf_k_pf_fill");
+      CU(bf_launch_pf_fill(p, g.dP, dbp, (double *)w.tri_qb.p, (double *)w.ws_qm.p, qmseq, scale_src, (double *)w.d_lnscale.p, w.d_counters + 1,
+                           p.ext == BF_EXT_IN_FILL ? r->pf : nullptr, sp), "launch bf_k_pf_fill");
       g.launches++;
-      if (!bf_pf_fill_does_ext(b->stride, b->B)) {
-        if (wide_ext(b->B, b->stride))
-          CU(bf_launch_q5_wide(g.dP, dbp, (const double *)w.tri_qb.p, (const double *)w.d_lnscale.p, r->pf, sp), "launch bf_k_q5_wide");
-        else
-          CU(bf_launch_pf_ext(g.dP, dbp, (const double *)w.tri_qb.p, (const double *)w.d_lnscale.p, r->pf, sp), "launch bf_k_pf_ext");
+      if (p.ext == BF_EXT_CTA) {
+        CU(bf_launch_q5_wide(g.dP, dbp, (const double *)w.tri_qb.p, (const double *)w.d_lnscale.p, r->pf, sp), "launch bf_k_q5_wide");
+        g.launches++;
+      } else if (p.ext == BF_EXT_WARP) {
+        CU(bf_launch_pf_ext(g.dP, dbp, (const double *)w.tri_qb.p, (const double *)w.d_lnscale.p, r->pf, sp), "launch bf_k_pf_ext");
         g.launches++;
       }
       if (want_out) {
-        int ogrid = 0;
-        CU(bf_out_grid(dbp, g.sm_count, &ogrid), "size bf_k_pf_out");
-        CU(w.ws_out.reserve((size_t)ogrid * bf_out_ws_slot(b->stride) * sizeof(double)), "cudaMalloc(outside workspace)");
+        BfPlan po;
+        CU(bf_plan_out(b->stride, b->B, g.sm_count, &po), "plan bf_k_pf_out");
+        CU(w.ws_out.reserve((size_t)po.grid * po.ws * sizeof(double)), "cudaMalloc(outside workspace)");
         if (b->want & BF_WANT_BPP) CU(cudaMemsetAsync(r->bpp, 0, (size_t)b->B * b->stride * b->stride * sizeof(double), st), "clear bpp");
-        CU(bf_launch_pf_out(g.dP, dbp, (const double *)w.tri_qb.p, qmseq, (double *)w.ws_out.p, (const double *)w.d_lnscale.p,
+        CU(bf_launch_pf_out(po, g.dP, dbp, (const double *)w.tri_qb.p, qmseq, (double *)w.ws_out.p, (const double *)w.d_lnscale.p,
                             (b->want & BF_WANT_DEFECT) ? b->targets : nullptr, b->n_targets, b->stride,
-                            (b->want & BF_WANT_DEFECT) ? r->defect : nullptr, (b->want & BF_WANT_BPP) ? r->bpp : nullptr, ogrid,
+                            (b->want & BF_WANT_DEFECT) ? r->defect : nullptr, (b->want & BF_WANT_BPP) ? r->bpp : nullptr,
                             w.d_counters + 2, st), "launch bf_k_pf_out");
         g.launches++;
       }
     } else {
-      int occ = bf_occupancy_pf(two, wstride);
-      int grid = std::min(b->B, g.sm_count * occ);
-      size_t slot = bf_pf_slot_doubles(wstride) * sizeof(double);
-      while (grid > g.sm_count && (size_t)grid * slot > ((size_t)64 << 30)) grid -= g.sm_count;
-      CU(w.ws_pf.reserve((size_t)grid * slot), "cudaMalloc(pf workspace)");
-      CU(bf_launch_pf(g.dP, dbp, two, (double *)w.ws_pf.p, wstride, grid, w.d_counters + 1, scale_src, r->pf, sp), "launch bf_k_pf");
+      CU(w.ws_pf.reserve((size_t)p.grid * p.ws * sizeof(double)), "cudaMalloc(pf workspace)");
+      CU(bf_launch_pf(p, g.dP, dbp, (double *)w.ws_pf.p, w.d_counters + 1, scale_src, r->pf, sp), "launch bf_k_pf");
       g.launches++;
     }
     if (timing) cudaEventRecord(w.ev[3], sp);
@@ -335,7 +323,6 @@ int bf_init(int device) {
   g.device = device;
   g.force_generic = bf_opt("BF_FORCE_GENERIC", 0) == 1;
   g.sm_count = prop.multiProcessorCount;
-  bf_fill_set_sms(g.sm_count);
   CU(cudaStreamCreateWithFlags(&g.stream, cudaStreamNonBlocking), "cudaStreamCreate");
   CU(g.w.create(), "create engine workspace");
   CU(bf_upload_constants(), "upload candidate table");

@@ -821,8 +821,6 @@ __global__ void __launch_bounds__(NW * 32, 1) bf_k_pf_cl(const BfParams *__restr
   cl_sync();
 }
 
-constexpr size_t kSmemBudgetCl = 232448 - 1024 - 256;
-
 int ilog2(int x) { int l = 0; while ((1 << l) < x) l++; return l; }
 
 bool make_geom(int nmax, int C, int BW, int elem_banks /*32: int, 16: double*/, ClGeom *out) {
@@ -854,7 +852,7 @@ int max_active_clusters(K kern, int C) {
   memset(&cfg, 0, sizeof cfg);
   cfg.gridDim = dim3((unsigned)(C * 64), 1, 1);
   cfg.blockDim = dim3(kNWcl * 32, 1, 1);
-  cfg.dynamicSmemBytes = kSmemBudgetCl;
+  cfg.dynamicSmemBytes = kSmemBudget;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
@@ -865,7 +863,7 @@ int max_active_clusters(K kern, int C) {
 }
 template <class K>
 cudaError_t cl_attrs(K kern) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudgetCl);
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
   if (e != cudaSuccess) return e;
   return cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
 }
@@ -893,13 +891,12 @@ const ClSlots &cl_slots(ClSlots &s, K kern) {
 int mfe_rounds_allowed(int nmax) { return nmax < 130 ? 0 : nmax < 230 ? 1 : nmax < 330 ? 2 : 3; }
 int pf_rounds_allowed(int nmax) { return nmax < 130 ? 0 : nmax < 180 ? 1 : nmax < 230 ? 2 : nmax < 350 ? 3 : 5; }
 
+// cforce: BF_CL_C (0: the rule's choice), bw: BF_CL_BW
 struct ClCfg { bool ok, dflt; int slots; ClGeom g; MfeClPlan pl; };
-ClCfg mfe_cl_cfg(int nmax, int B) {
+ClCfg mfe_cl_cfg(int nmax, int B, int cforce, int bw) {
   ClCfg c;
   c.ok = c.dflt = false; c.slots = 0;
   if (nmax < 1 || nmax > 2000) return c;
-  const int cforce = bf_opt("BF_CL_C", 0);
-  const int bw = bf_opt("BF_CL_BW", 32);
   if (bw != 16 && bw != 32) return c;
   const ClSlots &sl = cl_slots(g_slots_mfe, bf_k_mfe_cl<kNWcl, kNTcl>);
   int best_rounds = 1 << 30;
@@ -909,7 +906,7 @@ ClCfg mfe_cl_cfg(int nmax, int B) {
     if (!make_geom(nmax, C, bw, 32, &t.g)) continue;
     t.pl = mfe_cl_plan(nmax, t.g);
     t.slots = sl.n[t.g.logC];
-    if (t.pl.total > kSmemBudgetCl || t.slots < 1) continue;
+    if (t.pl.total > kSmemBudget || t.slots < 1) continue;
     const int rounds = ((B > 0 ? B : 1) + t.slots - 1) / t.slots;
     if (rounds < best_rounds) { best_rounds = rounds; c = t; c.ok = true; }   // ties: the smaller cluster (leaves SMs to the other stream)
   }
@@ -918,12 +915,10 @@ ClCfg mfe_cl_cfg(int nmax, int B) {
 }
 
 struct PfClCfg { bool ok, dflt; int slots; ClGeom g; PfClPlan pl; };
-PfClCfg pf_cl_cfg(int nmax, int B) {
+PfClCfg pf_cl_cfg(int nmax, int B, int cforce, int bw) {
   PfClCfg c;
   c.ok = c.dflt = false; c.slots = 0;
   if (nmax < 1 || nmax > 2000) return c;
-  const int cforce = bf_opt("BF_CL_C", 0);
-  const int bw = bf_opt("BF_CL_BW", 32);
   if (bw != 16 && bw != 32) return c;
   const ClSlots &sl = cl_slots(g_slots_pf, bf_k_pf_cl<kNWcl, kNTcl>);
   int best_rounds = 1 << 30;
@@ -933,7 +928,7 @@ PfClCfg pf_cl_cfg(int nmax, int B) {
     if (!make_geom(nmax, C, bw, 16, &t.g)) continue;
     t.pl = pf_cl_plan(nmax, t.g);
     t.slots = sl.n[t.g.logC];
-    if (t.pl.total > kSmemBudgetCl || t.slots < 1) continue;
+    if (t.pl.total > kSmemBudget || t.slots < 1) continue;
     const int rounds = ((B > 0 ? B : 1) + t.slots - 1) / t.slots;
     if (rounds < best_rounds) { best_rounds = rounds; c = t; c.ok = true; }
   }
@@ -959,70 +954,53 @@ cudaError_t cl_launch(K kern, int nclusters, int C, unsigned smem, cudaStream_t 
 }  // namespace
 
 // The cluster kernels take a batch when asked to (BF_CL=1, wherever they cover the length) or, by default, when the batch fits in
-// few rounds of the clusters in flight (see *_rounds_allowed); BF_CL=0 switches them off.
-bool bf_cl_mfe_use(int nmax, int B) {
-  const int m = bf_opt("BF_CL", -1);
-  if (m == 0) return false;
-  const ClCfg c = mfe_cl_cfg(nmax, B);
-  return c.ok && (m == 1 || c.dflt);
-}
-int bf_cl_mfe_csize(int nmax, int B) { const ClCfg c = mfe_cl_cfg(nmax, B); return c.ok ? c.g.C : 0; }
-size_t bf_cl_mfe_ws_slot(int nmax, int B) {   // ints per CLUSTER: entries of the pairable cells, one slab per CTA
-  const ClCfg c = mfe_cl_cfg(nmax, B);
-  if (!c.ok) return 0;
-  return (size_t)c.g.C * (((size_t)nmax * c.g.ncl * kEntW + 7) / 8 * 8);
-}
-cudaError_t bf_cl_mfe_grid(const BfBatchDev &b, int sms, int *grid) {
-  const ClCfg c = mfe_cl_cfg(b.stride, b.B);
-  if (!c.ok) return cudaErrorInvalidValue;
-  *grid = b.B < c.slots ? b.B : c.slots;
-  return cudaSuccess;
+// few rounds of the clusters in flight (see *_rounds_allowed); BF_CL=0 switches them off.  A plan is one cluster per sequence, as
+// many as run at once; its workspace is one slab of cell entries per CTA.
+bool bf_cl_mfe_plan(int nmax, int B, const BfOpts &o, BfPlan *p) {
+  if (o.cl == 0 || B <= 0) return false;
+  const ClCfg c = mfe_cl_cfg(nmax, B, o.cl_c, o.cl_bw);
+  if (!c.ok || !(o.cl == 1 || c.dflt)) return false;
+  p->family = BF_FAM_CLUSTER;
+  p->key = c.g.C;
+  p->bw = c.g.BW;
+  p->grid = B < c.slots ? B : c.slots;
+  p->smem = c.pl.total;
+  p->ws = (size_t)c.g.C * (((size_t)nmax * c.g.ncl * kEntW + 7) / 8 * 8);   // ints
+  return true;
 }
 
-cudaError_t bf_launch_mfe_cl(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *work_counter, cudaStream_t st) {
-  const ClCfg c = mfe_cl_cfg(b.stride, b.B);
-  if (!c.ok) return cudaErrorInvalidValue;
-  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
-  if (e != cudaSuccess) return e;
+cudaError_t bf_launch_mfe_cl(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int *work_counter,
+                             cudaStream_t st) {
+  ClGeom g;
+  make_geom(b.stride, p.key, p.bw, 32, &g);
   const uint32_t *taps = nullptr;
-  e = taps_device(c.g.RS, 32, &taps);
+  cudaError_t e = taps_device(g.RS, 32, &taps);
   if (e != cudaSuccess) return e;
-  const int ncluster = b.B < c.slots ? b.B : c.slots;
-  const size_t tri_slot = bf_tri_slot(b.stride), ent_slot = bf_cl_mfe_ws_slot(b.stride, b.B);
-  return cl_launch(bf_k_mfe_cl<kNWcl, kNTcl>, ncluster, c.g.C, c.pl.total, st, dP, b, ctri, ftri, tri_slot, ws, ent_slot, taps, c.pl, c.g,
-                   work_counter);
+  return cl_launch(bf_k_mfe_cl<kNWcl, kNTcl>, p.grid, g.C, (unsigned)p.smem, st, dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, p.ws, taps,
+                   mfe_cl_plan(b.stride, g), g, work_counter);
 }
 
 // ---------------------------------------------------------------------------------------------------- partition function
-bool bf_cl_pf_use(int nmax, int B) {
-  const int m = bf_opt("BF_CL", -1);
-  if (m == 0) return false;
-  const PfClCfg c = pf_cl_cfg(nmax, B);
-  return c.ok && (m == 1 || c.dflt);
+bool bf_cl_pf_plan(int nmax, int B, const BfOpts &o, BfPlan *p) {
+  if (o.cl == 0 || B <= 0) return false;
+  const PfClCfg c = pf_cl_cfg(nmax, B, o.cl_c, o.cl_bw);
+  if (!c.ok || !(o.cl == 1 || c.dflt)) return false;
+  p->family = BF_FAM_CLUSTER;
+  p->key = c.g.C;
+  p->bw = c.g.BW;
+  p->grid = B < c.slots ? B : c.slots;
+  p->smem = c.pl.total;
+  p->ws = (size_t)c.g.C * (((size_t)nmax * c.g.ncl * kEntDc + 7) / 8 * 8);   // doubles
+  return true;
 }
-int bf_cl_pf_csize(int nmax, int B) { const PfClCfg c = pf_cl_cfg(nmax, B); return c.ok ? c.g.C : 0; }
-size_t bf_cl_pf_ws_slot(int nmax, int B) {   // doubles per CLUSTER
-  const PfClCfg c = pf_cl_cfg(nmax, B);
-  if (!c.ok) return 0;
-  return (size_t)c.g.C * (((size_t)nmax * c.g.ncl * kEntDc + 7) / 8 * 8);
-}
-cudaError_t bf_cl_pf_grid(const BfBatchDev &b, int sms, int *grid) {
-  const PfClCfg c = pf_cl_cfg(b.stride, b.B);
-  if (!c.ok) return cudaErrorInvalidValue;
-  *grid = b.B < c.slots ? b.B : c.slots;
-  return cudaSuccess;
-}
-cudaError_t bf_launch_pf_cl(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                            double *lnscale, int sms, int *work_counter, cudaStream_t st) {
-  const PfClCfg c = pf_cl_cfg(b.stride, b.B);
-  if (!c.ok) return cudaErrorInvalidValue;
-  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
-  if (e != cudaSuccess) return e;
+
+cudaError_t bf_launch_pf_cl(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq,
+                            const int *mfe_for_scale, double *lnscale, int *work_counter, cudaStream_t st) {
+  ClGeom g;
+  make_geom(b.stride, p.key, p.bw, 16, &g);
   const uint32_t *taps = nullptr;
-  e = taps_device(c.g.RS, 16, &taps);
+  cudaError_t e = taps_device(g.RS, 16, &taps);
   if (e != cudaSuccess) return e;
-  const int ncluster = b.B < c.slots ? b.B : c.slots;
-  const size_t tri_slot = bf_tri_slot(b.stride), ent_slot = bf_cl_pf_ws_slot(b.stride, b.B);
-  return cl_launch(bf_k_pf_cl<kNWcl, kNTcl>, ncluster, c.g.C, c.pl.total, st, dP, b, qbtri, tri_slot, ws, ent_slot, qmseq, mfe_for_scale, lnscale,
-                   taps, c.pl, c.g, work_counter);
+  return cl_launch(bf_k_pf_cl<kNWcl, kNTcl>, p.grid, g.C, (unsigned)p.smem, st, dP, b, qbtri, bf_tri_slot(b.stride), ws, p.ws, qmseq,
+                   mfe_for_scale, lnscale, taps, pf_cl_plan(b.stride, g), g, work_counter);
 }

@@ -29,6 +29,13 @@ struct BfBatchDev {
   const uint8_t *nopair;    // B x stride or null; 1 = position may not pair ('x' hard constraint)
 };
 
+// Packed triangular DP table of one sequence, stored by anti-diagonal: entry (i,j), d = j-i >= 4, at tri_off(n, d) + i-1.
+BF_HD int tri_off(int n, int d) { return (d - 4) * n - (d * (d - 1) / 2 - 6); }
+BF_HD size_t tri_size(int n) { return n >= 5 ? (size_t)tri_off(n, n) : 0; }
+
+// dynamic shared memory a fold kernel's CTA may ask for: the 227 KB of sm_100 less its static tables and a reserve
+constexpr size_t kSmemBudget = 232448 - 1024 - 256;
+
 // per-sequence fold context held in shared memory
 struct BfCtx {
   int n, cp, W;

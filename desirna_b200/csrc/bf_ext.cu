@@ -18,8 +18,6 @@
 
 namespace {
 
-__host__ __device__ __forceinline__ int tri_off(int n, int d) { return (d - 4) * n - (d * (d - 1) / 2 - 6); }
-
 constexpr int kExtNW = 8;
 
 // tile row stride: even (so that consecutive lanes, which sit one row and one column apart, hit different banks)

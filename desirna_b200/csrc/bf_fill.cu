@@ -36,12 +36,6 @@ namespace {
 constexpr int kRing = 32;
 constexpr int kInfThr = BF_INF / 2;
 
-__host__ __device__ __forceinline__ int tri_off(int n, int d) {
-  // first entry of diagonal d (d >= 4)
-  return (d - 4) * n - (d * (d - 1) / 2 - 6);
-}
-__host__ __device__ __forceinline__ size_t tri_size(int n) { return n >= 5 ? (size_t)tri_off(n, n) : 0; }
-
 __device__ __forceinline__ size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // tile-major copy of a triangular table (blocked split): 4x4 tiles, tile (I,J) at tile_off(NT,I) + J-I, entry a*4+b
@@ -1249,7 +1243,18 @@ cudaError_t set_smem(K kern, size_t sm) {
   return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sm > 1024 ? sm : 1024));
 }
 
-constexpr size_t kSmemBudget = 232448 - 1024 - 256;  // dynamic budget per CTA (static tables + reserve taken off)
+// first-fit occupancy grid of a persistent kernel: every sequence its CTA, at most what the GPU runs at once
+template <typename K>
+cudaError_t occ_grid(K kern, int threads, size_t sm, int B, int sms, int *grid) {
+  cudaError_t e = set_smem(kern, sm);
+  if (e != cudaSuccess) return e;
+  int occ = 0;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, sm);
+  if (e != cudaSuccess) return e;
+  if (occ < 1) return cudaErrorInvalidConfiguration;
+  *grid = B < sms * occ ? B : sms * occ;
+  return cudaSuccess;
+}
 
 }  // namespace
 
@@ -1263,14 +1268,12 @@ struct FillCfg { int nw, pl; };
 
 // Small batches (a replica-exchange sub-step: B = replicas x targets, often far fewer sequences than the 148 x 2..3 CTA slots):
 // what matters is the latency of ONE sequence, so a CTA gets 16 warps instead of 8 when every sequence still gets its own SM.
-static int g_fill_sms = 148;
-void bf_fill_set_sms(int sms) { if (sms > 0) g_fill_sms = sms; }
-static bool want_wide(int B) { return B > 0 && B <= g_fill_sms && bf_opt("BF_WIDE", 1) != 0; }
+static bool want_wide(int B, int sms, const BfOpts &o) { return B > 0 && B <= sms && o.wide != 0; }
 
 static bool mfe_fits(int nmax, int nw, int pl) { return mfe_plan(nmax, nw, pl).total <= kSmemBudget; }
 static bool pf_fits(int nmax, int nw, int pl) { return pf_plan(nmax, nw, pl).total <= kSmemBudget; }
 
-static bool mfe_blk(int nmax, const FillCfg &c);
+static bool mfe_blk(int nmax, const FillCfg &c, int blk_min);
 // shared partial buffers (atomicMin) where they buy occupancy: CTAs per SM by shared memory, capped by the register limit (4 x 256 threads)
 static bool mfe_atom(int nmax, const FillCfg &c, bool blk) {
   auto occ = [&](bool atom) {
@@ -1281,14 +1284,15 @@ static bool mfe_atom(int nmax, const FillCfg &c, bool blk) {
   };
   return occ(true) > occ(false);
 }
-static FillCfg mfe_cfg(int nmax, int B = 0) {
-  if (want_wide(B))   // same placement rule, 16 warps
+// blk_min: BF_BLK_MIN (read only when wide)
+static FillCfg mfe_cfg(int nmax, bool wide, int blk_min) {
+  if (wide)   // same placement rule, 16 warps
     // one CTA per SM: nothing is gained by a small footprint, and with nothing else resident L2 latency is fully exposed --
     // keep on chip whatever fits (fML table + rings, else the rings), shared partial buffers if that is what makes it fit
     for (int pl : {kMfeFmSmem | kMfeRgSmem, kMfeRgSmem, 0}) {
       const FillCfg w{16, pl};
-      if (pl != 0 && nmax >= bf_opt("BF_BLK_MIN", 280)) continue;   // blocked split: the through-L2 layout measured faster (L=400)
-      if (mfe_plan(nmax, 16, pl, mfe_blk(nmax, w), true).total <= kSmemBudget) return w;
+      if (pl != 0 && nmax >= blk_min) continue;   // blocked split: the through-L2 layout measured faster (L=400)
+      if (mfe_plan(nmax, 16, pl, mfe_blk(nmax, w, blk_min), true).total <= kSmemBudget) return w;
     }
   // default (tuning sweep, profiles/r01_sweeps.md): rings on chip while >= 3 CTAs still fit on an SM (70 KB), else everything
   // through L2
@@ -1296,13 +1300,13 @@ static FillCfg mfe_cfg(int nmax, int B = 0) {
   if (mfe_fits(nmax, 8, pl)) return {8, pl};
   return {8, mfe_fits(nmax, 8, 0) ? 0 : -1};
 }
-static bool pf_blk(int nmax, const FillCfg &c);
+static bool pf_blk(int nmax, const FillCfg &c, int blk_min_pf);
 static bool pf_half(int nmax, const FillCfg &c);
-static FillCfg pf_cfg(int nmax, int B = 0) {
-  if (want_wide(B))   // as for the MFE: one CTA per SM, keep on chip what fits (qm/qm1 + generic ring, else the ring)
+static FillCfg pf_cfg(int nmax, bool wide, int blk_min_pf) {
+  if (wide)   // as for the MFE: one CTA per SM, keep on chip what fits (qm/qm1 + generic ring, else the ring)
     for (int pl : {kPfQmSmem | kPfQgSmem, kPfQgSmem, 0}) {
       const FillCfg w{16, pl};
-      if (pl != 0 && nmax >= bf_opt("BF_BLK_MIN_PF", 250)) continue;   // blocked split: through-L2 layout only
+      if (pl != 0 && nmax >= blk_min_pf) continue;   // blocked split: through-L2 layout only
       if (pf_plan(nmax, 16, pl, pf_half(nmax, w)).total <= kSmemBudget) return w;
     }
   const int pl = pf_plan(nmax, 8, kPfQgSmem).total <= 74 * 1024 ? kPfQgSmem : 0;
@@ -1312,121 +1316,139 @@ static FillCfg pf_cfg(int nmax, int B = 0) {
 
 // blocked split (tile-major mirror + block products): for the two default placements.  It pays once the split operands no longer
 // fit on chip (measured: L=100 3.86 -> 5.18 ms, L=200 16.1 -> 17.8 ms, L=400 143 -> 117 ms): long sequences only
-static bool mfe_blk(int nmax, const FillCfg &c) {
-  return (c.pl == 0 || c.pl == kMfeRgSmem) && nmax >= bf_opt("BF_BLK_MIN", 280) && mfe_plan(nmax, c.nw, c.pl, true).total <= kSmemBudget;
+static bool mfe_blk(int nmax, const FillCfg &c, int blk_min) {
+  return (c.pl == 0 || c.pl == kMfeRgSmem) && nmax >= blk_min && mfe_plan(nmax, c.nw, c.pl, true).total <= kSmemBudget;
 }
-
-// 0: length not covered by the fill path (the generic kernels take it); else 1 + placement flags
-int bf_fill_mfe_mode(int nmax) {
-  if (nmax < 1 || nmax > 2000) return 0;
-  return mfe_cfg(nmax).pl + 1;
-}
-int bf_fill_pf_mode(int nmax) {
-  if (nmax < 1 || nmax > 2000) return 0;
-  return pf_cfg(nmax).pl + 1;
-}
-// third-generation kernels (bf_fill3.cu) take every batch they cover; small batches (want_wide) get their 16-warp variants, and the
-// 16-warp round-1 kernels of this file only what those do not cover (BF_FILL3_SMALL=0: as before round 2's last session)
-// cluster-per-sequence kernels (bf_cluster.cu): small batches of long sequences (rule in bf_cluster.cu; BF_CL=0/1 overrides)
-static bool use_cl_mfe(int nmax, int B) { return B > 0 && bf_cl_mfe_use(nmax, B); }
-static bool small3(int B) { return want_wide(B) && bf_opt("BF_FILL3_SMALL", 1) != 0; }
-static bool use_fill3_mfe(int nmax, int B) { return !use_cl_mfe(nmax, B) && (!want_wide(B) || small3(B)) && bf_fill3_mfe_ok(nmax, small3(B)); }
-static bool use_cl_pf(int nmax, int B) { return B > 0 && bf_cl_pf_use(nmax, B); }
-static bool use_fill3_pf(int nmax, int B) { return !use_cl_pf(nmax, B) && (!want_wide(B) || small3(B)) && bf_fill3_pf_ok(nmax, small3(B)); }
-
-size_t bf_mfe_ws_slot(int nmax, int B) {  // ints of per-CTA HBM workspace: [rings when they are not on chip][tile-major fML mirror when blocked]
-  if (use_cl_mfe(nmax, B)) return bf_cl_mfe_ws_slot(nmax, B);
-  if (use_fill3_mfe(nmax, B)) return bf_fill3_mfe_ws_slot(nmax);
-  const FillCfg c = mfe_cfg(nmax, B);
-  if (c.pl < 0) return 0;
-  size_t o = 0;
-  if (!(c.pl & kMfeRgSmem)) o += ((size_t)3 * kRing * mfe_plan(nmax, c.nw, c.pl).rs + 7) / 8 * 8;
-  if (mfe_blk(nmax, c)) o += (tile_table_entries(nmax) + 7) / 8 * 8;
-  return o;
-}
-static bool pf_blk(int nmax, const FillCfg &c) { return c.pl == 0 && nmax >= bf_opt("BF_BLK_MIN_PF", 250); }
+static bool pf_blk(int nmax, const FillCfg &c, int blk_min_pf) { return c.pl == 0 && nmax >= blk_min_pf; }
 static bool pf_half(int nmax, const FillCfg &c) {
   // long sequences: with one partial buffer per warp only one CTA fits an SM; sharing buffers between warp pairs fits two
   if (c.nw == 16)   // one CTA per SM: share buffers between warp pairs only when the full set does not fit
     return c.pl == 0 && pf_plan(nmax, 16, 0, false).total > kSmemBudget;
   return c.pl == 0 && pf_plan(nmax, 8, 0, false).total > 113 * 1024 && pf_plan(nmax, 8, 0, true).total <= 113 * 1024;
 }
-size_t bf_pf_ws_slot(int nmax, int B) {  // doubles of per-CTA HBM workspace: [tables that are not on chip][blocked split: qm/qm1 mirrors, sums]
-  if (use_cl_pf(nmax, B)) return bf_cl_pf_ws_slot(nmax, B);
-  if (use_fill3_pf(nmax, B)) return bf_fill3_pf_ws_slot(nmax);
-  const FillCfg c = pf_cfg(nmax, B);
-  if (c.pl < 0) return 0;
-  size_t o = pf_ws_doubles(nmax, c.pl);
-  if (pf_blk(nmax, c)) o += 2 * ((tile_table_entries(nmax) + 7) / 8 * 8) + (size_t)3 * ((nmax + 3) / 4) * 16;
-  return (o + 7) / 8 * 8;
+
+// 0: length not covered by the fill path (the generic kernels take it); else 1 + placement flags.  Decided by the 8-warp
+// configuration, which does not depend on the batch.
+int bf_fill_mfe_mode(int nmax) {
+  if (nmax < 1 || nmax > 2000) return 0;
+  return mfe_cfg(nmax, false, 0).pl + 1;
+}
+int bf_fill_pf_mode(int nmax) {
+  if (nmax < 1 || nmax > 2000) return 0;
+  return pf_cfg(nmax, false, 0).pl + 1;
 }
 
-static int *g_f5_out = nullptr;   // where a 16-warp fill leaves f5 (set around the launch by bf_launch_mfe_fill)
-template <int NW, int PL, bool BLK = false, bool ATOM = false>
-static cudaError_t mfe_fill_t(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *grid_out, bool launch,
-                              int *counter, cudaStream_t st) {
-  auto kern = bf_k_mfe_fill<NW, PL, BLK, ATOM>;
-  const size_t sm = mfe_plan(b.stride, NW, PL, BLK, ATOM).total;
-  cudaError_t e = set_smem(kern, sm);
-  if (e != cudaSuccess) return e;
-  int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, sm);
-  if (e != cudaSuccess) return e;
-  if (occ < 1) return cudaErrorInvalidConfiguration;
-  const int grid = b.B < sms * occ ? b.B : sms * occ;
-  if (grid_out) *grid_out = grid;
-  if (!launch) return cudaSuccess;
-  kern<<<grid, NW * 32, sm, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, bf_mfe_ws_slot(b.stride, b.B), counter, NW == 16 ? g_f5_out : nullptr);
-  return cudaGetLastError();
-}
+// ---- the round-1 instantiations, exactly the combinations the rules above return
+using MfeFillK = void (*)(const BfParams *, BfBatchDev, int *, int *, size_t, int *, size_t, int *, int *);
+struct MfeFillVar { MfeFillK kern; int nw, pl; bool blk, atom; };
+#define BF_V(NW_, PL_, BLK_, ATOM_) {bf_k_mfe_fill<NW_, PL_, BLK_, ATOM_>, NW_, PL_, BLK_, ATOM_}
+static const MfeFillVar kMfeVars[] = {
+    BF_V(8, 0, false, false), BF_V(8, 0, false, true), BF_V(8, 0, true, false), BF_V(8, 0, true, true),
+    BF_V(8, kMfeRgSmem, false, false), BF_V(8, kMfeRgSmem, false, true), BF_V(8, kMfeRgSmem, true, false), BF_V(8, kMfeRgSmem, true, true),
+    BF_V(16, 0, false, true), BF_V(16, 0, true, false), BF_V(16, 0, true, true),
+    BF_V(16, kMfeRgSmem, false, false), BF_V(16, kMfeRgSmem, false, true),
+    BF_V(16, kMfeFmSmem | kMfeRgSmem, false, false), BF_V(16, kMfeFmSmem | kMfeRgSmem, false, true)};
+#undef BF_V
 
-static cudaError_t mfe_fill_dispatch(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *grid_out,
-                                     bool launch, int *counter, cudaStream_t st) {
-  const FillCfg c = mfe_cfg(b.stride, b.B);
+using PfFillK = void (*)(const BfParams *, BfBatchDev, double *, size_t, double *, size_t, double *, const int *, double *, int *, double *);
+struct PfFillVar { PfFillK kern; int nw, pl; bool half, blk; int minb; };
+#define BF_V(NW_, PL_, HALF_, BLK_, MINB_) {bf_k_pf_fill<NW_, PL_, HALF_, BLK_, MINB_>, NW_, PL_, HALF_, BLK_, MINB_}
+static const PfFillVar kPfVars[] = {
+    BF_V(16, kPfQmSmem | kPfQgSmem, false, false, 0), BF_V(16, kPfQgSmem, false, false, 0),
+    BF_V(16, 0, true, true, 0), BF_V(16, 0, true, false, 0), BF_V(16, 0, false, true, 0), BF_V(16, 0, false, false, 0),
+    BF_V(8, kPfQgSmem, false, false, 0), BF_V(8, 0, true, true, 0), BF_V(8, 0, true, false, 0), BF_V(8, 0, false, true, 0),
+    BF_V(8, 0, false, false, 4), BF_V(8, 0, false, false, 3), BF_V(8, 0, false, false, 0)};
+#undef BF_V
+
+static cudaError_t round1_mfe_plan(int nmax, int B, bool wide, const BfOpts &o, int sms, BfPlan *p) {
+  const FillCfg c = mfe_cfg(nmax, wide, o.blk_min);
   if (c.pl < 0) return cudaErrorInvalidValue;
-  const bool blk = mfe_blk(b.stride, c), atom = mfe_atom(b.stride, c, blk);
-#define BF_MFE_GO(NW_, PL_, BLK_, ATOM_) return mfe_fill_t<NW_, PL_, BLK_, ATOM_>(dP, b, ctri, ftri, ws, sms, grid_out, launch, counter, st)
-  if (c.pl == (kMfeFmSmem | kMfeRgSmem)) {   // 16 warps only, never blocked
-    if (atom) BF_MFE_GO(16, kMfeFmSmem | kMfeRgSmem, false, true);
-    BF_MFE_GO(16, kMfeFmSmem | kMfeRgSmem, false, false);
-  }
-  // the combinations the rules above return
-  switch ((c.nw == 16 ? 8 : 0) | (c.pl == 0 ? 0 : 4) | (blk ? 2 : 0) | (atom ? 1 : 0)) {
-    case 0: BF_MFE_GO(8, 0, false, false);
-    case 1: BF_MFE_GO(8, 0, false, true);
-    case 2: BF_MFE_GO(8, 0, true, false);
-    case 3: BF_MFE_GO(8, 0, true, true);
-    case 4: BF_MFE_GO(8, kMfeRgSmem, false, false);
-    case 5: BF_MFE_GO(8, kMfeRgSmem, false, true);
-    case 6: BF_MFE_GO(8, kMfeRgSmem, true, false);
-    case 7: BF_MFE_GO(8, kMfeRgSmem, true, true);
-    case 9: BF_MFE_GO(16, 0, false, true);
-    case 10: BF_MFE_GO(16, 0, true, false);
-    case 11: BF_MFE_GO(16, 0, true, true);
-    case 12: BF_MFE_GO(16, kMfeRgSmem, false, false);
-    case 13: BF_MFE_GO(16, kMfeRgSmem, false, true);
-  }
-#undef BF_MFE_GO
-  return cudaErrorInvalidValue;
+  const bool blk = mfe_blk(nmax, c, o.blk_min), atom = mfe_atom(nmax, c, blk);
+  int key = 0;
+  while (key < (int)(sizeof kMfeVars / sizeof kMfeVars[0]) &&
+         !(kMfeVars[key].nw == c.nw && kMfeVars[key].pl == c.pl && kMfeVars[key].blk == blk && kMfeVars[key].atom == atom)) key++;
+  if (key == (int)(sizeof kMfeVars / sizeof kMfeVars[0])) return cudaErrorInvalidValue;
+  p->family = BF_FAM_ROUND1;
+  p->key = key;
+  p->smem = mfe_plan(nmax, c.nw, c.pl, blk, atom).total;
+  // [rings when they are not on chip][tile-major fML mirror when blocked]
+  p->ws = 0;
+  if (!(c.pl & kMfeRgSmem)) p->ws += ((size_t)3 * kRing * mfe_plan(nmax, c.nw, c.pl).rs + 7) / 8 * 8;
+  if (blk) p->ws += (tile_table_entries(nmax) + 7) / 8 * 8;
+  return occ_grid(kMfeVars[key].kern, c.nw * 32, p->smem, B, sms, &p->grid);
 }
-cudaError_t bf_mfe_fill_grid(const BfBatchDev &b, int sms, int *grid) {
-  if (use_cl_mfe(b.stride, b.B)) return bf_cl_mfe_grid(b, sms, grid);
-  if (use_fill3_mfe(b.stride, b.B)) return bf_fill3_mfe_grid(b, sms, grid, small3(b.B));
-  return mfe_fill_dispatch(nullptr, b, nullptr, nullptr, nullptr, sms, grid, false, nullptr, nullptr);
-}
-// true: the fill kernel chosen for this batch also runs the exterior recursion and leaves f5 (B x (stride + 4) ints) for bf_k_trace
-bool bf_mfe_fill_does_ext(int nmax, int B) { return !use_cl_mfe(nmax, B) && !use_fill3_mfe(nmax, B) && mfe_cfg(nmax, B).nw == 16; }
 
-cudaError_t bf_launch_mfe_fill(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *work_counter,
-                               cudaStream_t st, int *f5_out) {
-  if (use_cl_mfe(b.stride, b.B)) return bf_launch_mfe_cl(dP, b, ctri, ftri, ws, sms, work_counter, st);
-  if (use_fill3_mfe(b.stride, b.B)) return bf_launch_mfe_fill3(dP, b, ctri, ftri, ws, sms, work_counter, st, small3(b.B));
+static cudaError_t round1_pf_plan(int nmax, int B, bool wide, const BfOpts &o, int sms, BfPlan *p) {
+  const FillCfg c = pf_cfg(nmax, wide, o.blk_min_pf);
+  if (c.pl < 0) return cudaErrorInvalidValue;
+  const bool half = pf_half(nmax, c), blk = pf_blk(nmax, c, o.blk_min_pf);
+  // everything through L2: occupancy is a register question.  Measured (profiles/r01_s4_sweep_pf_minb.log): 4 CTAs per SM pay up
+  // to ~135 nt, 3 up to ~185 nt; beyond, the tables of more sequences in flight no longer fit in L2 and the 2-CTA build wins
+  const int minb = c.nw == 8 && c.pl == 0 && !half && !blk ? (nmax <= 135 ? 4 : nmax <= 185 ? 3 : 0) : 0;
+  int key = 0;
+  while (key < (int)(sizeof kPfVars / sizeof kPfVars[0]) &&
+         !(kPfVars[key].nw == c.nw && kPfVars[key].pl == c.pl && kPfVars[key].half == half && kPfVars[key].blk == blk && kPfVars[key].minb == minb)) key++;
+  if (key == (int)(sizeof kPfVars / sizeof kPfVars[0])) return cudaErrorInvalidValue;
+  p->family = BF_FAM_ROUND1;
+  p->key = key;
+  p->smem = pf_plan(nmax, c.nw, c.pl, half).total;
+  // [tables that are not on chip][blocked split: qm/qm1 mirrors, sums]
+  size_t ws = pf_ws_doubles(nmax, c.pl);
+  if (blk) ws += 2 * ((tile_table_entries(nmax) + 7) / 8 * 8) + (size_t)3 * ((nmax + 3) / 4) * 16;
+  p->ws = (ws + 7) / 8 * 8;
+  return occ_grid(kPfVars[key].kern, c.nw * 32, p->smem, B, sms, &p->grid);
+}
+
+// exterior recursion of a fill that does not run it itself: one CTA per sequence for batches that leave SMs idle (BF_EXT_WIDE=0/1
+// overrides), else one warp per sequence
+static BfExtRoute ext_route(int stride, int B, int sms, const BfOpts &o) {
+  const bool cta = (o.ext_wide >= 0 ? o.ext_wide != 0 : B <= 2 * sms) && bf_ext_wide_ok(stride);
+  return cta ? BF_EXT_CTA : BF_EXT_WARP;
+}
+
+// The route of a fold pass: the generic kernels for two strands, BF_FORCE_GENERIC and lengths the fill path does not cover; else the
+// cluster kernels (rule in bf_cluster.cu; BF_CL=0/1 overrides), then the third-generation kernels (bf_fill3.cu), which take every
+// batch they cover -- small batches (want_wide) their 16-warp variants unless BF_FILL3_SMALL=0 --, then the round-1 kernels of this
+// file.
+cudaError_t bf_plan_mfe(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p) {
+  const BfOpts o = bf_opts();
+  *p = BfPlan{};
+  if (two || force_generic || bf_fill_mfe_mode(stride) == 0) return bf_gen_mfe_plan(stride, B, two, o, sms, p);
+  const bool wide = want_wide(B, sms, o), small = wide && o.fill3_small != 0;
+  cudaError_t e = cudaSuccess;
+  if (!bf_cl_mfe_plan(stride, B, o, p)) {
+    if (!wide || small) e = bf_fill3_mfe_plan(stride, B, small, o, sms, p);
+    if (e == cudaSuccess && p->family != BF_FAM_TAP) e = round1_mfe_plan(stride, B, wide, o, sms, p);
+  }
+  const bool in_fill = p->family == BF_FAM_ROUND1 && kMfeVars[p->key].nw == 16;
+  p->ext = in_fill ? BF_EXT_IN_FILL : ext_route(stride, B, sms, o);
+  return e;
+}
+
+cudaError_t bf_plan_pf(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p) {
+  const BfOpts o = bf_opts();
+  *p = BfPlan{};
+  if (two || force_generic || bf_fill_pf_mode(stride) == 0) return bf_gen_pf_plan(stride, B, two, o, sms, p);
+  const bool wide = want_wide(B, sms, o), small = wide && o.fill3_small != 0;
+  cudaError_t e = cudaSuccess;
+  if (!bf_cl_pf_plan(stride, B, o, p)) {
+    if (!wide || small) e = bf_fill3_pf_plan(stride, B, small, o, sms, p);
+    if (e == cudaSuccess && p->family != BF_FAM_TAP) e = round1_pf_plan(stride, B, wide, o, sms, p);
+  }
+  const bool in_fill = p->family == BF_FAM_ROUND1 && kPfVars[p->key].nw == 16;
+  p->ext = in_fill ? BF_EXT_IN_FILL : ext_route(stride, B, sms, o);
+  return e;
+}
+
+cudaError_t bf_launch_mfe_fill(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int *work_counter,
+                               int *f5_out, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
-  g_f5_out = f5_out;
-  e = mfe_fill_dispatch(dP, b, ctri, ftri, ws, sms, nullptr, true, work_counter, st);
-  g_f5_out = nullptr;
-  return e;
+  if (p.family == BF_FAM_CLUSTER) return bf_launch_mfe_cl(p, dP, b, ctri, ftri, ws, work_counter, st);
+  if (p.family == BF_FAM_TAP) return bf_launch_mfe_fill3(p, dP, b, ctri, ftri, ws, work_counter, st);
+  const MfeFillVar &v = kMfeVars[p.key];
+  v.kern<<<p.grid, v.nw * 32, p.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, p.ws, work_counter, f5_out);
+  return cudaGetLastError();
 }
 
 cudaError_t bf_launch_trace(const BfParams *dP, const BfBatchDev &b, const int *ctri, const int *ftri, int *out_mfe, char *out_ss,
@@ -1439,70 +1461,15 @@ cudaError_t bf_launch_trace(const BfParams *dP, const BfBatchDev &b, const int *
   return cudaGetLastError();
 }
 
-static double *g_pf_out5 = nullptr;   // where a 16-warp fill leaves the ensemble energies (set around the launch by bf_launch_pf_fill)
-template <int NW, int PL, bool HALF = false, bool BLK = false, int MINB = 0>
-static cudaError_t pf_fill_t(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale, double *lnscale,
-                             int sms, int *grid_out, bool launch, int *counter, cudaStream_t st) {
-  auto kern = bf_k_pf_fill<NW, PL, HALF, BLK, MINB>;
-  const size_t sm = pf_plan(b.stride, NW, PL, HALF).total;
-  cudaError_t e = set_smem(kern, sm);
-  if (e != cudaSuccess) return e;
-  int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, sm);
-  if (e != cudaSuccess) return e;
-  if (occ < 1) return cudaErrorInvalidConfiguration;
-  const int grid = b.B < sms * occ ? b.B : sms * occ;
-  if (grid_out) *grid_out = grid;
-  if (!launch) return cudaSuccess;
-  kern<<<grid, NW * 32, sm, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), ws, bf_pf_ws_slot(b.stride, b.B), qmseq, mfe_for_scale, lnscale, counter, NW == 16 ? g_pf_out5 : nullptr);
-  return cudaGetLastError();
-}
-static cudaError_t pf_fill_dispatch(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                                    double *lnscale, int sms, int *grid_out, bool launch, int *counter, cudaStream_t st) {
-  const FillCfg c = pf_cfg(b.stride, b.B);
-  if (c.pl < 0) return cudaErrorInvalidValue;
-  const bool half = pf_half(b.stride, c), blk = pf_blk(b.stride, c);
-#define BF_PF_GO(...) return pf_fill_t<__VA_ARGS__>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, grid_out, launch, counter, st)
-  if (c.nw == 16) {
-    if (c.pl == (kPfQmSmem | kPfQgSmem)) BF_PF_GO(16, kPfQmSmem | kPfQgSmem);
-    if (c.pl == kPfQgSmem) BF_PF_GO(16, kPfQgSmem);
-    if (half && blk) BF_PF_GO(16, 0, true, true);
-    if (half) BF_PF_GO(16, 0, true, false);
-    if (blk) BF_PF_GO(16, 0, false, true);
-    BF_PF_GO(16, 0);
-  }
-  if (c.pl == kPfQgSmem) BF_PF_GO(8, kPfQgSmem);
-  if (half && blk) BF_PF_GO(8, 0, true, true);
-  if (half) BF_PF_GO(8, 0, true, false);
-  if (blk) BF_PF_GO(8, 0, false, true);
-  // everything through L2: occupancy is a register question.  Measured (profiles/r01_s4_sweep_pf_minb.log): 4 CTAs per SM pay up
-  // to ~135 nt, 3 up to ~185 nt; beyond, the tables of more sequences in flight no longer fit in L2 and the 2-CTA build wins
-  if (b.stride <= 135) BF_PF_GO(8, 0, false, false, 4);
-  if (b.stride <= 185) BF_PF_GO(8, 0, false, false, 3);
-  BF_PF_GO(8, 0);
-#undef BF_PF_GO
-}
-
-// grid size the fill will use (the caller sizes the per-CTA workspace with it)
-cudaError_t bf_pf_fill_grid(const BfBatchDev &b, int sms, int *grid) {
-  if (use_cl_pf(b.stride, b.B)) return bf_cl_pf_grid(b, sms, grid);
-  if (use_fill3_pf(b.stride, b.B)) return bf_fill3_pf_grid(b, sms, grid, small3(b.B));
-  return pf_fill_dispatch(nullptr, b, nullptr, nullptr, nullptr, nullptr, nullptr, sms, grid, false, nullptr, nullptr);
-}
-
-// true: the fill kernel chosen for this batch also runs the exterior recursion and writes out5 (no bf_launch_pf_ext needed)
-bool bf_pf_fill_does_ext(int nmax, int B) { return !use_cl_pf(nmax, B) && !use_fill3_pf(nmax, B) && pf_cfg(nmax, B).nw == 16; }
-
-cudaError_t bf_launch_pf_fill(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *qmws, double *qmseq, const int *mfe_for_scale,
-                              double *lnscale, int sms, int *work_counter, cudaStream_t st, double *out5) {
-  if (use_cl_pf(b.stride, b.B)) return bf_launch_pf_cl(dP, b, qbtri, qmws, qmseq, mfe_for_scale, lnscale, sms, work_counter, st);
-  if (use_fill3_pf(b.stride, b.B)) return bf_launch_pf_fill3(dP, b, qbtri, qmws, qmseq, mfe_for_scale, lnscale, sms, work_counter, st, small3(b.B));
+cudaError_t bf_launch_pf_fill(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, double *qbtri, double *qmws, double *qmseq,
+                              const int *mfe_for_scale, double *lnscale, int *work_counter, double *out5, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
-  g_pf_out5 = out5;
-  e = pf_fill_dispatch(dP, b, qbtri, qmws, qmseq, mfe_for_scale, lnscale, sms, nullptr, true, work_counter, st);
-  g_pf_out5 = nullptr;
-  return e;
+  if (p.family == BF_FAM_CLUSTER) return bf_launch_pf_cl(p, dP, b, qbtri, qmws, qmseq, mfe_for_scale, lnscale, work_counter, st);
+  if (p.family == BF_FAM_TAP) return bf_launch_pf_fill3(p, dP, b, qbtri, qmws, qmseq, mfe_for_scale, lnscale, work_counter, st);
+  const PfFillVar &v = kPfVars[p.key];
+  v.kern<<<p.grid, v.nw * 32, p.smem, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), qmws, p.ws, qmseq, mfe_for_scale, lnscale, work_counter, out5);
+  return cudaGetLastError();
 }
 
 cudaError_t bf_launch_pf_ext(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *lnscale, double *out5,

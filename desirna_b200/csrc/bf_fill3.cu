@@ -804,16 +804,14 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 2 : 1) bf_k_pf_fill3(const 
   }
 }
 
-constexpr size_t kSmemBudget = 232448 - 1024 - 256;
-
 struct Mfe3Cfg { bool ok; int rs; size_t smem; };
 // small: a batch that leaves SMs idle (a replica-exchange sub-step) -- one 16-warp CTA (12 tap + 4 auxiliary warps) per sequence with the
 // whole shared memory of its SM; measured against the 16-warp round-1 kernels at B = 64 (profiles/r02_small_batch_fill3.txt): 36 nt 0.089 ->
 // 0.076 ms, 100 nt 0.340 -> 0.257, 148 nt 0.678 -> 0.427, 200 nt 1.07 -> 0.66, as long as the fML table fits on chip (~230 nt)
-Mfe3Cfg mfe3_cfg(int nmax, bool small) {
+Mfe3Cfg mfe3_cfg(int nmax, bool small, int fill3) {
   Mfe3Cfg c;
   c.ok = false;
-  if (nmax < 1 || bf_opt("BF_FILL3", 1) == 0) return c;
+  if (nmax < 1 || fill3 == 0) return c;
   c.rs = pick_rs(nmax, 32);
   // 8 warps: 6 tap + 2 auxiliary.  The fML table has to be on chip: with two auxiliary warps per CTA the split cannot hide L2
   // latency (measured: L = 120 7.8 ms per 4096 folds against 5.96 ms of the round-1 kernel, L = 200 33 against 16).  Three CTAs
@@ -823,65 +821,11 @@ Mfe3Cfg mfe3_cfg(int nmax, bool small) {
   return c;
 }
 
-}  // namespace
-
-bool bf_fill3_mfe_ok(int nmax, bool small) { return mfe3_cfg(nmax, small).ok; }
-size_t bf_fill3_mfe_ws_slot(int nmax) { return 2 * ((tri_size(nmax) * kEntWords + 7) / 8 * 8); }   // ints per CTA: entries of every cell, two sequences
-
-template <int NW, int NWI>
-static cudaError_t mfe3_launch(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, const Mfe3Cfg &c, int sms, int *counter,
-                               cudaStream_t st, int *grid_out) {
-  auto kern = bf_k_mfe_fill3<NW, NWI>;
-  static int occ_cache[4096];   // per stride: CTAs per SM (0 = not asked yet); the attribute is set once per instance
-  static bool attr_set = false;
-  cudaError_t e;
-  if (!attr_set) {
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
-    if (e != cudaSuccess) return e;
-    attr_set = true;
-  }
-  int occ_tmp = 0;
-  int &occ = b.stride < 4096 ? occ_cache[b.stride] : occ_tmp;
-  if (occ == 0) {
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, c.smem);
-    if (e != cudaSuccess) return e;
-    if (occ < 1) return cudaErrorInvalidConfiguration;
-  }
-  const int grid = b.B < sms * occ ? b.B : sms * occ;
-  if (grid_out) { *grid_out = grid; return cudaSuccess; }
-  const uint32_t *taps = nullptr;
-  e = taps_device(c.rs, 32, &taps);
-  if (e != cudaSuccess) return e;
-  kern<<<grid, NW * 32, c.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, bf_fill3_mfe_ws_slot(b.stride), taps, c.rs, counter);
-  return cudaGetLastError();
-}
-
-static cudaError_t mfe3_dispatch(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *work_counter,
-                                 cudaStream_t st, int *grid_out, bool small) {
-  const Mfe3Cfg c = mfe3_cfg(b.stride, small);
-  if (!c.ok) return cudaErrorInvalidValue;
-  if (small) return mfe3_launch<16, 12>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out);
-  return mfe3_launch<8, 6>(dP, b, ctri, ftri, ws, c, sms, work_counter, st, grid_out);
-}
-
-cudaError_t bf_fill3_mfe_grid(const BfBatchDev &b, int sms, int *grid, bool small) {
-  return mfe3_dispatch(nullptr, b, nullptr, nullptr, nullptr, sms, nullptr, nullptr, grid, small);
-}
-
-cudaError_t bf_launch_mfe_fill3(const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int sms, int *work_counter,
-                                cudaStream_t st, bool small) {
-  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
-  if (e != cudaSuccess) return e;
-  return mfe3_dispatch(dP, b, ctri, ftri, ws, sms, work_counter, st, nullptr, small);
-}
-
-// ---------------------------------------------------------------------------------------------------- partition function, host side
-namespace {
 struct Pf3Cfg { bool ok; int rs; bool qms, pair; size_t smem; int nw, nwi; };
-Pf3Cfg pf3_cfg(int nmax, bool small) {
+Pf3Cfg pf3_cfg(int nmax, bool small, int fill3) {
   Pf3Cfg c;
   c.ok = false;
-  if (nmax < 1 || bf_opt("BF_FILL3", 1) == 0) return c;
+  if (nmax < 1 || fill3 == 0) return c;
   c.rs = pick_rs(nmax, 16);
   // One CTA of 16 warps (12 tap + 4 auxiliary) per SM with qm / qm1 on chip while they fit (~105 nt), through L2 beyond.  Measured
   // at L = 100 (4096 folds): 16 warps on chip 5.01 ms, 12 warps with paired cells 5.13, two CTAs of 8 warps (qm / qm1 in L2) 5.14;
@@ -902,62 +846,89 @@ Pf3Cfg pf3_cfg(int nmax, bool small) {
   c.ok = c.smem <= kSmemBudget && nmax <= (small ? 230 : 150);
   return c;
 }
-}  // namespace
 
-bool bf_fill3_pf_ok(int nmax, bool small) { return pf3_cfg(nmax, small).ok; }
-size_t bf_fill3_pf_ws_slot(int nmax) {   // doubles per CTA: entries of every cell, qm and qm1
-  const size_t tri_pad = (tri_size(nmax) + 7) / 8 * 8;
-  return tri_pad * kEntD + 2 * tri_pad;
-}
+// The instantiations the rules return, each with its occupancy per stride (0 = not asked yet) and whether its shared-memory
+// attribute is set: asked once per instance.
+template <typename K>
+struct Fill3Inst {
+  K kern;
+  int nw, nwi;
+  bool qms, pair;
+  int occ_cache[4096];
+  bool attr_set;
+};
+using Mfe3K = void (*)(const BfParams *, BfBatchDev, int *, int *, size_t, int *, size_t, const uint32_t *, int, int *);
+using Pf3K = void (*)(const BfParams *, BfBatchDev, double *, size_t, double *, size_t, double *, const int *, double *, const uint32_t *, int, int *);
+Fill3Inst<Mfe3K> g_mfe3[] = {{bf_k_mfe_fill3<8, 6>, 8, 6, false, false, {}, false}, {bf_k_mfe_fill3<16, 12>, 16, 12, false, false, {}, false}};
+#define BF_I(NW_, NWI_, QMSM_, PAIR_) {bf_k_pf_fill3<NW_, NWI_, QMSM_, PAIR_>, NW_, NWI_, QMSM_, PAIR_, {}, false}
+Fill3Inst<Pf3K> g_pf3[] = {BF_I(8, 6, false, false), BF_I(16, 12, true, false), BF_I(16, 12, true, true), BF_I(16, 12, false, true),
+                           BF_I(16, 10, false, true)};
+#undef BF_I
 
-template <int NW, int NWI, bool QMSM, bool PAIR = false>
-static cudaError_t pf3_launch(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                              double *lnscale, const Pf3Cfg &c, int sms, int *counter, cudaStream_t st, int *grid_out) {
-  auto kern = bf_k_pf_fill3<NW, NWI, QMSM, PAIR>;
-  static int occ_cache[4096];
-  static bool attr_set = false;
+template <typename K>
+cudaError_t fill3_grid(Fill3Inst<K> &k, int stride, size_t smem, int B, int sms, int *grid) {
   cudaError_t e;
-  if (!attr_set) {
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
+  if (!k.attr_set) {
+    e = cudaFuncSetAttribute(k.kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
     if (e != cudaSuccess) return e;
-    attr_set = true;
+    k.attr_set = true;
   }
   int occ_tmp = 0;
-  int &occ = b.stride < 4096 ? occ_cache[b.stride] : occ_tmp;
+  int &occ = stride < 4096 ? k.occ_cache[stride] : occ_tmp;
   if (occ == 0) {
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, c.smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k.kern, k.nw * 32, smem);
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
   }
-  const int grid = b.B < sms * occ ? b.B : sms * occ;
-  if (grid_out) { *grid_out = grid; return cudaSuccess; }
+  *grid = B < sms * occ ? B : sms * occ;
+  return cudaSuccess;
+}
+
+}  // namespace
+
+cudaError_t bf_fill3_mfe_plan(int nmax, int B, bool small, const BfOpts &o, int sms, BfPlan *p) {
+  const Mfe3Cfg c = mfe3_cfg(nmax, small, o.fill3);
+  if (!c.ok) return cudaSuccess;
+  p->family = BF_FAM_TAP;
+  p->key = small ? 1 : 0;
+  p->smem = c.smem;
+  p->ws = 2 * ((tri_size(nmax) * kEntWords + 7) / 8 * 8);   // ints per CTA: entries of every cell, two sequences
+  return fill3_grid(g_mfe3[p->key], nmax, c.smem, B, sms, &p->grid);
+}
+
+cudaError_t bf_launch_mfe_fill3(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, int *ctri, int *ftri, int *ws, int *work_counter,
+                                cudaStream_t st) {
+  const int rs = pick_rs(b.stride, 32);
   const uint32_t *taps = nullptr;
-  e = taps_device(c.rs, 16, &taps);
+  cudaError_t e = taps_device(rs, 32, &taps);
   if (e != cudaSuccess) return e;
-  kern<<<grid, NW * 32, c.smem, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), ws, bf_fill3_pf_ws_slot(b.stride), qmseq, mfe_for_scale, lnscale,
-                                      taps, c.rs, counter);
+  const Fill3Inst<Mfe3K> &k = g_mfe3[p.key];
+  k.kern<<<p.grid, k.nw * 32, p.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, p.ws, taps, rs, work_counter);
   return cudaGetLastError();
 }
 
-static cudaError_t pf3_dispatch(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                                double *lnscale, int sms, int *counter, cudaStream_t st, int *grid_out, bool small) {
-  const Pf3Cfg c = pf3_cfg(b.stride, small);
-  if (!c.ok) return cudaErrorInvalidValue;
-#define BF_GO(NW_, NWI_, QMSM_, PAIR_)                                                                                                \
-  if (c.nw == NW_ && c.nwi == NWI_ && c.qms == QMSM_ && c.pair == PAIR_)                                                             \
-    return pf3_launch<NW_, NWI_, QMSM_, PAIR_>(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, c, sms, counter, st, grid_out)
-  BF_GO(8, 6, false, false); BF_GO(16, 12, true, false); BF_GO(16, 12, true, true); BF_GO(16, 12, false, true); BF_GO(16, 10, false, true);
-#undef BF_GO
-  return cudaErrorInvalidValue;
+cudaError_t bf_fill3_pf_plan(int nmax, int B, bool small, const BfOpts &o, int sms, BfPlan *p) {
+  const Pf3Cfg c = pf3_cfg(nmax, small, o.fill3);
+  if (!c.ok) return cudaSuccess;
+  const int n = (int)(sizeof g_pf3 / sizeof g_pf3[0]);
+  int key = 0;
+  while (key < n && !(g_pf3[key].nw == c.nw && g_pf3[key].nwi == c.nwi && g_pf3[key].qms == c.qms && g_pf3[key].pair == c.pair)) key++;
+  if (key == n) return cudaErrorInvalidValue;
+  p->family = BF_FAM_TAP;
+  p->key = key;
+  p->smem = c.smem;
+  const size_t tri_pad = (tri_size(nmax) + 7) / 8 * 8;
+  p->ws = tri_pad * kEntD + 2 * tri_pad;   // doubles per CTA: entries of every cell, qm and qm1
+  return fill3_grid(g_pf3[key], nmax, c.smem, B, sms, &p->grid);
 }
 
-cudaError_t bf_fill3_pf_grid(const BfBatchDev &b, int sms, int *grid, bool small) {
-  return pf3_dispatch(nullptr, b, nullptr, nullptr, nullptr, nullptr, nullptr, sms, nullptr, nullptr, grid, small);
-}
-
-cudaError_t bf_launch_pf_fill3(const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq, const int *mfe_for_scale,
-                               double *lnscale, int sms, int *work_counter, cudaStream_t st, bool small) {
-  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
+cudaError_t bf_launch_pf_fill3(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, double *qbtri, double *ws, double *qmseq,
+                               const int *mfe_for_scale, double *lnscale, int *work_counter, cudaStream_t st) {
+  const int rs = pick_rs(b.stride, 16);
+  const uint32_t *taps = nullptr;
+  cudaError_t e = taps_device(rs, 16, &taps);
   if (e != cudaSuccess) return e;
-  return pf3_dispatch(dP, b, qbtri, ws, qmseq, mfe_for_scale, lnscale, sms, work_counter, st, nullptr, small);
+  const Fill3Inst<Pf3K> &k = g_pf3[p.key];
+  k.kern<<<p.grid, k.nw * 32, p.smem, st>>>(dP, b, qbtri, bf_tri_slot(b.stride), ws, p.ws, qmseq, mfe_for_scale, lnscale, taps, rs, work_counter);
+  return cudaGetLastError();
 }

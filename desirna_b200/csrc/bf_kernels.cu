@@ -14,6 +14,7 @@
 // Recurrences: SURVEY.md A.4 (fill), A.5 (backtrack order), A.6 (inside), A.7 (two strands), A.8 (eval).
 #include "bf_kernels.h"
 
+#include <algorithm>
 #include <cstdlib>
 #include <type_traits>
 
@@ -1230,17 +1231,13 @@ cudaError_t bf_upload_constants() {
   return e;
 }
 
-size_t bf_mfe_slot_ints(int wstride) { return (size_t)6 * wstride * wstride; }      // c, fML, fML^T + the three inner-term variants of c
-size_t bf_pf_slot_doubles(int wstride) { return (size_t)6 * wstride * wstride; }   // qb, qm, qm1^T + the three variants of qb
+static size_t bf_mfe_slot_ints(int wstride) { return (size_t)6 * wstride * wstride; }      // c, fML, fML^T + the three inner-term variants of c
+static size_t bf_pf_slot_doubles(int wstride) { return (size_t)6 * wstride * wstride; }   // qb, qm, qm1^T + the three variants of qb
 
 // The generic kernels (two strands; any length the fill path does not cover) keep three W x W tables per CTA.  Short sequences --
 // the reference's two-strand examples are 17 & 18 nt -- fit in shared memory next to the per-sequence arrays, which takes the L2
 // round trip out of every table access.  Capped so that at least two CTAs share an SM.
-static bool gen_wide(int B) {
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return B > 0 && B <= sms && bf_opt("BF_WIDE", 1) != 0;
-}
+static bool gen_wide(int B, int sms, const BfOpts &o) { return B > 0 && B <= sms && o.wide != 0; }
 // the two-barrier variants: batches that leave SMs idle, i.e. latency matters (measured: 17 & 18 nt x 64 MFE 0.164 -> 0.150 ms, but
 // 50 & 50 nt x 4096 16.7 -> 25.5 ms)
 static bool gen_pre(int wstride, bool wide) { return wide && wstride - 2 <= kPreMax; }
@@ -1281,28 +1278,62 @@ static PfKernel pf_kernel_p(bool two, bool wide) {
 static MfeKernel mfe_kernel(bool two, bool wide, bool pre) { return pre ? mfe_kernel_p<true>(two, wide) : mfe_kernel_p<false>(two, wide); }
 static PfKernel pf_kernel(bool two, bool wide, bool pre) { return pre ? pf_kernel_p<true>(two, wide) : pf_kernel_p<false>(two, wide); }
 
-cudaError_t bf_launch_mfe(const BfParams *dP, const BfBatchDev &b, bool two, int *ws, int wstride, int grid, int *work_counter,
-                          int *out_mfe, char *out_ss, int ss_stride, cudaStream_t st) {
+// CTAs per SM of the 8-warp build: what sizes the grid of a large batch (1 when the query fails)
+template <typename K>
+static int gen_occupancy(K kern, size_t sm) {
+  int nb = 0;
+  if (sm > kOptIn) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, BF_THREADS, sm) != cudaSuccess) return 1;
+  return nb < 1 ? 1 : nb;
+}
+
+// key: two | wide << 1 | pre << 2.  A warp per cell: with few sequences (a CTA owns its SM) 16 warps per CTA halve the rounds per
+// diagonal.  The grid keeps the per-CTA workspace within a sane share of HBM (48 GB MFE, 64 GB PF).
+cudaError_t bf_gen_mfe_plan(int stride, int B, bool two, const BfOpts &o, int sms, BfPlan *p) {
+  const int wstride = stride + 2;
+  const bool wide = gen_wide(B, sms, o), pre = gen_pre(wstride, wide);
+  p->family = BF_FAM_GENERIC;
+  p->key = (two ? 1 : 0) | (wide ? 2 : 0) | (pre ? 4 : 0);
+  p->smem = mfe_smem_total(wstride, pre);
+  p->tables_off = mfe_tables_off(wstride, pre);
+  p->ws = bf_mfe_slot_ints(wstride);
+  p->grid = std::min(B, sms * gen_occupancy(mfe_kernel(two, false, false), mfe_smem_total(wstride, false)));
+  while (p->grid > sms && (size_t)p->grid * p->ws * sizeof(int) > ((size_t)48 << 30)) p->grid -= sms;
+  return cudaSuccess;
+}
+
+cudaError_t bf_gen_pf_plan(int stride, int B, bool two, const BfOpts &o, int sms, BfPlan *p) {
+  const int wstride = stride + 2;
+  const bool wide = gen_wide(B, sms, o), pre = gen_pre(wstride, wide);
+  p->family = BF_FAM_GENERIC;
+  p->key = (two ? 1 : 0) | (wide ? 2 : 0) | (pre ? 4 : 0);
+  p->smem = pf_smem_total(wstride, pre);
+  p->tables_off = pf_tables_off(wstride, pre);
+  p->ws = bf_pf_slot_doubles(wstride);
+  p->grid = std::min(B, sms * gen_occupancy(pf_kernel(two, false, false), pf_smem_total(wstride, false)));
+  while (p->grid > sms && (size_t)p->grid * p->ws * sizeof(double) > ((size_t)64 << 30)) p->grid -= sms;
+  return cudaSuccess;
+}
+
+cudaError_t bf_launch_mfe(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, int *ws, int *work_counter, int *out_mfe, char *out_ss,
+                          int ss_stride, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
-  // a warp per cell: with few sequences (a CTA owns its SM) 16 warps per CTA halve the rounds per diagonal
-  const bool wide = gen_wide(b.B), pre = gen_pre(wstride, wide);
-  const size_t sm = mfe_smem_total(wstride, pre);
-  auto kern = mfe_kernel(two, wide, pre);
-  if (sm > kOptIn) { e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); if (e != cudaSuccess) return e; }
-  kern<<<grid, (wide ? 16 : BF_WARPS) * 32, sm, st>>>(dP, b, ws, bf_mfe_slot_ints(wstride), wstride, work_counter, out_mfe, out_ss, ss_stride, mfe_tables_off(wstride, pre));
+  const bool wide = p.key & 2;
+  auto kern = mfe_kernel(p.key & 1, wide, p.key & 4);
+  if (p.smem > kOptIn) { e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem); if (e != cudaSuccess) return e; }
+  kern<<<p.grid, (wide ? 16 : BF_WARPS) * 32, p.smem, st>>>(dP, b, ws, p.ws, b.stride + 2, work_counter, out_mfe, out_ss, ss_stride, p.tables_off);
   return cudaGetLastError();
 }
 
-cudaError_t bf_launch_pf(const BfParams *dP, const BfBatchDev &b, bool two, double *ws, int wstride, int grid, int *work_counter,
-                         const int *mfe_for_scale, double *out5, cudaStream_t st) {
+cudaError_t bf_launch_pf(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, double *ws, int *work_counter, const int *mfe_for_scale,
+                         double *out5, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
-  const bool wide = gen_wide(b.B), pre = gen_pre(wstride, wide);
-  const size_t sm = pf_smem_total(wstride, pre);
-  auto kern = pf_kernel(two, wide, pre);
-  if (sm > kOptIn) { e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); if (e != cudaSuccess) return e; }
-  kern<<<grid, (wide ? 16 : BF_WARPS) * 32, sm, st>>>(dP, b, ws, bf_pf_slot_doubles(wstride), wstride, work_counter, mfe_for_scale, out5, pf_tables_off(wstride, pre));
+  const bool wide = p.key & 2;
+  auto kern = pf_kernel(p.key & 1, wide, p.key & 4);
+  if (p.smem > kOptIn) { e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem); if (e != cudaSuccess) return e; }
+  kern<<<p.grid, (wide ? 16 : BF_WARPS) * 32, p.smem, st>>>(dP, b, ws, p.ws, b.stride + 2, work_counter, mfe_for_scale, out5, p.tables_off);
   return cudaGetLastError();
 }
 
@@ -1313,21 +1344,4 @@ cudaError_t bf_launch_eval(const BfParams *dP, const BfBatchDev &b, const char *
   if (sm > kOptIn) { cudaError_t e = cudaFuncSetAttribute(bf_k_eval, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); if (e != cudaSuccess) return e; }
   bf_k_eval<<<b.B * n_targets, 128, sm, st>>>(dP, b, targets, n_targets, tstride, out_e);
   return cudaGetLastError();
-}
-
-int bf_occupancy_mfe(bool two, int wstride) {   // of the 8-warp kernels: what sizes the grid of a large batch
-  int nb = 0;
-  auto kern = mfe_kernel(two, false, false);
-  const size_t sm = mfe_smem_total(wstride, false);
-  if (sm > kOptIn) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, BF_THREADS, sm) != cudaSuccess) return 1;
-  return nb < 1 ? 1 : nb;
-}
-int bf_occupancy_pf(bool two, int wstride) {
-  int nb = 0;
-  auto kern = pf_kernel(two, false, false);
-  const size_t sm = pf_smem_total(wstride, false);
-  if (sm > kOptIn) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, BF_THREADS, sm) != cudaSuccess) return 1;
-  return nb < 1 ? 1 : nb;
 }

@@ -19,9 +19,6 @@
 
 namespace {
 
-__host__ __device__ __forceinline__ int tri_off(int n, int d) { return (d - 4) * n - (d * (d - 1) / 2 - 6); }
-__host__ __device__ __forceinline__ size_t tri_size(int n) { return n >= 5 ? (size_t)tri_off(n, n) : 0; }
-
 struct OutPlan {
   int rs;
   size_t o_wg, o_wb, o_w1, o_scl, o_q5, o_q3, o_prow, o_ppair, o_ap, o_bqm, o_bqm1, o_g, o_toff, o_pt, o_stk, o_S, total;
@@ -588,79 +585,62 @@ __global__ void __launch_bounds__(NW * 32) bf_k_pf_out2(const BfParams *__restri
 // ---- host side: v2 whenever its plan fits the CTA's shared memory (generic ring on chip when that still leaves two CTAs per
 // SM), else the first version
 namespace {
-constexpr size_t kOutSmemBudget = 232448 - 1024 - 256;
-int out_version(int nmax, bool *rgs, bool *hsm = nullptr, int B = 0, int sms = 148) {
-  if (hsm) *hsm = false;
+// B = 0: the variant without the on-chip H / qm / qm1 tables (what sizes the workspace)
+int out_version(int nmax, bool *rgs, bool *hsm, int B, int sms) {
+  *hsm = false;
   // H / qm / qm1 of the sequence on chip as well: measured against reading them through L2 (profiles/r02_outside_hsm.txt) -- ahead
   // while two CTAs still share an SM (<= ~60 nt: 3-5 %) and for batches that leave SMs idle (B = 64: 0.96 -> 0.82 ms at 100 nt);
   // behind for big batches once it costs the second CTA (4096 x 100 nt: 16.2 against 11.3 ms).
-  const bool want = out2_plan(nmax, 8, true, true).total <= 113 * 1024 || (B > 0 && B <= sms);
-  if (hsm && want && out2_plan(nmax, 8, true, true).total <= kOutSmemBudget) { *rgs = true; *hsm = true; return 2; }
+  const bool want = B > 0 && (out2_plan(nmax, 8, true, true).total <= 113 * 1024 || B <= sms);
+  if (want && out2_plan(nmax, 8, true, true).total <= kSmemBudget) { *rgs = true; *hsm = true; return 2; }
   if (out2_plan(nmax, 8, true).total <= 113 * 1024) { *rgs = true; return 2; }
-  if (out2_plan(nmax, 8, false).total <= kOutSmemBudget) { *rgs = false; return 2; }
+  if (out2_plan(nmax, 8, false).total <= kSmemBudget) { *rgs = false; return 2; }
   return 1;
 }
-template <bool RGS, bool HSM>
-cudaError_t out2_setup(const BfBatchDev &b, int sms, int *grid, size_t *smem) {
-  auto kern = bf_k_pf_out2<8, RGS, HSM>;
-  const size_t sm = out2_plan(b.stride, 8, RGS, HSM).total;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sm > 1024 ? sm : 1024));
-  if (e != cudaSuccess) return e;
-  int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, sm);
-  if (e != cudaSuccess) return e;
-  if (occ < 1) return cudaErrorInvalidConfiguration;
-  *grid = b.B < sms * occ ? b.B : sms * occ;
-  if (smem) *smem = sm;
-  return cudaSuccess;
-}
+
+// bf_k_pf_out2 without and with the generic ring on chip, and with H / qm / qm1 on chip as well
+using OutK = void (*)(const BfParams *, BfBatchDev, const double *, const double *, size_t, double *, size_t, const double *, const char *, int,
+                      int, double *, double *, int *);
+const OutK kOut2[] = {bf_k_pf_out2<8, false, false>, bf_k_pf_out2<8, true, false>, bf_k_pf_out2<8, true, true>};
 }  // namespace
 
-size_t bf_out_ws_slot(int nmax) {
-  bool rgs = false;
-  if (out_version(nmax, &rgs) == 2) return (out2_ws_doubles(nmax, rgs) + 7) / 8 * 8;
-  return 4 * ((tri_size(nmax) + 7) / 8 * 8);
-}
-
-cudaError_t bf_out_grid(const BfBatchDev &b, int sms, int *grid) {
+// key: 0 = bf_k_pf_out, else kOut2[key - 1].  The workspace is sized for the variant without H on chip, so with it the slab is
+// larger than it needs to be.
+cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p) {
+  *p = BfPlan{};
   bool rgs = false, hsm = false;
-  if (out_version(b.stride, &rgs, &hsm, b.B, sms) == 2)
-    return hsm ? out2_setup<true, true>(b, sms, grid, nullptr) : rgs ? out2_setup<true, false>(b, sms, grid, nullptr) : out2_setup<false, false>(b, sms, grid, nullptr);
-  auto kern = bf_k_pf_out<8>;
-  const size_t sm = out_plan(b.stride).total;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sm > 1024 ? sm : 1024));
+  p->ws = out_version(stride, &rgs, &hsm, 0, sms) == 2 ? (out2_ws_doubles(stride, rgs) + 7) / 8 * 8 : 4 * ((tri_size(stride) + 7) / 8 * 8);
+  const void *kern;
+  if (out_version(stride, &rgs, &hsm, B, sms) == 2) {
+    p->key = 1 + rgs + hsm;
+    p->smem = out2_plan(stride, 8, rgs, hsm).total;
+    kern = (const void *)kOut2[p->key - 1];
+  } else {
+    p->key = 0;
+    p->smem = out_plan(stride).total;
+    kern = (const void *)bf_k_pf_out<8>;
+  }
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(p->smem > 1024 ? p->smem : 1024));
   if (e != cudaSuccess) return e;
   int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, sm);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, p->smem);
   if (e != cudaSuccess) return e;
   if (occ < 1) return cudaErrorInvalidConfiguration;
-  *grid = b.B < sms * occ ? b.B : sms * occ;
+  p->grid = B < sms * occ ? B : sms * occ;
   return cudaSuccess;
 }
 
-cudaError_t bf_launch_pf_out(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, double *ws,
+cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, double *ws,
                              const double *lnscale, const char *targets, int n_targets, int tstride, double *out_defect, double *out_bpp,
-                             int grid, int *work_counter, cudaStream_t st) {
+                             int *work_counter, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
-  bool rgs = false, hsm = false;
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (out_version(b.stride, &rgs, &hsm, b.B, sms) == 2) {
-    const size_t sm = out2_plan(b.stride, 8, rgs, hsm).total, tslot = (tri_size(b.stride) + 7) / 8 * 8, wslot = bf_out_ws_slot(b.stride);
-    if (hsm)
-      bf_k_pf_out2<8, true, true><<<grid, 256, sm, st>>>(dP, b, qbtri, qmseq, tslot, ws, wslot, lnscale, targets, n_targets, tstride, out_defect,
-                                                         out_bpp, work_counter);
-    else if (rgs)
-      bf_k_pf_out2<8, true, false><<<grid, 256, sm, st>>>(dP, b, qbtri, qmseq, tslot, ws, wslot, lnscale, targets, n_targets, tstride, out_defect,
-                                                          out_bpp, work_counter);
-    else
-      bf_k_pf_out2<8, false, false><<<grid, 256, sm, st>>>(dP, b, qbtri, qmseq, tslot, ws, wslot, lnscale, targets, n_targets, tstride, out_defect,
-                                                           out_bpp, work_counter);
-    return cudaGetLastError();
-  }
-  const size_t sm = out_plan(b.stride).total;
-  bf_k_pf_out<8><<<grid, 256, sm, st>>>(dP, b, qbtri, qmseq, (tri_size(b.stride) + 7) / 8 * 8, ws, lnscale, targets, n_targets, tstride,
-                                        out_defect, out_bpp, work_counter);
+  const size_t tslot = (tri_size(b.stride) + 7) / 8 * 8;
+  if (p.key == 0)
+    bf_k_pf_out<8><<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, lnscale, targets, n_targets, tstride, out_defect, out_bpp,
+                                                work_counter);
+  else
+    kOut2[p.key - 1]<<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, p.ws, lnscale, targets, n_targets, tstride, out_defect,
+                                                  out_bpp, work_counter);
   return cudaGetLastError();
 }

@@ -10,6 +10,7 @@
 #include <mutex>
 #include <vector>
 
+#include "bf_device.cuh"
 #include "bf_kernels.h"
 
 namespace {
@@ -18,8 +19,6 @@ constexpr int kRing = 32;
 constexpr int kInfThr = BF_INF / 2;
 constexpr int kNSG = 12, kNS1 = 3, kNSB = 3, kNSlot = kNSG + kNS1 + kNSB + 1;   // + the slot of the nine special candidates
 
-__host__ __device__ __forceinline__ int tri_off(int n, int d) { return (d - 4) * n - (d * (d - 1) / 2 - 6); }
-__host__ __device__ __forceinline__ size_t tri_size(int n) { return n >= 5 ? (size_t)tri_off(n, n) : 0; }
 __device__ __forceinline__ int ptype_sp(const uint8_t *SP, int i, int j) { return bf_ptype_bases(SP[i], SP[j]); }
 
 // (u1, u2) of the nine non-decomposable interior candidates: stack, bulge-1 (2x), 1x1, 1x2, 2x1, 2x2, 2x3, 3x2
