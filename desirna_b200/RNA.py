@@ -12,6 +12,7 @@ DesiRNA.py:35).  A maintainer switches engines with `from desirna_b200 import RN
     fc.hc_add_from_db(db)                         sequence_utils.py:1181, 1198, 1214
     fc.exp_params_rescale(mfe)                    energy_scores.py:372   (numerical no-op here: the kernels rescale per sequence)
     fc.ensemble_defect(db)                        energy_scores.py:374
+    fc.pbacktrack([num_samples]), RNA.init_rand(seed)   stochastic backtracking (not called by DesiRNA; ViennaRNA's API)
     RNA.fold(seq) / RNA.co_pf_fold(seq)           energy_scores.py:354; dimer_multichain_energy.py:109, 113-114
 
 Conventions kept: energies come back as Python floats holding float32-rounded kcal/mol (ViennaRNA returns C
@@ -20,6 +21,7 @@ Results of one fold compound are cached, and a whole batch of compounds can be e
 through `prefetch()` -- that is how the lock-step replica loop keeps the GPU busy while callers still see
 the per-object API.  There is no CPU fallback: every number comes from libb200fold.so.
 """
+import random
 import struct
 
 import numpy as np
@@ -37,6 +39,14 @@ class _Cvar:
 
 
 cvar = _Cvar()
+
+# seeds of fc.pbacktrack(): each call draws the next one, so successive calls give new samples and init_rand(seed) repeats a run
+_rand = random.Random()
+
+
+def init_rand(seed=None):
+    """Seed the generator behind fc.pbacktrack() (ViennaRNA RNA.init_rand); no seed: from the system's entropy source."""
+    _rand.seed(seed)
 
 
 def params_load(path):
@@ -185,6 +195,16 @@ class fold_compound:
             out = self._run(E.WANT_MFE | E.WANT_PF | E.WANT_DEFECT, targets=[[db]])
             self._cache[key] = float(out["defect"][0])
         return self._cache[key]
+
+    def pbacktrack(self, num_samples=None, *_):
+        """vrna_pbacktrack: a secondary structure drawn from the Boltzmann ensemble, or a list of num_samples independent ones"""
+        if "&" in self.sequence:
+            raise NotImplementedError("pbacktrack on two-strand compounds is not part of the accelerated path")
+        if self._nopair is not None and any(self._nopair):
+            raise RuntimeError("fold_compound.pbacktrack() after hc_add_from_db(): sampling under hard constraints is not supported")
+        n = 1 if num_samples is None else int(num_samples)
+        out = _eng.sample([self.sequence], n, seed=_rand.getrandbits(64))[0]
+        return out[0] if num_samples is None else out
 
     def second_best_energy(self):
         """(MFE, energy of the second-best structure) in kcal/mol as C floats, or (MFE, None) when the sequence has a single

@@ -103,6 +103,7 @@ struct Engine {
   bool force_generic = false;                     // BF_FORCE_GENERIC=1: route single strands through the generic kernels too
   // staging for the host-buffer entry point
   DevBuf d_seq, d_len, d_cut, d_nopair, d_targets, d_mfe, d_ss, d_pf, d_eval, d_defect, d_bpp;
+  DevBuf d_q5, d_samples;  // bf_sample: exterior prefixes, drawn structures
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -150,8 +151,10 @@ int validate(const bf_batch_t *b, const bf_result_t *r) {
 // scale_override (device, B ints, dcal/mol): energies that set the partition function's per-nucleotide scale instead of this
 // call's own MFE.  The result does not depend on the scale beyond rounding, and without that dependency the partition function
 // runs on the workspace's second stream beside the MFE fill -- worth it when both grids fit the GPU together (small batches).
+// keep_qm: keep the per-sequence qm / qm1 tables (w.qm_seq) of the PF fill for a pass that reads them after this call (bf_sample);
+// the outside pass (BF_WANT_BPP / BF_WANT_DEFECT) keeps them in any case.
 int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two, cudaStream_t st, const int *scale_override = nullptr,
-               bool timing = true) {
+               bool timing = true, bool keep_qm = false) {
   if (b->B == 0) return BF_OK;
   BfBatchDev db;
   db.B = b->B; db.stride = b->stride; db.seq = b->seq; db.len = b->len; db.cut = b->cut; db.nopair = b->nopair;
@@ -206,11 +209,13 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     mfe_for_scale = out_mfe;
   }
   const bool want_out = (b->want & (BF_WANT_BPP | BF_WANT_DEFECT)) != 0;
+  const bool want_qm = want_out || keep_qm;
   if ((b->want & BF_WANT_PF) || want_out) {
     BfPlan p;
     CU(bf_plan_pf(b->stride, b->B, two, g.force_generic, g.sm_count, &p), "plan the PF fill");
-    if (want_out && p.family == BF_FAM_GENERIC)
-      return fail(BF_ERR_UNAVAILABLE, "base-pair probabilities / ensemble defect: single-strand sequences within the fill path's length range only");
+    if (want_qm && p.family == BF_FAM_GENERIC)
+      return fail(BF_ERR_UNAVAILABLE, want_out ? "base-pair probabilities / ensemble defect: single-strand sequences within the fill path's length range only"
+                                               : "sampling: single-strand sequences within the fill path's length range only");
     BfBatchDev dbp = db;
     dbp.nopair = nullptr;  // hard constraints are added after fc.pf() in the reference (sequence_utils.py:1181)
     // a constrained MFE is not a bound on the unconstrained ensemble: only use it for scaling when unconstrained
@@ -225,7 +230,7 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
       CU(w.d_lnscale.reserve((size_t)b->B * sizeof(double)), "cudaMalloc(lnscale)");
       CU(w.ws_qm.reserve((size_t)p.grid * p.ws * sizeof(double)), "cudaMalloc(qm workspace)");
       double *qmseq = nullptr;
-      if (want_out) {
+      if (want_qm) {
         CU(w.qm_seq.reserve((size_t)b->B * 2 * slot), "cudaMalloc(per-sequence qm/qm1)");
         qmseq = (double *)w.qm_seq.p;
       }
@@ -335,7 +340,8 @@ int bf_init(int device) {
 int bf_shutdown(void) {
   if (!g.inited) return BF_OK;
   cudaStreamSynchronize(g.stream);
-  for (DevBuf *b : {&g.d_defect, &g.d_bpp, &g.d_seq, &g.d_len, &g.d_cut, &g.d_nopair, &g.d_targets, &g.d_mfe, &g.d_ss, &g.d_pf, &g.d_eval, &g.d_in, &g.d_out, &g.d_zero}) b->release();
+  for (DevBuf *b : {&g.d_defect, &g.d_bpp, &g.d_seq, &g.d_len, &g.d_cut, &g.d_nopair, &g.d_targets, &g.d_mfe, &g.d_ss, &g.d_pf, &g.d_eval, &g.d_in, &g.d_out, &g.d_zero,
+                    &g.d_q5, &g.d_samples}) b->release();
   if (g.h_in) cudaFreeHost(g.h_in);
   if (g.h_out) cudaFreeHost(g.h_out);
   g.h_in = g.h_out = nullptr; g.h_in_cap = g.h_out_cap = g.zero_cap = 0;
@@ -552,6 +558,46 @@ int bf_second_best(const bf_batch_t *b, int32_t *e1_dcal, int32_t *e2_dcal) {
   CU(cudaMemcpyAsync(e1_dcal, d_e, B * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e1");
   CU(cudaMemcpyAsync(e2_dcal, d_e + B, B * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e2");
   CU(cudaStreamSynchronize(st), "bf_second_best");
+  return BF_OK;
+}
+
+int bf_sample(const bf_batch_t *b, int32_t n_samples, uint64_t seed, char *ss_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!b || !ss_out || n_samples < 1 || b->B < 0 || b->stride <= 0 || (b->B && (!b->seq || !b->len))) return fail(BF_ERR_ARG, "bf_sample: bad argument");
+  if (any_cut(b, b->cut)) return fail(BF_ERR_UNAVAILABLE, "bf_sample: single strands only");
+  if (b->nopair) return fail(BF_ERR_UNAVAILABLE, "bf_sample: the partition function does not honour hard constraints");
+  if (g.force_generic || bf_fill_pf_mode(b->stride) == 0) return fail(BF_ERR_UNAVAILABLE, "bf_sample: stride outside the fill path");
+  for (int i = 0; i < b->B; i++)
+    if (b->len[i] < 0 || b->len[i] > b->stride) return fail(BF_ERR_ARG, "sequence length exceeds stride");
+  if (b->B == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  const size_t B = b->B, S = b->stride, out_bytes = B * (size_t)n_samples * (S + 1);
+  CU(g.d_seq.reserve(B * S), "cudaMalloc(seq)");
+  CU(g.d_len.reserve(B * sizeof(int)), "cudaMalloc(len)");
+  CU(g.d_mfe.reserve(B * sizeof(int)), "cudaMalloc(mfe)");
+  CU(g.d_pf.reserve(B * 5 * sizeof(double)), "cudaMalloc(pf)");
+  CU(g.d_q5.reserve(B * (S + 1) * sizeof(double)), "cudaMalloc(q5)");
+  CU(g.d_samples.reserve(out_bytes), "cudaMalloc(samples)");
+  CU(cudaMemcpyAsync(g.d_seq.p, b->seq, B * S, cudaMemcpyHostToDevice, st), "H2D seq");
+  CU(cudaMemcpyAsync(g.d_len.p, b->len, B * sizeof(int), cudaMemcpyHostToDevice, st), "H2D len");
+  // the MFE sets the partition function's scale, as for base-pair probabilities; the fill keeps qm / qm1 for the walk
+  bf_batch_t db;
+  memset(&db, 0, sizeof(db));
+  db.B = b->B; db.stride = b->stride; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
+  db.want = BF_WANT_MFE | BF_WANT_PF;
+  bf_result_t dr;
+  memset(&dr, 0, sizeof(dr));
+  dr.mfe_dcal = (int32_t *)g.d_mfe.p; dr.pf = (double *)g.d_pf.p;
+  int rc = run_device(g.w, &db, &dr, false, st, nullptr, true, true);
+  if (rc) return rc;
+  BfBatchDev dev;
+  dev.B = b->B; dev.stride = b->stride; dev.seq = db.seq; dev.len = db.len; dev.cut = nullptr; dev.nopair = nullptr;
+  CU(bf_launch_sample(g.dP, dev, (const double *)g.w.tri_qb.p, (const double *)g.w.qm_seq.p, (const double *)g.w.d_lnscale.p, (double *)g.d_q5.p,
+                      n_samples, seed, (char *)g.d_samples.p, g.sm_count, st), "launch bf_k_sample");
+  g.launches += 2;
+  CU(cudaMemcpyAsync(ss_out, g.d_samples.p, out_bytes, cudaMemcpyDeviceToHost, st), "D2H samples");
+  CU(cudaStreamSynchronize(st), "bf_sample");
   return BF_OK;
 }
 

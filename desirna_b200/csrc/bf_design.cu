@@ -18,14 +18,6 @@ namespace {
 
 constexpr int kWPB = 4;  // warps (rows) per CTA
 
-__device__ __forceinline__ unsigned long long sm64(unsigned long long &s) {
-  s += 0x9E3779B97F4A7C15ull;
-  unsigned long long z = s;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
-__device__ __forceinline__ double u01(unsigned long long &s) { return (double)(sm64(s) >> 11) * (1.0 / 9007199254740992.0); }
 __device__ __forceinline__ int below(unsigned long long &s, int n) {
   const int k = (int)(u01(s) * (double)n);
   return k < n ? k : n - 1;

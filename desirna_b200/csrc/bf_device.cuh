@@ -85,6 +85,16 @@ __device__ __forceinline__ double bf_warp_sum(double v) {
   return v;
 }
 
+// splitmix64: the next 64-bit output of the stream whose state is s, and a uniform double in [0, 1) from it
+__device__ __forceinline__ unsigned long long sm64(unsigned long long &s) {
+  s += 0x9E3779B97F4A7C15ull;
+  unsigned long long z = s;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+__device__ __forceinline__ double u01(unsigned long long &s) { return (double)(sm64(s) >> 11) * (1.0 / 9007199254740992.0); }
+
 // ------------------------------------------------------------------ special hairpins
 BF_HD int bf_loop_key(const uint8_t *S, int i, int len, bool *valid) {
   int key = 0;

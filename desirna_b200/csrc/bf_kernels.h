@@ -108,6 +108,11 @@ cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchD
                              const double *lnscale, const char *targets, int n_targets, int tstride, double *out_defect, double *out_bpp,
                              int *work_counter, cudaStream_t st);
 
+// ---- stochastic backtracking (bf_sample.cu): n_samples structures per sequence drawn from the tables a PF fill with qmseq kept left
+// behind.  q5: B x (stride + 1) doubles of scratch; ss_out: B x n_samples x (stride + 1) chars, sample-major within a row.
+cudaError_t bf_launch_sample(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, const double *lnscale, double *q5,
+                             int n_samples, unsigned long long seed, char *ss_out, int sms, cudaStream_t st);
+
 // ---- suboptimal structures (bf_subopt.cu): host walk over the c / fML tables of the GPU fill
 #ifdef __cplusplus
 #include <string>

@@ -57,6 +57,7 @@ def lib():
         L.bf_second_best.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.bf_subopt.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                 C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.bf_sample.argtypes = [C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
         L.bf_debug_copy_table.argtypes = [C.c_int, C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         _lib = L
@@ -157,6 +158,28 @@ def second_best(seqs, nopair=None):
     e1, e2 = np.zeros(len(seqs), np.int32), np.zeros(len(seqs), np.int32)
     _check(lib().bf_second_best(C.byref(b), e1.ctypes.data, e2.ctypes.data))
     return e1, e2
+
+
+def sample(seqs, n_samples, seed=0):
+    """bf_sample: stochastic backtracking (ViennaRNA fc.pbacktrack()).  n_samples secondary structures of every single-strand
+    sequence, drawn independently from its Boltzmann ensemble; returns a list (per sequence) of lists of dot-bracket strings.
+    The samples are a function of (seed, sequence index, sample index) only: the same call repeats, and the first k samples of a
+    call with more are those of a call with k."""
+    ensure_ready()
+    buf, lens, cuts = pack([s.upper().replace("T", "U") for s in seqs])
+    b = bf_batch_t()
+    b.B, b.stride = len(seqs), buf.shape[1]
+    b.seq, b.len = buf.ctypes.data, lens.ctypes.data
+    b.cut = cuts.ctypes.data if cuts.any() else None
+    n_samples = int(n_samples)
+    out = np.zeros((len(seqs), max(n_samples, 1), b.stride + 1), np.uint8)
+    _check(lib().bf_sample(C.byref(b), n_samples, int(seed) & ((1 << 64) - 1), out.ctypes.data))
+    res = []
+    for r in range(len(seqs)):
+        n = int(lens[r])
+        raw = out[r, :, :n].tobytes().decode("ascii")
+        res.append([raw[k * n:(k + 1) * n] for k in range(n_samples)])
+    return res
 
 
 def set_option(key, value):

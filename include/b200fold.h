@@ -96,6 +96,15 @@ int bf_score_batch_device(const bf_batch_t *batch, bf_result_t *result, void *cu
 int bf_second_best(const bf_batch_t *batch, int32_t *e1_dcal, int32_t *e2_dcal);
 int bf_subopt(const char *seq, int32_t len, const uint8_t *nopair, int32_t delta_dcal, int32_t max_out, char *ss_out, int32_t *e_out,
               int32_t *n_out, int32_t *truncated);
+/* fc.pbacktrack(num_samples) (vrna_pbacktrack, RNAsubopt -p): stochastic backtracking.  n_samples secondary structures of every
+ * sequence of the batch (seq, len, stride as in bf_score_batch), each drawn independently from the Boltzmann ensemble of the
+ * partition function bf_score_batch computes (the MFE sets its scale, as for BF_WANT_BPP).  HOST buffers, synchronous.
+ * ss_out: B x n_samples x (stride+1) chars, sample-major within a row; sample k of row r at (r * n_samples + k) * (stride+1),
+ * len[r] characters of . ( ) and a NUL (the rest of the slot is NUL too).  The samples are a function of (seed, r, k) alone: the
+ * same call repeats, and the first k samples of a call with n > k are those of a call with k.
+ * BF_ERR_UNAVAILABLE: a row with cut > 0, a nopair mask (the partition function ignores constraints), a stride outside the fill
+ * path (> 2000) or BF_FORCE_GENERIC.  BF_ERR_ARG: n_samples < 1, null buffers, len > stride. */
+int bf_sample(const bf_batch_t *batch, int32_t n_samples, uint64_t seed, char *ss_out);
 
 /* device time (ms, CUDA events on the launch stream) of the mfe, pf and eval kernels of the most recent
  * bf_score_batch[_device] call; -1 for a kernel that did not run.  Blocks until those kernels finished. */
