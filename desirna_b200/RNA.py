@@ -13,6 +13,7 @@ DesiRNA.py:35).  A maintainer switches engines with `from desirna_b200 import RN
     fc.exp_params_rescale(mfe)                    energy_scores.py:372   (numerical no-op here: the kernels rescale per sequence)
     fc.ensemble_defect(db)                        energy_scores.py:374
     fc.pbacktrack([num_samples]), RNA.init_rand(seed)   stochastic backtracking (not called by DesiRNA; ViennaRNA's API)
+    fc.subopt_zuker()                             Zuker suboptimals (not called by DesiRNA; ViennaRNA's API)
     RNA.fold(seq) / RNA.co_pf_fold(seq)           energy_scores.py:354; dimer_multichain_energy.py:109, 113-114
 
 Conventions kept: energies come back as Python floats holding float32-rounded kcal/mol (ViennaRNA returns C
@@ -234,6 +235,25 @@ class fold_compound:
         for structure, e in found:
             cb(structure, f32(e / 100.0), data)
         cb(None, 0.0, data)
+
+    def subopt_zuker(self):
+        """vrna_subopt_zuker: for every base pair that some structure contains, a minimum-free-energy structure containing it
+        (each structure listed once), sorted by energy; hard constraints of hc_add_from_db() apply"""
+        if "&" in self.sequence:
+            raise NotImplementedError("subopt_zuker on two-strand compounds is not part of the accelerated path")
+        nopair = np.asarray(self._nopair, np.uint8) if self._nopair is not None and any(self._nopair) else None
+        return [subopt_solution(s, f32(e / 100.0)) for s, e in _eng.subopt_zuker(self.sequence, nopair)]
+
+
+class subopt_solution:
+    """one entry of fc.subopt_zuker(): .structure and .energy (kcal/mol, C float) as ViennaRNA's subopt_solution"""
+
+    def __init__(self, structure, energy):
+        self.structure = structure
+        self.energy = energy
+
+    def __repr__(self):
+        return "subopt_solution(%r, %r)" % (self.structure, self.energy)
 
 
 def fold(sequence):

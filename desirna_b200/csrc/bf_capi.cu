@@ -104,6 +104,7 @@ struct Engine {
   // staging for the host-buffer entry point
   DevBuf d_seq, d_len, d_cut, d_nopair, d_targets, d_mfe, d_ss, d_pf, d_eval, d_defect, d_bpp;
   DevBuf d_q5, d_samples;  // bf_sample: exterior prefixes, drawn structures
+  DevBuf d_epair;          // bf_pair_mfe: E_pair of every sequence
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -341,7 +342,7 @@ int bf_shutdown(void) {
   if (!g.inited) return BF_OK;
   cudaStreamSynchronize(g.stream);
   for (DevBuf *b : {&g.d_defect, &g.d_bpp, &g.d_seq, &g.d_len, &g.d_cut, &g.d_nopair, &g.d_targets, &g.d_mfe, &g.d_ss, &g.d_pf, &g.d_eval, &g.d_in, &g.d_out, &g.d_zero,
-                    &g.d_q5, &g.d_samples}) b->release();
+                    &g.d_q5, &g.d_samples, &g.d_epair}) b->release();
   if (g.h_in) cudaFreeHost(g.h_in);
   if (g.h_out) cudaFreeHost(g.h_out);
   g.h_in = g.h_out = nullptr; g.h_in_cap = g.h_out_cap = g.zero_cap = 0;
@@ -598,6 +599,86 @@ int bf_sample(const bf_batch_t *b, int32_t n_samples, uint64_t seed, char *ss_ou
   g.launches += 2;
   CU(cudaMemcpyAsync(ss_out, g.d_samples.p, out_bytes, cudaMemcpyDeviceToHost, st), "D2H samples");
   CU(cudaStreamSynchronize(st), "bf_sample");
+  return BF_OK;
+}
+
+int bf_pair_mfe(const bf_batch_t *b, int32_t *e_pair_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!b || !e_pair_out || b->B < 0 || b->stride <= 0 || (b->B && (!b->seq || !b->len))) return fail(BF_ERR_ARG, "bf_pair_mfe: bad argument");
+  if (any_cut(b, b->cut)) return fail(BF_ERR_UNAVAILABLE, "bf_pair_mfe: single strands only");
+  if (g.force_generic || bf_fill_mfe_mode(b->stride) == 0) return fail(BF_ERR_UNAVAILABLE, "bf_pair_mfe: stride outside the fill path");
+  for (int i = 0; i < b->B; i++)
+    if (b->len[i] < 0 || b->len[i] > b->stride) return fail(BF_ERR_ARG, "sequence length exceeds stride");
+  if (b->B == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  const size_t B = b->B, S = b->stride;
+  CU(g.d_seq.reserve(B * S), "cudaMalloc(seq)");
+  CU(g.d_len.reserve(B * sizeof(int)), "cudaMalloc(len)");
+  CU(g.d_mfe.reserve(B * sizeof(int)), "cudaMalloc(mfe)");
+  CU(g.d_epair.reserve(B * S * S * sizeof(int)), "cudaMalloc(e_pair)");
+  CU(cudaMemcpyAsync(g.d_seq.p, b->seq, B * S, cudaMemcpyHostToDevice, st), "H2D seq");
+  CU(cudaMemcpyAsync(g.d_len.p, b->len, B * sizeof(int), cudaMemcpyHostToDevice, st), "H2D len");
+  bf_batch_t db;
+  memset(&db, 0, sizeof(db));
+  db.B = b->B; db.stride = b->stride; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
+  if (b->nopair) {
+    CU(g.d_nopair.reserve(B * S), "cudaMalloc(nopair)");
+    CU(cudaMemcpyAsync(g.d_nopair.p, b->nopair, B * S, cudaMemcpyHostToDevice, st), "H2D nopair");
+    db.nopair = (const uint8_t *)g.d_nopair.p;
+  }
+  db.want = BF_WANT_MFE;
+  bf_result_t dr;
+  memset(&dr, 0, sizeof(dr));
+  dr.mfe_dcal = (int32_t *)g.d_mfe.p;
+  int rc = run_device(g.w, &db, &dr, false, st);
+  if (rc) return rc;
+  BfBatchDev dev;
+  dev.B = b->B; dev.stride = b->stride; dev.seq = db.seq; dev.len = db.len; dev.cut = nullptr; dev.nopair = db.nopair;
+  BfPlan p;
+  CU(bf_plan_mfe_out(b->stride, b->B, g.sm_count, &p), "plan bf_k_mfe_out");
+  CU(g.w.ws_out.reserve((size_t)p.grid * p.ws * sizeof(int)), "cudaMalloc(outside workspace)");
+  CU(bf_launch_mfe_out(p, g.dP, dev, (const int *)g.w.tri_c.p, (const int *)g.w.tri_f.p, (int *)g.w.ws_out.p, (int *)g.d_epair.p,
+                       g.w.d_counters + 2, st), "launch bf_k_mfe_out");
+  g.launches++;
+  CU(cudaMemcpyAsync(e_pair_out, g.d_epair.p, B * S * S * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e_pair");
+  CU(cudaStreamSynchronize(st), "bf_pair_mfe");
+  return BF_OK;
+}
+
+int bf_subopt_zuker(const char *seq, int32_t len, const uint8_t *nopair, int32_t max_out, char *ss_out, int32_t *e_out, int32_t *n_out,
+                    int32_t *truncated) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!seq || len <= 0 || !ss_out || !e_out || !n_out || max_out <= 0) return fail(BF_ERR_ARG, "bf_subopt_zuker: bad argument");
+  if (g.force_generic || bf_fill_mfe_mode(len) == 0) return fail(BF_ERR_UNAVAILABLE, "bf_subopt_zuker: length outside the fill path");
+  // E_pair of this one sequence; its MFE fill leaves the c / fML tables in the engine's table buffers
+  int32_t l32 = len;
+  bf_batch_t b;
+  memset(&b, 0, sizeof(b));
+  b.B = 1; b.stride = len; b.seq = seq; b.len = &l32; b.nopair = nopair;
+  std::vector<int> ep((size_t)len * len);
+  int rc = bf_pair_mfe(&b, ep.data());
+  if (rc) return rc;
+  const size_t slot = bf_tri_slot(len);
+  std::vector<int> c(slot), fm(slot);
+  CU(cudaMemcpy(c.data(), g.w.tri_c.p, slot * sizeof(int), cudaMemcpyDeviceToHost), "D2H c table");
+  CU(cudaMemcpy(fm.data(), g.w.tri_f.p, slot * sizeof(int), cudaMemcpyDeviceToHost), "D2H fML table");
+  std::vector<uint8_t> S(len + 2, 0), SP(len + 2, 0);
+  for (int k = 1; k <= len; k++) {
+    S[k] = (uint8_t)bf_base_code(seq[k - 1]);
+    SP[k] = (nopair && nopair[k - 1]) ? 0 : S[k];
+  }
+  std::vector<std::pair<int, std::string>> out;
+  bool trunc = false;
+  if (bf_zuker_host(g.hP, len, S.data(), SP.data(), c.data(), fm.data(), ep.data(), max_out, &out, &trunc) < 0)
+    return fail(BF_ERR_CUDA, "bf_subopt_zuker: E_pair disagrees with the MFE fill's tables");
+  for (size_t k = 0; k < out.size(); k++) {
+    e_out[k] = out[k].first;
+    memcpy(ss_out + k * (size_t)(len + 1), out[k].second.c_str(), (size_t)len + 1);
+  }
+  *n_out = (int32_t)out.size();
+  if (truncated) *truncated = trunc ? 1 : 0;
   return BF_OK;
 }
 

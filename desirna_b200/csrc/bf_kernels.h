@@ -45,6 +45,7 @@ struct BfPlan {
 cudaError_t bf_plan_mfe(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p);
 cudaError_t bf_plan_pf(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p);
 cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p);
+cudaError_t bf_plan_mfe_out(int stride, int B, int sms, BfPlan *p);   // p->ws: ints per CTA
 
 cudaError_t bf_upload_constants();
 
@@ -108,6 +109,11 @@ cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchD
                              const double *lnscale, const char *targets, int n_targets, int tstride, double *out_defect, double *out_bpp,
                              int *work_counter, cudaStream_t st);
 
+// ---- minimum-free-energy outside pass (bf_outside.cu): over the c / fML triangles an MFE fill of the same batch left behind.
+// e_pair: B x stride x stride ints, [i-1][j-1] = lowest energy of a structure containing (i,j), BF_INF elsewhere.
+cudaError_t bf_launch_mfe_out(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, const int *ctri, const int *ftri, int *ws, int *e_pair,
+                              int *work_counter, cudaStream_t st);
+
 // ---- stochastic backtracking (bf_sample.cu): n_samples structures per sequence drawn from the tables a PF fill with qmseq kept left
 // behind.  q5: B x (stride + 1) doubles of scratch; ss_out: B x n_samples x (stride + 1) chars, sample-major within a row.
 cudaError_t bf_launch_sample(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, const double *lnscale, double *q5,
@@ -120,4 +126,8 @@ cudaError_t bf_launch_sample(const BfParams *dP, const BfBatchDev &b, const doub
 #include <vector>
 int bf_wuchty_host(const BfParams *P, int n, const uint8_t *S, const uint8_t *SP, const int *c, const int *fm, int delta, int cap,
                    std::vector<std::pair<int, std::string>> *out, int *mfe_out, bool *truncated);
+// Zuker suboptimals: e_pair (n x n, [i-1][j-1]) from bf_launch_mfe_out over the same tables.  Returns the number of structures
+// (<= cap; *truncated when more pairs were left uncovered), or -1 if e_pair and the tables disagree.
+int bf_zuker_host(const BfParams *P, int n, const uint8_t *S, const uint8_t *SP, const int *c, const int *fm, const int *e_pair, int cap,
+                  std::vector<std::pair<int, std::string>> *out, bool *truncated);
 #endif

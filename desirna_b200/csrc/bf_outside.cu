@@ -1,4 +1,5 @@
-// bf_outside.cu -- outside pass of the partition function: base-pair probabilities and ensemble defect (sm_100a).
+// bf_outside.cu -- outside passes (sm_100a): of the partition function (base-pair probabilities, ensemble defect) and of the
+// minimum free energy (the best structure containing each pair, bf_k_mfe_out below).
 //
 // Replaces md.compute_bpp=1 + fc.pf() + fc.ensemble_defect(target) (utils/energy_scores.py:362-374 in the reference).
 // Formulated as the reverse-mode derivative of the inside recursion of bf_k_pf_fill in GATHER form, so that it runs
@@ -580,6 +581,181 @@ __global__ void __launch_bounds__(NW * 32) bf_k_pf_out2(const BfParams *__restri
   }
 }
 
+// =====================================================================================================
+//  Minimum-free-energy outside pass: for every pair (a,b) the lowest energy of the rest of a structure that contains it,
+//  Cout(a,b), over the packed c / fML triangles of the MFE fill, so that E_pair(a,b) = C(a,b) + Cout(a,b).
+//
+//    Cout(a,b) = min { f5[a-1] + ext(a,b) + f3[b+1],                                          exterior loop
+//                      Cout(i,j) + E_int(i,j;a,b)                      (a-i-1)+(j-b-1) <= 30,   enclosing interior loop
+//                      mlstem(a,b) + min( A(a,b), min_i fML(i+1,a-1) + Hall(i,b) ) }          enclosing multiloop
+//    G(i,j)    = Cout(i,j) + MLclosing + mlstem(closing (i,j))
+//    Hm(i,b)   = min_j G(i,j) + fML(b+1,j-1)                           right of the stem: a multiloop segment
+//    Hu(i,b)   = min(G(i,b+1), Hu(i,b+1) + MLbase)                     right of the stem: unpaired only
+//    Hall      = min(Hm, Hu),   A(a,b) = min(Hm(a-1,b), A(a-1,b) + MLbase)   (left of the stem unpaired, right a segment)
+//
+//  The min-plus twin of the PF pass's row accumulators: every term is O(n) per cell, the pass O(n^3).  Cells are processed a
+//  diagonal at a time from n-1 down to 4 (one barrier per diagonal), lanes on consecutive cells; the Cout, G and Hall triangles
+//  live in the CTA's HBM workspace, Hm / Hu / A in two-diagonal rings on chip.  f5 / f3 are computed first by warps 0 and 1.
+// =====================================================================================================
+constexpr int kMoutNW = 8;
+
+struct MoutPlan {
+  int rs;
+  size_t o_f5, o_f3, o_toff, o_hm, o_hu, o_ap, o_S, o_SP, total;
+};
+__host__ __device__ inline MoutPlan mout_plan(int nmax) {
+  MoutPlan p;
+  p.rs = (nmax + 8 + 3) / 4 * 4;
+  size_t o = 0;
+  p.o_f5 = o; o += (size_t)p.rs * sizeof(int);
+  p.o_f3 = o; o += (size_t)p.rs * sizeof(int);
+  p.o_toff = o; o += (size_t)p.rs * sizeof(int);
+  p.o_hm = o; o += (size_t)2 * p.rs * sizeof(int);
+  p.o_hu = o; o += (size_t)2 * p.rs * sizeof(int);
+  p.o_ap = o; o += (size_t)2 * p.rs * sizeof(int);
+  p.o_S = o; o += (nmax + 2 + 15) / 16 * 16;
+  p.o_SP = o; o += (nmax + 2 + 15) / 16 * 16;
+  p.total = o;
+  return p;
+}
+// ints of per-CTA HBM workspace: the Cout, G and Hall triangles
+__host__ __device__ inline size_t mout_ws_ints(int nmax) { return 3 * ((tri_size(nmax) + 7) / 8 * 8); }
+
+__global__ void __launch_bounds__(kMoutNW * 32) bf_k_mfe_out(const BfParams *__restrict__ P, BfBatchDev b, const int *__restrict__ ctri,
+                                                            const int *__restrict__ ftri, size_t tri_slot, int *ws, size_t ws_slot,
+                                                            int *e_pair, int *work_counter) {
+  extern __shared__ __align__(16) unsigned char dyn[];
+  __shared__ int s_seq;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int nmax = b.stride;
+  const MoutPlan pl = mout_plan(nmax);
+  const int RS = pl.rs;
+  const BfSmallI &T = P->si;
+  int *f5 = reinterpret_cast<int *>(dyn + pl.o_f5);
+  int *f3 = reinterpret_cast<int *>(dyn + pl.o_f3);
+  int *toff = reinterpret_cast<int *>(dyn + pl.o_toff);
+  int *HM = reinterpret_cast<int *>(dyn + pl.o_hm);
+  int *HU = reinterpret_cast<int *>(dyn + pl.o_hu);
+  int *AR = reinterpret_cast<int *>(dyn + pl.o_ap);
+  uint8_t *S = dyn + pl.o_S, *SP = dyn + pl.o_SP;
+  const size_t tri_pad = (tri_size(nmax) + 7) / 8 * 8;
+  int *CO = ws + (size_t)blockIdx.x * ws_slot, *GT = CO + tri_pad, *HA = GT + tri_pad;
+  const int mlbase = T.MLbase;
+
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) s_seq = atomicAdd(work_counter, 1);
+    __syncthreads();
+    const int sq = s_seq;
+    if (sq >= b.B) break;
+    const int n = b.len[sq];
+    const char *src = b.seq + (size_t)sq * b.stride;
+    const uint8_t *np = b.nopair ? b.nopair + (size_t)sq * b.stride : nullptr;
+    for (int k = tid; k <= n + 1; k += blockDim.x) {
+      const uint8_t s = (uint8_t)((k >= 1 && k <= n) ? bf_base_code(src[k - 1]) : 0);
+      S[k] = s;
+      SP[k] = (np && k >= 1 && k <= n && np[k - 1]) ? 0 : s;
+    }
+    for (int k = tid; k <= n; k += blockDim.x) toff[k] = (k >= 4) ? tri_off(n, k) : 0;
+    for (int k = tid; k < 2 * RS; k += blockDim.x) { HM[k] = BF_INF; HU[k] = BF_INF; AR[k] = BF_INF; }
+    int *out = e_pair + (size_t)sq * nmax * nmax;
+    for (size_t k = tid; k < (size_t)nmax * nmax; k += blockDim.x) out[k] = BF_INF;
+    const int *c = ctri + (size_t)sq * tri_slot, *fm = ftri + (size_t)sq * tri_slot;
+    __syncthreads();
+    auto ext = [&](int i, int j, int t) -> int { return bf_e_ext(T, t, (i > 1) ? S[i - 1] : -1, (j < n) ? S[j + 1] : -1); };
+    // exterior prefix f5 (warp 0) and suffix f3 (warp 1)
+    if (warp == 0) {
+      if (lane == 0) f5[0] = 0;
+      __syncwarp();
+      for (int j = 1; j <= n; j++) {
+        int e = BF_INF;
+        for (int i = 1 + lane; i < j - BF_TURN; i += 32) {
+          const int t = bf_ptype_bases(SP[i], SP[j]);
+          const int cc = t ? c[toff[j - i] + i - 1] : BF_INF;
+          if (cc < BF_INF) e = min(e, f5[i - 1] + cc + ext(i, j, t));
+        }
+        e = bf_warp_min(e);
+        if (lane == 0) f5[j] = min(e, f5[j - 1]);
+        __syncwarp();
+      }
+    } else if (warp == 1) {
+      if (lane == 0) f3[n + 1] = 0;
+      __syncwarp();
+      for (int i = n; i >= 1; i--) {
+        int e = BF_INF;
+        for (int j = i + BF_TURN + 1 + lane; j <= n; j += 32) {
+          const int t = bf_ptype_bases(SP[i], SP[j]);
+          const int cc = t ? c[toff[j - i] + i - 1] : BF_INF;
+          if (cc < BF_INF) e = min(e, cc + ext(i, j, t) + f3[j + 1]);
+        }
+        e = bf_warp_min(e);
+        if (lane == 0) f3[i] = min(e, f3[i + 1]);
+        __syncwarp();
+      }
+    }
+    __syncthreads();
+
+    for (int d = n - 1; d >= BF_TURN + 1; d--) {
+      const int ncell = n - d;
+      const int r0 = (d & 1) * RS, r1 = ((d + 1) & 1) * RS;
+      for (int a = tid + 1; a <= ncell; a += blockDim.x) {
+        const int bb = a + d;
+        // Hm: the stem ends at bb, the closing pair (a, j) of its multiloop, fML(bb+1, j-1) between
+        int hm = BF_INF;
+        for (int m = 6; bb + m <= n; m++) {
+          const int g = GT[toff[d + m] + a - 1], f = fm[toff[m - 2] + bb];
+          hm = min(hm, g + f);
+        }
+        if (hm >= BF_INF) hm = BF_INF;
+        int hu = BF_INF;
+        if (bb < n) hu = min(GT[toff[d + 1] + a - 1], HU[r1 + a] + mlbase);
+        if (hu >= BF_INF) hu = BF_INF;
+        int ap = BF_INF;
+        if (a > 1) ap = min(HM[r1 + a - 1], AR[r1 + a - 1] + mlbase);
+        if (ap >= BF_INF) ap = BF_INF;
+        const int o = toff[d] + a - 1;
+        const int t = bf_ptype_bases(SP[a], SP[bb]);
+        const int cab = t ? c[o] : BF_INF;
+        int e = BF_INF;
+        if (cab < BF_INF) {
+          e = f5[a - 1] + ext(a, bb, t) + f3[bb + 1];
+          // enclosing interior loops: outer pair (a-1-u1, bb+1+u2), s = u1 + u2
+          const int t2 = bf_rtype(t), sp1 = S[a - 1], sq1 = S[bb + 1];
+          const int smax = min(BF_MAXLOOP, n - 1 - d - 2);
+          for (int s = 0; s <= smax; s++) {
+            const int od = toff[d + 2 + s];
+            for (int u1 = max(0, s - (n - bb - 1)); u1 <= min(s, a - 2); u1++) {
+              const int i = a - 1 - u1, j = bb + 1 + s - u1;
+              const int co = CO[od + i - 1];
+              if (co >= BF_INF) continue;
+              const int to = bf_ptype_bases(S[i], S[j]);
+              e = min(e, co + bf_e_intloop(P, T, u1, s - u1, to, t2, S[i + 1], S[j - 1], sp1, sq1));
+            }
+          }
+          // enclosing multiloops: left of the stem unpaired (A) or a segment fML(i+1, a-1)
+          if (a > 1 && bb < n) {
+            int ml = ap;
+            for (int m = 6; m <= a - 1; m++) {
+              const int i = a - m;
+              ml = min(ml, fm[toff[m - 2] + i] + HA[toff[d + m] + i - 1]);
+            }
+            if (ml < BF_INF) e = min(e, ml + bf_e_mlstem(T, t, sp1, sq1));
+          }
+          if (e >= BF_INF) e = BF_INF;
+        }
+        CO[o] = e;
+        GT[o] = e < BF_INF ? e + T.MLclosing + bf_e_mlstem(T, bf_rtype(t), S[bb - 1], S[a + 1]) : BF_INF;
+        HA[o] = min(hm, hu);
+        HM[r0 + a] = hm;
+        HU[r0 + a] = hu;
+        AR[r0 + a] = ap;
+        if (e < BF_INF) out[(size_t)(a - 1) * nmax + (bb - 1)] = cab + e;
+      }
+      __syncthreads();
+    }
+  }
+}
+
 }  // namespace
 
 // ---- host side: v2 whenever its plan fits the CTA's shared memory (generic ring on chip when that still leaves two CTAs per
@@ -642,5 +818,27 @@ cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchD
   else
     kOut2[p.key - 1]<<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, p.ws, lnscale, targets, n_targets, tstride, out_defect,
                                                   out_bpp, work_counter);
+  return cudaGetLastError();
+}
+
+cudaError_t bf_plan_mfe_out(int stride, int B, int sms, BfPlan *p) {
+  *p = BfPlan{};
+  p->ws = mout_ws_ints(stride);
+  p->smem = mout_plan(stride).total;
+  cudaError_t e = cudaFuncSetAttribute(bf_k_mfe_out, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(p->smem > 1024 ? p->smem : 1024));
+  if (e != cudaSuccess) return e;
+  int occ = 0;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bf_k_mfe_out, kMoutNW * 32, p->smem);
+  if (e != cudaSuccess) return e;
+  if (occ < 1) return cudaErrorInvalidConfiguration;
+  p->grid = B < sms * occ ? B : sms * occ;
+  return cudaSuccess;
+}
+
+cudaError_t bf_launch_mfe_out(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, const int *ctri, const int *ftri, int *ws, int *e_pair,
+                              int *work_counter, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
+  if (e != cudaSuccess) return e;
+  bf_k_mfe_out<<<p.grid, kMoutNW * 32, p.smem, st>>>(dP, b, ctri, ftri, bf_tri_slot(b.stride), ws, p.ws, e_pair, work_counter);
   return cudaGetLastError();
 }

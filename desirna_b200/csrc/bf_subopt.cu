@@ -34,7 +34,7 @@ struct Walker {
   std::string ss;
   std::vector<std::pair<int, std::string>> *out;
   long long found = 0;
-  bool overflow = false;
+  bool overflow = false, first_only = false;   // first_only: stop at the first structure (bf_zuker_host's completions)
 
   int off(int d) const { return (d - 4) * n - (d * (d - 1) / 2 - 6); }
   int C(int i, int j) const { return (j - i > BF_TURN && i >= 1 && j <= n) ? c[off(j - i) + i - 1] : BF_INF; }
@@ -78,6 +78,7 @@ struct Walker {
       found++;
       if ((int)out->size() < cap) out->emplace_back(acc, ss);
       else overflow = true;
+      if (first_only) overflow = true;
       return;
     }
     const Iv v = st.back();
@@ -164,6 +165,111 @@ int bf_wuchty_host(const BfParams *P, int n, const uint8_t *S, const uint8_t *SP
   w.st.push_back({1, n, 0});
   w.rec(0, mfe);
   if (truncated) *truncated = w.overflow;
+  std::sort(out->begin(), out->end());
+  return (int)out->size();
+}
+
+// Zuker suboptimals (fc.subopt_zuker()): pairs in order of (E_pair, i, j); for each pair no listed structure contains yet, one
+// structure of energy E_pair containing it.  Its outside part is traced back from Cout = E_pair - C, the exterior, interior and
+// multiloop cases of bf_k_mfe_out tried in that order; what it leaves open (the pair itself, exterior prefixes and suffixes,
+// multiloop segments) is completed by the Walker above with the band closed at the sum of their optima, so that its first
+// leaf is an optimal completion.
+int bf_zuker_host(const BfParams *P, int n, const uint8_t *S, const uint8_t *SP, const int *c, const int *fm, const int *e_pair, int cap,
+                  std::vector<std::pair<int, std::string>> *out, bool *truncated) {
+  Walker w;
+  w.P = P; w.T = &P->si; w.n = n; w.S = S; w.SP = SP; w.c = c; w.fm = fm; w.cap = 1; w.first_only = true;
+  w.prepare();
+  const BfSmallI &T = P->si;
+  std::vector<int> f3(n + 2, 0);
+  for (int i = n; i >= 1; i--) {
+    int e = f3[i + 1];
+    for (int j = i + BF_TURN + 1; j <= n; j++) {
+      const int t = w.pt(i, j), cc = w.C(i, j);
+      if (t && cc < BF_INF) e = std::min(e, cc + w.ext(i, j, t) + f3[j + 1]);
+    }
+    f3[i] = e;
+  }
+  auto E = [&](int i, int j) { return e_pair[(size_t)(i - 1) * n + (j - 1)]; };
+  auto CO = [&](int i, int j) { return (i >= 1 && j <= n && E(i, j) < BF_INF) ? E(i, j) - w.C(i, j) : BF_INF; };
+  struct Pr { int e, i, j; };
+  std::vector<Pr> pairs;
+  for (int i = 1; i <= n; i++)
+    for (int j = i + BF_TURN + 1; j <= n; j++)
+      if (E(i, j) < BF_INF) pairs.push_back({E(i, j), i, j});
+  std::sort(pairs.begin(), pairs.end(), [](const Pr &x, const Pr &y) { return x.e != y.e ? x.e < y.e : x.i != y.i ? x.i < y.i : x.j < y.j; });
+  std::vector<char> covered((size_t)(n + 1) * (n + 1), 0);
+  const int ml = T.MLbase;
+  *truncated = false;
+  for (const Pr &pr : pairs) {
+    if (covered[(size_t)pr.i * (n + 1) + pr.j]) continue;
+    if ((int)out->size() >= cap) { *truncated = true; break; }
+    std::string ss(n, '.');
+    std::vector<Iv> open;
+    open.push_back({pr.i, pr.j, 2});
+    int a = pr.i, b = pr.j, v = CO(a, b);
+    for (;;) {
+      ss[a - 1] = '('; ss[b - 1] = ')';
+      const int t = w.pt(a, b);
+      if (v == w.f5[a - 1] + w.ext(a, b, t) + f3[b + 1]) {
+        if (a > 1) open.push_back({1, a - 1, 0});
+        for (int i = b + 1; i <= n;) {   // the suffix f3[b+1], traced here (the Walker's exterior kind is a prefix)
+          if (f3[i] == f3[i + 1]) { i++; continue; }
+          int j = i + BF_TURN + 1;
+          for (; j <= n; j++) {
+            const int tt = w.pt(i, j), cc = w.C(i, j);
+            if (tt && cc < BF_INF && f3[i] == cc + w.ext(i, j, tt) + f3[j + 1]) break;
+          }
+          if (j > n) return -1;
+          ss[i - 1] = '('; ss[j - 1] = ')';
+          open.push_back({i, j, 2});
+          i = j + 1;
+        }
+        break;
+      }
+      bool found = false;
+      for (int s = 0; s <= BF_MAXLOOP && !found; s++)
+        for (int u1 = 0; u1 <= s && !found; u1++) {
+          const int i = a - 1 - u1, j = b + 1 + s - u1;
+          if (i < 1 || j > n) continue;
+          const int co = CO(i, j);
+          if (co >= BF_INF) continue;
+          if (v == co + bf_e_intloop(P, T, u1, s - u1, w.pt(i, j), bf_rtype(t), S[i + 1], S[j - 1], S[a - 1], S[b + 1])) {
+            a = i; b = j; v = co; found = true;
+          }
+        }
+      if (found) continue;
+      const int stem = (a > 1 && b < n) ? bf_e_mlstem(T, t, S[a - 1], S[b + 1]) : BF_INF;
+      for (int i = a - 1; i >= 1 && !found && stem < BF_INF; i--)
+        for (int j = b + 1; j <= n && !found; j++) {
+          const int co = CO(i, j);
+          if (co >= BF_INF) continue;
+          const int base = co + T.MLclosing + bf_e_mlstem(T, bf_rtype(w.pt(i, j)), S[j - 1], S[i + 1]) + stem;
+          const int lu = (a - 1 - i) * ml, lf = w.M(i + 1, a - 1), ru = (j - 1 - b) * ml, rf = w.M(b + 1, j - 1);
+          const int opt[3][2] = {{lf, ru}, {lu, rf}, {lf, rf}};
+          for (int k = 0; k < 3 && !found; k++) {
+            if (opt[k][0] >= BF_INF || opt[k][1] >= BF_INF || v != base + opt[k][0] + opt[k][1]) continue;
+            if (k != 1) open.push_back({i + 1, a - 1, 1});
+            if (k != 0) open.push_back({b + 1, j - 1, 1});
+            a = i; b = j; v = co; found = true;
+          }
+        }
+      if (!found) return -1;
+    }
+    // complete the open intervals optimally
+    std::vector<std::pair<int, std::string>> one;
+    int rest = 0;
+    for (const Iv &iv : open) rest += w.best(iv);
+    w.st = open; w.ss = ss; w.out = &one; w.thr = rest; w.found = 0; w.overflow = false;
+    w.rec(0, rest);
+    if (one.empty()) return -1;
+    const std::string &s1 = one[0].second;
+    std::vector<int> stk;
+    for (int k = 1; k <= n; k++) {
+      if (s1[k - 1] == '(') stk.push_back(k);
+      else if (s1[k - 1] == ')') { covered[(size_t)stk.back() * (n + 1) + k] = 1; stk.pop_back(); }
+    }
+    out->emplace_back(pr.e, s1);
+  }
   std::sort(out->begin(), out->end());
   return (int)out->size();
 }

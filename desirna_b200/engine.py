@@ -58,6 +58,9 @@ def lib():
         L.bf_subopt.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                 C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.bf_sample.argtypes = [C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p]
+        L.bf_pair_mfe.argtypes = [C.c_void_p, C.c_void_p]
+        L.bf_subopt_zuker.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),
+                                      C.POINTER(C.c_int32)]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
         L.bf_debug_copy_table.argtypes = [C.c_int, C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         _lib = L
@@ -180,6 +183,48 @@ def sample(seqs, n_samples, seed=0):
         raw = out[r, :, :n].tobytes().decode("ascii")
         res.append([raw[k * n:(k + 1) * n] for k in range(n_samples)])
     return res
+
+
+def pair_mfe(seqs, nopair=None):
+    """bf_pair_mfe: int32 [B, stride, stride], entry [i-1, j-1] (i < j) the lowest energy in dcal/mol of any structure of single-strand
+    sequence b that contains the pair (i,j) -- the matrix of Zuker suboptimals (RNAsubopt -z); 10000000 where no structure contains it
+    and on and below the diagonal.  nopair: optional uint8 [B, stride] mask ('x' hard constraint), honoured as by the MFE."""
+    ensure_ready()
+    buf, lens, cuts = pack([s.upper().replace("T", "U") for s in seqs])
+    b = bf_batch_t()
+    b.B, b.stride = len(seqs), buf.shape[1]
+    b.seq, b.len = buf.ctypes.data, lens.ctypes.data
+    b.cut = cuts.ctypes.data if cuts.any() else None
+    if nopair is not None:
+        nopair = np.ascontiguousarray(nopair, np.uint8)
+        assert nopair.shape == buf.shape
+        b.nopair = nopair.ctypes.data
+    out = np.zeros((len(seqs), b.stride, b.stride), np.int32)
+    _check(lib().bf_pair_mfe(C.byref(b), out.ctypes.data))
+    return out
+
+
+def subopt_zuker(seq, nopair=None):
+    """bf_subopt_zuker: Zuker suboptimals of one single-strand sequence, [(structure, energy_dcal)] sorted by (energy, structure):
+    for every pair (i,j) that some structure contains, a structure of energy E_pair(i,j) that contains it."""
+    ensure_ready()
+    s = seq.upper().replace("T", "U").encode("ascii")
+    n = len(s)
+    mask = None
+    if nopair is not None:
+        mask = np.ascontiguousarray(nopair, np.uint8)
+        assert mask.shape == (n,)
+    # one structure per uncovered pair: grow the buffer until every pair is covered
+    cap = 1024
+    while True:
+        ss = np.zeros((cap, n + 1), np.uint8)
+        en = np.zeros(cap, np.int32)
+        cnt, trunc = C.c_int32(0), C.c_int32(0)
+        _check(lib().bf_subopt_zuker(s, n, mask.ctypes.data if mask is not None else None, cap, ss.ctypes.data, en.ctypes.data,
+                                     C.byref(cnt), C.byref(trunc)))
+        if not trunc.value:
+            return [(bytes(ss[k, :n]).decode("ascii"), int(en[k])) for k in range(cnt.value)]
+        cap *= 8
 
 
 def set_option(key, value):

@@ -105,6 +105,27 @@ int bf_subopt(const char *seq, int32_t len, const uint8_t *nopair, int32_t delta
  * BF_ERR_UNAVAILABLE: a row with cut > 0, a nopair mask (the partition function ignores constraints), a stride outside the fill
  * path (> 2000) or BF_FORCE_GENERIC.  BF_ERR_ARG: n_samples < 1, null buffers, len > stride. */
 int bf_sample(const bf_batch_t *batch, int32_t n_samples, uint64_t seed, char *ss_out);
+/* E_pair: for every base pair (i,j) of every sequence of the batch (seq, len, nopair, stride as in bf_score_batch), the lowest
+ * free energy of any secondary structure that contains it -- the MFE fill, then an outside pass in the minimum-free-energy
+ * semiring over the fill's tables (RNAsubopt -z computes the same matrix).  Same energy model as BF_WANT_MFE: a nopair mask is
+ * honoured as the MFE honours it.  HOST buffers, synchronous.
+ * e_pair_out: B x stride x stride int32 in dcal/mol, entry [i-1][j-1] for i < j (the layout of bpp); 10000000 where (i,j)
+ * cannot pair (not canonical, j - i <= 3, a masked position) or no structure contains it, on and below the diagonal and
+ * beyond len.
+ * BF_ERR_UNAVAILABLE: a row with cut > 0, a stride outside the fill path (> 2000) or BF_FORCE_GENERIC.
+ * BF_ERR_ARG: null buffers, len > stride. */
+int bf_pair_mfe(const bf_batch_t *batch, int32_t *e_pair_out);
+/* fc.subopt_zuker() (vrna_subopt_zuker, RNAsubopt -z): Zuker suboptimals of ONE single-strand sequence.  The pairs with a finite
+ * E_pair (bf_pair_mfe) are taken in order of (E_pair, i, j); for each pair no structure listed so far contains, one structure of
+ * energy E_pair that contains it is appended (inside part traced back from the fill's c table, outside part from the outside
+ * pass).  Every pair with a finite E_pair is therefore in some listed structure.  Output sorted by (energy, structure string);
+ * ss_out: max_out x (len+1) chars, e_out: max_out energies in dcal/mol, *n_out: structures written, *truncated: 1 if pairs were
+ * left uncovered after max_out structures.  nopair: optional len bytes (hard constraint 'x').
+ * Which of several structures of equal energy is listed for a pair is a choice of the traceback; ViennaRNA may list another one
+ * (no ViennaRNA output pins it).
+ * BF_ERR_UNAVAILABLE: len outside the fill path (> 2000) or BF_FORCE_GENERIC.  BF_ERR_ARG: null buffers, len <= 0, max_out <= 0. */
+int bf_subopt_zuker(const char *seq, int32_t len, const uint8_t *nopair, int32_t max_out, char *ss_out, int32_t *e_out, int32_t *n_out,
+                    int32_t *truncated);
 
 /* device time (ms, CUDA events on the launch stream) of the mfe, pf and eval kernels of the most recent
  * bf_score_batch[_device] call; -1 for a kernel that did not run.  Blocks until those kernels finished. */
