@@ -14,6 +14,7 @@ DesiRNA.py:35).  A maintainer switches engines with `from desirna_b200 import RN
     fc.ensemble_defect(db)                        energy_scores.py:374
     fc.pbacktrack([num_samples]), RNA.init_rand(seed)   stochastic backtracking (not called by DesiRNA; ViennaRNA's API)
     fc.subopt_zuker()                             Zuker suboptimals (not called by DesiRNA; ViennaRNA's API)
+    RNA.duplexfold(s1, s2)                        RNA-RNA hybridization, RNAduplex (not called by DesiRNA; ViennaRNA's API)
     RNA.fold(seq) / RNA.co_pf_fold(seq)           energy_scores.py:354; dimer_multichain_energy.py:109, 113-114
 
 Conventions kept: energies come back as Python floats holding float32-rounded kcal/mol (ViennaRNA returns C
@@ -254,6 +255,38 @@ class subopt_solution:
 
     def __repr__(self):
         return "subopt_solution(%r, %r)" % (self.structure, self.energy)
+
+
+class duplexT:
+    """result of RNA.duplexfold(), in ViennaRNA's duplexT convention as recalled (no ViennaRNA output pins it here):
+    .structure  'a-part&b-part', trimmed to the paired region plus one flanking nucleotide on each side where one exists;
+    .i          last position of the a-part, 1-based;
+    .j          first position of the b-part, 1-based;
+    .energy     kcal/mol (double)"""
+
+    def __init__(self, structure, energy, i, j):
+        self.structure = structure
+        self.energy = energy
+        self.i = i
+        self.j = j
+
+    def __repr__(self):
+        return "duplexT(%r, %r, i=%d, j=%d)" % (self.structure, self.energy, self.i, self.j)
+
+
+def duplexfold(s1, s2):
+    """vrna_duplexfold: the lowest-energy structure of strands s1 and s2 made of intermolecular pairs only (bf_duplex).  With no
+    possible intermolecular pair: the untrimmed all-dot structure, i = len(s1), j = 1 and energy 100000.0."""
+    e, ss = _eng.duplex([s1], [s2], pairs=[(0, 0)])
+    e, ss = int(e[0]), ss[0]
+    n1, n2 = len(s1), len(s2)
+    if e >= _eng.INF_DCAL:
+        return duplexT(ss, e / 100.0, n1, 1)
+    pa, pb = ss[:n1], ss[n1 + 1:]
+    # 1-based bounds: the paired region and one flanking nucleotide on each side where one exists
+    a0, a1 = max(pa.index("("), 1), min(pa.rindex("(") + 2, n1)
+    b0, b1 = max(pb.index(")"), 1), min(pb.rindex(")") + 2, n2)
+    return duplexT(pa[a0 - 1:a1] + "&" + pb[b0 - 1:b1], e / 100.0, a1, b0)
 
 
 def fold(sequence):

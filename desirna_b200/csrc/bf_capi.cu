@@ -105,6 +105,8 @@ struct Engine {
   DevBuf d_seq, d_len, d_cut, d_nopair, d_targets, d_mfe, d_ss, d_pf, d_eval, d_defect, d_bpp;
   DevBuf d_q5, d_samples;  // bf_sample: exterior prefixes, drawn structures
   DevBuf d_epair;          // bf_pair_mfe: E_pair of every sequence
+  // bf_duplex: strands, pair list, per-pair c-table offsets, c tables / HBM rings, energies, structures
+  DevBuf d_dxa, d_dxb, d_dxlen, d_dxpairs, d_dxoff, d_dxws, d_dxe, d_dxss;
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -342,7 +344,8 @@ int bf_shutdown(void) {
   if (!g.inited) return BF_OK;
   cudaStreamSynchronize(g.stream);
   for (DevBuf *b : {&g.d_defect, &g.d_bpp, &g.d_seq, &g.d_len, &g.d_cut, &g.d_nopair, &g.d_targets, &g.d_mfe, &g.d_ss, &g.d_pf, &g.d_eval, &g.d_in, &g.d_out, &g.d_zero,
-                    &g.d_q5, &g.d_samples, &g.d_epair}) b->release();
+                    &g.d_q5, &g.d_samples, &g.d_epair, &g.d_dxa, &g.d_dxb, &g.d_dxlen, &g.d_dxpairs, &g.d_dxoff, &g.d_dxws, &g.d_dxe,
+                    &g.d_dxss}) b->release();
   if (g.h_in) cudaFreeHost(g.h_in);
   if (g.h_out) cudaFreeHost(g.h_out);
   g.h_in = g.h_out = nullptr; g.h_in_cap = g.h_out_cap = g.zero_cap = 0;
@@ -643,6 +646,120 @@ int bf_pair_mfe(const bf_batch_t *b, int32_t *e_pair_out) {
   g.launches++;
   CU(cudaMemcpyAsync(e_pair_out, g.d_epair.p, B * S * S * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e_pair");
   CU(cudaStreamSynchronize(st), "bf_pair_mfe");
+  return BF_OK;
+}
+
+namespace {
+constexpr int kDuplexMaxLen = 2000;                   // per strand, as for the fill path
+constexpr int kDuplexMaxStride = 1 << 16;             // bytes per strand row: keeps a structure slot far below the per-launch budget
+constexpr long long kDuplexChunk = 1 << 16;           // pairs per launch at most
+constexpr size_t kDuplexWsInts = (size_t)64 << 20;    // c tables / HBM rings of one launch: 256 MB
+constexpr size_t kDuplexSsBytes = (size_t)256 << 20;  // structures of one launch
+
+int check_strands(const bf_strands_t &s) {
+  if (s.n < 0 || s.stride <= 0 || s.stride > kDuplexMaxStride || (s.n && (!s.seq || !s.len))) return fail(BF_ERR_ARG, "bf_duplex: bad strand set");
+  for (int k = 0; k < s.n; k++) {
+    if (s.len[k] < 0 || s.len[k] > s.stride) return fail(BF_ERR_ARG, "bf_duplex: strand length exceeds stride");
+    if (s.len[k] > kDuplexMaxLen) return fail(BF_ERR_ARG, "bf_duplex: strand longer than 2000 nt");
+  }
+  return BF_OK;
+}
+}  // namespace
+
+int bf_duplex(const bf_duplex_t *q, int32_t *e_dcal, char *ss_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!q || !e_dcal || (q->pairs && q->n_pairs < 0)) return fail(BF_ERR_ARG, "bf_duplex: bad argument");
+  int rc = check_strands(q->a);
+  if (!rc) rc = check_strands(q->b);
+  if (rc) return rc;
+  const long long P = q->pairs ? q->n_pairs : (long long)q->a.n * q->b.n;
+  if (q->pairs)
+    for (long long p = 0; p < P; p++)
+      if (q->pairs[2 * p] < 0 || q->pairs[2 * p] >= q->a.n || q->pairs[2 * p + 1] < 0 || q->pairs[2 * p + 1] >= q->b.n)
+        return fail(BF_ERR_ARG, "bf_duplex: pair index out of range");
+  if (P == 0) return BF_OK;
+  const bool want_ss = ss_out != nullptr;
+  const int sa = q->a.stride, sb = q->b.stride, ss_stride = sa + sb + 2;
+  auto len_of = [&](long long p, int *n1, int *n2) {
+    const int ia = q->pairs ? q->pairs[2 * p] : (int)(p / q->b.n), ib = q->pairs ? q->pairs[2 * p + 1] : (int)(p % q->b.n);
+    *n1 = q->a.len[ia]; *n2 = q->b.len[ib];
+  };
+  BfDuplexDev d;
+  d.stride_a = sa; d.stride_b = sb; d.nb = q->b.n;
+  d.amax = *std::max_element(q->a.len, q->a.len + q->a.n);
+  d.bmax = *std::max_element(q->b.len, q->b.len + q->b.n);
+  if (q->pairs) {
+    d.ring_w = 0;
+    for (long long p = 0; p < P; p++) { int n1, n2; len_of(p, &n1, &n2); d.ring_w = std::max(d.ring_w, std::min(n1, n2)); }
+  } else {
+    d.ring_w = std::min(d.amax, d.bmax);
+  }
+  const bool gring = bf_duplex_gring(d);
+  const size_t ring_slot = bf_duplex_ring_slot(d.ring_w);
+  cudaStream_t st = g.stream;
+  CU(g.d_dxa.reserve((size_t)q->a.n * sa), "cudaMalloc(duplex a)");
+  CU(g.d_dxb.reserve((size_t)q->b.n * sb), "cudaMalloc(duplex b)");
+  CU(g.d_dxlen.reserve((size_t)(q->a.n + q->b.n) * sizeof(int)), "cudaMalloc(duplex len)");
+  CU(cudaMemcpyAsync(g.d_dxa.p, q->a.seq, (size_t)q->a.n * sa, cudaMemcpyHostToDevice, st), "H2D duplex a");
+  CU(cudaMemcpyAsync(g.d_dxb.p, q->b.seq, (size_t)q->b.n * sb, cudaMemcpyHostToDevice, st), "H2D duplex b");
+  int *dlen = (int *)g.d_dxlen.p;
+  CU(cudaMemcpyAsync(dlen, q->a.len, q->a.n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D duplex len a");
+  CU(cudaMemcpyAsync(dlen + q->a.n, q->b.len, q->b.n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D duplex len b");
+  d.seq_a = (const char *)g.d_dxa.p; d.seq_b = (const char *)g.d_dxb.p;
+  d.len_a = dlen; d.len_b = dlen + q->a.n;
+  d.pairs = nullptr;
+  if (q->pairs) {
+    CU(g.d_dxpairs.reserve((size_t)P * 2 * sizeof(int)), "cudaMalloc(duplex pairs)");
+    CU(cudaMemcpyAsync(g.d_dxpairs.p, q->pairs, (size_t)P * 2 * sizeof(int), cudaMemcpyHostToDevice, st), "H2D duplex pairs");
+    d.pairs = (const int *)g.d_dxpairs.p;
+  }
+  // chunks of consecutive pairs whose c tables (structures) or HBM rings fit the workspace budget
+  const long long cap = want_ss ? std::min<long long>(kDuplexChunk, (long long)(kDuplexSsBytes / ss_stride)) : kDuplexChunk;
+  std::vector<long long> off;
+  for (long long p0 = 0; p0 < P;) {
+    long long p1 = p0;
+    size_t ws = 0, used = 0;   // c-table ints; c tables and rings
+    off.clear();
+    if (want_ss || gring) {
+      while (p1 < P && p1 - p0 < cap) {
+        int n1, n2;
+        len_of(p1, &n1, &n2);
+        const size_t tab = want_ss ? (size_t)n1 * n2 : 0, need = tab + (gring ? ring_slot : 0);
+        if (p1 > p0 && used + need > kDuplexWsInts) break;
+        if (want_ss) off.push_back((long long)ws);
+        ws += tab;
+        used += need;
+        p1++;
+      }
+    } else {
+      p1 = std::min(P, p0 + cap);
+    }
+    const int np = (int)(p1 - p0);
+    int *ctab = nullptr, *gws = nullptr;
+    const long long *doff = nullptr;
+    if (want_ss || gring) {
+      CU(g.d_dxws.reserve((ws + (gring ? (size_t)np * ring_slot : 0)) * sizeof(int)), "cudaMalloc(duplex workspace)");
+      gws = (int *)g.d_dxws.p;
+      if (want_ss) {
+        ctab = gws + (gring ? (size_t)np * ring_slot : 0);
+        CU(g.d_dxoff.reserve(off.size() * sizeof(long long)), "cudaMalloc(duplex offsets)");
+        CU(cudaMemcpyAsync(g.d_dxoff.p, off.data(), off.size() * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D duplex offsets");
+        doff = (const long long *)g.d_dxoff.p;
+      }
+    }
+    CU(g.d_dxe.reserve((size_t)np * sizeof(int)), "cudaMalloc(duplex energies)");
+    if (want_ss) CU(g.d_dxss.reserve((size_t)np * ss_stride), "cudaMalloc(duplex structures)");
+    d.p0 = p0; d.np = np;
+    CU(bf_launch_duplex(g.dP, d, gring, gws, (int *)g.d_dxe.p, ctab, doff, want_ss ? (char *)g.d_dxss.p : nullptr, ss_stride, st),
+       "launch bf_k_duplex");
+    g.launches++;
+    CU(cudaMemcpyAsync(e_dcal + p0, g.d_dxe.p, (size_t)np * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H duplex energies");
+    if (want_ss)
+      CU(cudaMemcpyAsync(ss_out + (size_t)p0 * ss_stride, g.d_dxss.p, (size_t)np * ss_stride, cudaMemcpyDeviceToHost, st), "D2H duplex structures");
+    p0 = p1;
+  }
+  CU(cudaStreamSynchronize(st), "bf_duplex");
   return BF_OK;
 }
 

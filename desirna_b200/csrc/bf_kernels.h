@@ -119,6 +119,26 @@ cudaError_t bf_launch_mfe_out(const BfPlan &p, const BfParams *dP, const BfBatch
 cudaError_t bf_launch_sample(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, const double *lnscale, double *q5,
                              int n_samples, unsigned long long seed, char *ss_out, int sms, cudaStream_t st);
 
+// ---- RNA-RNA hybridization (bf_duplex.cu): duplex MFE of np pairs (a strand, b strand), pairs p0 .. p0 + np - 1 of the call
+struct BfDuplexDev {
+  const char *seq_a, *seq_b;   // strands, rows of stride_a / stride_b bytes
+  int stride_a, stride_b;
+  const int *len_a, *len_b;
+  const int *pairs;            // 2 per pair (index into a, index into b), or null: the grid, pair p = (p / nb, p % nb)
+  int nb;
+  long long p0;
+  int np;
+  int amax, bmax;              // longest a / b strand of the launch
+  int ring_w;                  // largest min(len a, len b) of the launch: the ring's width
+};
+// true: the c ring of this launch does not fit shared memory and lives in HBM, bf_duplex_ring_slot(ring_w) ints per pair
+bool bf_duplex_gring(const BfDuplexDev &d);
+size_t bf_duplex_ring_slot(int ring_w);
+// e_out: np energies (BF_INF: no pair possible).  ss_out (null: energies only): np x ss_stride chars, a's characters, '&', b's, NUL;
+// then ctab holds each pair's n1 x n2 c table at ctab_off[pair - p0] ints.
+cudaError_t bf_launch_duplex(const BfParams *dP, const BfDuplexDev &d, bool gring, int *gring_ws, int *e_out, int *ctab,
+                             const long long *ctab_off, char *ss_out, int ss_stride, cudaStream_t st);
+
 // ---- suboptimal structures (bf_subopt.cu): host walk over the c / fML tables of the GPU fill
 #ifdef __cplusplus
 #include <string>

@@ -34,6 +34,14 @@ class bf_result_t(C.Structure):
                 ("eval_dcal", C.c_void_p), ("defect", C.c_void_p), ("bpp", C.c_void_p)]
 
 
+class bf_strands_t(C.Structure):
+    _fields_ = [("n", C.c_int32), ("stride", C.c_int32), ("seq", C.c_void_p), ("len", C.c_void_p)]
+
+
+class bf_duplex_t(C.Structure):
+    _fields_ = [("a", bf_strands_t), ("b", bf_strands_t), ("n_pairs", C.c_int32), ("pairs", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -61,6 +69,7 @@ def lib():
         L.bf_pair_mfe.argtypes = [C.c_void_p, C.c_void_p]
         L.bf_subopt_zuker.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]
+        L.bf_duplex.argtypes = [C.POINTER(bf_duplex_t), C.c_void_p, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
         L.bf_debug_copy_table.argtypes = [C.c_int, C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         _lib = L
@@ -225,6 +234,43 @@ def subopt_zuker(seq, nopair=None):
         if not trunc.value:
             return [(bytes(ss[k, :n]).decode("ascii"), int(en[k])) for k in range(cnt.value)]
         cap *= 8
+
+
+def duplex(seqs_a, seqs_b, pairs=None, structures=True):
+    """bf_duplex: RNA-RNA hybridization (ViennaRNA's duplexfold recurrence, RNAduplex), intermolecular pairs only.  The duplex MFE
+    in dcal/mol of every requested pair of strands (10000000: no intermolecular pair is possible).  pairs: [(index into seqs_a,
+    index into seqs_b)], or None for the full grid.  Returns int32 energies, shape [P] or [len(seqs_a), len(seqs_b)] for the grid;
+    with structures, (energies, structures): 'a-part&b-part' strings, full length, '(' in a and ')' in b, in the same layout (a
+    list, or a list of rows for the grid).  Each strand holds at most 2000 nt; T is read as U."""
+    if any("&" in s for s in seqs_a) or any("&" in s for s in seqs_b):
+        raise ValueError("engine.duplex: a strand may not contain '&' (pass the two strands separately)")
+    ensure_ready()
+    q = bf_duplex_t()
+    keep = []
+    for st, seqs in ((q.a, seqs_a), (q.b, seqs_b)):
+        buf, lens, _ = pack([s.upper().replace("T", "U") for s in seqs])
+        st.n, st.stride, st.seq, st.len = len(seqs), buf.shape[1], buf.ctypes.data, lens.ctypes.data
+        keep += [buf, lens]
+    la, lb = keep[1], keep[3]
+    if pairs is None:
+        P, shape = len(seqs_a) * len(seqs_b), (len(seqs_a), len(seqs_b))
+        ia, ib = np.repeat(np.arange(len(seqs_a)), len(seqs_b)), np.tile(np.arange(len(seqs_b)), len(seqs_a))
+    else:
+        pr = np.ascontiguousarray(np.asarray(pairs, np.int32).reshape(-1, 2))
+        P, shape = pr.shape[0], (pr.shape[0],)
+        q.n_pairs, q.pairs = P, pr.ctypes.data
+        keep.append(pr)
+        ia, ib = pr[:, 0], pr[:, 1]
+    e = np.zeros(P, np.int32)
+    ss = np.zeros((P, q.a.stride + q.b.stride + 2), np.uint8) if structures else None
+    _check(lib().bf_duplex(C.byref(q), e.ctypes.data, ss.ctypes.data if structures else None))
+    e = e.reshape(shape)
+    if not structures:
+        return e
+    out = [bytes(ss[p, :int(la[ia[p]]) + int(lb[ib[p]]) + 1]).decode("ascii") for p in range(P)]
+    if pairs is None:
+        out = [out[r * len(seqs_b):(r + 1) * len(seqs_b)] for r in range(len(seqs_a))]
+    return e, out
 
 
 def set_option(key, value):

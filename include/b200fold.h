@@ -127,6 +127,32 @@ int bf_pair_mfe(const bf_batch_t *batch, int32_t *e_pair_out);
 int bf_subopt_zuker(const char *seq, int32_t len, const uint8_t *nopair, int32_t max_out, char *ss_out, int32_t *e_out, int32_t *n_out,
                     int32_t *truncated);
 
+/* RNA.duplexfold(s1, s2) / RNAduplex: RNA-RNA hybridization, counting intermolecular pairs only (not called by DesiRNA).
+ * For every requested (a, b) pair of strands, the lowest energy of a duplex structure: a chain of pairs a[k]-b[l], canonical,
+ * k increasing and l decreasing, with at most 30 unpaired nucleotides between consecutive pairs, scored as bf_score_batch's
+ * two-strand eval scores that structure on a&b (DuplexInit, the outer exterior stem, interior loops, the nick loop closed by the
+ * innermost pair).  This is ViennaRNA's duplexfold recurrence as published; no ViennaRNA output pins it here.
+ * Ties: the innermost pair is the first minimum in the order i (in a) ascending, then j (in b) descending; the backtrack from
+ * (i,j) takes the first (k,l) that reproduces the energy, k = i-1 downwards, then l = j+1 upwards.
+ * pairs: n_pairs x 2 (index into a, index into b), or NULL for the full grid a.n x b.n, a-major (n_pairs is then ignored).
+ * e_dcal: one energy per pair in dcal/mol; 10000000 where no intermolecular pair is possible.
+ * ss_out: NULL (energies only) or per pair a.stride + b.stride + 2 chars: a's len characters, '&', b's len characters, NUL
+ * (the rest of the slot NUL too).  Pairs are '(' in a and ')' in b, full length, not trimmed; all dots where there is no pair.
+ * HOST buffers, synchronous.  BF_ERR_ARG: null buffers, len < 0 or > stride, a strand longer than 2000 nt, a pair index out of
+ * range, n_pairs < 0, a stride above 65536. */
+typedef struct {
+  int32_t n;           /* strands */
+  int32_t stride;      /* bytes between consecutive rows of seq, >= every len, <= 65536 */
+  const char *seq;     /* n x stride ASCII ACGU (T accepted) */
+  const int32_t *len;  /* n lengths, 0 .. 2000 */
+} bf_strands_t;
+typedef struct {
+  bf_strands_t a, b;
+  int32_t n_pairs;
+  const int32_t *pairs;
+} bf_duplex_t;
+int bf_duplex(const bf_duplex_t *q, int32_t *e_dcal, char *ss_out);
+
 /* device time (ms, CUDA events on the launch stream) of the mfe, pf and eval kernels of the most recent
  * bf_score_batch[_device] call; -1 for a kernel that did not run.  Blocks until those kernels finished. */
 int bf_last_kernel_ms(double out[3]);
