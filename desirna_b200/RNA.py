@@ -15,6 +15,8 @@ DesiRNA.py:35).  A maintainer switches engines with `from desirna_b200 import RN
     fc.pbacktrack([num_samples]), RNA.init_rand(seed)   stochastic backtracking (not called by DesiRNA; ViennaRNA's API)
     fc.subopt_zuker()                             Zuker suboptimals (not called by DesiRNA; ViennaRNA's API)
     RNA.duplexfold(s1, s2)                        RNA-RNA hybridization, RNAduplex (not called by DesiRNA; ViennaRNA's API)
+    RNA.pfl_fold_up(seq, ulength, W, L)           accessibility, RNAplfold -u (not called by DesiRNA; ViennaRNA's API; conventions recalled)
+    RNA.pfl_fold(seq, W, L, cutoff)               RNAplfold pair probabilities (not called by DesiRNA; ViennaRNA's API; conventions recalled)
     RNA.fold(seq) / RNA.co_pf_fold(seq)           energy_scores.py:354; dimer_multichain_energy.py:109, 113-114
 
 Conventions kept: energies come back as Python floats holding float32-rounded kcal/mol (ViennaRNA returns C
@@ -287,6 +289,53 @@ def duplexfold(s1, s2):
     a0, a1 = max(pa.index("("), 1), min(pa.rindex("(") + 2, n1)
     b0, b1 = max(pb.index(")"), 1), min(pb.rindex(")") + 2, n2)
     return duplexT(pa[a0 - 1:a1] + "&" + pb[b0 - 1:b1], e / 100.0, a1, b0)
+
+
+def _plfold_span(sequence, window_size, max_bp_span):
+    n = len(sequence)
+    W, L = min(int(window_size), n), min(int(max_bp_span), n)
+    if W != L:
+        raise NotImplementedError("RNAplfold with a maximum base-pair span below the window size is not supported (L must equal W)")
+    return W
+
+
+def pfl_fold_up(sequence, ulength, window_size, max_bp_span):
+    """RNAplfold -u (ViennaRNA RNA.pfl_fold_up), span = window: n+1 lists of ulength+1 floats, [i][u] the window-averaged probability
+    that the u nucleotides ending at i (i-u+1 .. i, 1-based) are unpaired.  Row 0, column 0 and entries with u > i are 0.0.  This
+    pU layout is ViennaRNA's as recalled; no ViennaRNA output pins it here."""
+    n, U = len(sequence), int(ulength)
+    out = [[0.0] * (U + 1) for _ in range(n + 1)]
+    if n == 0 or U < 1:
+        return out
+    W = _plfold_span(sequence, window_size, max_bp_span)
+    mu = min(U, W, n)
+    _, pu = _eng.plfold([sequence], W, mu, pairs=False)[0]
+    for i in range(1, n + 1):
+        row = out[i]
+        for u in range(1, min(mu, i) + 1):
+            row[u] = float(pu[i - u, u - 1])
+    return out
+
+
+class ep:
+    """one pair probability of RNA.pfl_fold: .i < .j (1-based), .p, .type (0: a base pair)"""
+
+    def __init__(self, i, j, p, type=0):
+        self.i, self.j, self.p, self.type = i, j, p, type
+
+    def __repr__(self):
+        return f"ep({self.i}, {self.j}, {self.p:.6g})"
+
+
+def pfl_fold(sequence, w, L, cutoff):
+    """RNAplfold pair probabilities (ViennaRNA RNA.pfl_fold), span = window: the pairs whose window-averaged probability is at least
+    cutoff, as ep objects in (i, j) order.  Conventions recalled; no ViennaRNA output pins them here."""
+    n = len(sequence)
+    if n == 0:
+        return []
+    W = _plfold_span(sequence, w, L)
+    band, _ = _eng.plfold([sequence], W, 1, pairs=True)[0]
+    return [ep(i + 1, i + 1 + d, float(band[i, d])) for i in range(n) for d in range(band.shape[1]) if band[i, d] > 0.0 and band[i, d] >= cutoff]
 
 
 def fold(sequence):

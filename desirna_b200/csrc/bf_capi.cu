@@ -18,7 +18,7 @@
 // choice is made (BF_FORCE_GENERIC at bf_init, BF_DESIGN_OVERLAP at bf_design_create, the others at every call), so that a host
 // program can flip them between calls on one engine.
 static const char *const kOptions[] = {"BF_CL", "BF_CL_C", "BF_CL_BW", "BF_EXT_WIDE", "BF_WIDE", "BF_FILL3", "BF_FILL3_SMALL",
-                                       "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP"};
+                                       "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP", "BF_PLFOLD_MB"};
 
 int bf_opt(const char *name, int dflt) {
   const char *v = getenv(name);
@@ -105,6 +105,8 @@ struct Engine {
   DevBuf d_seq, d_len, d_cut, d_nopair, d_targets, d_mfe, d_ss, d_pf, d_eval, d_defect, d_bpp;
   DevBuf d_q5, d_samples;  // bf_sample: exterior prefixes, drawn structures
   DevBuf d_epair;          // bf_pair_mfe: E_pair of every sequence
+  // bf_unpaired / bf_plfold: kept outside triangles, bf_k_unpaired's workspace, P_u of every row; per-strand window tables, averages
+  DevBuf d_keep, d_upws, d_pu, d_pfstr, d_pfbpp, d_pfpu;
   // bf_duplex: strands, pair list, per-pair c-table offsets, c tables / HBM rings, energies, structures
   DevBuf d_dxa, d_dxb, d_dxlen, d_dxpairs, d_dxoff, d_dxws, d_dxe, d_dxss;
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
@@ -156,8 +158,10 @@ int validate(const bf_batch_t *b, const bf_result_t *r) {
 // runs on the workspace's second stream beside the MFE fill -- worth it when both grids fit the GPU together (small batches).
 // keep_qm: keep the per-sequence qm / qm1 tables (w.qm_seq) of the PF fill for a pass that reads them after this call (bf_sample);
 // the outside pass (BF_WANT_BPP / BF_WANT_DEFECT) keeps them in any case.
+// keep_out (device, B x 3 x bf_tri_slot doubles): run the outside pass and keep its bqb / bqm / qm1-outside triangles (bf_unpaired).
+// plan_B > 0: choose the kernels as for a batch of plan_B rows (bf_plfold: every chunk of a call runs the same kernels).
 int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two, cudaStream_t st, const int *scale_override = nullptr,
-               bool timing = true, bool keep_qm = false) {
+               bool timing = true, bool keep_qm = false, double *keep_out = nullptr, int plan_B = 0) {
   if (b->B == 0) return BF_OK;
   BfBatchDev db;
   db.B = b->B; db.stride = b->stride; db.seq = b->seq; db.len = b->len; db.cut = b->cut; db.nopair = b->nopair;
@@ -182,7 +186,7 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     if (!out_mfe) { CU(w.d_mfe_scratch.reserve((size_t)b->B * sizeof(int)), "cudaMalloc(mfe scratch)"); out_mfe = (int *)w.d_mfe_scratch.p; }
     char *out_ss = (b->want & BF_WANT_SS) ? r->mfe_ss : nullptr;
     BfPlan p;
-    CU(bf_plan_mfe(b->stride, b->B, two, g.force_generic, g.sm_count, &p), "plan the MFE fill");
+    CU(bf_plan_mfe(b->stride, plan_B > 0 ? plan_B : b->B, two, g.force_generic, g.sm_count, &p), "plan the MFE fill");
     if (timing) cudaEventRecord(w.ev[0], st);
     if (p.family != BF_FAM_GENERIC) {
       const size_t slot = bf_tri_slot(b->stride) * sizeof(int);
@@ -211,11 +215,11 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
     w.ran[0] = timing;
     mfe_for_scale = out_mfe;
   }
-  const bool want_out = (b->want & (BF_WANT_BPP | BF_WANT_DEFECT)) != 0;
+  const bool want_out = (b->want & (BF_WANT_BPP | BF_WANT_DEFECT)) != 0 || keep_out;
   const bool want_qm = want_out || keep_qm;
   if ((b->want & BF_WANT_PF) || want_out) {
     BfPlan p;
-    CU(bf_plan_pf(b->stride, b->B, two, g.force_generic, g.sm_count, &p), "plan the PF fill");
+    CU(bf_plan_pf(b->stride, plan_B > 0 ? plan_B : b->B, two, g.force_generic, g.sm_count, &p), "plan the PF fill");
     if (want_qm && p.family == BF_FAM_GENERIC)
       return fail(BF_ERR_UNAVAILABLE, want_out ? "base-pair probabilities / ensemble defect: single-strand sequences within the fill path's length range only"
                                                : "sampling: single-strand sequences within the fill path's length range only");
@@ -249,13 +253,13 @@ int run_device(Workspace &w, const bf_batch_t *b, const bf_result_t *r, bool two
       }
       if (want_out) {
         BfPlan po;
-        CU(bf_plan_out(b->stride, b->B, g.sm_count, &po), "plan bf_k_pf_out");
+        CU(bf_plan_out(b->stride, plan_B > 0 ? plan_B : b->B, g.sm_count, &po, keep_out != nullptr), "plan bf_k_pf_out");
         CU(w.ws_out.reserve((size_t)po.grid * po.ws * sizeof(double)), "cudaMalloc(outside workspace)");
         if (b->want & BF_WANT_BPP) CU(cudaMemsetAsync(r->bpp, 0, (size_t)b->B * b->stride * b->stride * sizeof(double), st), "clear bpp");
         CU(bf_launch_pf_out(po, g.dP, dbp, (const double *)w.tri_qb.p, qmseq, (double *)w.ws_out.p, (const double *)w.d_lnscale.p,
                             (b->want & BF_WANT_DEFECT) ? b->targets : nullptr, b->n_targets, b->stride,
                             (b->want & BF_WANT_DEFECT) ? r->defect : nullptr, (b->want & BF_WANT_BPP) ? r->bpp : nullptr,
-                            w.d_counters + 2, st), "launch bf_k_pf_out");
+                            w.d_counters + 2, st, keep_out), "launch bf_k_pf_out");
         g.launches++;
       }
     } else {
@@ -646,6 +650,143 @@ int bf_pair_mfe(const bf_batch_t *b, int32_t *e_pair_out) {
   g.launches++;
   CU(cudaMemcpyAsync(e_pair_out, g.d_epair.p, B * S * S * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H e_pair");
   CU(cudaStreamSynchronize(st), "bf_pair_mfe");
+  return BF_OK;
+}
+
+namespace {
+// The accessibility pipeline on a batch already on the device (seq, len, stride): MFE (it sets the scale), PF fill with qm / qm1 kept,
+// the outside pass keeping its triangles in g.d_keep, then bf_k_unpaired into d_pu when d_pu is not null.  plan_B: as for run_device.
+int unpaired_device(const bf_batch_t *db, int max_u, double *d_pu, cudaStream_t st, int plan_B = 0) {
+  const size_t B = db->B, S = db->stride;
+  CU(g.d_mfe.reserve(B * sizeof(int)), "cudaMalloc(mfe)");
+  CU(g.d_pf.reserve(B * 5 * sizeof(double)), "cudaMalloc(pf)");
+  CU(g.d_keep.reserve(B * 3 * bf_tri_slot(db->stride) * sizeof(double)), "cudaMalloc(outside triangles)");
+  bf_result_t dr;
+  memset(&dr, 0, sizeof(dr));
+  dr.mfe_dcal = (int32_t *)g.d_mfe.p; dr.pf = (double *)g.d_pf.p;
+  int rc = run_device(g.w, db, &dr, false, st, nullptr, true, true, (double *)g.d_keep.p, plan_B);
+  if (rc || !d_pu) return rc;
+  const size_t slot = bf_unpaired_ws_bytes(db->stride);
+  const size_t ws = std::min<size_t>(std::min<size_t>(B, 8 * (size_t)g.sm_count) * slot, std::max<size_t>(slot, (size_t)1 << 30));
+  CU(g.d_upws.reserve(ws), "cudaMalloc(unpaired workspace)");
+  CU(cudaMemsetAsync(d_pu, 0, B * S * max_u * sizeof(double), st), "clear pu");
+  BfBatchDev dev;
+  dev.B = db->B; dev.stride = db->stride; dev.seq = db->seq; dev.len = db->len; dev.cut = nullptr; dev.nopair = nullptr;
+  CU(bf_launch_unpaired(g.dP, dev, (const double *)g.w.tri_qb.p, (const double *)g.w.qm_seq.p, (const double *)g.d_keep.p,
+                        (const double *)g.w.d_lnscale.p, (double *)g.d_upws.p, ws, max_u, d_pu, g.w.d_counters + 3, g.sm_count, st),
+     "launch bf_k_unpaired");
+  g.launches++;
+  return BF_OK;
+}
+}  // namespace
+
+int bf_unpaired(const bf_batch_t *b, int32_t max_u, double *pu_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!b || !pu_out || b->B < 0 || b->stride <= 0 || (b->B && (!b->seq || !b->len))) return fail(BF_ERR_ARG, "bf_unpaired: bad argument");
+  if (max_u < 1 || max_u > b->stride) return fail(BF_ERR_ARG, "bf_unpaired: max_u outside 1 .. stride");
+  if (any_cut(b, b->cut)) return fail(BF_ERR_UNAVAILABLE, "bf_unpaired: single strands only");
+  if (b->nopair) return fail(BF_ERR_UNAVAILABLE, "bf_unpaired: the partition function does not honour hard constraints");
+  if (g.force_generic || bf_fill_pf_mode(b->stride) == 0) return fail(BF_ERR_UNAVAILABLE, "bf_unpaired: stride outside the fill path");
+  for (int i = 0; i < b->B; i++)
+    if (b->len[i] < 0 || b->len[i] > b->stride) return fail(BF_ERR_ARG, "sequence length exceeds stride");
+  if (b->B == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  const size_t B = b->B, S = b->stride;
+  CU(g.d_seq.reserve(B * S), "cudaMalloc(seq)");
+  CU(g.d_len.reserve(B * sizeof(int)), "cudaMalloc(len)");
+  CU(g.d_pu.reserve(B * S * max_u * sizeof(double)), "cudaMalloc(pu)");
+  CU(cudaMemcpyAsync(g.d_seq.p, b->seq, B * S, cudaMemcpyHostToDevice, st), "H2D seq");
+  CU(cudaMemcpyAsync(g.d_len.p, b->len, B * sizeof(int), cudaMemcpyHostToDevice, st), "H2D len");
+  bf_batch_t db;
+  memset(&db, 0, sizeof(db));
+  db.B = b->B; db.stride = b->stride; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
+  db.want = BF_WANT_MFE | BF_WANT_PF;
+  int rc = unpaired_device(&db, max_u, (double *)g.d_pu.p, st);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(pu_out, g.d_pu.p, B * S * max_u * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H pu");
+  CU(cudaStreamSynchronize(st), "bf_unpaired");
+  return BF_OK;
+}
+
+int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp_out, double *pu_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!s || (!bpp_out && !pu_out) || s->n < 0 || s->stride <= 0 || (s->n && (!s->seq || !s->len))) return fail(BF_ERR_ARG, "bf_plfold: bad argument");
+  for (int r = 0; r < s->n; r++)
+    if (s->len[r] < 0 || s->len[r] > s->stride) return fail(BF_ERR_ARG, "bf_plfold: strand length exceeds stride");
+  if (winsize < 1 || max_u < 1 || max_u > winsize) return fail(BF_ERR_ARG, "bf_plfold: winsize < 1 or max_u outside 1 .. winsize");
+  if (winsize > 2000) return fail(BF_ERR_UNAVAILABLE, "bf_plfold: window longer than 2000 nt");
+  if (g.force_generic) return fail(BF_ERR_UNAVAILABLE, "bf_plfold: BF_FORCE_GENERIC");
+  const int n = s->n, S = s->stride;
+  // windows: strand r has nwin = len - W' + 1 of length W' = min(W, len), global indices win0[r] .. win0[r] + nwin - 1
+  std::vector<int> tab(3 * (size_t)n);   // len, win0, wlen
+  long long total = 0;
+  int wstride = 1;
+  for (int r = 0; r < n; r++) {
+    const int len = s->len[r], wl = std::min<int>(winsize, len);
+    if (total > INT32_MAX - len) return fail(BF_ERR_ARG, "bf_plfold: more than 2^31 windows");
+    tab[r] = len; tab[n + r] = (int)total; tab[2 * n + r] = wl;
+    total += len > 0 ? len - wl + 1 : 0;
+    wstride = std::max(wstride, wl);
+  }
+  if (bf_fill_pf_mode(wstride) == 0) return fail(BF_ERR_UNAVAILABLE, "bf_plfold: window longer than the PF fill path covers");
+  if (n == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  const size_t bpp_bytes = (size_t)n * S * winsize * sizeof(double), pu_bytes = (size_t)n * S * max_u * sizeof(double);
+  CU(g.d_pfstr.reserve(tab.size() * sizeof(int)), "cudaMalloc(plfold strands)");
+  CU(cudaMemcpyAsync(g.d_pfstr.p, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice, st), "H2D plfold strands");
+  if (bpp_out) { CU(g.d_pfbpp.reserve(bpp_bytes), "cudaMalloc(plfold bpp)"); CU(cudaMemsetAsync(g.d_pfbpp.p, 0, bpp_bytes, st), "clear plfold bpp"); }
+  if (pu_out) { CU(g.d_pfpu.reserve(pu_bytes), "cudaMalloc(plfold pu)"); CU(cudaMemsetAsync(g.d_pfpu.p, 0, pu_bytes, st), "clear plfold pu"); }
+  // chunks of consecutive windows within the memory budget: per window the fill's c / fML (ints) and qb / qm / qm1 triangles, the three
+  // kept outside triangles, P_u and the sequence
+  const size_t per = bf_tri_slot(wstride) * (2 * sizeof(int) + 6 * sizeof(double)) + (size_t)wstride * (1 + (pu_out ? max_u * sizeof(double) : 0));
+  const size_t budget = (size_t)std::max(1, bf_opt("BF_PLFOLD_MB", 1024)) << 20;
+  const long long cap = std::max<long long>(1, std::min<long long>(1 << 16, (long long)(budget / per)));
+  const long long chunk = std::min<long long>(cap, std::max<long long>(total, 1));
+  CU(g.d_seq.reserve((size_t)chunk * wstride), "cudaMalloc(seq)");
+  CU(g.d_len.reserve((size_t)chunk * sizeof(int)), "cudaMalloc(len)");
+  if (pu_out) CU(g.d_pu.reserve((size_t)chunk * wstride * max_u * sizeof(double)), "cudaMalloc(pu)");
+  std::vector<char> hseq((size_t)chunk * wstride, 0);
+  std::vector<int> hlen((size_t)chunk);
+  const int *dstr = (const int *)g.d_pfstr.p;
+  int r = 0;
+  for (long long w0 = 0; w0 < total; w0 += chunk) {
+    const int nw = (int)std::min<long long>(chunk, total - w0);
+    while (tab[n + r] + (long long)(tab[r] > 0 ? tab[r] - tab[2 * n + r] + 1 : 0) <= w0) r++;   // strand of window w0
+    const int r0 = r;
+    int rr = r0;
+    for (int k = 0; k < nw; k++) {
+      const long long gw = w0 + k;
+      while (tab[n + rr] + (long long)(tab[rr] > 0 ? tab[rr] - tab[2 * n + rr] + 1 : 0) <= gw) rr++;
+      const int sidx = (int)(gw - tab[n + rr]), wl = tab[2 * n + rr];
+      memcpy(&hseq[(size_t)k * wstride], s->seq + (size_t)rr * S + sidx, wl);
+      memset(&hseq[(size_t)k * wstride + wl], 0, wstride - wl);
+      hlen[k] = wl;
+    }
+    CU(cudaMemcpyAsync(g.d_seq.p, hseq.data(), (size_t)nw * wstride, cudaMemcpyHostToDevice, st), "H2D windows");
+    CU(cudaMemcpyAsync(g.d_len.p, hlen.data(), (size_t)nw * sizeof(int), cudaMemcpyHostToDevice, st), "H2D window lengths");
+    bf_batch_t db;
+    memset(&db, 0, sizeof(db));
+    db.B = nw; db.stride = wstride; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
+    db.want = BF_WANT_MFE | BF_WANT_PF;
+    // planned for the whole call, so that the kernels -- and with them every window's values -- do not depend on the chunking
+    int rc = unpaired_device(&db, max_u, pu_out ? (double *)g.d_pu.p : nullptr, st, (int)std::max<long long>(total, 1));
+    if (rc) return rc;
+    BfPlfoldDev d;
+    d.len = dstr; d.win0 = dstr + n; d.wlen = dstr + 2 * n;
+    d.stride = S; d.winsize = winsize; d.max_u = max_u;
+    d.r0 = r0; d.r1 = rr + 1; d.w0 = w0; d.nw = nw; d.wstride = wstride;
+    CU(bf_launch_plfold_avg(d, (const double *)g.w.tri_qb.p, (const double *)g.d_keep.p, pu_out ? (const double *)g.d_pu.p : nullptr,
+                            bpp_out ? (double *)g.d_pfbpp.p : nullptr, pu_out ? (double *)g.d_pfpu.p : nullptr, st),
+       "launch bf_k_plfold_avg");
+    g.launches++;
+    // the host staging buffers are rewritten for the next chunk: the copies above must have read them
+    CU(cudaStreamSynchronize(st), "bf_plfold chunk");
+  }
+  if (bpp_out) CU(cudaMemcpyAsync(bpp_out, g.d_pfbpp.p, bpp_bytes, cudaMemcpyDeviceToHost, st), "D2H plfold bpp");
+  if (pu_out) CU(cudaMemcpyAsync(pu_out, g.d_pfpu.p, pu_bytes, cudaMemcpyDeviceToHost, st), "D2H plfold pu");
+  CU(cudaStreamSynchronize(st), "bf_plfold");
   return BF_OK;
 }
 

@@ -44,7 +44,7 @@ struct BfPlan {
 
 cudaError_t bf_plan_mfe(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p);
 cudaError_t bf_plan_pf(int stride, int B, bool two, bool force_generic, int sms, BfPlan *p);
-cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p);
+cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p, bool keep = false);   // keep: for bf_launch_pf_out's keep
 cudaError_t bf_plan_mfe_out(int stride, int B, int sms, BfPlan *p);   // p->ws: ints per CTA
 
 cudaError_t bf_upload_constants();
@@ -105,9 +105,31 @@ cudaError_t bf_launch_f5_wide(const BfParams *dP, const BfBatchDev &b, const int
 cudaError_t bf_launch_q5_wide(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *lnscale, double *out5, cudaStream_t st);
 
 // ---- outside pass: base-pair probabilities and ensemble defect (bf_outside.cu)
+// keep (plan made with keep): B x 3 x bf_tri_slot doubles, per sequence the packed bqb, bqm and qm1-outside triangles (bf_unpaired.cu)
 cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, double *ws,
                              const double *lnscale, const char *targets, int n_targets, int tstride, double *out_defect, double *out_bpp,
-                             int *work_counter, cudaStream_t st);
+                             int *work_counter, cudaStream_t st, double *keep = nullptr);
+
+// ---- accessibility (bf_unpaired.cu): probabilities of unpaired stretches from the tables of a PF fill (qb, qm / qm1 kept) and of the
+// outside pass with keep.  pu_out: B x stride x max_u doubles, [r][i-1][u-1] = P(i .. i+u-1 unpaired), 0 where i+u-1 > len.
+cudaError_t bf_launch_unpaired(const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, const double *keep,
+                               const double *lnscale, double *ws, size_t ws_bytes, int max_u, double *pu_out, int *work_counter, int sms,
+                               cudaStream_t st);
+size_t bf_unpaired_ws_bytes(int stride);   // HBM workspace of one CTA of bf_k_unpaired
+// RNAplfold window averages: windows w0 .. w0 + nw - 1 of the call (strand-major, window s of strand r is global window win0[r] + s - 1)
+// have been folded as rows 0 .. nw - 1 of a batch of stride wstride (qb, keep; pu: nw x wstride x max_u).  Strands r0 .. r1 - 1 hold
+// them.  Each output element adds its windows of this chunk in ascending order to its running sum and divides by its window count in
+// the chunk that holds its last window, so the result does not depend on where the chunks end.
+struct BfPlfoldDev {
+  const int *len, *win0, *wlen;   // per strand: length, first global window, window length min(W, len)
+  int stride;                      // of the strands and of the outputs
+  int winsize, max_u;              // bpp row width W, pu row width
+  int r0, r1;                      // strands of this chunk
+  long long w0;                    // first global window of this chunk
+  int nw, wstride;
+};
+cudaError_t bf_launch_plfold_avg(const BfPlfoldDev &d, const double *qbtri, const double *keep, const double *pu, double *bpp_acc,
+                                 double *pu_acc, cudaStream_t st);
 
 // ---- minimum-free-energy outside pass (bf_outside.cu): over the c / fML triangles an MFE fill of the same batch left behind.
 // e_pair: B x stride x stride ints, [i-1][j-1] = lowest energy of a structure containing (i,j), BF_INF elsewhere.

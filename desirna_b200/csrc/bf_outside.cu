@@ -48,10 +48,13 @@ __host__ __device__ inline OutPlan out_plan(int nmax) {
   return p;
 }
 
-template <int NW>
+// KEEP: also write the outside values bf_k_unpaired reads, per sequence three packed triangles at keep + sq * 3 * tri_slot:
+// bqb, bqm and bqm1 without its bu * bqm1(a,b+1) self-recursion (qm1(a,b)'s outside value as its parents use it)
+template <int NW, bool KEEP = false>
 __global__ void __launch_bounds__(NW * 32) bf_k_pf_out(const BfParams *__restrict__ P, BfBatchDev b, const double *qbtri, const double *qmseq,
                                                        size_t tri_slot, double *ws, const double *lnscale, const char *targets,
-                                                       int n_targets, int tstride, double *out_defect, double *out_bpp, int *work_counter) {
+                                                       int n_targets, int tstride, double *out_defect, double *out_bpp, int *work_counter,
+                                                       double *keep) {
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ int s_seq, s_bad;
   __shared__ double s_red[NW];
@@ -206,6 +209,10 @@ __global__ void __launch_bounds__(NW * 32) bf_k_pf_out(const BfParams *__restric
           bqb += accg * T.x_mmI[t2][sq1][sp1] + acc1 * T.x_mm1nI[t2][sq1][sp1] + accb * (t > 2 ? xtau : 1.0) + accs;
         }
         const int o = toff[d] + a - 1;
+        if (KEEP) {
+          double *K = keep + (size_t)sq * 3 * tri_slot;
+          K[o] = bqb; K[tri_slot + o] = bqm; K[2 * tri_slot + o] = bqm + u2 + ap;
+        }
         H[o] = hab;
         BQM[r0 + a] = bqm;
         AP[r0 + a] = ap;
@@ -300,10 +307,11 @@ __host__ __device__ inline size_t out2_ws_doubles(int nmax, bool rgs) {
   for (int idx_ = (warp), flip_ = 0, s = (smax) - idx_; s >= 0;                                  \
        idx_ += flip_ ? 2 * (warp) + 1 : 2 * ((NW) - 1 - (warp)) + 1, flip_ ^= 1, s = (smax) - idx_)
 
-template <int NW, bool RGS, bool HSM>
+template <int NW, bool RGS, bool HSM, bool KEEP = false>   // KEEP: as for bf_k_pf_out
 __global__ void __launch_bounds__(NW * 32) bf_k_pf_out2(const BfParams *__restrict__ P, BfBatchDev b, const double *qbtri, const double *qmseq,
                                                         size_t tri_slot, double *ws, size_t ws_slot, const double *lnscale, const char *targets,
-                                                        int n_targets, int tstride, double *out_defect, double *out_bpp, int *work_counter) {
+                                                        int n_targets, int tstride, double *out_defect, double *out_bpp, int *work_counter,
+                                                        double *keep) {
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ int s_seq, s_bad, s_np[2];
   __shared__ double s_red[NW];
@@ -478,6 +486,10 @@ __global__ void __launch_bounds__(NW * 32) bf_k_pf_out2(const BfParams *__restri
             bqb += enc;
           }
           const int o = toff[dd] + a - 1;
+          if (KEEP) {
+            double *K = keep + (size_t)sq * 3 * tri_slot;
+            K[o] = bqb; K[tri_slot + o] = bqm; K[2 * tri_slot + o] = bqm + u2 + ap;
+          }
           H[o] = hab;
           BQM[r0 + a] = bqm;
           AP[r0 + a] = ap;
@@ -774,15 +786,19 @@ int out_version(int nmax, bool *rgs, bool *hsm, int B, int sms) {
   return 1;
 }
 
-// bf_k_pf_out2 without and with the generic ring on chip, and with H / qm / qm1 on chip as well
+// bf_k_pf_out2 without and with the generic ring on chip, and with H / qm / qm1 on chip as well; then the same with KEEP
 using OutK = void (*)(const BfParams *, BfBatchDev, const double *, const double *, size_t, double *, size_t, const double *, const char *, int,
-                      int, double *, double *, int *);
-const OutK kOut2[] = {bf_k_pf_out2<8, false, false>, bf_k_pf_out2<8, true, false>, bf_k_pf_out2<8, true, true>};
+                      int, double *, double *, int *, double *);
+const OutK kOut2[] = {bf_k_pf_out2<8, false, false>, bf_k_pf_out2<8, true, false>, bf_k_pf_out2<8, true, true>,
+                      bf_k_pf_out2<8, false, false, true>, bf_k_pf_out2<8, true, false, true>, bf_k_pf_out2<8, true, true, true>};
+using Out1K = void (*)(const BfParams *, BfBatchDev, const double *, const double *, size_t, double *, const double *, const char *, int, int,
+                       double *, double *, int *, double *);
+const Out1K kOut1[] = {bf_k_pf_out<8>, bf_k_pf_out<8, true>};
 }  // namespace
 
-// key: 0 = bf_k_pf_out, else kOut2[key - 1].  The workspace is sized for the variant without H on chip, so with it the slab is
-// larger than it needs to be.
-cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p) {
+// key: 0 = bf_k_pf_out, else kOut2[key - 1]; + 4 with keep (the KEEP instantiation).  The workspace is sized for the variant without
+// H on chip, so with it the slab is larger than it needs to be.
+cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p, bool keep) {
   *p = BfPlan{};
   bool rgs = false, hsm = false;
   p->ws = out_version(stride, &rgs, &hsm, 0, sms) == 2 ? (out2_ws_doubles(stride, rgs) + 7) / 8 * 8 : 4 * ((tri_size(stride) + 7) / 8 * 8);
@@ -790,12 +806,13 @@ cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p) {
   if (out_version(stride, &rgs, &hsm, B, sms) == 2) {
     p->key = 1 + rgs + hsm;
     p->smem = out2_plan(stride, 8, rgs, hsm).total;
-    kern = (const void *)kOut2[p->key - 1];
+    kern = (const void *)kOut2[p->key - 1 + (keep ? 3 : 0)];
   } else {
     p->key = 0;
     p->smem = out_plan(stride).total;
-    kern = (const void *)bf_k_pf_out<8>;
+    kern = (const void *)kOut1[keep];
   }
+  if (keep) p->key += 4;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(p->smem > 1024 ? p->smem : 1024));
   if (e != cudaSuccess) return e;
   int occ = 0;
@@ -808,16 +825,17 @@ cudaError_t bf_plan_out(int stride, int B, int sms, BfPlan *p) {
 
 cudaError_t bf_launch_pf_out(const BfPlan &p, const BfParams *dP, const BfBatchDev &b, const double *qbtri, const double *qmseq, double *ws,
                              const double *lnscale, const char *targets, int n_targets, int tstride, double *out_defect, double *out_bpp,
-                             int *work_counter, cudaStream_t st) {
+                             int *work_counter, cudaStream_t st, double *keep) {
   cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
   if (e != cudaSuccess) return e;
   const size_t tslot = (tri_size(b.stride) + 7) / 8 * 8;
-  if (p.key == 0)
-    bf_k_pf_out<8><<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, lnscale, targets, n_targets, tstride, out_defect, out_bpp,
-                                                work_counter);
+  const int k = p.key & 3, kp = p.key >> 2;
+  if (k == 0)
+    kOut1[kp]<<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, lnscale, targets, n_targets, tstride, out_defect, out_bpp,
+                                           work_counter, keep);
   else
-    kOut2[p.key - 1]<<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, p.ws, lnscale, targets, n_targets, tstride, out_defect,
-                                                  out_bpp, work_counter);
+    kOut2[k - 1 + 3 * kp]<<<p.grid, 256, p.smem, st>>>(dP, b, qbtri, qmseq, tslot, ws, p.ws, lnscale, targets, n_targets, tstride, out_defect,
+                                                      out_bpp, work_counter, keep);
   return cudaGetLastError();
 }
 

@@ -70,6 +70,8 @@ def lib():
         L.bf_subopt_zuker.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]
         L.bf_duplex.argtypes = [C.POINTER(bf_duplex_t), C.c_void_p, C.c_void_p]
+        L.bf_unpaired.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
+        L.bf_plfold.argtypes = [C.POINTER(bf_strands_t), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
         L.bf_debug_copy_table.argtypes = [C.c_int, C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         _lib = L
@@ -271,6 +273,39 @@ def duplex(seqs_a, seqs_b, pairs=None, structures=True):
     if pairs is None:
         out = [out[r * len(seqs_b):(r + 1) * len(seqs_b)] for r in range(len(seqs_a))]
     return e, out
+
+
+def unpaired(seqs, max_u):
+    """bf_unpaired: float64 [B, stride, max_u], entry [b, i-1, u-1] the probability that positions i .. i+u-1 (1-based) of
+    single-strand sequence b are all unpaired, in the ensemble of WANT_BPP (RNAplfold -u over the whole sequence); 0 where
+    i+u-1 > len.  T is read as U."""
+    ensure_ready()
+    buf, lens, cuts = pack([s.upper().replace("T", "U") for s in seqs])
+    b = bf_batch_t()
+    b.B, b.stride = len(seqs), buf.shape[1]
+    b.seq, b.len = buf.ctypes.data, lens.ctypes.data
+    b.cut = cuts.ctypes.data if cuts.any() else None
+    out = np.zeros((len(seqs), b.stride, max(int(max_u), 1)), np.float64)
+    _check(lib().bf_unpaired(C.byref(b), int(max_u), out.ctypes.data))
+    return out
+
+
+def plfold(seqs, winsize, max_u=31, pairs=True):
+    """bf_plfold: RNAplfold with span = window size over single strands.  Returns one (band, pu) per sequence of length n:
+    band float64 [n, winsize], band[i-1, d] the mean pair probability of (i, i+d) over the windows that hold both (None unless
+    pairs), and pu float64 [n, max_u], pu[i-1, u-1] the mean probability that i .. i+u-1 is unpaired over the windows that hold
+    it.  T is read as U."""
+    if any("&" in s for s in seqs):
+        raise ValueError("engine.plfold: single strands only (a sequence contains '&')")
+    ensure_ready()
+    buf, lens, _ = pack([s.upper().replace("T", "U") for s in seqs])
+    st = bf_strands_t()
+    st.n, st.stride, st.seq, st.len = len(seqs), buf.shape[1], buf.ctypes.data, lens.ctypes.data
+    W, U = int(winsize), int(max_u)
+    band = np.zeros((len(seqs), st.stride, max(W, 1)), np.float64) if pairs else None
+    pu = np.zeros((len(seqs), st.stride, max(U, 1)), np.float64)
+    _check(lib().bf_plfold(C.byref(st), W, U, band.ctypes.data if pairs else None, pu.ctypes.data))
+    return [(band[r, :int(lens[r])] if pairs else None, pu[r, :int(lens[r])]) for r in range(len(seqs))]
 
 
 def set_option(key, value):

@@ -153,6 +153,31 @@ typedef struct {
 } bf_duplex_t;
 int bf_duplex(const bf_duplex_t *q, int32_t *e_dcal, char *ss_out);
 
+/* Accessibility (not called by DesiRNA; RNAplfold -u, RNA.pfl_fold_up).  HOST buffers, synchronous.
+ * Global: for a sequence of length n, P_u(i, u) is the probability that none of positions i .. i+u-1 is paired, in exactly the
+ * ensemble of bf_score_batch's BF_WANT_PF / BF_WANT_BPP (loaded parameters, dangles = 2, pf_smooth, the per-nucleotide scale taken
+ * from the MFE).  Equivalently P_u(i, u) = Z(positions i .. i+u-1 may not pair) / Z.  Values are clamped to [0, 1] against rounding.
+ * pu_out: B x stride x max_u doubles, [r][i-1][u-1] = P_u(i, u); 0 where i+u-1 > len.
+ * BF_ERR_UNAVAILABLE: a row with cut > 0, a nopair mask (the partition function ignores constraints), a stride the PF fill path does
+ * not cover (as for BF_WANT_BPP; at present above 668) or BF_FORCE_GENERIC.  BF_ERR_ARG: null buffers, len > stride, max_u outside
+ * 1 .. stride. */
+int bf_unpaired(const bf_batch_t *batch, int32_t max_u, double *pu_out);
+/* RNAplfold with span = window size (RNA.pfl_fold / RNA.pfl_fold_up).  For a strand of length n let W' = min(winsize, n); the windows
+ * are the substrings s .. s+W'-1, s = 1 .. n-W'+1, each folded as an isolated sequence under the global model above (its end
+ * nucleotides have no outside neighbours).
+ *   pbar(i, j):    the mean, over the windows that contain both i and j, of that window's pair probability;
+ *   pbar_u(i, u):  the mean, over the windows that contain i .. i+u-1, of that window's P_u.
+ * All windows of all strands of s run through one pipeline, in chunks of consecutive windows within a fixed memory budget; every chunk
+ * runs the kernels chosen for the whole call and each average is summed in window order, so the result does not depend on the
+ * chunking.  Not pinned by any ViennaRNA output here: whether
+ * ViennaRNA's window folds let exterior-loop dangles see the nucleotides just outside the window, and the shim's output conventions.
+ * A maximum base-pair span smaller than the window is not supported.
+ * bpp_out: NULL or n x stride x winsize doubles, [r][i-1][d] = pbar(i, i+d); 0 where d < 4, i+d > len or d >= W'.
+ * pu_out:  NULL or n x stride x max_u doubles, [r][i-1][u-1] = pbar_u(i, u); 0 where i+u-1 > len.
+ * BF_ERR_ARG: both outputs NULL, null strands, len < 0 or > stride, winsize < 1, max_u outside 1 .. winsize.
+ * BF_ERR_UNAVAILABLE: winsize > 2000, a window W' longer than the PF fill path covers (as for bf_unpaired), or BF_FORCE_GENERIC. */
+int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp_out, double *pu_out);
+
 /* device time (ms, CUDA events on the launch stream) of the mfe, pf and eval kernels of the most recent
  * bf_score_batch[_device] call; -1 for a kernel that did not run.  Blocks until those kernels finished. */
 int bf_last_kernel_ms(double out[3]);
@@ -175,6 +200,7 @@ int bf_sm_count(void);
  *   "blk_min" / "blk_min_pf" N: the round-1 MFE / PF fills use the blocked split from N nt on (default 280 / 250);
  *   "force_generic" 1: single strands on the generic kernels too (read by bf_init);
  *   "design_overlap" 0: the device design loop always folds MFE, then PF.
+ *   "plfold_mb" N: memory budget of one bf_plfold chunk in MB (default 1024); the result does not depend on it.
  * Any other key is refused with BF_ERR_ARG. */
 int bf_set_option(const char *key, int value);
 /* Test hook: copy one engine-internal DP table of the most recent call to host memory.
