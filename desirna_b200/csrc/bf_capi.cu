@@ -109,6 +109,8 @@ struct Engine {
   DevBuf d_keep, d_upws, d_pu, d_pfstr, d_pfbpp, d_pfpu;
   // bf_duplex: strands, pair list, per-pair c-table offsets, c tables / HBM rings, energies, structures
   DevBuf d_dxa, d_dxb, d_dxlen, d_dxpairs, d_dxoff, d_dxws, d_dxe, d_dxss;
+  // bf_interact (strands and pair list in the bf_duplex buffers above): opening-energy tables of each side, per-unit slots, results
+  DevBuf d_ixeda, d_ixedb, d_ixslot, d_ixres;
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -709,13 +711,10 @@ int bf_unpaired(const bf_batch_t *b, int32_t max_u, double *pu_out) {
   return BF_OK;
 }
 
-int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp_out, double *pu_out) {
-  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
-  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
-  if (!s || (!bpp_out && !pu_out) || s->n < 0 || s->stride <= 0 || (s->n && (!s->seq || !s->len))) return fail(BF_ERR_ARG, "bf_plfold: bad argument");
-  for (int r = 0; r < s->n; r++)
-    if (s->len[r] < 0 || s->len[r] > s->stride) return fail(BF_ERR_ARG, "bf_plfold: strand length exceeds stride");
-  if (winsize < 1 || max_u < 1 || max_u > winsize) return fail(BF_ERR_ARG, "bf_plfold: winsize < 1 or max_u outside 1 .. winsize");
+namespace {
+// The RNAplfold pipeline on host strands s (checked by the caller): leaves the window averages in g.d_pfbpp (want_bpp: n x stride x
+// winsize) and g.d_pfpu (want_pu: n x stride x max_u) on the device.
+int plfold_device(const bf_strands_t *s, int32_t winsize, int32_t max_u, bool want_bpp, bool want_pu) {
   if (winsize > 2000) return fail(BF_ERR_UNAVAILABLE, "bf_plfold: window longer than 2000 nt");
   if (g.force_generic) return fail(BF_ERR_UNAVAILABLE, "bf_plfold: BF_FORCE_GENERIC");
   const int n = s->n, S = s->stride;
@@ -736,17 +735,17 @@ int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp
   const size_t bpp_bytes = (size_t)n * S * winsize * sizeof(double), pu_bytes = (size_t)n * S * max_u * sizeof(double);
   CU(g.d_pfstr.reserve(tab.size() * sizeof(int)), "cudaMalloc(plfold strands)");
   CU(cudaMemcpyAsync(g.d_pfstr.p, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice, st), "H2D plfold strands");
-  if (bpp_out) { CU(g.d_pfbpp.reserve(bpp_bytes), "cudaMalloc(plfold bpp)"); CU(cudaMemsetAsync(g.d_pfbpp.p, 0, bpp_bytes, st), "clear plfold bpp"); }
-  if (pu_out) { CU(g.d_pfpu.reserve(pu_bytes), "cudaMalloc(plfold pu)"); CU(cudaMemsetAsync(g.d_pfpu.p, 0, pu_bytes, st), "clear plfold pu"); }
+  if (want_bpp) { CU(g.d_pfbpp.reserve(bpp_bytes), "cudaMalloc(plfold bpp)"); CU(cudaMemsetAsync(g.d_pfbpp.p, 0, bpp_bytes, st), "clear plfold bpp"); }
+  if (want_pu) { CU(g.d_pfpu.reserve(pu_bytes), "cudaMalloc(plfold pu)"); CU(cudaMemsetAsync(g.d_pfpu.p, 0, pu_bytes, st), "clear plfold pu"); }
   // chunks of consecutive windows within the memory budget: per window the fill's c / fML (ints) and qb / qm / qm1 triangles, the three
   // kept outside triangles, P_u and the sequence
-  const size_t per = bf_tri_slot(wstride) * (2 * sizeof(int) + 6 * sizeof(double)) + (size_t)wstride * (1 + (pu_out ? max_u * sizeof(double) : 0));
+  const size_t per = bf_tri_slot(wstride) * (2 * sizeof(int) + 6 * sizeof(double)) + (size_t)wstride * (1 + (want_pu ? max_u * sizeof(double) : 0));
   const size_t budget = (size_t)std::max(1, bf_opt("BF_PLFOLD_MB", 1024)) << 20;
   const long long cap = std::max<long long>(1, std::min<long long>(1 << 16, (long long)(budget / per)));
   const long long chunk = std::min<long long>(cap, std::max<long long>(total, 1));
   CU(g.d_seq.reserve((size_t)chunk * wstride), "cudaMalloc(seq)");
   CU(g.d_len.reserve((size_t)chunk * sizeof(int)), "cudaMalloc(len)");
-  if (pu_out) CU(g.d_pu.reserve((size_t)chunk * wstride * max_u * sizeof(double)), "cudaMalloc(pu)");
+  if (want_pu) CU(g.d_pu.reserve((size_t)chunk * wstride * max_u * sizeof(double)), "cudaMalloc(pu)");
   std::vector<char> hseq((size_t)chunk * wstride, 0);
   std::vector<int> hlen((size_t)chunk);
   const int *dstr = (const int *)g.d_pfstr.p;
@@ -771,19 +770,34 @@ int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp
     db.B = nw; db.stride = wstride; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
     db.want = BF_WANT_MFE | BF_WANT_PF;
     // planned for the whole call, so that the kernels -- and with them every window's values -- do not depend on the chunking
-    int rc = unpaired_device(&db, max_u, pu_out ? (double *)g.d_pu.p : nullptr, st, (int)std::max<long long>(total, 1));
+    int rc = unpaired_device(&db, max_u, want_pu ? (double *)g.d_pu.p : nullptr, st, (int)std::max<long long>(total, 1));
     if (rc) return rc;
     BfPlfoldDev d;
     d.len = dstr; d.win0 = dstr + n; d.wlen = dstr + 2 * n;
     d.stride = S; d.winsize = winsize; d.max_u = max_u;
     d.r0 = r0; d.r1 = rr + 1; d.w0 = w0; d.nw = nw; d.wstride = wstride;
-    CU(bf_launch_plfold_avg(d, (const double *)g.w.tri_qb.p, (const double *)g.d_keep.p, pu_out ? (const double *)g.d_pu.p : nullptr,
-                            bpp_out ? (double *)g.d_pfbpp.p : nullptr, pu_out ? (double *)g.d_pfpu.p : nullptr, st),
+    CU(bf_launch_plfold_avg(d, (const double *)g.w.tri_qb.p, (const double *)g.d_keep.p, want_pu ? (const double *)g.d_pu.p : nullptr,
+                            want_bpp ? (double *)g.d_pfbpp.p : nullptr, want_pu ? (double *)g.d_pfpu.p : nullptr, st),
        "launch bf_k_plfold_avg");
     g.launches++;
     // the host staging buffers are rewritten for the next chunk: the copies above must have read them
     CU(cudaStreamSynchronize(st), "bf_plfold chunk");
   }
+  return BF_OK;
+}
+}  // namespace
+
+int bf_plfold(const bf_strands_t *s, int32_t winsize, int32_t max_u, double *bpp_out, double *pu_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!s || (!bpp_out && !pu_out) || s->n < 0 || s->stride <= 0 || (s->n && (!s->seq || !s->len))) return fail(BF_ERR_ARG, "bf_plfold: bad argument");
+  for (int r = 0; r < s->n; r++)
+    if (s->len[r] < 0 || s->len[r] > s->stride) return fail(BF_ERR_ARG, "bf_plfold: strand length exceeds stride");
+  if (winsize < 1 || max_u < 1 || max_u > winsize) return fail(BF_ERR_ARG, "bf_plfold: winsize < 1 or max_u outside 1 .. winsize");
+  int rc = plfold_device(s, winsize, max_u, bpp_out != nullptr, pu_out != nullptr);
+  if (rc || s->n == 0) return rc;
+  cudaStream_t st = g.stream;
+  const size_t bpp_bytes = (size_t)s->n * s->stride * winsize * sizeof(double), pu_bytes = (size_t)s->n * s->stride * max_u * sizeof(double);
   if (bpp_out) CU(cudaMemcpyAsync(bpp_out, g.d_pfbpp.p, bpp_bytes, cudaMemcpyDeviceToHost, st), "D2H plfold bpp");
   if (pu_out) CU(cudaMemcpyAsync(pu_out, g.d_pfpu.p, pu_bytes, cudaMemcpyDeviceToHost, st), "D2H plfold pu");
   CU(cudaStreamSynchronize(st), "bf_plfold");
@@ -901,6 +915,151 @@ int bf_duplex(const bf_duplex_t *q, int32_t *e_dcal, char *ss_out) {
     p0 = p1;
   }
   CU(cudaStreamSynchronize(st), "bf_duplex");
+  return BF_OK;
+}
+
+namespace {
+constexpr int kInteractMaxSpan = 64;
+constexpr long long kInteractSlots = 8 << 20;          // (pair, k1) slots of one launch: 192 MB
+constexpr size_t kInteractSsBytes = (size_t)256 << 20;  // structures of one launch
+
+int max_len(const bf_strands_t &s) { return s.n ? *std::max_element(s.len, s.len + s.n) : 0; }
+
+// Accessibility mode acc (-1 none, 0 global, W > 0 window) of strand set s with max_u = span, when it is available
+int interact_acc_check(const bf_strands_t &s, int acc, int span) {
+  if (acc < -1) return fail(BF_ERR_ARG, "bf_interact: accessibility mode below -1");
+  if (acc > 0 && acc < span) return fail(BF_ERR_ARG, "bf_interact: window shorter than max_span");
+  if (acc < 0) return BF_OK;
+  if (g.force_generic) return fail(BF_ERR_UNAVAILABLE, "bf_interact: accessibility under BF_FORCE_GENERIC");
+  const int m = acc == 0 ? max_len(s) : std::min(acc, max_len(s));
+  if (acc > 2000 || (m > 0 && bf_fill_pf_mode(m) == 0)) return fail(BF_ERR_UNAVAILABLE, "bf_interact: strand or window longer than the PF fill path covers");
+  return BF_OK;
+}
+
+// The opening energies of one side on the device, [strand][k-1][u-1], *rows positions x span per strand: P_u from bf_k_unpaired
+// (global) or the RNAplfold pipeline (window), turned into ED by bf_k_interact_ed.
+int interact_ed(const bf_strands_t &s, int acc, int span, DevBuf &ed, int *rows, cudaStream_t st) {
+  const size_t n = s.n;
+  const double *pu;
+  if (acc == 0) {
+    const int S = std::max(1, max_len(s));
+    std::vector<char> h(n * S, 0);
+    for (size_t r = 0; r < n; r++) memcpy(&h[r * S], s.seq + r * s.stride, s.len[r]);
+    CU(g.d_seq.reserve(n * S), "cudaMalloc(seq)");
+    CU(g.d_len.reserve(n * sizeof(int)), "cudaMalloc(len)");
+    CU(g.d_pu.reserve(n * S * span * sizeof(double)), "cudaMalloc(pu)");
+    CU(cudaMemcpyAsync(g.d_seq.p, h.data(), n * S, cudaMemcpyHostToDevice, st), "H2D seq");
+    CU(cudaMemcpyAsync(g.d_len.p, s.len, n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D len");
+    bf_batch_t db;
+    memset(&db, 0, sizeof(db));
+    db.B = s.n; db.stride = S; db.seq = (const char *)g.d_seq.p; db.len = (const int32_t *)g.d_len.p;
+    db.want = BF_WANT_MFE | BF_WANT_PF;
+    int rc = unpaired_device(&db, span, (double *)g.d_pu.p, st);
+    if (rc) return rc;
+    pu = (const double *)g.d_pu.p;
+    *rows = S;
+  } else {
+    int rc = plfold_device(&s, acc, span, false, true);
+    if (rc) return rc;
+    pu = (const double *)g.d_pfpu.p;
+    *rows = s.stride;
+  }
+  const size_t cnt = n * *rows * span;
+  CU(ed.reserve(cnt * sizeof(double)), "cudaMalloc(opening energies)");
+  CU(bf_launch_interact_ed(pu, (double *)ed.p, cnt, g.hP->kT, st), "launch bf_k_interact_ed");
+  g.launches++;
+  // the host staging vector above goes out of scope
+  CU(cudaStreamSynchronize(st), "bf_interact accessibility");
+  return BF_OK;
+}
+}  // namespace
+
+int bf_interact(const bf_interact_t *q, double *e, int32_t *h_dcal, double *ed, int32_t *site, char *ss_out) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!q || !e || (q->pairs && q->n_pairs < 0)) return fail(BF_ERR_ARG, "bf_interact: bad argument");
+  int rc = check_strands(q->a);
+  if (!rc) rc = check_strands(q->b);
+  if (rc) return rc;
+  const int span = q->max_span;
+  if (span < 1 || span > kInteractMaxSpan) return fail(BF_ERR_ARG, "bf_interact: max_span outside 1 .. 64");
+  const long long P = q->pairs ? q->n_pairs : (long long)q->a.n * q->b.n;
+  if (q->pairs)
+    for (long long p = 0; p < P; p++)
+      if (q->pairs[2 * p] < 0 || q->pairs[2 * p] >= q->a.n || q->pairs[2 * p + 1] < 0 || q->pairs[2 * p + 1] >= q->b.n)
+        return fail(BF_ERR_ARG, "bf_interact: pair index out of range");
+  if ((rc = interact_acc_check(q->a, q->acc_a, span)) || (rc = interact_acc_check(q->b, q->acc_b, span))) return rc;
+  if (P == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  BfInteractDev d;
+  d.span = span;
+  d.ed_a = d.ed_b = nullptr;
+  d.rows_a = d.rows_b = 0;
+  if (q->acc_a >= 0) {
+    if ((rc = interact_ed(q->a, q->acc_a, span, g.d_ixeda, &d.rows_a, st))) return rc;
+    d.ed_a = (const double *)g.d_ixeda.p;
+  }
+  if (q->acc_b >= 0) {
+    const bool same = q->acc_b == q->acc_a && q->b.n == q->a.n && q->b.stride == q->a.stride && q->b.seq == q->a.seq && q->b.len == q->a.len;
+    if (same) {
+      d.ed_b = d.ed_a; d.rows_b = d.rows_a;
+    } else {
+      if ((rc = interact_ed(q->b, q->acc_b, span, g.d_ixedb, &d.rows_b, st))) return rc;
+      d.ed_b = (const double *)g.d_ixedb.p;
+    }
+  }
+  const int sa = q->a.stride, sb = q->b.stride, ss_stride = sa + sb + 2;
+  CU(g.d_dxa.reserve((size_t)q->a.n * sa), "cudaMalloc(interact a)");
+  CU(g.d_dxb.reserve((size_t)q->b.n * sb), "cudaMalloc(interact b)");
+  CU(g.d_dxlen.reserve((size_t)(q->a.n + q->b.n) * sizeof(int)), "cudaMalloc(interact len)");
+  CU(cudaMemcpyAsync(g.d_dxa.p, q->a.seq, (size_t)q->a.n * sa, cudaMemcpyHostToDevice, st), "H2D interact a");
+  CU(cudaMemcpyAsync(g.d_dxb.p, q->b.seq, (size_t)q->b.n * sb, cudaMemcpyHostToDevice, st), "H2D interact b");
+  int *dlen = (int *)g.d_dxlen.p;
+  CU(cudaMemcpyAsync(dlen, q->a.len, q->a.n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D interact len a");
+  CU(cudaMemcpyAsync(dlen + q->a.n, q->b.len, q->b.n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D interact len b");
+  d.seq_a = (const char *)g.d_dxa.p; d.seq_b = (const char *)g.d_dxb.p;
+  d.stride_a = sa; d.stride_b = sb;
+  d.len_a = dlen; d.len_b = dlen + q->a.n;
+  d.nb = q->b.n;
+  d.amax = std::max(1, max_len(q->a));
+  d.bmax = std::max(1, max_len(q->b));
+  d.pairs = nullptr;
+  if (q->pairs) {
+    CU(g.d_dxpairs.reserve((size_t)P * 2 * sizeof(int)), "cudaMalloc(interact pairs)");
+    CU(cudaMemcpyAsync(g.d_dxpairs.p, q->pairs, (size_t)P * 2 * sizeof(int), cudaMemcpyHostToDevice, st), "H2D interact pairs");
+    d.pairs = (const int *)g.d_dxpairs.p;
+  }
+  // launches of consecutive pairs whose (pair, k1) slots and structures fit the per-launch budgets
+  long long cap = std::min<long long>(1 << 16, kInteractSlots / d.amax);
+  if (ss_out) cap = std::min<long long>(cap, (long long)(kInteractSsBytes / ss_stride));
+  cap = std::max<long long>(cap, 1);
+  const long long np_max = std::min(cap, P);
+  CU(g.d_ixslot.reserve((size_t)np_max * d.amax * sizeof(BfInteractSlot)), "cudaMalloc(interact slots)");
+  CU(g.d_ixres.reserve((size_t)np_max * (4 * sizeof(double) + sizeof(long long) + 5 * sizeof(int))), "cudaMalloc(interact results)");
+  if (ss_out) CU(g.d_dxss.reserve((size_t)np_max * ss_stride), "cudaMalloc(interact structures)");
+  BfInteractOut out;
+  out.e = (double *)g.d_ixres.p;
+  out.ed = out.e + np_max;
+  out.rank = (long long *)(out.ed + 2 * np_max);
+  out.h = (int *)(out.rank + np_max);
+  out.site = out.h + np_max;
+  for (long long p0 = 0; p0 < P; p0 += cap) {
+    const int np = (int)std::min(cap, P - p0);
+    d.p0 = p0; d.np = np;
+    d.ia0 = q->pairs ? 0 : (int)(p0 / d.nb);
+    d.ib0 = q->pairs ? 0 : (int)(p0 % d.nb);
+    CU(bf_launch_interact(g.dP, d, (BfInteractSlot *)g.d_ixslot.p, out, ss_out ? (char *)g.d_dxss.p : nullptr, ss_stride,
+                          g.w.d_counters + 4, g.sm_count, st),
+       "launch bf_k_interact");
+    g.launches += ss_out ? 3 : 2;
+    CU(cudaMemcpyAsync(e + p0, out.e, (size_t)np * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H interact energies");
+    if (h_dcal) CU(cudaMemcpyAsync(h_dcal + p0, out.h, (size_t)np * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H interact H");
+    if (ed) CU(cudaMemcpyAsync(ed + 2 * p0, out.ed, (size_t)np * 2 * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H interact ED");
+    if (site) CU(cudaMemcpyAsync(site + 4 * p0, out.site, (size_t)np * 4 * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H interact sites");
+    if (ss_out)
+      CU(cudaMemcpyAsync(ss_out + (size_t)p0 * ss_stride, g.d_dxss.p, (size_t)np * ss_stride, cudaMemcpyDeviceToHost, st), "D2H interact structures");
+  }
+  CU(cudaStreamSynchronize(st), "bf_interact");
   return BF_OK;
 }
 

@@ -161,6 +161,36 @@ size_t bf_duplex_ring_slot(int ring_w);
 cudaError_t bf_launch_duplex(const BfParams *dP, const BfDuplexDev &d, bool gring, int *gring_ws, int *e_out, int *ctab,
                              const long long *ctab_off, char *ss_out, int ss_stride, cudaStream_t st);
 
+// ---- accessibility-aware RNA-RNA interaction (bf_interact.cu): the best site of np pairs, pairs p0 .. p0 + np - 1 of the call
+struct BfInteractDev {
+  const char *seq_a, *seq_b;   // strands, rows of stride_a / stride_b bytes
+  int stride_a, stride_b;
+  const int *len_a, *len_b;
+  const int *pairs;            // as BfDuplexDev
+  int nb;
+  long long p0;
+  int ia0, ib0;                // the grid's pair p0: (p0 / nb, p0 % nb)
+  int np;
+  int amax, bmax;              // longest a / b strand of the call: units per pair, staging sizes
+  int span;                    // max_span, 1 .. 64
+  const double *ed_a, *ed_b;   // opening energies [strand][k-1][u-1], rows_a / rows_b positions x span; null: no accessibility
+  int rows_a, rows_b;
+};
+struct BfInteractSlot { double e; long long rank; int h, pad; };   // best site of one (pair, k1) unit; rank -1: none
+// per pair of the launch: E, H (BF_INF: no site), packed rank (-1: no site); ed (2 per pair) and site (k1, km, lm, l1) or null
+struct BfInteractOut {
+  double *e;
+  int *h;
+  long long *rank;
+  double *ed;
+  int *site;
+};
+// slots: np x amax.  ss_out (null: energies only): np x ss_stride chars in bf_duplex's layout.
+cudaError_t bf_launch_interact(const BfParams *dP, const BfInteractDev &d, BfInteractSlot *slots, const BfInteractOut &out, char *ss_out,
+                               int ss_stride, int *work_counter, int sms, cudaStream_t st);
+// ed[x] = -(kT / 1000) ln pu[x] (kcal/mol), +inf where pu[x] <= 0; kT in cal/mol
+cudaError_t bf_launch_interact_ed(const double *pu, double *ed, size_t n, double kT, cudaStream_t st);
+
 // ---- suboptimal structures (bf_subopt.cu): host walk over the c / fML tables of the GPU fill
 #ifdef __cplusplus
 #include <string>

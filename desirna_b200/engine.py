@@ -42,6 +42,11 @@ class bf_duplex_t(C.Structure):
     _fields_ = [("a", bf_strands_t), ("b", bf_strands_t), ("n_pairs", C.c_int32), ("pairs", C.c_void_p)]
 
 
+class bf_interact_t(C.Structure):
+    _fields_ = [("a", bf_strands_t), ("b", bf_strands_t), ("n_pairs", C.c_int32), ("pairs", C.c_void_p), ("max_span", C.c_int32),
+                ("acc_a", C.c_int32), ("acc_b", C.c_int32)]
+
+
 _lib = None
 
 
@@ -70,6 +75,7 @@ def lib():
         L.bf_subopt_zuker.argtypes = [C.c_char_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]
         L.bf_duplex.argtypes = [C.POINTER(bf_duplex_t), C.c_void_p, C.c_void_p]
+        L.bf_interact.argtypes = [C.POINTER(bf_interact_t), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.bf_unpaired.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
         L.bf_plfold.argtypes = [C.POINTER(bf_strands_t), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
@@ -273,6 +279,58 @@ def duplex(seqs_a, seqs_b, pairs=None, structures=True):
     if pairs is None:
         out = [out[r * len(seqs_b):(r + 1) * len(seqs_b)] for r in range(len(seqs_a))]
     return e, out
+
+
+def interact(seqs_a, seqs_b, pairs=None, max_span=25, acc_a=0, acc_b=0, structures=True):
+    """bf_interact: accessibility-aware RNA-RNA interaction, the best site of every requested pair of strands.  A site is a duplex
+    chain as in engine.duplex whose span on each strand is at most max_span (1 .. 64; the default is RNAup's -w 25); its score is
+    E = H / 100 + ED_a + ED_b in kcal/mol, H the chain's hybridization energy in dcal/mol and ED = -kT ln P_u the free energy
+    that opens the site on each strand.  acc_a / acc_b choose P_u: -1 none (ED = 0), 0 the global ensemble of the whole strand
+    (engine.unpaired), W > 0 RNAplfold window averages with span W >= max_span (engine.plfold).  pairs: [(index into seqs_a,
+    index into seqs_b)], or None for the full grid.
+
+    Returns a dict of numpy arrays, each of shape [P] or [len(seqs_a), len(seqs_b)] plus a trailing axis where noted: 'e'
+    (float64, +inf where no site exists), 'h' (int32, 10000000 where none), 'ed_a', 'ed_b' (float64), 'site' (int32, [..., 4]:
+    1-based k1, km in a and lm, l1 in b, 0 where none) and, with structures, 'structures': full-length 'a-part&b-part' strings
+    as engine.duplex returns them.  Each strand holds at most 2000 nt; T is read as U.
+
+    ViennaRNA's Python API has no call with this model: RNAup's pf_interact is a partition-function model over all sites, while
+    this returns the single site of least E, as RNAplex -a and IntaRNA's MFE mode do, so there is no RNA.py counterpart."""
+    if any("&" in s for s in seqs_a) or any("&" in s for s in seqs_b):
+        raise ValueError("engine.interact: a strand may not contain '&' (pass the two strands separately)")
+    ensure_ready()
+    q = bf_interact_t()
+    keep = []
+    for st, seqs in ((q.a, seqs_a), (q.b, seqs_b)):
+        buf, lens, _ = pack([s.upper().replace("T", "U") for s in seqs])
+        st.n, st.stride, st.seq, st.len = len(seqs), buf.shape[1], buf.ctypes.data, lens.ctypes.data
+        keep += [buf, lens]
+    la, lb = keep[1], keep[3]
+    q.max_span, q.acc_a, q.acc_b = int(max_span), int(acc_a), int(acc_b)
+    if pairs is None:
+        P, shape = len(seqs_a) * len(seqs_b), (len(seqs_a), len(seqs_b))
+        ia, ib = np.repeat(np.arange(len(seqs_a)), len(seqs_b)), np.tile(np.arange(len(seqs_b)), len(seqs_a))
+    else:
+        pr = np.ascontiguousarray(np.asarray(pairs, np.int32).reshape(-1, 2))
+        P, shape = pr.shape[0], (pr.shape[0],)
+        q.n_pairs, q.pairs = P, pr.ctypes.data
+        keep.append(pr)
+        ia, ib = pr[:, 0], pr[:, 1]
+    e = np.zeros(P, np.float64)
+    h = np.zeros(P, np.int32)
+    ed = np.zeros((P, 2), np.float64)
+    site = np.zeros((P, 4), np.int32)
+    ss = np.zeros((P, q.a.stride + q.b.stride + 2), np.uint8) if structures else None
+    _check(lib().bf_interact(C.byref(q), e.ctypes.data, h.ctypes.data, ed.ctypes.data, site.ctypes.data,
+                             ss.ctypes.data if structures else None))
+    out = {"e": e.reshape(shape), "h": h.reshape(shape), "ed_a": ed[:, 0].reshape(shape).copy(), "ed_b": ed[:, 1].reshape(shape).copy(),
+           "site": site.reshape(shape + (4,))}
+    if structures:
+        st = [bytes(ss[p, :int(la[ia[p]]) + int(lb[ib[p]]) + 1]).decode("ascii") for p in range(P)]
+        if pairs is None:
+            st = [st[r * len(seqs_b):(r + 1) * len(seqs_b)] for r in range(len(seqs_a))]
+        out["structures"] = st
+    return out
 
 
 def unpaired(seqs, max_u):

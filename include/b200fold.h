@@ -153,6 +153,42 @@ typedef struct {
 } bf_duplex_t;
 int bf_duplex(const bf_duplex_t *q, int32_t *e_dcal, char *ss_out);
 
+/* Accessibility-aware RNA-RNA interaction (RNAup / RNAplex -a / IntaRNA's site model; not called by DesiRNA).  HOST buffers,
+ * synchronous.
+ * A site of strands a and b is a duplex chain as in bf_duplex: pairs (k1,l1), ..., (km,lm) of a[k] with b[l], k increasing, l
+ * decreasing, at most 30 unpaired nucleotides between consecutive pairs, with both spans km - k1 + 1 and l1 - lm + 1 at most
+ * max_span (1 .. 64).  Its hybridization energy H (dcal/mol) is bf_duplex's energy of that chain: the engine's two-strand eval of
+ * the structure on a&b (DuplexInit, the outer exterior stem, the interior loops, the nick loop closed by the innermost pair, with
+ * neighbours only where they exist).  Its opening energies are
+ *   ED_a = -(kT/1000) ln P_u^a(k1, km - k1 + 1),   ED_b = -(kT/1000) ln P_u^b(lm, l1 - lm + 1)     (kcal/mol)
+ * with kT the loaded parameter set's, in cal/mol (the partition function's), and P_u from each side's accessibility mode:
+ *   acc = -1: none, ED = 0;  acc = 0: global, bf_unpaired's ensemble of the whole strand;  acc = W > 0: bf_plfold's window average
+ *   with span = W (W >= max_span).  Where P_u <= 0 the site does not exist.
+ * Its score is E = (double)H / 100.0 + ED_a + ED_b, evaluated in that order in double.  For each requested pair of strands the
+ * result is the site of least E; ties go to the first site in the order k1 ascending, l1 descending, km ascending, lm descending.
+ * The structure is traced back inside the table of that start with bf_duplex's rule (the first (k,l) reproducing the cell, k = i-1
+ * downwards, then l = j+1 upwards).  With no accessibility on either side and max_span >= both lengths, 100 E is bf_duplex's energy.
+ * The accessibility of each side is computed once per call on the device (once for both when a and b are the same strand set and
+ * mode); P_u and ED stay on the device.
+ * Outputs per pair (pairs: n_pairs x 2 (index into a, index into b), or NULL for the full grid a.n x b.n, a-major):
+ *   e:      E in kcal/mol, +inf where no site exists;
+ *   h_dcal: NULL or H, 10000000 where no site exists;
+ *   ed:     NULL or 2 doubles, ED_a and ED_b (0 where no site exists);
+ *   site:   NULL or 4 ints, 1-based k1, km, lm, l1 (0 where no site exists);
+ *   ss_out: NULL or a.stride + b.stride + 2 chars in bf_duplex's layout, all dots where no site exists.
+ * This is not RNAup's partition-function interaction (RNAup -b): a single best site, no intramolecular structure inside it.
+ * BF_ERR_ARG: null q or e, a bad strand set (as bf_duplex), max_span outside 1 .. 64, acc < -1, a window below max_span,
+ * n_pairs < 0, a pair index out of range.  BF_ERR_UNAVAILABLE: global accessibility of a strand longer than the PF fill path covers,
+ * a window longer than the fill path covers, accessibility under BF_FORCE_GENERIC. */
+typedef struct {
+  bf_strands_t a, b;       /* as bf_duplex; strands <= 2000 nt */
+  int32_t n_pairs;         /* with pairs == NULL: the full a-major grid */
+  const int32_t *pairs;
+  int32_t max_span;        /* 1 .. 64 */
+  int32_t acc_a, acc_b;    /* -1 none, 0 global, W > 0 RNAplfold window W (W >= max_span) */
+} bf_interact_t;
+int bf_interact(const bf_interact_t *q, double *e, int32_t *h_dcal, double *ed, int32_t *site, char *ss_out);
+
 /* Accessibility (not called by DesiRNA; RNAplfold -u, RNA.pfl_fold_up).  HOST buffers, synchronous.
  * Global: for a sequence of length n, P_u(i, u) is the probability that none of positions i .. i+u-1 is paired, in exactly the
  * ensemble of bf_score_batch's BF_WANT_PF / BF_WANT_BPP (loaded parameters, dangles = 2, pf_smooth, the per-nucleotide scale taken
