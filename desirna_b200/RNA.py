@@ -14,6 +14,8 @@ DesiRNA.py:35).  A maintainer switches engines with `from desirna_b200 import RN
     fc.ensemble_defect(db)                        energy_scores.py:374
     fc.pbacktrack([num_samples]), RNA.init_rand(seed)   stochastic backtracking (not called by DesiRNA; ViennaRNA's API)
     fc.subopt_zuker()                             Zuker suboptimals (not called by DesiRNA; ViennaRNA's API)
+    fc.path_findpath_saddle(s1, s2, width)        findpath saddle (not called by DesiRNA; ViennaRNA's API; conventions recalled)
+    fc.path_findpath(s1, s2, width)               findpath refolding path (not called by DesiRNA; ViennaRNA's API; conventions recalled)
     RNA.duplexfold(s1, s2)                        RNA-RNA hybridization, RNAduplex (not called by DesiRNA; ViennaRNA's API)
     RNA.pfl_fold_up(seq, ulength, W, L)           accessibility, RNAplfold -u (not called by DesiRNA; ViennaRNA's API; conventions recalled)
     RNA.pfl_fold(seq, W, L, cutoff)               RNAplfold pair probabilities (not called by DesiRNA; ViennaRNA's API; conventions recalled)
@@ -246,6 +248,42 @@ class fold_compound:
             raise NotImplementedError("subopt_zuker on two-strand compounds is not part of the accelerated path")
         nopair = np.asarray(self._nopair, np.uint8) if self._nopair is not None and any(self._nopair) else None
         return [subopt_solution(s, f32(e / 100.0)) for s, e in _eng.subopt_zuker(self.sequence, nopair)]
+
+    def path_findpath_saddle(self, s1, s2, width=1):
+        """vrna_path_findpath_saddle: the saddle energy (int, dcal/mol) of the best direct refolding path from s1 to s2 found by the
+        breadth-limited search of width `width` (engine.findpath).  The width schedule, direction alternation and tie order are
+        ViennaRNA's as recalled; no ViennaRNA output pins them here."""
+        if "&" in self.sequence:
+            raise NotImplementedError("path_findpath_saddle on two-strand compounds is not part of the accelerated path")
+        return int(_eng.findpath([self.sequence], [s1], [s2], width, path=False)[0])
+
+    def path_findpath(self, s1, s2, width=1):
+        """vrna_path_findpath: the best direct refolding path from s1 to s2, a list of path objects (.s structure, .en kcal/mol) from
+        s1 to s2, with the structures expanded from the moves.  Conventions recalled as for path_findpath_saddle."""
+        if "&" in self.sequence:
+            raise NotImplementedError("path_findpath on two-strand compounds is not part of the accelerated path")
+        _, res = _eng.findpath([self.sequence], [s1], [s2], width)
+        moves, pe = res[0]
+        ss = list(s1)
+        out = [path(s1, f32(int(pe[0]) / 100.0))]
+        for (i, j), e in zip(moves.tolist(), pe[1:].tolist()):
+            if i > 0:
+                ss[i - 1], ss[j - 1] = "(", ")"
+            else:
+                ss[-i - 1], ss[-j - 1] = ".", "."
+            out.append(path("".join(ss), f32(int(e) / 100.0)))
+        return out
+
+
+class path:
+    """one step of fc.path_findpath(): .s (structure) and .en (kcal/mol, C float) as ViennaRNA's path object"""
+
+    def __init__(self, s, en):
+        self.s = s
+        self.en = en
+
+    def __repr__(self):
+        return "path(%r, %r)" % (self.s, self.en)
 
 
 class subopt_solution:

@@ -18,7 +18,8 @@
 // choice is made (BF_FORCE_GENERIC at bf_init, BF_DESIGN_OVERLAP at bf_design_create, the others at every call), so that a host
 // program can flip them between calls on one engine.
 static const char *const kOptions[] = {"BF_CL", "BF_CL_C", "BF_CL_BW", "BF_EXT_WIDE", "BF_WIDE", "BF_FILL3", "BF_FILL3_SMALL",
-                                       "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP", "BF_PLFOLD_MB"};
+                                       "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP", "BF_PLFOLD_MB",
+                                       "BF_FINDPATH_MB"};
 
 int bf_opt(const char *name, int dflt) {
   const char *v = getenv(name);
@@ -111,6 +112,9 @@ struct Engine {
   DevBuf d_dxa, d_dxb, d_dxlen, d_dxpairs, d_dxoff, d_dxws, d_dxe, d_dxss;
   // bf_interact (strands and pair list in the bf_duplex buffers above): opening-energy tables of each side, per-unit slots, results
   DevBuf d_ixeda, d_ixedb, d_ixslot, d_ixres;
+  // bf_findpath: sequences, lengths, pair tables, move lists and counts, back-pointer offsets, per-CTA workspaces, back-pointers, per-run
+  // saddles and start energies, results
+  DevBuf d_fpseq, d_fplen, d_fppt, d_fpmv, d_fpnd, d_fpoff, d_fpws, d_fpbp, d_fprun, d_fpout;
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -1060,6 +1064,134 @@ int bf_interact(const bf_interact_t *q, double *e, int32_t *h_dcal, double *ed, 
       CU(cudaMemcpyAsync(ss_out + (size_t)p0 * ss_stride, g.d_dxss.p, (size_t)np * ss_stride, cudaMemcpyDeviceToHost, st), "D2H interact structures");
   }
   CU(cudaStreamSynchronize(st), "bf_interact");
+  return BF_OK;
+}
+
+namespace {
+// pair table of dot-bracket db (n chars) into pt[0 .. n+1]; false when it is not a balanced '.', '(', ')' string with j - i >= 4
+bool findpath_parse(const char *db, int n, short *pt, std::vector<int> &stk) {
+  stk.clear();
+  for (int i = 0; i <= n + 1; i++) pt[i] = 0;
+  for (int i = 1; i <= n; i++) {
+    const char c = db[i - 1];
+    if (c == '(') stk.push_back(i);
+    else if (c == ')') {
+      if (stk.empty()) return false;
+      const int o = stk.back();
+      stk.pop_back();
+      if (i - o < 4) return false;
+      pt[o] = (short)i; pt[i] = (short)o;
+    } else if (c != '.') return false;
+  }
+  return stk.empty();
+}
+}  // namespace
+
+int bf_findpath(const bf_findpath_t *q, int32_t *saddle_dcal, int32_t *n_moves, int32_t *moves, int32_t *path_e) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!q || !saddle_dcal || q->n < 0 || q->stride < 1) return fail(BF_ERR_ARG, "bf_findpath: bad argument");
+  if (q->stride > BF_FINDPATH_MAX_LEN) return fail(BF_ERR_ARG, "bf_findpath: stride above 2000");
+  if (q->width < 1 || q->width > BF_FINDPATH_MAX_WIDTH) return fail(BF_ERR_ARG, "bf_findpath: width outside 1 .. 1024");
+  const int n = q->n, S = q->stride;
+  if (n && (!q->seq || !q->len || !q->s1 || !q->s2)) return fail(BF_ERR_ARG, "bf_findpath: null sequence or structure buffer");
+  // pair tables, move lists (pairs of s1 only, ascending i, then pairs of s2 only) and their counts
+  std::vector<short> pt((size_t)n * 2 * (S + 2));
+  std::vector<int> mv((size_t)n * S, 0), nd((size_t)n * 2), stk;
+  int nmax = 1, kmax = 0;
+  for (int r = 0; r < n; r++) {
+    const int len = q->len[r];
+    if (len < 0 || len > S) return fail(BF_ERR_ARG, "bf_findpath: length outside 0 .. stride");
+    for (int i = 0; i < len; i++)
+      if (!bf_base_code(q->seq[(size_t)r * S + i])) return fail(BF_ERR_ARG, "bf_findpath: sequence character other than ACGUT");
+    short *p1 = &pt[(size_t)r * 2 * (S + 2)], *p2 = p1 + S + 2;
+    if (!findpath_parse(q->s1 + (size_t)r * S, len, p1, stk) || !findpath_parse(q->s2 + (size_t)r * S, len, p2, stk))
+      return fail(BF_ERR_ARG, "bf_findpath: structure not balanced, a character other than '.()', or a pair with j - i < 4");
+    int *m = &mv[(size_t)r * S], k = 0;
+    for (int i = 1; i <= len; i++) if (p1[i] > i && p2[i] != p1[i]) m[k++] = i << 16 | p1[i];
+    nd[2 * r] = k;
+    for (int i = 1; i <= len; i++) if (p2[i] > i && p1[i] != p2[i]) m[k++] = i << 16 | p2[i];
+    nd[2 * r + 1] = k - nd[2 * r];
+    nmax = std::max(nmax, len);
+    kmax = std::max(kmax, k);
+    if (n_moves) n_moves[r] = k;
+  }
+  if (n == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  const int W = q->width, R = bf_findpath_runs(W), kw = std::max(1, (kmax + 63) / 64);
+  // per-instance pair tables are interleaved (s1, s2); the kernel reads them through two pointers with a stride of two tables
+  std::vector<short> pt1((size_t)n * (S + 2)), pt2((size_t)n * (S + 2));
+  for (int r = 0; r < n; r++) {
+    memcpy(&pt1[(size_t)r * (S + 2)], &pt[(size_t)r * 2 * (S + 2)], (S + 2) * sizeof(short));
+    memcpy(&pt2[(size_t)r * (S + 2)], &pt[(size_t)r * 2 * (S + 2) + S + 2], (S + 2) * sizeof(short));
+  }
+  const size_t ptb = (size_t)n * (S + 2) * sizeof(short);
+  CU(g.d_fpseq.reserve((size_t)n * S), "cudaMalloc(findpath seq)");
+  CU(g.d_fplen.reserve((size_t)n * sizeof(int)), "cudaMalloc(findpath len)");
+  CU(g.d_fppt.reserve(2 * ptb), "cudaMalloc(findpath pair tables)");
+  CU(g.d_fpmv.reserve((size_t)n * S * sizeof(int)), "cudaMalloc(findpath moves)");
+  CU(g.d_fpnd.reserve((size_t)n * 2 * sizeof(int)), "cudaMalloc(findpath counts)");
+  CU(cudaMemcpyAsync(g.d_fpseq.p, q->seq, (size_t)n * S, cudaMemcpyHostToDevice, st), "H2D findpath seq");
+  CU(cudaMemcpyAsync(g.d_fplen.p, q->len, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D findpath len");
+  CU(cudaMemcpyAsync(g.d_fppt.p, pt1.data(), ptb, cudaMemcpyHostToDevice, st), "H2D findpath s1");
+  CU(cudaMemcpyAsync((char *)g.d_fppt.p + ptb, pt2.data(), ptb, cudaMemcpyHostToDevice, st), "H2D findpath s2");
+  CU(cudaMemcpyAsync(g.d_fpmv.p, mv.data(), (size_t)n * S * sizeof(int), cudaMemcpyHostToDevice, st), "H2D findpath move lists");
+  CU(cudaMemcpyAsync(g.d_fpnd.p, nd.data(), (size_t)n * 2 * sizeof(int), cudaMemcpyHostToDevice, st), "H2D findpath counts");
+  // within a memory budget: the grid's per-CTA workspaces (shaped by the whole call, so that the kernel's work does not depend on the
+  // split) and the back-pointers of the instances of one launch
+  const size_t budget = (size_t)std::max(1, bf_opt("BF_FINDPATH_MB", 1024)) << 20;
+  const long long cap = bf_findpath_cap(W, kmax);
+  const size_t ws_cta = bf_findpath_ws_bytes(W, nmax, kw, cap);
+  const int grid_max = (int)std::max<long long>(1, std::min<long long>((long long)g.sm_count * bf_findpath_occupancy(), (long long)(budget / ws_cta)));
+  const long long wsum = bf_findpath_width_sum(W);
+  std::vector<long long> off((size_t)n + 1, 0);
+  for (int r = 0; r < n; r++) off[r + 1] = off[r] + (long long)(nd[2 * r] + nd[2 * r + 1]) * wsum;
+  // launches of consecutive instances whose back-pointers fit the budget (at least one instance each)
+  std::vector<int> cut{0};
+  for (int r = 1; r < n; r++)
+    if ((size_t)(off[r + 1] - off[cut.back()]) * sizeof(int2) > budget) cut.push_back(r);
+  cut.push_back(n);
+  long long bp_max = 0;
+  int n_max = 0;
+  for (size_t c = 0; c + 1 < cut.size(); c++) {
+    bp_max = std::max(bp_max, off[cut[c + 1]] - off[cut[c]]);
+    n_max = std::max(n_max, cut[c + 1] - cut[c]);
+  }
+  CU(g.d_fpoff.reserve((size_t)n * sizeof(long long)), "cudaMalloc(findpath offsets)");
+  CU(g.d_fpws.reserve((size_t)grid_max * ws_cta), "cudaMalloc(findpath workspaces)");
+  CU(g.d_fpbp.reserve((size_t)std::max<long long>(bp_max, 1) * sizeof(int2)), "cudaMalloc(findpath back-pointers)");
+  CU(g.d_fprun.reserve((size_t)n_max * R * 2 * sizeof(int)), "cudaMalloc(findpath runs)");
+  CU(g.d_fpout.reserve((size_t)n_max * (1 + 2 * S + S + 1) * sizeof(int)), "cudaMalloc(findpath results)");
+  std::vector<long long> loff((size_t)n);
+  for (size_t c = 0; c + 1 < cut.size(); c++)
+    for (int r = cut[c]; r < cut[c + 1]; r++) loff[r] = off[r] - off[cut[c]];
+  CU(cudaMemcpyAsync(g.d_fpoff.p, loff.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D findpath offsets");
+  int *o_sad = (int *)g.d_fpout.p, *o_mv = o_sad + n_max, *o_pe = o_mv + (size_t)n_max * 2 * S;
+  for (size_t c = 0; c + 1 < cut.size(); c++) {
+    const int r0 = cut[c], nl = cut[c + 1] - r0;
+    BfFindpathDev d;
+    d.n = nl; d.stride = S;
+    d.seq = (const char *)g.d_fpseq.p + (size_t)r0 * S;
+    d.len = (const int *)g.d_fplen.p + r0;
+    d.pt1 = (const short *)g.d_fppt.p + (size_t)r0 * (S + 2);
+    d.pt2 = (const short *)((const char *)g.d_fppt.p + ptb) + (size_t)r0 * (S + 2);
+    d.mv = (const int *)g.d_fpmv.p + (size_t)r0 * S;
+    d.nd = (const int *)g.d_fpnd.p + 2 * r0;
+    d.width = W; d.nmax = nmax; d.kw = kw; d.cap = cap;
+    d.bp = (int2 *)g.d_fpbp.p;
+    d.bp_off = (const long long *)g.d_fpoff.p + r0;
+    d.run_sad = (int *)g.d_fprun.p; d.run_e0 = d.run_sad + (size_t)n_max * R;
+    const int grid = (int)std::min<long long>(grid_max, (long long)nl * R);
+    if (moves) CU(cudaMemsetAsync(o_mv, 0, (size_t)nl * 2 * S * sizeof(int), st), "clear findpath moves");
+    if (path_e) CU(cudaMemsetAsync(o_pe, 0, (size_t)nl * (S + 1) * sizeof(int), st), "clear findpath energies");
+    CU(bf_launch_findpath(g.dP, d, (unsigned char *)g.d_fpws.p, grid, g.w.d_counters + 5, o_sad, moves ? o_mv : nullptr, path_e ? o_pe : nullptr, st),
+       "launch bf_k_findpath");
+    g.launches += 2;
+    CU(cudaMemcpyAsync(saddle_dcal + r0, o_sad, (size_t)nl * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H findpath saddles");
+    if (moves) CU(cudaMemcpyAsync(moves + (size_t)r0 * 2 * S, o_mv, (size_t)nl * 2 * S * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H findpath moves");
+    if (path_e) CU(cudaMemcpyAsync(path_e + (size_t)r0 * (S + 1), o_pe, (size_t)nl * (S + 1) * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H findpath energies");
+  }
+  CU(cudaStreamSynchronize(st), "bf_findpath");
   return BF_OK;
 }
 

@@ -191,6 +191,31 @@ cudaError_t bf_launch_interact(const BfParams *dP, const BfInteractDev &d, BfInt
 // ed[x] = -(kT / 1000) ln pu[x] (kcal/mol), +inf where pu[x] <= 0; kT in cal/mol
 cudaError_t bf_launch_interact_ed(const double *pu, double *ed, size_t n, double kT, cudaStream_t st);
 
+// ---- direct refolding paths (bf_findpath.cu): the breadth-limited findpath search of n instances, all runs of width W
+#define BF_FINDPATH_MAX_LEN 2000
+#define BF_FINDPATH_MAX_WIDTH 1024
+struct BfFindpathDev {
+  int n, stride;               // instances of the launch; row stride of seq and mv (pair tables: stride + 2)
+  const char *seq;             // n x stride
+  const int *len;              // n
+  const short *pt1, *pt2;      // pair tables of s1 / s2, n x (stride + 2), index 0 .. len + 1, 0 = unpaired
+  const int *mv;               // n x stride: (i << 16 | j) of the pairs of s1 not in s2 (ascending i), then of s2 not in s1
+  const int *nd;               // n x 2: the two counts
+  int width, nmax, kw;         // W; workspace shape: longest strand, 64-bit words of the longest move bitset
+  long long cap;               // candidate keys per CTA (a power of two >= W x the most moves)
+  int2 *bp;                    // back-pointers (parent rank << 16 | move, E) of every run, level-major, from bp_off[r]
+  const long long *bp_off;     // n
+  int *run_sad, *run_e0;       // n x bf_findpath_runs(W): saddle and start energy of each run
+};
+size_t bf_findpath_ws_bytes(int width, int nmax, int kw, long long cap);   // one CTA's workspace
+long long bf_findpath_cap(int width, int kmax);
+int bf_findpath_runs(int width);
+int bf_findpath_width_sum(int width);   // sum of w over the runs: back-pointers per instance = moves x this
+int bf_findpath_occupancy();
+// ws: grid x bf_findpath_ws_bytes.  saddle: n; moves (n x stride x 2) and path_e (n x (stride + 1)) or null.
+cudaError_t bf_launch_findpath(const BfParams *dP, const BfFindpathDev &d, unsigned char *ws, int grid, int *work_counter, int *saddle,
+                               int *moves, int *path_e, cudaStream_t st);
+
 // ---- suboptimal structures (bf_subopt.cu): host walk over the c / fML tables of the GPU fill
 #ifdef __cplusplus
 #include <string>

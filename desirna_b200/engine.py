@@ -47,6 +47,11 @@ class bf_interact_t(C.Structure):
                 ("acc_a", C.c_int32), ("acc_b", C.c_int32)]
 
 
+class bf_findpath_t(C.Structure):
+    _fields_ = [("n", C.c_int32), ("stride", C.c_int32), ("seq", C.c_void_p), ("len", C.c_void_p), ("s1", C.c_void_p), ("s2", C.c_void_p),
+                ("width", C.c_int32)]
+
+
 _lib = None
 
 
@@ -76,6 +81,7 @@ def lib():
                                       C.POINTER(C.c_int32)]
         L.bf_duplex.argtypes = [C.POINTER(bf_duplex_t), C.c_void_p, C.c_void_p]
         L.bf_interact.argtypes = [C.POINTER(bf_interact_t), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.bf_findpath.argtypes = [C.POINTER(bf_findpath_t), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.bf_unpaired.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
         L.bf_plfold.argtypes = [C.POINTER(bf_strands_t), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
@@ -331,6 +337,37 @@ def interact(seqs_a, seqs_b, pairs=None, max_span=25, acc_a=0, acc_b=0, structur
             st = [st[r * len(seqs_b):(r + 1) * len(seqs_b)] for r in range(len(seqs_a))]
         out["structures"] = st
     return out
+
+
+def findpath(seqs, s1, s2, width=1, path=True):
+    """bf_findpath: direct refolding paths (ViennaRNA's findpath), a breadth-limited search over the paths from s1[r] to s2[r] that
+    remove the pairs of s1 that s2 lacks and add the pairs of s2 that s1 lacks, one pair per step.  width: W, 1 .. 1024; the call
+    runs widths 1, 2, 4, ... below W, then W, each in both directions, and keeps the path of least saddle (definition in
+    include/b200fold.h).  Energies are the engine's eval (dcal/mol); sequences are single strands of at most 2000 nt, T read as U.
+
+    Returns saddles (int32 [n], dcal/mol) and, with path=True, also a list (per instance) of (moves, path_e): moves an int32 [k, 2]
+    array of 1-based (i, j), positive for an insertion and negative for a deletion, path_e an int32 [k + 1] array of the energies of
+    the structures along the path, E(s1) first."""
+    if any("&" in s for s in seqs):
+        raise ValueError("engine.findpath: single strands only")
+    ensure_ready()
+    n = len(seqs)
+    buf, lens, _ = pack([s.upper().replace("T", "U") for s in seqs])
+    S = buf.shape[1]
+    if len(s1) != n or len(s2) != n or any(len(s1[r]) != lens[r] or len(s2[r]) != lens[r] for r in range(n)):
+        raise ValueError("engine.findpath: one s1 and one s2 of the sequence's length per sequence")
+    t1 = pack_targets([[x] for x in s1], S).reshape(n, S) if n else np.zeros((0, S), np.uint8)
+    t2 = pack_targets([[x] for x in s2], S).reshape(n, S) if n else np.zeros((0, S), np.uint8)
+    q = bf_findpath_t()
+    q.n, q.stride, q.seq, q.len, q.s1, q.s2, q.width = n, S, buf.ctypes.data, lens.ctypes.data, t1.ctypes.data, t2.ctypes.data, int(width)
+    sad = np.zeros(n, np.int32)
+    k = np.zeros(n, np.int32)
+    mv = np.zeros((n, S, 2), np.int32) if path else None
+    pe = np.zeros((n, S + 1), np.int32) if path else None
+    _check(lib().bf_findpath(C.byref(q), sad.ctypes.data, k.ctypes.data, mv.ctypes.data if path else None, pe.ctypes.data if path else None))
+    if not path:
+        return sad
+    return sad, [(mv[r, :k[r]].copy(), pe[r, :k[r] + 1].copy()) for r in range(n)]
 
 
 def unpaired(seqs, max_u):

@@ -189,6 +189,46 @@ typedef struct {
 } bf_interact_t;
 int bf_interact(const bf_interact_t *q, double *e, int32_t *h_dcal, double *ed, int32_t *site, char *ss_out);
 
+/* Direct refolding paths (ViennaRNA's findpath: fc.path_findpath_saddle / fc.path_findpath; not called by DesiRNA).  HOST buffers,
+ * synchronous.
+ * Each instance r has a single-strand sequence (ACGU, T accepted, len[r] <= stride <= 2000), two structures s1 and s2 of len[r]
+ * characters ('.', '(' and ')' only, balanced, every pair with j - i >= 4; pairs need not be canonical) and the call's width W,
+ * 1 .. 1024.
+ * E(x) is the energy of structure x exactly as bf_score_batch with BF_WANT_EVAL returns it: int dcal/mol, non-standard pairs
+ * scored as type 7.
+ * One run (a -> b, width w): the moves are the deletions D = pairs of a not in b, ascending i, then the insertions I = pairs of b
+ * not in a, ascending i, indexed 0 .. k-1 with k = |D| + |I|.  A state is a set of moves done; its structure is a minus the
+ * deleted pairs plus the inserted pairs, and it is valid when no position is in two pairs and no two pairs cross.
+ *   Level 0 is {a}, with saddle E(a).
+ *   Level t+1 holds every valid one-move successor of the states kept at level t, with saddle = max(parent saddle, E(child)).
+ *   Successors with the same move set are one state; it keeps the least (saddle, parent rank, move index).
+ *   States are ordered by (saddle, E, parent rank, move index); the first w are kept, and their positions are their ranks.
+ * A level is never empty (while a deletion remains it is valid; once all are done every remaining insertion is compatible), so
+ * level k is exactly {b}.
+ * Runs of a call: w = 1, 2, 4, ... (the powers of two below W), then W; each w runs forward (s1 -> s2), then reverse (s2 -> s1).
+ * The result is the run with the least saddle; ties go to the first run in that order.
+ * The path is reported from s1 to s2 (a reverse run's path is reversed, so its deletions become insertions):
+ *   saddle_dcal: n saddles (dcal/mol), = max(path_e);
+ *   n_moves:     NULL or n counts k;
+ *   moves:       NULL or n x stride x 2: move m of instance r is (i, j), 1-based, positive for an insertion and negative for a
+ *                deletion (ViennaRNA's vrna_move_t sign convention); 0 past k;
+ *   path_e:      NULL or n x (stride + 1): E of the k + 1 structures of the path, E(s1) first; 0 past k.
+ * Every intermediate is a valid secondary structure.  The saddle does not increase from W' to W for every power of two W' <= W (the
+ * runs of W' are a subset of those of W), and when W is at least the largest level it is the optimum over all direct paths.
+ * Not pinned: ViennaRNA's exact width schedule, direction alternation and tie order are recalled; no ViennaRNA output in the tree
+ * pins them.
+ * BF_ERR_ARG: null q or saddle_dcal, n < 0, stride < 1 or > 2000, len < 0 or > stride, width outside 1 .. 1024, a sequence
+ * character other than ACGUT, an unbalanced structure, another character, a pair with j - i < 4.  BF_ERR_NOT_INIT before bf_init or
+ * before parameters are loaded. */
+typedef struct {
+  int32_t n, stride;       /* instances; bytes between rows of seq, s1 and s2 */
+  const char *seq;         /* n x stride */
+  const int32_t *len;      /* n */
+  const char *s1, *s2;     /* n x stride dot-bracket */
+  int32_t width;           /* W, 1 .. 1024 */
+} bf_findpath_t;
+int bf_findpath(const bf_findpath_t *q, int32_t *saddle_dcal, int32_t *n_moves, int32_t *moves, int32_t *path_e);
+
 /* Accessibility (not called by DesiRNA; RNAplfold -u, RNA.pfl_fold_up).  HOST buffers, synchronous.
  * Global: for a sequence of length n, P_u(i, u) is the probability that none of positions i .. i+u-1 is paired, in exactly the
  * ensemble of bf_score_batch's BF_WANT_PF / BF_WANT_BPP (loaded parameters, dangles = 2, pf_smooth, the per-nucleotide scale taken
