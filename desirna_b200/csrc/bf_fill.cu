@@ -491,37 +491,40 @@ __global__ void __launch_bounds__(WPB * 32) bf_k_trace(const BfParams *__restric
   if (lane == 0) f5[0] = 0;
   __syncwarp();
   // f5[j] = min(f5[j-1], min_i f5[i-1] + c(i,j) + Ext(i,j)): a serial chain over j whose table look-ups do not depend on f5.
-  // The terms of column j+1 are fetched (L2 latency) while column j is reduced; K = 32-wide chunks of i per lane.
+  // The table entries of column j+PD are fetched while column j is reduced (PD columns of look-ups in flight: one column's
+  // reduction is far shorter than a table load that misses in L2), the exterior terms are added when the column is reduced;
+  // K = 32-wide chunks of i per lane.
   auto chain = [&](auto kc) {
-    constexpr int K = decltype(kc)::value;
-    int cur[K], nxt[K];
+    constexpr int K = decltype(kc)::value, PD = 16 / K;
+    int cc[PD][K];
     auto fetch = [&](int j, int *v) {
 #pragma unroll
       for (int c = 0; c < K; c++) {
         const int i = 1 + lane + 32 * c;
-        int val = BF_INF;
-        if (i < j - BF_TURN) {
-          const int t = ptype_sp(SP, i, j);
-          if (t) {
-            const int cc = C_(i, j);
-            if (cc < BF_INF) val = cc + ext_e(i, j, t);
-          }
-        }
-        v[c] = val;
+        v[c] = (j <= n && i < j - BF_TURN && ptype_sp(SP, i, j)) ? C_(i, j) : BF_INF;
       }
     };
-    fetch(1, cur);
-    for (int j = 1; j <= n; j++) {
-      if (j < n) fetch(j + 1, nxt);
-      int e = BF_INF;
 #pragma unroll
-      for (int c = 0; c < K; c++)
-        if (cur[c] < BF_INF) e = min(e, f5[lane + 32 * c] + cur[c]);
-      e = bf_warp_min(e);
-      if (lane == 0) f5[j] = min(e, f5[j - 1]);
-      __syncwarp();
+    for (int p = 0; p < PD; p++) fetch(1 + p, cc[p]);
+    for (int j0 = 1; j0 <= n; j0 += PD) {
 #pragma unroll
-      for (int c = 0; c < K; c++) cur[c] = nxt[c];
+      for (int p = 0; p < PD; p++) {
+        const int j = j0 + p;
+        if (j > n) break;
+        int e = BF_INF;
+#pragma unroll
+        for (int c = 0; c < K; c++) {
+          const int i = 1 + lane + 32 * c;
+          if (cc[p][c] < BF_INF) {   // set only for i < j - TURN with a pair type
+            const int v = cc[p][c] + ext_e(i, j, ptype_sp(SP, i, j));
+            if (v < BF_INF) e = min(e, f5[i - 1] + v);
+          }
+        }
+        fetch(j + PD, cc[p]);
+        e = bf_warp_min(e);
+        if (lane == 0) f5[j] = min(e, f5[j - 1]);
+        __syncwarp();
+      }
     }
   };
   if (f5_in) {   // the 16-warp fill already ran the recursion

@@ -60,16 +60,18 @@ constexpr bool kPrepassInPhases = false;
 // shared-memory plan of the MFE fill
 // ---------------------------------------------------------------------------------------------
 struct Mfe3Plan {
-  size_t o_S, o_SP, o_np, o_ring, o_dml, o_fm, o_stg, o_tmpe, o_ps, o_cl, o_pp, total;
+  size_t o_S, o_SP, o_np, o_ring, o_dml, o_fm, o_stg, o_tmpe, o_stc, o_ps, o_cl, o_pp, total;
 };
 __host__ __device__ inline Mfe3Plan mfe3_plan(int nmax, int rs, int nw, int nwa) {
   Mfe3Plan p;
   size_t o = 0;
   p.o_ring = o; o += ((size_t)3 * kRing * rs + rs) * sizeof(int);   // three rings + one neutral row
-  p.o_dml = o; o += (size_t)4 * rs * sizeof(int);
+  // split minima: phase d reads row d-2 while the combine writes row d-1, so two rows suffice
+  p.o_dml = o; o += (size_t)2 * rs * sizeof(int);
   p.o_fm = o; o += (tri_size(nmax) + 4) * sizeof(int);
   p.o_stg = o; o += (size_t)2 * 3 * rs * sizeof(int);               // newest ring row, staged by the tap warps (double-buffered)
   p.o_tmpe = o; o += (size_t)2 * rs * sizeof(int);                  // c + MLstem of the newest diagonal
+  p.o_stc = o; o += (size_t)2 * rs * sizeof(int);                   // c of the newest diagonal (follows TMPE: reset together)
   p.o_ps = o; o += (size_t)2 * nwa * rs * sizeof(int);
   // per-sequence state exists twice: the auxiliary warps prepare the next sequence while the current one is folded
   p.o_np = o; o += (size_t)2 * ((nmax + 4) / 4 * 4) * sizeof(unsigned short);
@@ -94,10 +96,11 @@ __device__ __forceinline__ int lds_s32(unsigned addr) {
 // =====================================================================================================
 // Phase d of the diagonal loop (one barrier per phase):
 //   tap warps [0, NWI):  every pairable cell of diagonal d -- 487 decomposable interior candidates + 9 special ones (taps), hairpin,
-//                        multiloop closing (split minima of diagonal d-2) -> c(i,j); written to the HBM table, to the staging row of
-//                        the rings and, with its multiloop-stem term, to TMPE
-//   aux warps [NWI, NW): diagonal d-1: staging row -> rings, fML (needs c of d-1, the split minima of d-1 and fML of d-2);
-//                        then their share of the split points of diagonal d
+//                        multiloop closing (split minima of diagonal d-2) -> c(i,j); staged in STC, in the staging row of the rings
+//                        and, with its multiloop-stem term, in TMPE
+//   aux warps [NWI, NW): diagonal d-1: staging row -> rings, STC -> c table in HBM (every cell, INF where nothing was staged: one
+//                        coalesced row store instead of a scalar store per pairable cell), fML (needs c of d-1, the split minima of
+//                        d-1 and fML of d-2); then their share of the split points of diagonal d
 // Ring row d must not be written while phase d still reads row d-32 (same slot): hence the staging row.
 template <int NW, int NWI>
 __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_mfe_fill3(const BfParams *__restrict__ P, BfBatchDev b, int *ctri, int *ftri, size_t tri_slot,
@@ -117,6 +120,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
   int *fms = reinterpret_cast<int *>(dyn + pl.o_fm);
   int *STG = reinterpret_cast<int *>(dyn + pl.o_stg);
   int *TMPE = reinterpret_cast<int *>(dyn + pl.o_tmpe);
+  int *STC = reinterpret_cast<int *>(dyn + pl.o_stc);
   int *PS = reinterpret_cast<int *>(dyn + pl.o_ps);
   const BfSmallI &T = P->si;
   const bool tapw = warp < NWI;
@@ -158,9 +162,9 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
     return n1;
   };
   // pre-pass of one diagonal by one warp: per-cell constants (everything that depends on the sequence only) of its pairable cells,
-  // compacted, into the slot's half of the workspace; INF into the c table for the cells that cannot pair.  First the pairable
-  // cells are compacted (ballot), then the look-ups run with every lane busy.
-  auto prepass_diag = [&](int d, int slot, int n1, int *cgo, unsigned short *cl) {
+  // compacted, into the slot's half of the workspace.  First the pairable cells are compacted (ballot), then the look-ups run with
+  // every lane busy.
+  auto prepass_diag = [&](int d, int slot, int n1, unsigned short *cl) {
     const uint8_t *S1 = dyn + pl.o_S + slot * seq_pad, *SP1 = dyn + pl.o_SP + slot * seq_pad;
     unsigned short *NP1 = reinterpret_cast<unsigned short *>(dyn + pl.o_np) + slot * np_pad;
     int *ent1 = ent_base + (size_t)slot * (ent_slot / 2);
@@ -171,7 +175,6 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
       const bool in = i <= n1 - d;
       const int t = in ? bf_ptype_bases(SP1[i], SP1[i + d]) : 0;
       const unsigned mk = __ballot_sync(BF_FULL, t != 0);
-      if (in && !t) cgo[od + i - 1] = BF_INF;
       if (t) cl[count + __popc(mk & ((1u << lane) - 1))] = (unsigned short)i;
       count += __popc(mk);
     }
@@ -214,21 +217,20 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
   // (all warps, before any tap list is in use: their scratch lists live in the tap warps' list area)
   unsigned short *cl_all = reinterpret_cast<unsigned short *>(dyn + pl.o_cl) + (size_t)warp * ((nmax + 7) / 8 * 8);
   unsigned short *cl_aux = reinterpret_cast<unsigned short *>(dyn + pl.o_pp) + (size_t)(warp >= NWI ? warp - NWI : 0) * ((nmax + 7) / 8 * 8);
-  for (int d = BF_TURN + 1 + warp; d <= n - 1; d += NW) prepass_diag(d, 0, n, ctri + (size_t)sq * tri_slot, cl_all);
+  for (int d = BF_TURN + 1 + warp; d <= n - 1; d += NW) prepass_diag(d, 0, n, cl_all);
 
   for (;;) {
     __syncthreads();   // the state of sequence sq (slot cur) is complete; nobody reads s_seq or the other slot any more
     if (tid == 0) s_seq = atomicAdd(work_counter, 1);
     for (int k = tid; k < 3 * kRing * RS + RS; k += blockDim.x) RG[k] = BF_INF;
-    for (int k = tid; k < 4 * RS; k += blockDim.x) DML[k] = BF_INF;
+    for (int k = tid; k < 2 * RS; k += blockDim.x) DML[k] = BF_INF;
     for (int k = tid; k < 6 * RS; k += blockDim.x) STG[k] = BF_INF;
-    for (int k = tid; k < 2 * RS; k += blockDim.x) TMPE[k] = BF_INF;
+    for (int k = tid; k < 4 * RS; k += blockDim.x) TMPE[k] = BF_INF;   // TMPE and STC
     __syncthreads();
     // the next sequence: its codes now, its pre-pass diagonal by diagonal on the auxiliary warps during the phases below
     const int sqn = s_seq;
     const bool have_next = sqn < b.B;
     const int n1 = have_next ? load_seq(sqn, cur ^ 1) : 0;
-    int *cgo_next = ctri + (size_t)(have_next ? sqn : 0) * tri_slot;
     int pd = BF_TURN + 1 + (warp - NWI);   // next pre-pass diagonal of this auxiliary warp
     const unsigned short *NP = reinterpret_cast<const unsigned short *>(dyn + pl.o_np) + cur * np_pad;
     const int *ent = ent_base + (size_t)cur * (ent_slot / 2);
@@ -265,10 +267,11 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
         // ------------------------------------------------------------ tap warps: c(i,j) of every pairable cell of diagonal d
         if (d <= n - 1) {
           const int np = NP[d];
-          const int od = tri_off(n, d);
-          const unsigned sdml = (unsigned)__cvta_generic_to_shared(DML + ((d - 2) & 3) * RS + 1);
-          // lanes 0..2 write the staged ring row (generic, 1xn, bulge variant), lane 3 the fML candidate: lane's target array
-          const unsigned stail = (unsigned)__cvta_generic_to_shared(lane < 3 ? STG + (buf * 3 + lane) * RS : TMPE + buf * RS);
+          const unsigned sdml = (unsigned)__cvta_generic_to_shared(DML + ((d - 2) & 1) * RS + 1);
+          // lanes 0..2 write the staged ring row (generic, 1xn, bulge variant), lane 3 the fML candidate, lane 4 c itself: lane's
+          // target array, and the mask that drops the entry word lane 4 would add
+          const unsigned stail = (unsigned)__cvta_generic_to_shared(lane < 3 ? STG + (buf * 3 + lane) * RS : lane == 3 ? TMPE + buf * RS : STC + buf * RS);
+          const int tlmask = lane == 4 ? 0 : -1;
           const int smax = min(BF_MAXLOOP, d - 6);
           const int mi = smax + 1 < 0 ? 0 : smax + 1;
           const int ng = __ldg(meta + mi), n1 = __ldg(meta + 32 + mi), nb = __ldg(meta + 64 + mi);
@@ -281,7 +284,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
             const int *p = wl;
             for (int c = warp; c < np; c += NWI, p += kEntWords) {
               const int4 ea = *reinterpret_cast<const int4 *>(p);   // i, mismatchI, mismatch1nI, hairpin
-              const int ic = ea.x, mlc = p[4], tau = p[7], esp = p[lsp], etl = p[ltl];
+              const int ic = ea.x, mlc = p[4], tau = p[7], esp = p[lsp], etl = p[ltl] & tlmask;
               // the cell index is the same in every lane: taken through REDUX it lands in a uniform register, and a tap load
               // becomes LDS [R + UR] -- the lane's byte offset in a register, the cell's ring address uniform
               const unsigned i4 = 4u * (unsigned)__reduce_min_sync(BF_FULL, ic);
@@ -301,8 +304,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
               if (dm < kInfThr) tot = min(tot, dm + mlc);            // multiloop closed by (i,j)
               const bool fin = tot < kInfThr;
               const int v = (fin && etl < kInfThr) ? tot + etl : BF_INF;
-              if (lane < 4) asm volatile("st.shared.s32 [%0], %1;" ::"r"(stail + i4), "r"(v) : "memory");
-              if (lane == 0) cg_out[od + (int)(i4 >> 2) - 1] = fin ? tot : BF_INF;
+              if (lane < 5) asm volatile("st.shared.s32 [%0], %1;" ::"r"(stail + i4), "r"(v) : "memory");
             }
           };
           using std::integral_constant;
@@ -324,7 +326,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
         // ------------------------------------------------------------ diagonal d-1: staging row -> rings, fML
         if (d > BF_TURN + 1) {
           const int dd = d - 1, ncell = n - dd, pb = dd & 1;
-          int *stg = STG + pb * 3 * RS, *tmpe = TMPE + pb * RS;
+          int *stg = STG + pb * 3 * RS, *tmpe = TMPE + pb * RS, *stc = STC + pb * RS;
           const int *ps = PS + pb * NWA * RS;
           const int row = (dd & (kRing - 1)) * RS;
           const int o0 = tri_off(n, dd), om = dd > BF_TURN + 1 ? tri_off(n, dd - 1) : 0;
@@ -334,15 +336,16 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
 #pragma unroll
             for (int w = 0; w < NWA; w++) sp = min(sp, ps[w * RS + cell]);
             if (sp >= kInfThr) sp = BF_INF;
-            const int eg = stg[i], e1 = stg[RS + i], eb = stg[2 * RS + i], te = tmpe[i];
-            stg[i] = BF_INF; stg[RS + i] = BF_INF; stg[2 * RS + i] = BF_INF; tmpe[i] = BF_INF;   // only pairable cells are written
+            const int eg = stg[i], e1 = stg[RS + i], eb = stg[2 * RS + i], te = tmpe[i], cv = stc[i];
+            stg[i] = BF_INF; stg[RS + i] = BF_INF; stg[2 * RS + i] = BF_INF; tmpe[i] = BF_INF; stc[i] = BF_INF;   // only pairable cells are written
             CG[row + i] = eg; C1[row + i] = e1; CB[row + i] = eb;
+            cg_out[o0 + i - 1] = cv;
             int m = min(sp, te);
             if (dd > BF_TURN + 1) m = min(m, min(fms[om + i], fms[om + i - 1]) + T.MLbase);
             if (m >= kInfThr) m = BF_INF;
             fg_out[o0 + i - 1] = m;
             fms[o0 + i - 1] = m;
-            DML[(dd & 3) * RS + i] = sp;
+            DML[(dd & 1) * RS + i] = sp;
           }
         }
         if (d <= n - 1) {
@@ -393,7 +396,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
         // (measured: two auxiliary warps cannot hide it -- 780 instructions per 32 pairable cells, 3.07 against 2.57 ms per 4096
         // folds at L = 100 -- so by default all warps do it between two sequences, below)
         if (kPrepassInPhases && have_next && pd <= n1 - 1) {
-          prepass_diag(pd, cur ^ 1, n1, cgo_next, cl_aux);
+          prepass_diag(pd, cur ^ 1, n1, cl_aux);
           pd += NWA;
         }
       }
@@ -402,7 +405,7 @@ __global__ void __launch_bounds__(NW * 32, NW <= 8 ? 3 : NW <= 12 ? 2 : 1) bf_k_
     if (!have_next) break;
     // what the auxiliary warps did not reach (a next sequence much longer than this one): all warps
     for (int d = BF_TURN + 1 + (kPrepassInPhases ? NWA * (n - BF_TURN > 0 ? n - BF_TURN : 0) : 0) + warp; d <= n1 - 1; d += NW)
-      prepass_diag(d, cur ^ 1, n1, cgo_next, cl_all);
+      prepass_diag(d, cur ^ 1, n1, cl_all);
     sq = sqn;
     n = n1;
     cur ^= 1;
