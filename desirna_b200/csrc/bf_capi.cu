@@ -2,6 +2,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -19,7 +20,7 @@
 // program can flip them between calls on one engine.
 static const char *const kOptions[] = {"BF_CL", "BF_CL_C", "BF_CL_BW", "BF_EXT_WIDE", "BF_WIDE", "BF_FILL3", "BF_FILL3_SMALL",
                                        "BF_BLK_MIN", "BF_BLK_MIN_PF", "BF_FORCE_GENERIC", "BF_DESIGN_OVERLAP", "BF_PLFOLD_MB",
-                                       "BF_FINDPATH_MB"};
+                                       "BF_FINDPATH_MB", "BF_KINFOLD_MB"};
 
 int bf_opt(const char *name, int dflt) {
   const char *v = getenv(name);
@@ -115,6 +116,8 @@ struct Engine {
   // bf_findpath: sequences, lengths, pair tables, move lists and counts, back-pointer offsets, per-CTA workspaces, back-pointers, per-run
   // saddles and start energies, results
   DevBuf d_fpseq, d_fplen, d_fppt, d_fpmv, d_fpnd, d_fpoff, d_fpws, d_fpbp, d_fprun, d_fpout;
+  // bf_kinfold: sequences, lengths, start / stop pair tables, rate table, snapshot times, per-CTA workspaces, outputs of one launch
+  DevBuf d_kfseq, d_kflen, d_kfpt, d_kfrate, d_kfsnap, d_kfws, d_kfout;
   // small batches (a replica-exchange sub-step scored through the host-buffer call): inputs packed into one pinned block and one H2D
   // copy, results into one device block and one D2H copy
   DevBuf d_in, d_out, d_zero;
@@ -1192,6 +1195,126 @@ int bf_findpath(const bf_findpath_t *q, int32_t *saddle_dcal, int32_t *n_moves, 
     if (path_e) CU(cudaMemcpyAsync(path_e + (size_t)r0 * (S + 1), o_pe, (size_t)nl * (S + 1) * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H findpath energies");
   }
   CU(cudaStreamSynchronize(st), "bf_findpath");
+  return BF_OK;
+}
+
+int bf_kinfold(const bf_kinfold_t *q, int32_t *status, double *t_end, int64_t *steps, int32_t *e_end, char *ss_end, int32_t *e_snap,
+               char *ss_snap) {
+  if (!g.inited) return fail(BF_ERR_NOT_INIT, "bf_init has not been called");
+  if (!g.have_params) return fail(BF_ERR_NOT_INIT, "no energy parameters loaded");
+  if (!q || !status || q->n < 0 || q->n_traj < 1 || q->stride < 1) return fail(BF_ERR_ARG, "bf_kinfold: bad argument");
+  if (q->stride > BF_KINFOLD_MAX_LEN) return fail(BF_ERR_ARG, "bf_kinfold: stride above 2000");
+  if (q->rule < 0 || q->rule > 2) return fail(BF_ERR_ARG, "bf_kinfold: rule outside 0 .. 2");
+  if (q->max_steps < 1) return fail(BF_ERR_ARG, "bf_kinfold: max_steps below 1");
+  if (q->n_snap < 0) return fail(BF_ERR_ARG, "bf_kinfold: n_snap below 0");
+  const bool timed = q->rule != 2;
+  if (timed && !(std::isfinite(q->t_max) && q->t_max > 0)) return fail(BF_ERR_ARG, "bf_kinfold: t_max not finite and positive");
+  if (timed && q->n_snap > 0) {
+    if (!q->t_snap) return fail(BF_ERR_ARG, "bf_kinfold: null snapshot times");
+    for (int s = 0; s < q->n_snap; s++)
+      if (!(q->t_snap[s] >= 0 && q->t_snap[s] <= q->t_max) || (s && q->t_snap[s] < q->t_snap[s - 1]))
+        return fail(BF_ERR_ARG, "bf_kinfold: snapshot times not ascending in [0, t_max]");
+  }
+  const int n = q->n, S = q->stride, T = q->n_traj, ns = q->n_snap;
+  if (n && (!q->seq || !q->len)) return fail(BF_ERR_ARG, "bf_kinfold: null sequence buffer");
+  // start and stop pair tables; every pair canonical.  gmax: the most groups of 32 valid moves any step can have (every move is a
+  // canonical pair with j - i >= 4)
+  std::vector<short> pt((size_t)n * 2 * (S + 2), 0);
+  std::vector<int> stk;
+  std::vector<uint8_t> code(S + 2);
+  int nmax = 1;
+  long long npmax = 1;
+  for (int r = 0; r < n; r++) {
+    const int len = q->len[r];
+    const char *seq = q->seq + (size_t)r * S;
+    if (len < 0 || len > S) return fail(BF_ERR_ARG, "bf_kinfold: length outside 0 .. stride");
+    for (int i = 1; i <= len; i++)
+      if (!(code[i] = (uint8_t)bf_base_code(seq[i - 1]))) return fail(BF_ERR_ARG, "bf_kinfold: sequence character other than ACGUT");
+    for (int w = 0; w < 2; w++) {
+      const char *db = w ? q->stop : q->start;
+      if (!db) continue;
+      short *p = &pt[((size_t)r * 2 + w) * (S + 2)];
+      if (!findpath_parse(db + (size_t)r * S, len, p, stk))
+        return fail(BF_ERR_ARG, "bf_kinfold: structure not balanced, a character other than '.()', or a pair with j - i < 4");
+      for (int i = 1; i <= len; i++)
+        if (p[i] > i && !bf_ptype_bases(code[i], code[p[i]])) return fail(BF_ERR_ARG, "bf_kinfold: a non-canonical pair");
+    }
+    // canonical partners j >= i + 4 of every i, from counts of each base at and after i + 4
+    long long np = 0, cnt[5] = {0, 0, 0, 0, 0};
+    for (int i = len - 4; i >= 1; i--) {
+      cnt[code[i + 4]]++;
+      for (int b = 1; b <= 4; b++) np += bf_ptype_bases(code[i], b) ? cnt[b] : 0;
+    }
+    nmax = std::max(nmax, len);
+    npmax = std::max(npmax, np);
+  }
+  if (n == 0) return BF_OK;
+  cudaStream_t st = g.stream;
+  std::vector<short> pts((size_t)n * 2 * (S + 2));   // all start tables, then all stop tables
+  for (int r = 0; r < n; r++)
+    for (int w = 0; w < 2; w++)
+      memcpy(&pts[((size_t)w * n + r) * (S + 2)], &pt[((size_t)r * 2 + w) * (S + 2)], (S + 2) * sizeof(short));
+  std::vector<double> rate(65536);
+  const double kT = g.hP->kT;
+  for (int x = 0; x < 65536; x++) {
+    const double de = (double)(x - 32768);
+    rate[x] = q->rule == 0 ? std::exp(-de * 10.0 / (2.0 * kT)) : std::min(1.0, std::exp(-de * 10.0 / kT));
+  }
+  const size_t ptb = (size_t)n * (S + 2) * sizeof(short);
+  CU(g.d_kfseq.reserve((size_t)n * S), "cudaMalloc(kinfold seq)");
+  CU(g.d_kflen.reserve((size_t)n * sizeof(int)), "cudaMalloc(kinfold len)");
+  CU(g.d_kfpt.reserve(2 * ptb), "cudaMalloc(kinfold pair tables)");
+  CU(g.d_kfrate.reserve(65536 * sizeof(double)), "cudaMalloc(kinfold rates)");
+  CU(g.d_kfsnap.reserve((size_t)std::max(ns, 1) * sizeof(double)), "cudaMalloc(kinfold snapshot times)");
+  CU(cudaMemcpyAsync(g.d_kfseq.p, q->seq, (size_t)n * S, cudaMemcpyHostToDevice, st), "H2D kinfold seq");
+  CU(cudaMemcpyAsync(g.d_kflen.p, q->len, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st), "H2D kinfold len");
+  CU(cudaMemcpyAsync(g.d_kfpt.p, pts.data(), 2 * ptb, cudaMemcpyHostToDevice, st), "H2D kinfold pair tables");
+  CU(cudaMemcpyAsync(g.d_kfrate.p, rate.data(), 65536 * sizeof(double), cudaMemcpyHostToDevice, st), "H2D kinfold rates");
+  if (timed && ns) CU(cudaMemcpyAsync(g.d_kfsnap.p, q->t_snap, (size_t)ns * sizeof(double), cudaMemcpyHostToDevice, st), "H2D kinfold snapshot times");
+  // half the budget for the grid's workspaces, half for the outputs of one launch
+  const size_t budget = (size_t)std::max(1, bf_opt("BF_KINFOLD_MB", 1024)) << 20;
+  const int gmax = timed ? (int)((npmax + 31) / 32) : 1;
+  const size_t ws_cta = bf_kinfold_ws_bytes(gmax, nmax);
+  const int occ = bf_kinfold_occupancy(nmax);
+  const int grid_max = (int)std::max<long long>(1, std::min<long long>((long long)g.sm_count * occ, (long long)(budget / 2 / ws_cta)));
+  const size_t per_u = 2 * sizeof(double) + 2 * sizeof(int) + (S + 1) + (size_t)ns * (sizeof(int) + S + 1);
+  const long long units = (long long)n * T;
+  const long long nl_max = std::min<long long>(units, std::max<long long>(1, (long long)(budget / 2 / per_u)));
+  CU(g.d_kfws.reserve((size_t)grid_max * ws_cta), "cudaMalloc(kinfold workspaces)");
+  CU(g.d_kfout.reserve((size_t)nl_max * per_u + 1024), "cudaMalloc(kinfold results)");
+  char *ob = (char *)g.d_kfout.p;
+  double *o_t = (double *)ob;
+  long long *o_steps = (long long *)(o_t + nl_max);
+  int *o_status = (int *)(o_steps + nl_max), *o_e = o_status + nl_max, *o_esnap = o_e + nl_max;
+  char *o_ss = (char *)(o_esnap + (size_t)nl_max * ns), *o_sssnap = o_ss + (size_t)nl_max * (S + 1);
+  for (long long u0 = 0; u0 < units; u0 += nl_max) {
+    const int nl = (int)std::min<long long>(nl_max, units - u0);
+    BfKinfoldDev d;
+    d.stride = S; d.T = T;
+    d.seq = (const char *)g.d_kfseq.p;
+    d.len = (const int *)g.d_kflen.p;
+    d.start = (const short *)g.d_kfpt.p;
+    d.stop = q->stop ? (const short *)((const char *)g.d_kfpt.p + ptb) : nullptr;
+    d.rate = (const double *)g.d_kfrate.p;
+    d.rule = q->rule; d.t_max = q->t_max; d.seed = q->seed; d.max_steps = q->max_steps;
+    d.n_snap = ns; d.t_snap = (const double *)g.d_kfsnap.p;
+    d.u0 = u0; d.nu = nl; d.nmax = nmax; d.gmax = gmax;
+    d.status = o_status; d.t_end = o_t; d.steps = o_steps; d.e_end = o_e; d.ss_end = o_ss; d.e_snap = o_esnap; d.ss_snap = o_sssnap;
+    const int grid = (int)std::min<long long>(grid_max, (nl + 7) / 8);
+    CU(bf_launch_kinfold(g.dP, d, (unsigned char *)g.d_kfws.p, grid, g.w.d_counters + 6, st), "launch bf_k_kinfold");
+    g.launches++;
+    CU(cudaMemcpyAsync(status + u0, o_status, (size_t)nl * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H kinfold status");
+    if (t_end) CU(cudaMemcpyAsync(t_end + u0, o_t, (size_t)nl * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H kinfold times");
+    if (steps) CU(cudaMemcpyAsync(steps + u0, o_steps, (size_t)nl * sizeof(long long), cudaMemcpyDeviceToHost, st), "D2H kinfold steps");
+    if (e_end) CU(cudaMemcpyAsync(e_end + u0, o_e, (size_t)nl * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H kinfold energies");
+    if (ss_end) CU(cudaMemcpyAsync(ss_end + u0 * (S + 1), o_ss, (size_t)nl * (S + 1), cudaMemcpyDeviceToHost, st), "D2H kinfold structures");
+    if (e_snap && ns)
+      CU(cudaMemcpyAsync(e_snap + u0 * ns, o_esnap, (size_t)nl * ns * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H kinfold snapshot energies");
+    if (ss_snap && ns)
+      CU(cudaMemcpyAsync(ss_snap + u0 * ns * (S + 1), o_sssnap, (size_t)nl * ns * (S + 1), cudaMemcpyDeviceToHost, st),
+         "D2H kinfold snapshot structures");
+  }
+  CU(cudaStreamSynchronize(st), "bf_kinfold");
   return BF_OK;
 }
 

@@ -216,6 +216,38 @@ int bf_findpath_occupancy();
 cudaError_t bf_launch_findpath(const BfParams *dP, const BfFindpathDev &d, unsigned char *ws, int grid, int *work_counter, int *saddle,
                                int *moves, int *path_e, cudaStream_t st);
 
+// ---- folding kinetics (bf_kinfold.cu): trajectories u0 .. u0 + nu - 1 of the call, trajectory u = r x T + k
+#define BF_KINFOLD_MAX_LEN 2000
+struct BfKinfoldDev {
+  int stride, T;               // row stride of seq (pair tables: stride + 2); trajectories per instance
+  const char *seq;             // instances x stride
+  const int *len;              // per instance
+  const short *start, *stop;   // pair tables, instances x (stride + 2), index 0 .. len + 1; stop may be null
+  const double *rate;          // 65536 rates, k(dE) at [dE + 32768]
+  int rule;                    // 0 Kawasaki, 1 Metropolis, 2 steepest descent
+  double t_max;
+  unsigned long long seed;
+  long long max_steps;
+  int n_snap;
+  const double *t_snap;        // n_snap ascending times
+  long long u0;
+  int nu;
+  int nmax, gmax;              // longest strand of the call; groups of one warp's workspace
+  // outputs of the launch's trajectories, indexed by u - u0
+  int *status;
+  double *t_end;
+  long long *steps;
+  int *e_end;
+  char *ss_end;                // (stride + 1) per trajectory
+  int *e_snap;                 // n_snap per trajectory
+  char *ss_snap;               // n_snap x (stride + 1) per trajectory
+};
+size_t bf_kinfold_smem(int nmax);       // dynamic shared memory of one CTA
+size_t bf_kinfold_ws_bytes(int gmax, int nmax);   // HBM workspace of one CTA
+int bf_kinfold_occupancy(int nmax);
+// ws: grid x bf_kinfold_ws_bytes(d.gmax, d.nmax)
+cudaError_t bf_launch_kinfold(const BfParams *dP, const BfKinfoldDev &d, unsigned char *ws, int grid, int *work_counter, cudaStream_t st);
+
 // ---- suboptimal structures (bf_subopt.cu): host walk over the c / fML tables of the GPU fill
 #ifdef __cplusplus
 #include <string>

@@ -52,6 +52,12 @@ class bf_findpath_t(C.Structure):
                 ("width", C.c_int32)]
 
 
+class bf_kinfold_t(C.Structure):
+    _fields_ = [("n", C.c_int32), ("stride", C.c_int32), ("seq", C.c_void_p), ("len", C.c_void_p), ("start", C.c_void_p),
+                ("stop", C.c_void_p), ("n_traj", C.c_int32), ("rule", C.c_int32), ("t_max", C.c_double), ("seed", C.c_uint64),
+                ("max_steps", C.c_int64), ("n_snap", C.c_int32), ("t_snap", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -82,6 +88,7 @@ def lib():
         L.bf_duplex.argtypes = [C.POINTER(bf_duplex_t), C.c_void_p, C.c_void_p]
         L.bf_interact.argtypes = [C.POINTER(bf_interact_t), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.bf_findpath.argtypes = [C.POINTER(bf_findpath_t), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.bf_kinfold.argtypes = [C.POINTER(bf_kinfold_t)] + [C.c_void_p] * 7
         L.bf_unpaired.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
         L.bf_plfold.argtypes = [C.POINTER(bf_strands_t), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
         L.bf_set_option.argtypes = [C.c_char_p, C.c_int]
@@ -368,6 +375,68 @@ def findpath(seqs, s1, s2, width=1, path=True):
     if not path:
         return sad
     return sad, [(mv[r, :k[r]].copy(), pe[r, :k[r] + 1].copy()) for r in range(n)]
+
+
+KINFOLD_RULES = {"kawasaki": 0, "metropolis": 1, "descent": 2}
+
+
+def kinfold(seqs, start=None, stop=None, n_traj=1, rule="kawasaki", t_max=500.0, seed=0, t_snap=None, max_steps=10**6,
+            structures=True):
+    """bf_kinfold: folding kinetics over single-pair moves (insert or delete one canonical pair; no shift moves), n_traj
+    trajectories per sequence.  rule: "kawasaki" (k = exp(-dE / 2kT)) or "metropolis" (k = min(1, exp(-dE / kT))), simulated
+    with Gillespie's method up to time t_max, or "descent", the deterministic steepest-descent walk to a local minimum.  start:
+    one structure per sequence or None (open chain); stop: one structure per sequence or None, absorbing (a "hit").  t_snap:
+    ascending times in [0, t_max] at which the occupied state is recorded.  The trajectories are a function of (seed, sequence
+    index, trajectory index) alone.  Definition in include/b200fold.h; single strands of at most 2000 nt, T read as U.
+
+    Returns a dict of numpy arrays shaped [len(seqs), n_traj, ...]: 'status' (int32: 0 t_max reached or, for descent, a local
+    minimum; 1 stop structure reached; 2 max_steps moves), 't_end' (float64), 'steps' (int64), 'e_end' (int32, dcal/mol) and,
+    with t_snap, 'e_snap' (int32 [..., n_snap]; 10000000 after a cap and for descent); with structures also 'ss_end' and
+    'ss_snap' (str, '' where e_snap is 10000000).
+
+    ViennaRNA's Python module has no Kinfold, so there is no RNA.py counterpart."""
+    if any("&" in s for s in seqs):
+        raise ValueError("engine.kinfold: single strands only")
+    if rule not in KINFOLD_RULES:
+        raise ValueError("engine.kinfold: rule must be one of " + ", ".join(KINFOLD_RULES))
+    ensure_ready()
+    n, T = len(seqs), int(n_traj)
+    buf, lens, _ = pack([s.upper().replace("T", "U") for s in seqs])
+    S = buf.shape[1]
+    q = bf_kinfold_t()
+    q.n, q.stride, q.seq, q.len, q.n_traj, q.rule = n, S, buf.ctypes.data, lens.ctypes.data, T, KINFOLD_RULES[rule]
+    q.t_max, q.seed, q.max_steps = float(t_max), int(seed) & ((1 << 64) - 1), int(max_steps)
+    keep = []
+    for name, dbs in (("start", start), ("stop", stop)):
+        if dbs is None:
+            continue
+        if len(dbs) != n or any(len(dbs[r]) != lens[r] for r in range(n)):
+            raise ValueError(f"engine.kinfold: one {name} structure of the sequence's length per sequence")
+        tb = pack_targets([[x] for x in dbs], S).reshape(n, S) if n else np.zeros((0, S), np.uint8)
+        keep.append(tb)
+        setattr(q, name, tb.ctypes.data)
+    ts = np.ascontiguousarray(t_snap if t_snap is not None else [], np.float64).reshape(-1)
+    q.n_snap, q.t_snap = ts.size, ts.ctypes.data if ts.size else None
+    ns, U = ts.size, n * max(T, 1)
+    status = np.zeros(U, np.int32)
+    t_end = np.zeros(U, np.float64)
+    steps = np.zeros(U, np.int64)
+    e_end = np.zeros(U, np.int32)
+    e_snap = np.zeros((U, ns), np.int32)
+    ss_end = np.zeros((U, S + 1), np.uint8) if structures else None
+    ss_snap = np.zeros((U, ns, S + 1), np.uint8) if structures and ns else None
+    _check(lib().bf_kinfold(C.byref(q), status.ctypes.data, t_end.ctypes.data, steps.ctypes.data, e_end.ctypes.data,
+                            ss_end.ctypes.data if ss_end is not None else None, e_snap.ctypes.data if ns else None,
+                            ss_snap.ctypes.data if ss_snap is not None else None))
+    shape = (n, T)
+    out = {"status": status.reshape(shape), "t_end": t_end.reshape(shape), "steps": steps.reshape(shape), "e_end": e_end.reshape(shape)}
+    if ns:
+        out["e_snap"] = e_snap.reshape(shape + (ns,))
+    if structures:
+        out["ss_end"] = ss_end.view(f"S{S + 1}").reshape(shape).astype(str)
+        if ns:
+            out["ss_snap"] = ss_snap.view(f"S{S + 1}").reshape(shape + (ns,)).astype(str)
+    return out
 
 
 def unpaired(seqs, max_u):

@@ -229,6 +229,63 @@ typedef struct {
 } bf_findpath_t;
 int bf_findpath(const bf_findpath_t *q, int32_t *saddle_dcal, int32_t *n_moves, int32_t *moves, int32_t *path_e);
 
+/* Folding kinetics (Kinfold-style trajectories; not called by DesiRNA).  HOST buffers, synchronous.
+ * States: the secondary structures of one strand whose pairs are all canonical (AU, CG, GU either way) with j - i >= 4, no position
+ * in two pairs, no two pairs crossing.  E(x) is the energy of x exactly as bf_score_batch with BF_WANT_EVAL returns it (int dcal/mol).
+ * Moves of x: deleting any pair of x; inserting a canonical pair (i, j), j - i >= 4, i and j unpaired, crossing no pair of x (both
+ * in the same loop).  No shift moves.  The canonical move order is (i, j) ascending; a pair is in x or not, so one list holds both.
+ * Rate of a move x -> y: k(dE), dE = E(y) - E(x), kT = the loaded parameter set's kT (cal/mol), taken from a table over integer
+ * dE in [-32768, 32767] built on the host in double:
+ *   rule 0, Kawasaki:   k = exp(-dE * 10 / (2 kT));
+ *   rule 1, Metropolis: k = min(1, exp(-dE * 10 / kT)).
+ * Stochastic step (Gillespie's direct method), at state x and time t:
+ *   the valid moves in canonical order are cut into consecutive groups of 32.  Within a group the rates v[0 .. 31] (0 past the last
+ *   move) are combined by a 5-step inclusive scan: for o = 1, 2, 4, 8, 16, v[l] += v[l - o] for l >= o, all at once.  A running
+ *   double R starts at 0 and adds each group's v[31] in group order; K is the final R, and the running prefix of move l of group g
+ *   is R(before g) + v[l].
+ *   Each step draws u1, then u2, from the trajectory's splitmix64 stream, seeded from (seed, instance r, trajectory k) alone as
+ *   bf_sample seeds (seed, row, sample).  dt = -ln(1 - u1) / K.  If t + dt > t_max, the trajectory ends at t_max in x.  Otherwise
+ *   t += dt and the move taken is the first whose running prefix exceeds u2 K (the last valid move if none does, by rounding).
+ *   K = 0 (no move): x is absorbing until t_max.
+ * Steepest descent (rule 2): each step takes the move of least dE, ties to the first in canonical order, and only if dE < 0; the
+ * walk ends at a local minimum.  t stays 0; seed, t_max and the snapshot times are not read.
+ * Stop structure (optional, per instance): absorbing; reaching it ends the trajectory with status 1 at that time.
+ * max_steps moves end a trajectory with status 2 (unless its last move reached the stop structure).
+ * Inputs: n instances (seq, len, stride as in bf_findpath, len <= stride <= 2000); start (NULL: the open chain) and stop (NULL:
+ * none), n x stride dot-brackets; n_traj trajectories per instance; rule; t_max; seed; max_steps; n_snap ascending snapshot times
+ * in [0, t_max].
+ * Outputs, per trajectory u = r * n_traj + k (caller-owned, NULL to skip, except status):
+ *   status:  0 t_max reached (rule 2: a local minimum), 1 stop structure reached, 2 max_steps moves;
+ *   t_end:   the time the trajectory ended (t_max, the time of the hit or of the last move; 0 for rule 2);
+ *   steps:   moves made;
+ *   e_end, ss_end: E and the structure at the end, ss_end stride + 1 chars per trajectory, NUL-padded;
+ *   e_snap, ss_snap: n_snap per trajectory, the state occupied at t_s (the state entered at the last move at or before t_s).  After
+ *   a hit that is the stop structure; after a cap, and for rule 2, 10000000 and an empty string.
+ * Device workspaces and outputs stay within a fixed budget (1 GB; bf_set_option "kinfold_mb"); a call that does not fit runs in
+ * several launches and its results do not depend on the split.
+ * Not reproduced: Kinfold's defaults -- shift moves, its multiloop and dangle options, --noLP, growth (--grow), energy cutoffs.  Its
+ * time unit (k0 = 1) and default --time 500 are recalled; no Kinfold output in the tree pins them.
+ * BF_ERR_ARG: null q or status, n < 0, n_traj < 1, stride outside 1 .. 2000, len < 0 or > stride, a sequence character other than
+ * ACGUT, an unbalanced start or stop structure or another character, a non-canonical pair or one with j - i < 4, rule outside
+ * 0 .. 2, t_max not finite or <= 0 (rules 0, 1), n_snap < 0, snapshot times not ascending or outside [0, t_max] (rules 0, 1),
+ * max_steps < 1.  BF_ERR_NOT_INIT before bf_init or before parameters are loaded. */
+typedef struct {
+  int32_t n, stride;       /* instances; bytes between rows of seq, start and stop */
+  const char *seq;         /* n x stride */
+  const int32_t *len;      /* n */
+  const char *start;       /* n x stride dot-bracket, or NULL: the open chain */
+  const char *stop;        /* n x stride dot-bracket, or NULL: none */
+  int32_t n_traj;          /* trajectories per instance, >= 1 */
+  int32_t rule;            /* 0 Kawasaki, 1 Metropolis, 2 steepest descent */
+  double t_max;
+  uint64_t seed;
+  int64_t max_steps;
+  int32_t n_snap;
+  const double *t_snap;    /* n_snap ascending times */
+} bf_kinfold_t;
+int bf_kinfold(const bf_kinfold_t *q, int32_t *status, double *t_end, int64_t *steps, int32_t *e_end, char *ss_end, int32_t *e_snap,
+               char *ss_snap);
+
 /* Accessibility (not called by DesiRNA; RNAplfold -u, RNA.pfl_fold_up).  HOST buffers, synchronous.
  * Global: for a sequence of length n, P_u(i, u) is the probability that none of positions i .. i+u-1 is paired, in exactly the
  * ensemble of bf_score_batch's BF_WANT_PF / BF_WANT_BPP (loaded parameters, dangles = 2, pf_smooth, the per-nucleotide scale taken
@@ -277,6 +334,7 @@ int bf_sm_count(void);
  *   "force_generic" 1: single strands on the generic kernels too (read by bf_init);
  *   "design_overlap" 0: the device design loop always folds MFE, then PF.
  *   "plfold_mb" N: memory budget of one bf_plfold chunk in MB (default 1024); the result does not depend on it.
+ *   "kinfold_mb" N: memory budget of bf_kinfold's device workspaces and outputs in MB (default 1024); the result does not depend on it.
  * Any other key is refused with BF_ERR_ARG. */
 int bf_set_option(const char *key, int value);
 /* Test hook: copy one engine-internal DP table of the most recent call to host memory.
